@@ -13,6 +13,12 @@ names.  `cpu_baseline` = the CPU oracle on a bounded sample of the same workload
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--ksp minres|fgmres|gmres]
     python bench.py --impl reference ...      # CPU oracle arm (the reference's algorithm)
+    python bench.py --dump-outputs DIR ...    # also write the last timed solve's results as DIR/<name>.npy
+
+--dump-outputs writes what a caller of the timed solve receives: the solution blocks (v.npy, zeta.npy; for the Stokes
+workload also mu.npy, p.npy) and the residual history of the solve (residual_history.npy), all float64.  A solution
+block larger than DUMP_SAMPLE entries is sampled at fixed, seeded (time block, dof) positions in global numbering, so
+two builds, or two GPU counts, can be compared entry for entry.
 """
 import argparse
 import json
@@ -104,6 +110,35 @@ class ClockSampler:
     def summary(self):
         return {"sm_mhz": statistics.median(self.samples) if self.samples else None,
                 "sm_max_mhz": self.max_mhz, "reasons": sorted(self.reasons)}
+
+
+DUMP_SAMPLE = 1 << 20        # entries kept of each dumped solution block: 8 MB in float64
+
+
+def sample_blocks(u, parts, dist=None):
+    """{name: float64 sample} of the (blocks, n) arrays stored block-major in the rank-local device vector u.
+    parts = [(name, offset of the rank's (blocks, n_local) array in u, blocks, n, row_begin, n_local)].  The sample is
+    drawn in global (block, dof) numbering and summed over ranks, each entry being owned by exactly one rank."""
+    import torch
+    out = {}
+    for name, offset, blocks, n, rb, nl in parts:
+        size = blocks * n
+        g = np.arange(size) if size <= DUMP_SAMPLE else \
+            np.unique(np.random.default_rng(0).integers(0, size, DUMP_SAMPLE))
+        t, j = np.divmod(g, n)
+        own = np.flatnonzero((j >= rb) & (j < rb + nl))
+        vals = torch.zeros(g.size, dtype=torch.float64, device=u.device)
+        vals[torch.from_numpy(own).to(u.device)] = u[torch.from_numpy(offset + t[own] * nl + j[own] - rb).to(u.device)]
+        if dist is not None:
+            dist.all_reduce(vals)
+        out[name] = vals.cpu().numpy()
+    return out
+
+
+def write_outputs(directory, arrays):
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def solver_parameters(ksp, rtol, restart=30):
@@ -284,6 +319,11 @@ def run_stokes(args):
         torch.cuda.synchronize()
     launches = s.kernel_launches() - l0
     value = ev0.elapsed_time(ev1) * 1e-3 / args.steps
+    if args.dump_outputs:
+        N, n_v, n_p = s.N, s.n_v, s.n_p
+        parts = [("v", 0, N, n_v, 0, n_v), ("zeta", N * n_v, N, n_v, 0, n_v),
+                 ("mu", 2 * N * n_v, N, n_p, 0, n_p), ("p", 2 * N * n_v + N * n_p, N, n_p, 0, n_p)]
+        write_outputs(args.dump_outputs, {**sample_blocks(u_last, parts), "residual_history": info.history})
     r0, r1 = s.to_host_blocks(b_dev - s.apply(u_last))
     r0[:, q["bdofs"]] = 0.0
     r1 = r1 - r1.mean(axis=1, keepdims=True)
@@ -350,7 +390,14 @@ def main():
                          "library defaults otherwise")
     ap.add_argument("--no_cpu_baseline", action="store_true")
     ap.add_argument("--no_alt", action="store_true", help="skip the FGMRES + triangular PC side measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the solution blocks (a fixed, seeded sample of at most DUMP_SAMPLE entries each) and "
+                         "the residual history of the last timed solve as DIR/<name>.npy, float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the results of the timed GPU solve (--impl b200)")
     if args.workload == "c3":
         # config C3 and the reference's default Krylov parameters (control/control.py:3260-3266): GMRES(10)
         if args.nx == 1024 and args.n_t == 64:
@@ -444,6 +491,11 @@ def main():
     total_s = max_over_ranks(ev0.elapsed_time(ev1) * 1e-3)
     value = total_s / args.steps
     res_norm = s.residual_norm(b_dev, u_last)
+    if args.dump_outputs:
+        blocks = (s.N, s.n, s.row_begin, s.n_local)
+        out = sample_blocks(u_last, [("v", 0, *blocks), ("zeta", s.N * s.n_local, *blocks)], dist)
+        if rank == 0:
+            write_outputs(args.dump_outputs, {**out, "residual_history": infos[-1].history})
 
     # ---- end to end through the public API with host buffers
     solve_e2e()

@@ -37,6 +37,37 @@ def test_one_gpu_records_cover_the_bench_configurations():
     assert bench.known_iterations(_args(nx=999))[1].startswith("assumed")
 
 
+def test_dump_sample_is_the_same_for_any_row_partition(tmp_path, monkeypatch):
+    """--dump-outputs: the sample is drawn in global (block, dof) numbering, so one rank and a row partition over two
+    ranks dump the same entries; small blocks are written whole."""
+    import numpy as np
+    import torch
+    monkeypatch.setattr(bench, "DUMP_SAMPLE", 50)
+    N, n = 7, 13
+    rng = np.random.default_rng(3)
+    v, zeta = rng.standard_normal((N, n)), rng.standard_normal((N, n))
+    whole = bench.sample_blocks(torch.from_numpy(np.concatenate([v.ravel(), zeta.ravel()])),
+                                [("v", 0, N, n, 0, n), ("zeta", N * n, N, n, 0, n)])
+    assert 0 < whole["v"].size <= 50 and np.all(np.isin(whole["v"], v)) and np.all(np.isin(whole["zeta"], zeta))
+    split = {"v": 0.0, "zeta": 0.0}
+    for rb, nl in ((0, 7), (7, 6)):                    # two ranks; their sum plays the all-reduce
+        u = torch.from_numpy(np.concatenate([v[:, rb:rb + nl].ravel(), zeta[:, rb:rb + nl].ravel()]))
+        part = bench.sample_blocks(u, [("v", 0, N, n, rb, nl), ("zeta", N * nl, N, n, rb, nl)])
+        split = {k: split[k] + part[k] for k in split}
+    assert all(np.array_equal(whole[k], split[k]) for k in split)
+    small = bench.sample_blocks(torch.arange(6, dtype=torch.float64), [("p", 0, 2, 3, 0, 3)])
+    assert np.array_equal(small["p"], np.arange(6.0))
+    bench.write_outputs(str(tmp_path / "out"), {**whole, "residual_history": [1.0, 0.5]})
+    assert sorted(os.listdir(tmp_path / "out")) == ["residual_history.npy", "v.npy", "zeta.npy"]
+    assert np.load(tmp_path / "out" / "residual_history.npy").dtype == np.float64
+
+
+def test_steps_must_be_positive():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                         timeout=120)
+    assert out.returncode == 2 and "--steps must be at least 1" in out.stderr
+
+
 def test_reference_arm_prints_the_contract_line():
     """`bench.py --impl reference` (the CPU arm: C / OpenMP port of the reference's algorithm) on a small problem."""
     so = os.path.join(ROOT, "oracle", "_build", "liboracle.so")
