@@ -95,6 +95,7 @@ SIGNATURES = {
     "ctl_objective_host": (C.c_int, [_H, _F64P, _F64P, _F64P, C.POINTER(C.c_double)]),
     "ctl_objective": (C.c_int, [_H, _F64P, _F64P, _F64P, C.POINTER(C.c_double)]),
     "ctl_build_rhs": (C.c_int, [_H, _F64P, _F64P, _F64P, _F64P]),
+    "ctl_lift_bc": (C.c_int, [_H, _F64P, _F64P, C.c_int]),
     "ctl_amg_num_hierarchies": (C.c_int32, [_H]),
     "ctl_amg_num_levels": (C.c_int32, [_H, C.c_int32]),
     "ctl_amg_level_size": (C.c_int, [_H, C.c_int32, C.c_int32, _I32P, C.POINTER(C.c_int64),
@@ -115,6 +116,7 @@ SIGNATURES = {
     "ctl_stokes_set_pc_callback": (C.c_int, [_H, PC_CALLBACK, C.c_void_p]),
     "ctl_stokes_solve": (C.c_int, [_H, _F64P, _F64P, C.POINTER(ctl_krylov_options),
                                    C.POINTER(ctl_solve_result)]),
+    "ctl_stokes_lift_bc": (C.c_int, [_H, _F64P, _F64P]),
     "ctl_stokes_time": (C.c_int, [_H, C.c_int, C.POINTER(C.c_double)]),
     "ctl_amg_setup_probe": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.POINTER(ctl_pc_options),
                                       C.POINTER(C.c_int32), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

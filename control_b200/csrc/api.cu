@@ -113,6 +113,7 @@ int ctl_destroy(ctl_handle h)
     ctl_pc_free(h);
     ctl_krylov_free(h);
     ctl_comm_free(h);
+    ctl_lift_invalidate(h);
     for (double *p : h->pool) cudaFree(p);
     cudaFree(h->d_indptr);
     cudaFree(h->d_indices);
@@ -151,6 +152,7 @@ int ctl_set_pattern(ctl_handle h, const int32_t *indptr, const int32_t *indices,
     h->h_K.clear();
     h->h_KT.clear();
     h->loc = HostCSR();
+    ctl_lift_invalidate(h);
     h->assembled = false;
     return CTL_OK;
 }
@@ -181,6 +183,7 @@ int ctl_set_values(ctl_handle h, int which, int level, const double *values)
     } else {
         CTL_CHECK(false, CTL_ERR_ARG, "ctl_set_values: unknown matrix id");
     }
+    ctl_lift_invalidate(h);             // the lifting reads M and K: rebuilt on the next ctl_lift_bc
     h->assembled = false;
     return CTL_OK;
 }
@@ -194,6 +197,7 @@ int ctl_set_bc(ctl_handle h, const int32_t *dofs, int32_t count)
         CTL_CHECK(dofs[i] >= 0 && dofs[i] < h->n, CTL_ERR_ARG, "ctl_set_bc: dof out of range");
         h->h_bcmask[dofs[i]] = 1;
     }
+    ctl_lift_invalidate(h);
     h->assembled = false;
     return CTL_OK;
 }

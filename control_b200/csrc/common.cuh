@@ -103,6 +103,7 @@ struct ctl_handle_s {
     std::shared_ptr<struct PcState> pc;
     std::shared_ptr<struct KrylovState> ks;
     std::shared_ptr<struct CommState> comm;
+    std::shared_ptr<struct LiftState> lift;   // boundary-column CSR of ctl_lift_bc (lift.cu); null = build on next use
     ctl_pc_callback pc_cb = nullptr;
     void *pc_cb_user = nullptr;
 
@@ -128,6 +129,12 @@ void ctl_pc_free(ctl_handle_s *h);        // pc.cu
 void ctl_krylov_free(ctl_handle_s *h);    // krylov.cu
 void ctl_comm_free(ctl_handle_s *h);      // comm.cu
 int ctl_pc_invalidate(ctl_handle_s *h);   // pc.cu: matrices changed, rebuild on next setup
+void ctl_lift_invalidate(ctl_handle_s *h);   // lift.cu: M, K or the Dirichlet dofs changed
+// lift.cu: the constrained-velocity columns of the divergence matrix B (n_p x n_v host CSR, values before
+// elimination; columns in the ctl_set_bc list of the velocity handle h), and b_1_0 -= T_2(tau B g) on them
+int ctl_lift_div_setup(ctl_handle_s *h, const int32_t *B_indptr, const int32_t *B_indices, const double *B_values,
+                       int n_p, std::shared_ptr<struct LiftState> *out);
+int ctl_lift_div_apply(ctl_handle_s *h, const struct LiftState *S, const double *g, double *b10, int n_p);
 // comm.cu
 int ctl_halo_exchange(ctl_handle_s *h, const double *x_tf);            // both panels -> d_halo
 int ctl_halo_exchange_panel(ctl_handle_s *h, const double *panel_tf);  // one panel -> d_halo[0]

@@ -34,6 +34,7 @@ enum { T_NONE = 0, T_ONE = 1, T_TWO = 2 };
 struct ctl_stokes_s {
     ctl_handle_s *hv = nullptr, *hp = nullptr;
     DevCSR B, BT;                 // B with the constrained velocity COLUMNS zeroed, and its transpose
+    std::shared_ptr<LiftState> lift_div;   // the constrained columns of B before zeroing (ctl_stokes_lift_bc)
     ctl_stokes_pc_options opts{};
     bool pc_ready = false;
     std::shared_ptr<SellPattern> fine_p;
@@ -509,15 +510,18 @@ int ctl_stokes_create(ctl_handle velocity, ctl_handle pressure, const int32_t *B
     const int64_t nnz = B.indptr[n_p];
     B.indices.assign(B_indices, B_indices + nnz);
     B.values.assign(B_values, B_values + nnz);
-    for (int64_t k = 0; k < nnz; ++k) {
+    for (int64_t k = 0; k < nnz; ++k)
         CTL_CHECK(B.indices[k] >= 0 && B.indices[k] < n_v, CTL_ERR_ARG, "ctl_stokes_create: column index out of range");
+    std::shared_ptr<LiftState> lift_div;       // kept for the lifting of inhomogeneous velocity data
+    CTL_TRY(ctl_lift_div_setup(velocity, B_indptr, B_indices, B_values, n_p, &lift_div));
+    for (int64_t k = 0; k < nnz; ++k)
         if (velocity->h_bcmask[B.indices[k]]) B.values[k] = 0.0;      // the operator sees x with bcs zeroed
-    }
     HostCSR BT;
     csr_transpose(B, BT);
     ctl_stokes_s *S = new ctl_stokes_s();
     S->hv = velocity;
     S->hp = pressure;
+    S->lift_div = lift_div;
     int rc = upload_csr(h, B, S->B);
     if (rc == CTL_OK) rc = upload_csr(h, BT, S->BT);
     S->colsum_blocks = ceil_div(n_p, COLSUM_ROWS);
@@ -549,6 +553,18 @@ int ctl_stokes_destroy(ctl_stokes S)
     for (cudaEvent_t e : S->ks.events) cudaEventDestroy(e);
     delete S;
     return CTL_OK;
+}
+
+int ctl_stokes_lift_bc(ctl_stokes S, const double *g, double *b)
+{
+    if (!S) return CTL_ERR_ARG;
+    ctl_handle_s *h = S->hv;
+    CTL_CHECK(h->assembled, CTL_ERR_STATE, "ctl_stokes_lift_bc: the velocity handle is not assembled");
+    if (h->h_bc.empty()) return CTL_OK;
+    CTL_CHECK(g && b, CTL_ERR_ARG, "ctl_stokes_lift_bc: null g or b (the velocity handle has Dirichlet dofs)");
+    CTL_TRY(ctl_lift_bc(h, g, b, CTL_LAYOUT_BLOCK_MAJOR));              // velocity rows: [2N blocks of n_v]
+    CTL_CUDA(cudaSetDevice(h->cfg.device));
+    return ctl_lift_div_apply(h, S->lift_div.get(), g, b + 2 * (size_t)h->N * h->n_loc, S->hp->n_loc);   // b_1_0
 }
 
 int64_t ctl_stokes_vec_len(ctl_stokes S) { return S ? 2ll * S->hv->N * ((int64_t)S->hv->n_loc + S->hp->n_loc) : 0; }

@@ -149,6 +149,18 @@ class StokesSystem:
         self._call(fn, b_dev.data_ptr(), u_dev.data_ptr())
         return u_dev
 
+    def lift_bc_device(self, g, b_dev):
+        """Lift inhomogeneous velocity Dirichlet data into the outer device right-hand side ``b_dev`` (block-major,
+        ``vec_len()`` entries) in place (``ctl_stokes_lift_bc``): velocity rows as ``MultiBlockSystem.lift_bc_device``,
+        divergence rows ``b_1_0 -= tau B g`` then T_2 for CN (control/control.py:4107-4119, 4207-4219).  ``g``:
+        (n_t, len(bc_dofs_v)) host array or CUDA tensor.  Returns ``b_dev``."""
+        if b_dev.numel() != self.vec_len() or b_dev.dtype != torch.float64 or not b_dev.is_cuda \
+                or not b_dev.is_contiguous():
+            raise ValueError("lift_bc_device needs a contiguous float64 CUDA vector of vec_len() entries")
+        g_dev = self.velocity._bc_values_device(g)
+        self._call(self._lib.ctl_stokes_lift_bc, g_dev.data_ptr(), b_dev.data_ptr())
+        return b_dev
+
     def time_divergence_products(self, reps=20):
         """Average milliseconds and algorithmic bytes of the batched ``tau B X`` / ``Y += tau B^T X``
         panel products (``ctl_stokes_time``)."""

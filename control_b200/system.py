@@ -446,10 +446,11 @@ class MultiBlockSystem:
         self._call(self._lib.ctl_objective, v_dev.data_ptr(), zeta_dev.data_ptr(), v_hat_dev.data_ptr(), C.byref(out))
         return float(out.value)
 
-    def build_rhs_device(self, v_hat_dev, f_nodal_dev, v_0=None):
+    def build_rhs_device(self, v_hat_dev, f_nodal_dev, v_0=None, bc_values=None):
         """Block-major device right-hand side of ``linear_solve`` from nodal data on the device
         (n_t levels x n_local each: this rank's rows); ``v_0``: host initial condition (all n entries) or None
-        (``ctl_build_rhs``)."""
+        (``ctl_build_rhs``).  ``bc_values``: None (homogeneous Dirichlet data) or the (n_t, len(bc_dofs))
+        boundary values of the state, lifted in with ``lift_bc_device``."""
         need = self.n_t * self.n_local
         for t in (v_hat_dev, f_nodal_dev):
             if t.numel() != need or t.dtype != torch.float64 or not t.is_cuda or not t.is_contiguous():
@@ -460,7 +461,33 @@ class MultiBlockSystem:
         v0 = None if v_0 is None else np.ascontiguousarray(v_0, dtype=np.float64)
         self._call(self._lib.ctl_build_rhs, v_hat_dev.data_ptr(), f_nodal_dev.data_ptr(),
                    None if v0 is None else v0.ctypes.data, b.data_ptr())
+        if bc_values is not None:
+            self.lift_bc_device(bc_values, b)
         return b
+
+    def _bc_values_device(self, g):
+        """(n_t, len(bc_dofs)) boundary values -- host array or CUDA tensor -- as a contiguous float64 device tensor."""
+        shape = (self.n_t, int(self.bc_dofs.size))
+        if isinstance(g, torch.Tensor) and g.is_cuda:
+            g_dev = g.to(self.device, torch.float64).contiguous()
+        else:
+            g_dev = torch.from_numpy(np.ascontiguousarray(_as_host_f64(g), dtype=np.float64)).to(self.device)
+        if g_dev.numel() != shape[0] * shape[1] or (g_dev.dim() == 2 and tuple(g_dev.shape) != shape):
+            raise ValueError(f"bc values must have shape {shape} (n_t, len(bc_dofs))")
+        return g_dev
+
+    def lift_bc_device(self, g, b_dev, layout=L.CTL_LAYOUT_BLOCK_MAJOR):
+        """Lift inhomogeneous Dirichlet data into the device right-hand side ``b_dev`` in place (``ctl_lift_bc``): the
+        terms the reference adds through ``v_inhom`` (control/control.py:2993-3124 BE, 3137-3212 CN), with the K
+        values the system holds, T_1 / T_2 applied, constrained rows untouched.  ``g``: (n_t, len(bc_dofs)) host array
+        or CUDA tensor, columns in the order of ``bc_dofs`` (what ``Control.Instationary._dirichlet_data`` returns);
+        every rank passes all of it.  Returns ``b_dev``."""
+        if b_dev.numel() != self.vec_len(layout) or b_dev.dtype != torch.float64 or not b_dev.is_cuda \
+                or not b_dev.is_contiguous():
+            raise ValueError("lift_bc_device needs a contiguous float64 CUDA vector of vec_len(layout) entries")
+        g_dev = self._bc_values_device(g)
+        self._call(self._lib.ctl_lift_bc, g_dev.data_ptr(), b_dev.data_ptr(), layout)
+        return b_dev
 
     def objective(self, v, zeta, v_hat):
         v = np.ascontiguousarray(v, dtype=np.float64)

@@ -202,14 +202,29 @@ int ctl_objective_host(ctl_handle h, const double *v_host, const double *zeta_ho
  * receives J_h. */
 int ctl_objective(ctl_handle h, const double *v, const double *zeta, const double *v_hat,
                   double *out_host);
-/* ---- right-hand sides of linear_solve from NODAL data (control/control.py:2980-3243, homogeneous
- *      Dirichlet data): v_hat, f_nodal are DEVICE arrays of n_t levels x n (the reference's
+/* ---- right-hand sides of linear_solve from NODAL data (control/control.py:2980-3243) for homogeneous
+ *      Dirichlet data; inhomogeneous data are added afterwards with ctl_lift_bc.  v_hat, f_nodal are DEVICE arrays
+ *      of n_t levels x n (the reference's
  *      cofunctions are M v_hat_i, M f_i for interpolated data); v_0_host: the initial condition
  *      (n doubles, host: ALL n entries on every rank) or NULL = 0; b: DEVICE block-major output (this rank's
  *      rows), T_1 / T_2 applied.  Several ranks: v_hat, f_nodal hold this rank's rows (n_t x n_local); the ghost
  *      entries the products gather are fetched from their owners. */
 int ctl_build_rhs(ctl_handle h, const double *v_hat, const double *f_nodal, const double *v_0_host,
                   double *b);
+/* ---- lifting of inhomogeneous, time-dependent Dirichlet data of the state (the reference's `v_inhom`,
+ *      control/control.py:2993-3124 BE, 3137-3212 CN): b <- b - T(L(g)) on the unconstrained rows, where L(g) is what
+ *      the boundary values contribute through the constrained COLUMNS of M and K to the rows of linear_solve
+ *      (BE: L_0[i] = tau M g_i for i < n_t-1, L_1[i] = tau K_i g_i + M g_i - M g_{i-1}; CN: L_0[i] = h M (g_{i+1} + g_i),
+ *      L_1[i] = (h K_{i+1} + M) g_{i+1} + (h K_i - M) g_i, the g_0 terms dropped, h = tau/2) and T = (T_1, T_2) for
+ *      CN, the identity for BE.  Constrained rows of b are not touched.  The lifting is additive, so it composes with
+ *      ctl_build_rhs, a host-built b, and the b handed to ctl_nonlinear_residual (with K_i at the iterate: after new
+ *      ctl_set_values + ctl_assemble the next call uses the new values).
+ *      g: DEVICE, n_t levels x n_bc (level-major), columns in the order of the ctl_set_bc list; every rank passes all
+ *         n_t x n_bc values (no communication).
+ *      b: DEVICE, in and out, this rank's rows in `layout`.
+ *      Errors: CTL_ERR_STATE before ctl_assemble; CTL_ERR_ARG for an unknown layout, or a NULL g / b when the handle
+ *      has Dirichlet dofs.  With no Dirichlet dofs the call does nothing.  Asynchronous on the handle's stream. */
+int ctl_lift_bc(ctl_handle h, const double *g, double *b, int layout);
 
 /* ---- AMG introspection (tests compare the hierarchy with the oracle's) */
 int32_t ctl_amg_num_hierarchies(ctl_handle h);
@@ -276,6 +291,12 @@ int ctl_stokes_set_pc_callback(ctl_stokes s, ctl_pc_callback fn, void *user);
  * opts->pc: CTL_PC_NONE or CTL_PC_BUILTIN */
 int ctl_stokes_solve(ctl_stokes s, const double *b, double *u, const ctl_krylov_options *opts,
                      ctl_solve_result *result);
+/* lifting of inhomogeneous velocity Dirichlet data into an outer right-hand side b (DEVICE, block-major, in and out):
+ * the velocity rows as ctl_lift_bc on the velocity handle, and the divergence rows b_1_0[i] -= tau B g_{i+1} (CN) /
+ * tau B g_i (BE), then T_2 for CN (control/control.py:4107-4119, 4207-4219), with the constrained columns of B as
+ * handed to ctl_stokes_create.  g: DEVICE, n_t x n_bc of the velocity handle, level-major.  Error codes as
+ * ctl_lift_bc, reported through ctl_last_error(velocity). */
+int ctl_stokes_lift_bc(ctl_stokes s, const double *g, double *b);
 /* time `reps` back-to-back launches of the batched divergence products on one time panel (CUDA
  * events on the stream; the panels exceed L2 at config C4).  out[0] = tau B X, average ms;
  * out[1] = its algorithmic bytes (12 nnz_B + 4 (n_p + 1) + 8 N (n_v + n_p)); out[2] = Y += tau B^T X,
