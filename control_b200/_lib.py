@@ -117,6 +117,7 @@ SIGNATURES = {
     "ctl_stokes_solve": (C.c_int, [_H, _F64P, _F64P, C.POINTER(ctl_krylov_options),
                                    C.POINTER(ctl_solve_result)]),
     "ctl_stokes_lift_bc": (C.c_int, [_H, _F64P, _F64P]),
+    "ctl_stokes_nonlinear_residual": (C.c_int, [_H, _F64P, _F64P, _F64P, C.POINTER(C.c_double)]),
     "ctl_stokes_time": (C.c_int, [_H, C.c_int, C.POINTER(C.c_double)]),
     "ctl_amg_setup_probe": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.POINTER(ctl_pc_options),
                                       C.POINTER(C.c_int32), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -359,10 +359,18 @@ class Control:
                                             max_non_linear_iter=10, relative_non_linear_tol=10.0**-5,
                                             absolute_non_linear_tol=10.0**-8, print_error_linear=False,
                                             print_error_non_linear=True, create_output=False, plots=False,
-                                            amg=None, amg_p=None):
+                                            amg=None, amg_p=None, device_loop=None):
             """control/control.py:4886-5219: Picard loop of Navier-Stokes control.  Every outer iteration
             re-linearises the forward operator around the new velocity on both spaces, hands the values to
-            the GPU and solves the outer Stokes-type system for the increment there."""
+            the GPU and solves the outer Stokes-type system for the increment there.
+
+            ``device_loop``: True keeps the iterate, the residual and the increments in HBM
+            (``_incompressible_non_linear_solve_device``; in-built preconditioner only, so ``P=`` raises
+            ``ValueError``); False or None runs the host loop, which evaluates the residual on the host and moves the
+            whole outer vector both ways every iteration.  None stays the host loop for now because the stand-in
+            systems that exercise both loops on inhomogeneous data have no device methods."""
+            if device_loop and P is not None:
+                raise ValueError("device_loop=True runs the in-built preconditioner; it does not take P=")
             if space_p is None:
                 space_p = getattr(self, "_space_p", None)
                 if space_p is None:
@@ -385,6 +393,13 @@ class Control:
             v_d = self.construct_v_d()
             g = self._dirichlet_data()
             self._v, self._zeta = v_old.copy(), zeta_old.copy()
+            if device_loop:
+                if nullspace_p not in (None, "constant"):
+                    raise ValueError("only the constant pressure nullspace is supported")
+                return self._incompressible_non_linear_solve_device(
+                    space_p, v_old, zeta_old, p_old, mu_old, v_0, v_d, f, g, solver_parameters, Multigrid,
+                    lambda_v_bounds, lambda_p_bounds, max_non_linear_iter, relative_non_linear_tol,
+                    absolute_non_linear_tol, print_error_linear, print_error_non_linear, amg, amg_p)
 
             def res_eval():                                             # 4979-5072
                 r00, r01 = self.non_linear_res_eval(v_old, zeta_old, v_0, v_d, f)
@@ -432,6 +447,106 @@ class Control:
                     break
             return k
 
+        def _incompressible_non_linear_solve_device(self, space_p, v_old, zeta_old, p_old, mu_old, v_0, v_d, f, g,
+                                                    solver_parameters, Multigrid, lambda_v_bounds, lambda_p_bounds,
+                                                    max_non_linear_iter, rel_tol, abs_tol, print_error_linear,
+                                                    print_error_non_linear, amg, amg_p):
+            """The loop of control/control.py:4886-5219 with device-resident iterates.  The right-hand side of the
+            data is built once (velocity rows as ``incompressible_linear_solve`` builds them, pressure rows zero).
+            Per outer iteration: the increment solve reads the residual where it lies, the velocity state goes to the
+            host (N n_v doubles) for the assembly of ``D_v_i`` / ``D_p_i``, their values come back
+            (``set_forward``), a copy of b is lifted with g (``lift_bc_device``), and the residual is
+            ``ctl_stokes_nonlinear_residual``: b - A_raw x with the RAW coupling products, as ``res_eval`` has them
+            (no ConstantNullspace corrections), and the norm of its untransformed parts."""
+            from .stokes import StokesSystem
+            n_t, tau, CN = self._n_t, self.tau, self._CN
+            N = n_t - 1 if CN else n_t
+            n_p = space_p["M_p"].shape[0]
+            times = self._times()
+            bd = self._bc_dofs
+            linear = self._is_linear()
+            fp = space_p.get("forward_matrix_p")
+            if not linear and fp is None:
+                raise ValueError("a non-linear forward operator needs space_p['forward_matrix_p']")
+
+            def forward(v):                                             # D_v_i, D_p_i at the state, 3780-3789
+                if linear:
+                    return self._forward_matrix, None
+                return ([self.construct_D_v(v[i], t) for i, t in enumerate(times)],
+                        [fp(v[i], t, self._Gauss_Newton) for i, t in enumerate(times)])
+
+            def rhs(v_init):                                            # 3961-4243, homogeneous data
+                K0 = self._forward_matrix if linear else self.construct_D_v(v_init, self._time_interval[0])
+                b_0_0, b_0_1 = build_rhs(self._M, K0, tau, n_t, CN, bd, v_d, f, v_init)
+                return system.to_device(np.concatenate([b_0_0, b_0_1]), np.zeros((2 * N, n_p)))
+            if solver_parameters is None:                               # 4291-4297
+                solver_parameters = {"linear_solver": "fgmres", "fgmres_restart": 10, "maximum_iterations": 100,
+                                     "relative_tolerance": 1.0e-6, "absolute_tolerance": 0.0,
+                                     "monitor_convergence": print_error_linear}
+            K, D_p = forward(v_old)
+            if getattr(self, "_stokes", None) is None:
+                self._stokes = StokesSystem(self._M, K, space_p["B"], space_p["M_p"], space_p["K_p"], n_t=n_t,
+                                            beta=self._beta, CN=CN, time_interval=self._time_interval,
+                                            bc_dofs_v=bd, device=self._dev["device"], D_p=D_p)
+            elif not linear:
+                self._stokes.set_forward(K, D_p)
+            system = self._stokes
+            if g is None:
+                b_dev = b_hom = rhs(v_0)
+            else:
+                b_hom, b_dev = self._lifted_rhs_pair(system, rhs, v_old, v_0, g)
+            x_dev = system.to_device(np.concatenate([v_old[1:], zeta_old[:-1]] if CN else [v_old, zeta_old]),
+                                     np.concatenate([mu_old, p_old]))
+            r_dev = system.new_vector()
+            norm_0 = system.nonlinear_residual(b_dev, x_dev, r_dev)
+            norm_k, k = norm_0, 0
+            self.non_linear_history = [norm_0]
+            self.inner_iterations = []
+            if print_error_non_linear:
+                print(f"Initial non-linear residual: {norm_0:.16e}")
+            while norm_k > rel_tol * norm_0 and norm_k > abs_tol:
+                system.setup_preconditioner(lambda_v_bounds=lambda_v_bounds, lambda_p_bounds=lambda_p_bounds, amg=amg,
+                                            amg_p=amg_p, Multigrid=Multigrid)
+                d_dev = system.new_vector()
+                self.last_ksp = system.solve_device(r_dev, d_dev, solver_parameters=solver_parameters)
+                if not solver_parameters.get("preconditioner", False) and self.last_ksp.reason <= 0:
+                    raise RuntimeError("Solver failed to converge")
+                if solver_parameters.get("monitor_convergence", True):
+                    for it, r_norm in enumerate(self.last_ksp.history):
+                        print(f"KSP: iteration {it:d}, residual norm {r_norm:.16e}")
+                self.inner_iterations.append(self.last_ksp.its)
+                x_dev += d_dev
+                v_blocks = system.velocity_state_to_host(x_dev)
+                if CN:
+                    v_old[1:] = v_blocks
+                else:
+                    v_old = v_blocks
+                if g is not None:                                       # 5127-5160
+                    v_old[:, bd] = g
+                if not linear:
+                    system.set_forward(*forward(v_old))
+                if g is not None:
+                    b_dev = system.lift_bc_device(g, b_hom.clone())
+                norm_k = system.nonlinear_residual(b_dev, x_dev, r_dev)
+                k += 1
+                self.non_linear_history.append(norm_k)
+                if print_error_non_linear:
+                    print(f"Non-linear solver: iteration {k:d}, non-linear residual norm {norm_k:.16e}")
+                if k + 1 > max_non_linear_iter:
+                    break
+            x_0, x_1 = system.to_host_blocks(x_dev)
+            if CN:
+                v_old[1:], zeta_old[:-1] = x_0[:N], x_0[N:]
+            else:
+                v_old, zeta_old = x_0[:N].copy(), x_0[N:].copy()
+            if k > 0:
+                if g is not None:
+                    v_old[:, bd] = g
+                self._bc(zeta_old)
+            self._v, self._zeta = v_old.copy(), zeta_old.copy()
+            self._p, self._mu = x_1[N:].copy(), x_1[:N].copy()
+            return k
+
         # ------------------------------------------------------------------ non_linear_solve
         def non_linear_res_eval(self, v_old, zeta_old, v_0, v_d, f):
             """control/control.py:2442-2818: right-hand side minus the KKT operator applied to
@@ -472,10 +587,21 @@ class Control:
         def non_linear_solve(self, *, P=None, solver_parameters=None, Multigrid=False, lambda_v_bounds=None,
                              max_non_linear_iter=10, relative_non_linear_tol=10.0**-5,
                              absolute_non_linear_tol=10.0**-8, print_error_linear=False,
-                             print_error_non_linear=True, create_output=False, plots=False, **amg):
+                             print_error_non_linear=True, create_output=False, plots=False, device_loop=None, **amg):
             """control/control.py:3377-3590: Picard / Gauss-Newton loop.  Every outer iteration
             hands new ``K_i`` values to the GPU (``MultiBlockSystem.set_K``) and solves for
-            the increment."""
+            the increment.
+
+            ``device_loop``: True keeps the iterate, the residual and the increments in HBM
+            (``_non_linear_solve_device``), with homogeneous or inhomogeneous Dirichlet data; it needs the in-built
+            preconditioner and one rank, so ``P=`` or ``world > 1`` raise ``ValueError``.  False runs the host loop.
+            None keeps the device loop for homogeneous data, the in-built preconditioner, one rank and a non-linear
+            forward operator, and the host loop otherwise: the stand-in systems that exercise both loops on
+            inhomogeneous data have no device methods."""
+            if device_loop and P is not None:
+                raise ValueError("device_loop=True runs the in-built preconditioner; it does not take P=")
+            if device_loop and self._dev["world"] > 1:
+                raise ValueError("device_loop=True runs on one rank")
             n_t, n = self._n_t, self._n
             g = self._dirichlet_data()
             v_old = self._v.copy()
@@ -487,10 +613,11 @@ class Control:
             f = self.construct_f()
             v_d = self.construct_v_d()
             self._v, self._zeta = v_old.copy(), zeta_old.copy()
-            if P is None and g is None and self._dev["world"] == 1 and not self._is_linear():
-                # homogeneous Dirichlet data, in-built preconditioner, one rank: the iterate, the residual and the
-                # increments stay in HBM; only the state crosses the boundary, because the forward form D_v(v_i)
-                # is assembled on the caller's side (Firedrake's) of it
+            if device_loop is None:
+                device_loop = P is None and g is None and self._dev["world"] == 1 and not self._is_linear()
+            if device_loop:
+                # the iterate, the residual and the increments stay in HBM; only the state crosses the boundary,
+                # because the forward form D_v(v_i) is assembled on the caller's side (Firedrake's) of it
                 return self._non_linear_solve_device(v_old, zeta_old, v_0, v_d, f, solver_parameters, Multigrid,
                                                      lambda_v_bounds, max_non_linear_iter, relative_non_linear_tol,
                                                      absolute_non_linear_tol, print_error_linear,
@@ -531,17 +658,25 @@ class Control:
             back (``set_K``), the residual is ``ctl_nonlinear_residual`` (right-hand side of ``linear_solve`` for
             the data, built ONCE, minus the fused operator at the iterate: the identity of
             tests/test_oracle.py::test_non_linear_residual_is_rhs_minus_operator), and the increment solve reads
-            it where it lies."""
+            it where it lies.  Inhomogeneous Dirichlet data g (INTEGRATION.md section 6): the residual takes a copy
+            of b lifted with the K_i of the iterate (``lift_bc_device``), and g is written into the iterate."""
             n_t, n, CN = self._n_t, self._n, self._CN
             times = self._times()
-            K0 = self.construct_D_v(v_0, self._time_interval[0])
-            b_0, b_1 = build_rhs(self._M, K0, self.tau, n_t, CN, self._bc_dofs, v_d, f, v_0)
+            g = self._dirichlet_data()
+            bd = self._bc_dofs
+
+            def rhs(v_init):
+                K0 = self.construct_D_v(v_init, self._time_interval[0])
+                return system.to_device(*build_rhs(self._M, K0, self.tau, n_t, CN, bd, v_d, f, v_init))
             if solver_parameters is None:                       # control.py:3260-3266
                 solver_parameters = {"linear_solver": "gmres", "gmres_restart": 10, "maximum_iterations": 50,
                                      "relative_tolerance": 1.0e-6, "absolute_tolerance": 0.0,
                                      "monitor_convergence": print_error_linear}
             system = self._ensure_system([self.construct_D_v(v_old[i], times[i]) for i in range(n_t)])
-            b_dev = system.to_device(b_0, b_1)
+            if g is None:
+                b_dev = rhs(v_0)
+            else:
+                b_hom, b_dev = self._lifted_rhs_pair(system, rhs, v_old, v_0, g)
             x_dev = system.to_device(*((v_old[1:], zeta_old[:-1]) if CN else (v_old, zeta_old)))
             r_dev = system.new_vector()
             norm_0 = system.nonlinear_residual(b_dev, x_dev, r_dev)
@@ -564,7 +699,11 @@ class Control:
                     v_old[1:] = v_blocks
                 else:
                     v_old = v_blocks.copy()
+                if g is not None:                               # control.py:3480-3483
+                    v_old[:, bd] = g
                 system.set_K([self.construct_D_v(v_old[i], times[i]) for i in range(n_t)])
+                if g is not None:
+                    b_dev = system.lift_bc_device(g, b_hom.clone())
                 norm_k = system.nonlinear_residual(b_dev, x_dev, r_dev)
                 k += 1
                 self.non_linear_history.append(norm_k)
@@ -577,9 +716,28 @@ class Control:
                 v_old[1:], zeta_old[:-1] = x_0, x_1
             else:
                 v_old, zeta_old = x_0.copy(), x_1.copy()
+            if g is not None and k > 0:
+                v_old[:, bd] = g
             self._bc(zeta_old)
             self._v, self._zeta = v_old.copy(), zeta_old.copy()
             return k
+
+        def _lifted_rhs_pair(self, system, rhs, v_old, v_0, g):
+            """Device right-hand sides of a non-linear loop with inhomogeneous Dirichlet data g: the homogeneous b that
+            every residual after the first lifts a copy of (for CN its initial condition is v_0 with g_0 on the
+            boundary, because the loop writes g into every level of the iterate, level 0 included), and the b of the
+            first residual, lifted with the boundary values the starting iterate carries.  ``rhs(v_init)`` builds a
+            homogeneous device right-hand side."""
+            b_first = rhs(v_0)
+            b_hom = b_first
+            if self._CN:
+                v_0g = v_0.copy()
+                v_0g[self._bc_dofs] = g[0]
+                b_hom = rhs(v_0g)
+            g_it = np.ascontiguousarray(v_old[:, self._bc_dofs])
+            if np.any(g_it):
+                b_first = system.lift_bc_device(g_it, b_first.clone())
+            return b_hom, b_first
 
 
 from .stationary import Stationary as _Stationary  # noqa: E402

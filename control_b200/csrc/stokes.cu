@@ -46,6 +46,8 @@ struct ctl_stokes_s {
     double *d_part = nullptr;     // partial column sums, [2 panels][blocks][ld]
     double *d_mean = nullptr;     // [2 sets][2 panels][ld]
     int colsum_blocks = 0;
+    double *d_res_part = nullptr; // per-block partial norms of ctl_stokes_nonlinear_residual, then the norm
+    int res_blocks = 0;
     std::vector<double *> pool;   // outer-length scratch vectors
     KrylovState ks;
     ctl_pc_callback pc_cb = nullptr;   // user preconditioner P= of incompressible_linear_solve (control/control.py:4686-4689)
@@ -168,6 +170,85 @@ __global__ void colsum_finish_kernel(const double *__restrict__ part, double *__
     double s = 0.0;
     for (int b = 0; b < blocks; ++b) s += part[(size_t)b * ld + c];
     mean[blockIdx.x * ld + c] = s / (double)n_rows;
+}
+
+// Epilogue of ctl_stokes_nonlinear_residual, one pass over the four panels of an internal-layout outer vector
+// (rows [0, 2 n_v): velocity, then 2 n_p pressure rows):
+//   velocity rows  R[r, :] <- b[r, :] - R[r, :], zero on constrained rows (R holds A_raw x there)
+//   pressure rows  R already holds b_p - tau T(B x_v); read only
+//   part[block]    sum over the block's rows of w ||T^-1 R[r, :]||^2, w = 1 (velocity) / w_p = 1 / tau^2 (pressure);
+//                  T^-1 (CN only) is T_1^-1 on the first velocity and the second pressure panel, T_2^-1 on the other
+//                  two -- the T each panel carries in stokes_apply_tf
+// Every lane takes part in both scans so that rows of different panels may share a warp.
+template <int G, int CPL>
+__global__ void __launch_bounds__(256) stokes_residual_kernel(const double *__restrict__ b, double *R,
+                                                             const uint8_t *__restrict__ bcmask,
+                                                             double *__restrict__ part, int n_v, int n_p, int N,
+                                                             int ld, int cn, double w_p)
+{
+    __shared__ double sh[8];
+    const int n_rows = 2 * n_v + 2 * n_p;
+    const RowMap m = row_map<G, CPL>(n_rows);
+    const size_t off = (size_t)m.r * ld + m.c0;
+    const bool vel = m.r < 2 * n_v;
+    double v[CPL];
+#pragma unroll
+    for (int q = 0; q < CPL / 2; ++q) {
+        const double2 o = *reinterpret_cast<const double2 *>(R + off + 2 * q);
+        v[2 * q] = o.x;
+        v[2 * q + 1] = o.y;
+    }
+    if (vel) {
+        double s[CPL];
+        load_cols<CPL>(b + off, s);
+        const bool bc = bcmask[m.r < n_v ? m.r : m.r - n_v] != 0;
+#pragma unroll
+        for (int q = 0; q < CPL; ++q) v[q] = bc ? 0.0 : s[q] - v[q];
+    }
+#pragma unroll
+    for (int q = 0; q < CPL; ++q)
+        if (m.c0 + q >= N) v[q] = 0.0;
+    if (vel && m.live) store_cols<CPL>(R + off, v);
+    if (cn) {
+        const bool one = vel ? m.r < n_v : m.r >= 2 * n_v + n_p;
+        double a[CPL], c[CPL];
+#pragma unroll
+        for (int q = 0; q < CPL; ++q) a[q] = c[q] = v[q];
+        t1_inv<G, CPL>(a, m.l);
+        t2_inv<G, CPL>(c, m.l);
+#pragma unroll
+        for (int q = 0; q < CPL; ++q) v[q] = one ? a[q] : c[q];
+    }
+    double s = 0.0;
+#pragma unroll
+    for (int q = 0; q < CPL; ++q)
+        if (m.c0 + q < N) s = fma(v[q], v[q], s);
+    s = m.live ? (vel ? s : w_p * s) : 0.0;
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) s += __shfl_down_sync(0xffffffffu, s, d);
+    if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = s;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double t = 0.0;
+        for (int w = 0; w < 8; ++w) t += sh[w];
+        part[blockIdx.x] = t;
+    }
+}
+
+// out = sqrt(sum_b part[b]) in a fixed order (one block of 256 threads)
+__global__ void __launch_bounds__(256) residual_finish_kernel(const double *__restrict__ part, int blocks,
+                                                              double *__restrict__ out)
+{
+    __shared__ double sh[256];
+    double s = 0.0;
+    for (int b = threadIdx.x; b < blocks; b += 256) s += part[b];
+    sh[threadIdx.x] = s;
+    __syncthreads();
+    for (int w = 128; w > 0; w >>= 1) {
+        if (threadIdx.x < w) sh[threadIdx.x] += sh[threadIdx.x + w];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) *out = sqrt(sh[0]);
 }
 
 // out = v - mean_v (+ mean_w), both panels (2 * n_rows rows of ld columns)
@@ -527,6 +608,9 @@ int ctl_stokes_create(ctl_handle velocity, ctl_handle pressure, const int32_t *B
     S->colsum_blocks = ceil_div(n_p, COLSUM_ROWS);
     if (rc == CTL_OK && cudaMalloc((void **)&S->d_part, sizeof(double) * 2 * S->colsum_blocks * h->ld) != cudaSuccess) rc = CTL_ERR_CUDA;
     if (rc == CTL_OK && cudaMalloc((void **)&S->d_mean, sizeof(double) * 4 * h->ld) != cudaSuccess) rc = CTL_ERR_CUDA;
+    S->res_blocks = blocks_for(2 * (velocity->n_loc + pressure->n_loc), h->ld);
+    if (rc == CTL_OK && cudaMalloc((void **)&S->d_res_part, sizeof(double) * (S->res_blocks + 1)) != cudaSuccess)
+        rc = CTL_ERR_CUDA;
     if (rc != CTL_OK) {
         ctl_stokes_destroy(S);
         return rc;
@@ -548,6 +632,7 @@ int ctl_stokes_destroy(ctl_stokes S)
     cudaFree(S->ts_x);
     cudaFree(S->d_part);
     cudaFree(S->d_mean);
+    cudaFree(S->d_res_part);
     for (double *p : S->pool) cudaFree(p);
     for (double *p : S->ks.basis) cudaFree(p);
     for (cudaEvent_t e : S->ks.events) cudaEventDestroy(e);
@@ -565,6 +650,58 @@ int ctl_stokes_lift_bc(ctl_stokes S, const double *g, double *b)
     CTL_TRY(ctl_lift_bc(h, g, b, CTL_LAYOUT_BLOCK_MAJOR));              // velocity rows: [2N blocks of n_v]
     CTL_CUDA(cudaSetDevice(h->cfg.device));
     return ctl_lift_div_apply(h, S->lift_div.get(), g, b + 2 * (size_t)h->N * h->n_loc, S->hp->n_loc);   // b_1_0
+}
+
+// Residual of the Navier-Stokes Picard loop (res_eval, control/control.py:4979-5072) on device vectors.  The
+// reference takes it with the RAW coupling products (r00 -= tau B^T mu, r01 -= tau B^T p, r10 = -B v, r11 = -B zeta),
+// so this is b - A_raw x: the operator of stokes_apply_tf without the ConstantNullspace corrections of the pressure
+// parts, which would shift the residual by the per-block means of mu and p.  Norm: that of the untransformed,
+// unscaled parts, ||T^-1 r_v||^2 + ||T^-1 r_p||^2 / tau^2.
+int ctl_stokes_nonlinear_residual(ctl_stokes S, const double *b, const double *x, double *r, double *norm_host)
+{
+    if (!S) return CTL_ERR_ARG;
+    ctl_handle_s *h = S->hv, *hp = S->hp;
+    CTL_CHECK(b && x && r && norm_host, CTL_ERR_ARG, "ctl_stokes_nonlinear_residual: null argument");
+    CTL_CHECK(r != b && r != x, CTL_ERR_ARG, "ctl_stokes_nonlinear_residual: r must not alias b or x");
+    CTL_CHECK(h->assembled && hp->assembled, CTL_ERR_STATE,
+              "ctl_stokes_nonlinear_residual: the velocity and pressure handles are not assembled");
+    CTL_CUDA(cudaSetDevice(h->cfg.device));
+    const bool cn = h->cfg.CN != 0;
+    const double tau = h->cfg.tau;
+    const int n_v = h->n_loc, n_p = hp->n_loc, ld = h->ld;
+    const size_t pv = (size_t)n_v * ld, pp = (size_t)n_p * ld;
+    const int64_t lv = h->vec_len();
+    double *partials = nullptr, *scalars = nullptr;
+    CTL_TRY(vec_workspace(h, &partials, &scalars));                             // pinned staging of vec_read_scalars
+    double *bt = nullptr, *xt = nullptr, *yt = nullptr;
+    CTL_TRY(outer_get(S, &bt));
+    CTL_TRY(outer_get(S, &xt));
+    CTL_TRY(outer_get(S, &yt));
+    int rc = outer_to_tf(S, b, bt);
+    if (rc == CTL_OK) rc = outer_to_tf(S, x, xt);
+    if (rc == CTL_OK) rc = ctl_kkt_apply_tf(h, xt, yt);                          // block_00 with D_v at the iterate
+    for (int q = 0; q < 2 && rc == CTL_OK; ++q)                                   // + tau T(B^T x_p), raw x_p
+        rc = panel_spmm(S, S->BT, xt + lv + q * pp, nullptr, yt + q * pv, tau, 1.0,
+                        cn ? (q == 0 ? T_ONE : T_TWO) : T_NONE, T_NONE, true);
+    for (int q = 0; q < 2 && rc == CTL_OK; ++q)                                   // r_p = b_p - tau T(B x_v)
+        rc = panel_spmm(S, S->B, xt + q * pv, bt + lv + q * pp, yt + lv + q * pp, tau, -1.0,
+                        cn ? (q == 0 ? T_TWO : T_ONE) : T_NONE, T_NONE, false);
+    if (rc == CTL_OK) {
+        DISPATCH_G(ld, (stokes_residual_kernel<GG, CC><<<S->res_blocks, 256, 0, h->stream>>>(
+                           bt, yt, h->d_bcmask, S->d_res_part, n_v, n_p, h->N, ld, cn ? 1 : 0, 1.0 / (tau * tau))));
+        residual_finish_kernel<<<1, 256, 0, h->stream>>>(S->d_res_part, S->res_blocks, S->d_res_part + S->res_blocks);
+        h->launches += 2;
+        if (cudaGetLastError() != cudaSuccess) {
+            ctl_set_error(h, "ctl_stokes_nonlinear_residual: kernel launch failed");
+            rc = CTL_ERR_CUDA;
+        }
+    }
+    if (rc == CTL_OK) rc = outer_to_bm(S, yt, r);
+    if (rc == CTL_OK) rc = vec_read_scalars(h, S->d_res_part + S->res_blocks, 1, norm_host);
+    S->pool.push_back(bt);
+    S->pool.push_back(xt);
+    S->pool.push_back(yt);
+    return rc;
 }
 
 int64_t ctl_stokes_vec_len(ctl_stokes S) { return S ? 2ll * S->hv->N * ((int64_t)S->hv->n_loc + S->hp->n_loc) : 0; }

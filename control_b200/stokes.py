@@ -102,6 +102,21 @@ class StokesSystem:
         L0 = 2 * self.N * self.n_v
         return a[:L0].reshape(2 * self.N, self.n_v), a[L0:].reshape(2 * self.N, self.n_p)
 
+    def velocity_state_to_host(self, x_dev):
+        """The N velocity-state blocks of an outer device vector (its first N n_v entries) as a host array of shape
+        (N, n_v): all a Picard loop needs to assemble ``D_v_i`` / ``D_p_i`` at the iterate."""
+        self._check_vec(x_dev, "velocity_state_to_host")
+        return x_dev[:self.N * self.n_v].cpu().numpy().reshape(self.N, self.n_v)
+
+    def new_vector(self):
+        """A zero outer device vector (block-major, ``vec_len()`` entries)."""
+        return torch.zeros(self.vec_len(), dtype=torch.float64, device=self.device)
+
+    def _check_vec(self, t, what):
+        if not isinstance(t, torch.Tensor) or t.numel() != self.vec_len() or t.dtype != torch.float64 \
+                or not t.is_cuda or not t.is_contiguous():
+            raise ValueError(f"{what} needs contiguous float64 CUDA vectors of vec_len() entries")
+
     # ------------------------------------------------------------------ operator / preconditioner
     def apply(self, x_dev, y_dev=None):
         """y = A x (MultiBlockSystemMatrix.mult, preconditioner/preconditioner.py:375-543)."""
@@ -160,6 +175,20 @@ class StokesSystem:
         g_dev = self.velocity._bc_values_device(g)
         self._call(self._lib.ctl_stokes_lift_bc, g_dev.data_ptr(), b_dev.data_ptr())
         return b_dev
+
+    def nonlinear_residual(self, b_dev, x_dev, r_dev):
+        """Residual of the Navier-Stokes Picard loop on outer device vectors (``ctl_stokes_nonlinear_residual``;
+        replaces ``res_eval`` of control/control.py:4979-5072): fills ``r_dev = b - A_raw x`` -- the right-hand side
+        of the increment solve, constrained velocity rows zero -- and returns the norm the reference's loop tests,
+        that of the untransformed parts (r00, r01, r10, r11).  ``A_raw`` is the outer operator with ``D_v`` at the
+        iterate (call ``set_forward`` first) and the RAW coupling products: unlike ``apply`` it does not centre the
+        pressure parts, because the reference's residual does not."""
+        for t in (b_dev, x_dev, r_dev):
+            self._check_vec(t, "nonlinear_residual")
+        out = C.c_double()
+        self._call(self._lib.ctl_stokes_nonlinear_residual, b_dev.data_ptr(), x_dev.data_ptr(), r_dev.data_ptr(),
+                   C.byref(out))
+        return float(out.value)
 
     def time_divergence_products(self, reps=20):
         """Average milliseconds and algorithmic bytes of the batched ``tau B X`` / ``Y += tau B^T X``

@@ -297,6 +297,17 @@ int ctl_stokes_solve(ctl_stokes s, const double *b, double *u, const ctl_krylov_
  * handed to ctl_stokes_create.  g: DEVICE, n_t x n_bc of the velocity handle, level-major.  Error codes as
  * ctl_lift_bc, reported through ctl_last_error(velocity). */
 int ctl_stokes_lift_bc(ctl_stokes s, const double *g, double *b);
+/* Residual of the Navier-Stokes Picard loop (res_eval of incompressible_non_linear_solve, control/control.py:
+ * 4979-5072) on DEVICE vectors of ctl_stokes_vec_len doubles, outer block-major layout: r = b - A_raw x, with A_raw
+ * the fused KKT operator on the velocity blocks (the K values the velocity handle holds: D_v at the iterate, after
+ * ctl_set_values / ctl_assemble), plus tau T(B^T x_p) on the velocity rows and tau T(B x_v) on the pressure rows,
+ * WITHOUT the ConstantNullspace corrections of ctl_stokes_apply -- the reference's residual uses raw products.
+ * Constrained velocity rows of r are zero; D_p does not enter.  *norm_host = sqrt(||T^-1 r_v||^2 +
+ * ||T^-1 r_p||^2 / tau^2), the norm of the untransformed, unscaled parts (r00, r01, r10, r11) the loop tests (T_1 on
+ * the first N velocity blocks and the last N pressure blocks, T_2 on the others; identity for BE).  b and x are not
+ * modified; r must not alias them.  CTL_ERR_ARG for null or aliased pointers, CTL_ERR_STATE if a handle is not
+ * assembled; messages through ctl_last_error(velocity). */
+int ctl_stokes_nonlinear_residual(ctl_stokes s, const double *b, const double *x, double *r, double *norm_host);
 /* time `reps` back-to-back launches of the batched divergence products on one time panel (CUDA
  * events on the stream; the panels exceed L2 at config C4).  out[0] = tau B X, average ms;
  * out[1] = its algorithmic bytes (12 nnz_B + 4 (n_p + 1) + 8 N (n_v + n_p)); out[2] = Y += tau B^T X,
