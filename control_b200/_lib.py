@@ -72,6 +72,7 @@ SIGNATURES = {
     "ctl_set_pattern": (C.c_int, [_H, C.c_void_p, C.c_void_p, C.c_int64]),
     "ctl_set_values": (C.c_int, [_H, C.c_int, C.c_int, C.c_void_p]),
     "ctl_set_bc": (C.c_int, [_H, C.c_void_p, C.c_int32]),
+    "ctl_set_block_size": (C.c_int, [_H, C.c_int32]),
     "ctl_assemble": (C.c_int, [_H]),
     "ctl_n_blocks": (C.c_int32, [_H]),
     "ctl_ld": (C.c_int32, [_H]),
@@ -82,6 +83,7 @@ SIGNATURES = {
     "ctl_kkt_apply": (C.c_int, [_H, _F64P, _F64P, C.c_int]),
     "ctl_pc_default_options": (C.c_int, [C.POINTER(ctl_pc_options)]),
     "ctl_pc_setup": (C.c_int, [_H, C.POINTER(ctl_pc_options)]),
+    "ctl_pc_block_size": (C.c_int32, [_H]),
     "ctl_pc_apply": (C.c_int, [_H, _F64P, _F64P, C.c_int]),
     "ctl_pc_fn": (C.c_int, [_H, _F64P, _F64P, C.c_int]),
     "ctl_set_pc_callback": (C.c_int, [_H, PC_CALLBACK, C.c_void_p]),

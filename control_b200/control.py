@@ -105,16 +105,26 @@ class Control:
     class Instationary:
         def __init__(self, M, forward_matrix, *, desired_state=None, force_f=None, force_function=None,
                      beta=1.0e-3, Gauss_Newton=False, CN=True, n_t=20, initial_condition=None,
-                     time_interval=(0.0, 1.0), bc_dofs=(), bc_values=None, device=None, rank=0, world=1):
+                     time_interval=(0.0, 1.0), bc_dofs=(), bc_values=None, device=None, rank=0, world=1,
+                     block_size=1):
             """``M``: mass matrix (scipy CSR).  ``forward_matrix(v_i, t, gauss_newton)`` -> CSR
             on M's pattern: the matrix ``D_v`` of ``construct_D_v`` (control.py:1887-1896) at
             state ``v_i`` and time ``t``; a plain CSR matrix means a linear, time-independent
             operator.  ``desired_state(t)`` -> (M @ v_hat(t), v_hat(t)), the two returns of
             the reference's callable (control.py:1929-1931); ``force_f(t)`` -> M @ f(t).
             ``bc_values``: None (homogeneous Dirichlet data) or a callable ``t -> values at bc_dofs``
-            (the reference's time-dependent ``bcs_v(space, t)``, control/control.py:1504-1530)."""
+            (the reference's time-dependent ``bcs_v(space, t)``, control/control.py:1504-1530).
+            ``block_size``: block size of the state space (``M.petscmat.getBlockSize()``; dofs interleaved as
+            ``bs * node + comp``), passed to every device system this instance creates -- the heat-type system and
+            the velocity system of the Stokes / Navier-Stokes solves -- whose preconditioners then run their time
+            sweeps on the scalar block when the matrices are ``I_bs (x) S``.  One GPU only."""
             if force_f is not None and force_function is not None:
                 raise TypeError("give either force_f or force_function")
+            if int(block_size) not in (1, 2, 3):
+                raise ValueError(f"block_size must be 1, 2 or 3, not {block_size}")
+            if int(block_size) > 1 and world > 1:
+                raise ValueError("block_size > 1 runs on one GPU: block-scalar sweeps are not available with world > 1")
+            self._block_size = int(block_size)
             self._M = M.tocsr()
             self._forward_matrix = forward_matrix
             self._desired_state = desired_state
@@ -177,12 +187,16 @@ class Control:
             if self._system is None:
                 self._system = MultiBlockSystem(self._M, K, n_t=self._n_t, beta=self._beta, CN=self._CN,
                                                 time_interval=self._time_interval, bc_dofs=self._bc_dofs,
-                                                **self._dev)
+                                                **self._block_kw("block_size"), **self._dev)
                 if self._dev["world"] > 1:
                     self._system.init_comm()
             else:
                 self._system.set_K(K)
             return self._system
+
+        def _block_kw(self, name):
+            # the block size only travels when it is not the default, so stand-in systems need not know it
+            return {name: self._block_size} if self._block_size != 1 else {}
 
         def close(self):
             if self._system is not None:
@@ -324,7 +338,8 @@ class Control:
             if getattr(self, "_stokes", None) is None:
                 self._stokes = StokesSystem(self._M, K, space_p["B"], space_p["M_p"], space_p["K_p"], n_t=n_t,
                                             beta=self._beta, CN=CN, time_interval=self._time_interval,
-                                            bc_dofs_v=self._bc_dofs, device=self._dev["device"], D_p=D_p)
+                                            bc_dofs_v=self._bc_dofs, device=self._dev["device"], D_p=D_p,
+                                            **self._block_kw("velocity_block_size"))
             elif not self._is_linear():
                 self._stokes.set_forward(K, D_p)
             system = self._stokes
@@ -487,7 +502,8 @@ class Control:
             if getattr(self, "_stokes", None) is None:
                 self._stokes = StokesSystem(self._M, K, space_p["B"], space_p["M_p"], space_p["K_p"], n_t=n_t,
                                             beta=self._beta, CN=CN, time_interval=self._time_interval,
-                                            bc_dofs_v=bd, device=self._dev["device"], D_p=D_p)
+                                            bc_dofs_v=bd, device=self._dev["device"], D_p=D_p,
+                                            **self._block_kw("velocity_block_size"))
             elif not linear:
                 self._stokes.set_forward(K, D_p)
             system = self._stokes

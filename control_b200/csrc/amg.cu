@@ -34,16 +34,17 @@ static int dev_alloc(ctl_handle_s *h, double **p, size_t n)
     return CTL_OK;
 }
 
-// work vectors of one level (after the matrices and dinv are in place)
+// work vectors of one level (after the matrices and dinv are in place): n rows of L.A.nc components each
 int amg_level_vectors(ctl_handle_s *h, AmgLevelDev &L, int level)
 {
-    CTL_TRY(dev_alloc(h, &L.r, L.n));
-    CTL_TRY(dev_alloc(h, &L.t0, L.n));
-    CTL_TRY(dev_alloc(h, &L.t1, L.n));
-    CTL_TRY(dev_alloc(h, &L.t2, L.n));
+    const size_t nv = (size_t)L.n * L.A.nc;
+    CTL_TRY(dev_alloc(h, &L.r, nv));
+    CTL_TRY(dev_alloc(h, &L.t0, nv));
+    CTL_TRY(dev_alloc(h, &L.t1, nv));
+    CTL_TRY(dev_alloc(h, &L.t2, nv));
     if (level > 0) {
-        CTL_TRY(dev_alloc(h, &L.x, L.n));
-        CTL_TRY(dev_alloc(h, &L.b, L.n));
+        CTL_TRY(dev_alloc(h, &L.x, nv));
+        CTL_TRY(dev_alloc(h, &L.b, nv));
     }
     return CTL_OK;
 }
@@ -51,20 +52,22 @@ int amg_level_vectors(ctl_handle_s *h, AmgLevelDev &L, int level)
 int64_t amg_cycle_bytes(const AmgHierarchyDev &H)
 {
     // per cycle and level: 2 nu smoother products (2 nu - 1 on the zero-guess side) + residual, restriction,
-    // prolongation; each product streams its matrix once plus the vectors it touches
+    // prolongation; each product streams its matrix once plus the vectors it touches.  A block hierarchy (nc
+    // components) streams each matrix once and every vector but the Jacobi diagonal nc times.
     const AmgParams &p = H.params;
     const int nl = (int)H.dev.size();
+    const int64_t nc = H.nc;
     int64_t bytes = 0;
     for (int l = 0; l < nl; ++l) {
         const AmgLevelDev &L = H.dev[l];
         if (l + 1 < nl) {
             const int nu_l = (l == 0 && p.nu_fine > 0) ? p.nu_fine : p.nu;
-            bytes += (L.A.bytes_per_pass + 40ll * L.n) * (2 * nu_l);
-            bytes += L.P.bytes_per_pass + L.R.bytes_per_pass + 32ll * L.n;
+            bytes += (L.A.bytes_per_pass + (8ll + 32ll * nc) * L.n) * (2 * nu_l);
+            bytes += L.P.bytes_per_pass + L.R.bytes_per_pass + 32ll * nc * L.n;
         } else if (L.Ainv) {
             bytes += 8ll * L.n * L.n;
         } else {
-            bytes += (L.A.bytes_per_pass + 40ll * L.n) * p.nu;
+            bytes += (L.A.bytes_per_pass + (8ll + 32ll * nc) * L.n) * p.nu;
         }
     }
     return bytes;
@@ -82,6 +85,7 @@ int amg_build(ctl_handle_s *h, const HostCSR &A0, const AmgParams &p,
     }
     const int nl = (int)H.host.size();
     H.dev.assign(nl, AmgLevelDev());
+    CTL_CHECK(H.nc == 1 || h->cfg.world == 1, CTL_ERR_ARG, "amg_build: block hierarchies run on one GPU only");
     if (h->cfg.world > 1) {
         CTL_CHECK(nl > 1, CTL_ERR_ARG, "amg_build: the problem is too small for a multi-rank hierarchy (single level)");
         CTL_TRY(amg_build_distributed(h, p, fine_pattern, H));
@@ -93,11 +97,13 @@ int amg_build(ctl_handle_s *h, const HostCSR &A0, const AmgParams &p,
             Ld.rho = Lh.rho;
             if (l == 0 && fine_pattern) CTL_TRY(sell_set_values(h, fine_pattern, Lh.A.values.data(), Ld.A));
             else CTL_TRY(sell_from_csr(h, Lh.A, Ld.A));
-            CTL_TRY(ctl_upload(h, &Ld.dinv, Lh.dinv.data(), (size_t)Ld.n));
+            Ld.A.nc = H.nc;
+            CTL_TRY(ctl_upload(h, &Ld.dinv, Lh.dinv.data(), (size_t)Ld.n));      // one entry per row: shared by the components
             CTL_TRY(amg_level_vectors(h, Ld, l));
             if (l + 1 < nl) {
                 CTL_TRY(sell_from_csr(h, Lh.P, Ld.P));
                 CTL_TRY(sell_from_csr(h, Lh.R, Ld.R));
+                Ld.P.nc = Ld.R.nc = H.nc;
             } else if (!Lh.Ainv.empty()) {
                 CTL_TRY(dense_inverse_upload(h, Lh.Ainv, Ld.n, &Ld.Ainv, &Ld.Ainv_ld));
             } else if (Lh.coarse_inverse) {
@@ -107,9 +113,10 @@ int amg_build(ctl_handle_s *h, const HostCSR &A0, const AmgParams &p,
     }
     H.bytes_per_cycle = amg_cycle_bytes(H);
     if (p.acc_lo > 0.0) {
-        CTL_TRY(dev_alloc(h, &H.acc_r, H.dev[0].n));
-        CTL_TRY(dev_alloc(h, &H.acc_z, H.dev[0].n));
-        CTL_TRY(dev_alloc(h, &H.acc_p, H.dev[0].n));
+        const size_t nv = (size_t)H.dev[0].n * H.nc;
+        CTL_TRY(dev_alloc(h, &H.acc_r, nv));
+        CTL_TRY(dev_alloc(h, &H.acc_z, nv));
+        CTL_TRY(dev_alloc(h, &H.acc_p, nv));
     }
     return CTL_OK;
 }
@@ -164,12 +171,12 @@ static int smooth(ctl_handle_s *h, const AmgParams &p, AmgLevelDev &L, int l, co
     };
     if (zero && nu == 1) {
         const HaloPush push = halo_push(L.px);
-        return vec_dinv_scale(h, L.dinv, b.x, x_out, scale, L.n, push);
+        return vec_dinv_scale(h, L.dinv, b.x, x_out, scale, L.n, push, L.A.nc);
     }
     if (!zero && nu == 1 && x_in == x_out) {      // the one step would overwrite the vector it gathers
         CTL_CHECK(!L.px, CTL_ERR_STATE, "smooth: degree 1 in place is not available on several GPUs");
         CTL_TRY(sell_cheb_step(h, L.A, L.dinv, b.x, nullptr, GVec(x_in), L.t0, 0.0, 1.0, scale));
-        return vec_copy_n(h, x_out, L.t0, L.n);
+        return vec_copy_n(h, x_out, L.t0, L.n * L.A.nc);
     }
     int k0;      // first step that still has to be taken
     if (zero) {
@@ -207,7 +214,7 @@ static int vcycle(ctl_handle_s *h, AmgHierarchyDev &H, int l, const GVec &b, dou
     AmgLevelDev &L = H.dev[l];
     const int last = (int)H.dev.size() - 1;
     if (l == last) {
-        if (L.Ainv) return dense_gemv(h, L.Ainv, b.x, x, L.n, L.Ainv_ld);
+        if (L.Ainv) return dense_gemv(h, L.Ainv, b.x, x, L.n, L.Ainv_ld, L.A.nc);
         return smooth(h, H.params, L, l, b, x_is_zero ? nullptr : x, x);
     }
     AmgLevelDev &C = H.dev[l + 1];
@@ -266,7 +273,7 @@ int amg_solve(ctl_handle_s *h, AmgHierarchyDev &H, const double *b, double *x, b
     }
     // Chebyshev semi-iteration on (V-cycle * A) over [acc_lo, acc_hi]: oracle/amg.py::solve (one GPU only)
     CTL_CHECK(!L0.px, CTL_ERR_STATE, "amg_solve: accelerated cycles are not available on several GPUs");
-    const int n = L0.n;
+    const int n = L0.n * H.nc;      // the vector work runs over every component
     double scale;
     std::vector<double> om;
     cheb_coefficients(p.acc_lo, p.acc_hi, p.cycles, &scale, om);

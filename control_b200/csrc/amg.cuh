@@ -22,6 +22,8 @@ struct AmgLevelDev {
 
 struct AmgHierarchyDev {
     AmgParams params;
+    int nc = 1;                          // components: the levels are the scalar S of I_nc (x) S and every level vector
+                                         // holds nc interleaved components per row (set before amg_build; one GPU)
     std::vector<AmgLevelHost> host;      // kept for introspection (ctl_amg_get_csr)
     std::vector<AmgLevelDev> dev;
     std::vector<std::shared_ptr<struct HaloSpace>> spaces;   // multi-GPU: exchange geometry of the levels >= 1 (halo.cu)

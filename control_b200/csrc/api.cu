@@ -188,6 +188,18 @@ int ctl_set_values(ctl_handle h, int which, int level, const double *values)
     return CTL_OK;
 }
 
+int ctl_set_block_size(ctl_handle h, int32_t bs)
+{
+    CTL_CHECK(h, CTL_ERR_ARG, "ctl_set_block_size: null handle");
+    CTL_CHECK(bs >= 1 && bs <= 3, CTL_ERR_ARG, "ctl_set_block_size: the block size must be 1, 2 or 3");
+    CTL_CHECK(h->n % bs == 0, CTL_ERR_ARG, "ctl_set_block_size: n is not a multiple of the block size");
+    CTL_CHECK(bs == 1 || h->cfg.world == 1, CTL_ERR_ARG, "ctl_set_block_size: block-scalar sweeps run on one GPU (world 1)");
+    CTL_CUDA(cudaSetDevice(h->cfg.device));
+    h->block_size = bs;
+    ctl_pc_free(h);                     // set up again with the new block size
+    return CTL_OK;
+}
+
 int ctl_set_bc(ctl_handle h, const int32_t *dofs, int32_t count)
 {
     CTL_CHECK(h && (dofs || count == 0) && count >= 0, CTL_ERR_ARG, "ctl_set_bc: bad argument");

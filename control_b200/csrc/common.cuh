@@ -61,6 +61,7 @@ struct ctl_handle_s {
     int64_t launches = 0;
     bool assembled = false;
     bool use_pdl = true;       // programmatic dependent launch for the chains of small sweep kernels (CTL_NO_PDL=1 disables)
+    int block_size = 1;        // ctl_set_block_size: interleaved components of the space, dof = block_size node + comp
 
     // host copies of what the caller handed over (global numbering)
     std::vector<int> h_indptr, h_indices;

@@ -81,6 +81,74 @@ std::vector<double> local_values(ctl_handle_s *h, const std::vector<double> &glo
     return v;
 }
 
+// ---- block-scalar sweeps (ctl_set_block_size): sweep matrices of the form I_bs (x) S on interleaved dofs,
+// dof = bs node + comp, are set up and run as the scalar S on bs components
+// The scalar pattern: the entries of the component-0 rows that lie in component-0 columns, numbered by node; src[p] is
+// the global entry the scalar entry p is read from.
+struct ScalarPattern {
+    HostCSR A;                     // values unused
+    std::vector<int64_t> src;
+};
+
+void scalar_pattern(const ctl_handle_s *h, int bs, ScalarPattern &out)
+{
+    const std::vector<int> &ip = h->h_indptr, &ix = h->h_indices;
+    const int nn = h->n / bs;
+    out.A.n_rows = out.A.n_cols = nn;
+    out.A.indptr.assign(nn + 1, 0);
+    out.A.indices.clear();
+    out.src.clear();
+    for (int i = 0; i < nn; ++i) {
+        const int r = bs * i;
+        for (int k = ip[r]; k < ip[r + 1]; ++k)
+            if (ix[k] % bs == 0) {
+                out.A.indices.push_back(ix[k] / bs);
+                out.src.push_back(k);
+            }
+        out.A.indptr[i + 1] = (int)out.A.indices.size();
+    }
+}
+
+std::vector<double> scalar_values(const ScalarPattern &sp, const std::vector<double> &global_vals)
+{
+    std::vector<double> v(sp.src.size());
+    for (size_t p = 0; p < v.size(); ++p) v[p] = global_vals[sp.src[p]];
+    return v;
+}
+
+HostCSR scalar_csr(const ScalarPattern &sp, const std::vector<double> &global_vals)
+{
+    HostCSR A = sp.A;
+    A.values = scalar_values(sp, global_vals);
+    return A;
+}
+
+// Values on the global pattern have the structure I_bs (x) S when no entry couples two components and the bs component
+// blocks are equal entry for entry, bitwise; an absent entry and a stored zero both count as 0.  (A Dirichlet list that
+// constrains only some components of a node breaks it: the constrained rows are identity rows.)
+bool has_block_structure(const ctl_handle_s *h, int bs, const std::vector<double> &vals)
+{
+    const std::vector<int> &ip = h->h_indptr, &ix = h->h_indices;
+    std::vector<std::pair<int, uint64_t>> first, other;
+    for (int i = 0; i < h->n / bs; ++i) {
+        for (int comp = 0; comp < bs; ++comp) {
+            const int r = bs * i + comp;
+            std::vector<std::pair<int, uint64_t>> &lst = comp == 0 ? first : other;
+            lst.clear();
+            for (int k = ip[r]; k < ip[r + 1]; ++k) {
+                const double v = vals[k];
+                if (v == 0.0) continue;
+                if (ix[k] % bs != comp) return false;
+                uint64_t bits;
+                std::memcpy(&bits, &v, sizeof(bits));
+                lst.emplace_back(ix[k] / bs, bits);
+            }
+            if (comp > 0 && other != first) return false;
+        }
+    }
+    return true;
+}
+
 }  // namespace
 
 void ctl_pc_free(ctl_handle_s *h)
@@ -436,8 +504,6 @@ int ctl_pc_setup(ctl_handle h, const ctl_pc_options *opts)
     }
 
     lap("transposition map, mass dinv");
-    CTL_TRY(sell_build_pattern(h, h->loc, st.fine));
-    lap("fine SELL pattern");
     // multi-GPU: exchange geometry of everything that gathers through the mesh pattern, and the two level-0
     // exchange streams (iterates, right-hand sides) every hierarchy shares
     if (h->cfg.world > 1) {
@@ -460,15 +526,6 @@ int ctl_pc_setup(ctl_handle h, const ctl_pc_options *opts)
     auto mesh_matrix = [&](SellMat &m) {
         if (h->cfg.world > 1) m.n_own = h->n_loc;
     };
-    std::vector<double> vals;
-    combine_global(h, 0, false, 0.0, 1.0, false, vals);
-    {
-        const std::vector<double> lv = local_values(h, vals);
-        CTL_TRY(sell_set_values(h, st.fine, lv.data(), st.Msell));
-        mesh_matrix(st.Msell);
-    }
-
-    lap("mass matrix values");
     // distinct diagonal blocks -> AMG hierarchies; distinct off-diagonal blocks -> SELL
     const bool per_level = h->h_K.size() > 1;
     const bool sym = h->k_symmetric;
@@ -529,6 +586,59 @@ int ctl_pc_setup(ctl_handle h, const ctl_pc_options *opts)
         pending.push_back({0, false, 0.0, 1.0});
         st.h_mass = (int)pending.size() - 1;
     }
+    // block-scalar sweeps: only when EVERY sweep matrix (M, each distinct diagonal and off-diagonal block, the mass
+    // hierarchy) has the structure I_bs (x) S; otherwise the whole handle takes the vector path.  Checked on the values
+    // the set-up forms anyway, in parallel, before anything is built.
+    st.bs = 1;
+    if (h->block_size > 1) {
+        const int bsz = h->block_size, nh = (int)pending.size(), n_off = (int)pending_off.size();
+        const int n_tasks = 1 + nh + n_off;
+        std::atomic<int> next{0};
+        std::atomic<bool> ok{true};
+        auto check = [&]() {
+            std::vector<double> v;
+            for (int i = next.fetch_add(1); i < n_tasks && ok.load(); i = next.fetch_add(1)) {
+                if (i == 0) {
+                    combine_global(h, 0, false, 0.0, 1.0, false, v);
+                } else if (i <= nh) {
+                    const PendingHier &q = pending[i - 1];
+                    combine_global(h, q.level, q.transposed, q.w, q.m_coef, true, v);
+                } else {
+                    const PendingOff &o = pending_off[i - 1 - nh];
+                    combine_global(h, o.level, o.transposed, o.w, o.m_coef, false, v);
+                }
+                if (!has_block_structure(h, bsz, v)) ok = false;
+            }
+        };
+        int n_threads = std::max(1, (int)std::thread::hardware_concurrency());
+        if (const char *e = getenv("CTL_SETUP_THREADS")) n_threads = std::max(1, atoi(e));
+        n_threads = std::min(std::min(n_threads, n_tasks), 32);
+        std::vector<std::thread> pool;
+        for (int t = 1; t < n_threads; ++t) pool.emplace_back(check);
+        check();
+        for (auto &t : pool) t.join();
+        if (ok) st.bs = bsz;
+        lap("block structure check");
+    }
+    ScalarPattern spat;
+    if (st.bs > 1) {
+        // same depth as the vector hierarchy: the levels of S are half (a third) as large
+        scalar_pattern(h, st.bs, spat);
+        st.amg.coarse_max = (opts->amg_coarse_max + st.bs - 1) / st.bs;
+        CTL_TRY(sell_build_pattern(h, spat.A, st.fine));
+    } else {
+        CTL_TRY(sell_build_pattern(h, h->loc, st.fine));
+    }
+    lap("fine SELL pattern");
+    {
+        std::vector<double> vals;
+        combine_global(h, 0, false, 0.0, 1.0, false, vals);
+        const std::vector<double> lv = st.bs > 1 ? scalar_values(spat, vals) : local_values(h, vals);
+        CTL_TRY(sell_set_values(h, st.fine, lv.data(), st.Msell));
+        st.Msell.nc = st.bs;
+        mesh_matrix(st.Msell);
+    }
+    lap("mass matrix values");
     // host setup of all hierarchies in parallel, then the device uploads one after the other
     {
         const int nh = (int)pending.size(), n_off = (int)pending_off.size();
@@ -548,14 +658,15 @@ int ctl_pc_setup(ctl_handle h, const ctl_pc_options *opts)
                     const PendingOff &o = pending_off[i - nh];
                     std::vector<double> v;
                     combine_global(h, o.level, o.transposed, o.w, o.m_coef, false, v);
-                    off_values[i - nh] = local_values(h, v);
+                    off_values[i - nh] = st.bs > 1 ? scalar_values(spat, v) : local_values(h, v);
                     continue;
                 }
                 try {
                     std::vector<double> v;
                     combine_global(h, pending[i].level, pending[i].transposed, pending[i].w, pending[i].m_coef, true, v);
                     // the workers share the host: each hierarchy gets its share of the threads
-                    amg_setup_host(global_csr(h, v), st.amg, st.hier[i].host, std::max(1, hw_threads / n_threads));
+                    amg_setup_host(st.bs > 1 ? scalar_csr(spat, v) : global_csr(h, v), st.amg, st.hier[i].host,
+                                   std::max(1, hw_threads / n_threads));
                 } catch (const std::exception &e) {
                     errors[i] = e.what();
                 }
@@ -571,12 +682,14 @@ int ctl_pc_setup(ctl_handle h, const ctl_pc_options *opts)
         lap("host AMG set-up (all)");
         for (int i = 0; i < nh; ++i) {
             CTL_CHECK(errors[i].empty(), CTL_ERR_STATE, errors[i]);
+            st.hier[i].nc = st.bs;
             CTL_TRY(amg_build(h, st.hier[i].host[0].A, st.amg, st.fine, st.hier[i]));
         }
         lap("formats, uploads, inverse");
         st.off.assign(n_off, SellMat());
         for (int i = 0; i < n_off; ++i) {
             CTL_TRY(sell_set_values(h, st.fine, off_values[i].data(), st.off[i]));
+            st.off[i].nc = st.bs;
             mesh_matrix(st.off[i]);
             off_values[i] = std::vector<double>();
         }
@@ -652,9 +765,13 @@ int ctl_amg_get_aggregates(ctl_handle h, int32_t hi, int32_t lvl, int32_t *agg)
     return CTL_OK;
 }
 
+int32_t ctl_pc_block_size(ctl_handle h) { return (h && h->pc && h->pc->ready) ? h->pc->bs : -1; }
+
 int ctl_amg_solve(ctl_handle h, int32_t hi, const double *b, double *x)
 {
     CTL_CHECK(h && h->pc && hi >= 0 && hi < (int)h->pc->hier.size() && b && x, CTL_ERR_ARG, "ctl_amg_solve: bad argument");
+    CTL_CHECK(h->pc->hier[hi].nc != 2 || (((uintptr_t)b | (uintptr_t)x) & 15) == 0, CTL_ERR_ARG,
+              "ctl_amg_solve: a block-size-2 hierarchy needs 16-byte aligned vectors");
     CTL_CUDA(cudaSetDevice(h->cfg.device));
     CTL_TRY(halo_epoch_begin(h));
     CTL_TRY(amg_solve(h, h->pc->hier[hi], b, x, false));
@@ -668,8 +785,8 @@ int ctl_time_amg(ctl_handle h, int32_t hi, int reps, int flush_l2, double *out)
     CTL_CUDA(cudaSetDevice(h->cfg.device));
     AmgHierarchyDev &H = h->pc->hier[hi];
     AmgLevelDev &L0 = H.dev[0];
-    const int n = L0.n;
-    const size_t nv = (size_t)n + L0.n_ghost;      // ghost entries behind the owned ones (multi-GPU; left at zero)
+    const int n = L0.n, nc = H.nc;
+    const size_t nv = (size_t)n * nc + L0.n_ghost;      // ghost entries behind the owned ones (multi-GPU; left at zero)
     // Cold-cache timing of the two fine-level kernels: INPUTS LARGER THAN L2.  Each launch works on its own set of
     // vectors (dinv, b, p_prev, p_cur, out), and the sets rotate through more than twice the 126 MB of L2, so no
     // launch finds its operands there.  (Round 1 overwrote a 256 MB buffer between launches instead: that leaves
@@ -685,12 +802,12 @@ int ctl_time_amg(ctl_handle h, int32_t hi, int reps, int flush_l2, double *out)
     if (flush_l2) CTL_CUDA(cudaMalloc((void **)&flush, flush_bytes));
     auto vec = [&](int set, int k) { return sets + ((size_t)set * kSetVecs + k) * nv; };      // k: 0 dinv 1 b 2 x 3 p 4 out
     {
-        std::vector<double> hb(n);
-        for (int i = 0; i < n; ++i) hb[i] = std::sin(0.37 * i) + 0.1;
-        for (int s = 0; s < n_sets; ++s) {
-            CTL_CUDA(cudaMemcpy(vec(s, 0), L0.dinv, nv * sizeof(double), cudaMemcpyDeviceToDevice));
-            CTL_CUDA(cudaMemcpy(vec(s, 1), hb.data(), (size_t)n * sizeof(double), cudaMemcpyHostToDevice));
-            CTL_CUDA(cudaMemcpy(vec(s, 3), hb.data(), (size_t)n * sizeof(double), cudaMemcpyHostToDevice));
+        std::vector<double> hb((size_t)n * nc);
+        for (size_t i = 0; i < hb.size(); ++i) hb[i] = std::sin(0.37 * i) + 0.1;
+        for (int s = 0; s < n_sets; ++s) {      // (the Jacobi diagonal has one entry per row, whatever nc)
+            CTL_CUDA(cudaMemcpy(vec(s, 0), L0.dinv, ((size_t)n + L0.n_ghost) * sizeof(double), cudaMemcpyDeviceToDevice));
+            CTL_CUDA(cudaMemcpy(vec(s, 1), hb.data(), hb.size() * sizeof(double), cudaMemcpyHostToDevice));
+            CTL_CUDA(cudaMemcpy(vec(s, 3), hb.data(), hb.size() * sizeof(double), cudaMemcpyHostToDevice));
         }
     }
     double *b = vec(0, 1), *x = vec(0, 2);
@@ -711,7 +828,7 @@ int ctl_time_amg(ctl_handle h, int32_t hi, int reps, int flush_l2, double *out)
             if (!with_kernel) continue;
             const int64_t l0 = h->launches;
             const int s = r % n_sets;
-            const GVec gp = L0.px ? GVec(vec(s, 3), vec(s, 3) + n) : GVec(vec(s, 3));
+            const GVec gp = L0.px ? GVec(vec(s, 3), vec(s, 3) + (size_t)n * nc) : GVec(vec(s, 3));
             if (which == 0) r2 = sell_cheb_step(h, L0.A, vec(s, 0), vec(s, 1), vec(s, 2), gp, vec(s, 4), 0.3, 0.7, 0.1);
             else if (which == 1) r2 = sell_spmv(h, L0.A, gp, vec(s, 4), vec(s, 1), SELL_RESIDUAL);
             else r2 = amg_solve(h, H, b, x);
@@ -731,9 +848,9 @@ int ctl_time_amg(ctl_handle h, int32_t hi, int reps, int flush_l2, double *out)
     }
     const double mat = (double)L0.A.bytes_per_pass;      // matrix stream of the format in use (sell_format.h)
     out[0] = acc[0] / reps;
-    out[1] = mat + 40.0 * n;                 // matrix + dinv, b, p_prev, p_cur, out
+    out[1] = mat + (8.0 + 32.0 * nc) * n;    // matrix + dinv, b, p_prev, p_cur, out (the vectors nc times, dinv once)
     out[2] = acc[1] / reps;
-    out[3] = mat + 24.0 * n;                 // matrix + b, x, r
+    out[3] = mat + 24.0 * nc * n;            // matrix + b, x, r
     out[4] = acc[2] / reps;
     out[5] = (double)H.bytes_per_cycle * H.params.cycles;
     out[6] = (double)launches_solve;

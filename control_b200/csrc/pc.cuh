@@ -21,10 +21,12 @@ struct PcState {
     ctl_pc_options opts{};
     bool ready = false;
     AmgParams amg;
+    int bs = 1;                             // block size the sweeps run with (ctl_set_block_size; 1 when the matrices
+                                            // lack the structure I_bs (x) S): S on bs interleaved components
 
     double *d_mass_dinv = nullptr;          // 1 / diag(assemble(M, bcs))
 
-    std::shared_ptr<SellPattern> fine;      // SELL pattern of the mesh matrix (local rows)
+    std::shared_ptr<SellPattern> fine;      // SELL pattern of the mesh matrix (local rows; of S when bs > 1)
     SellMat Msell;                          // M with constrained rows and columns zeroed
     std::vector<SellMat> off;               // distinct sub/super-diagonal blocks of L_hat
     std::vector<AmgHierarchyDev> hier;      // distinct diagonal blocks of L_hat (+ mass matrix)

@@ -282,6 +282,92 @@ __device__ __forceinline__ double dvec_get(const DVec &v, int c, unsigned seq_hi
     return __ldcg(v.ghost + (c - v.n_own));
 }
 
+// ---- several components per row (block-scalar sweeps, one GPU: no ghosts, no push).  The matrix is the scalar S
+// of I_NC (x) S; a row of S produces NC results and every gather loads the NC interleaved values of a node
+// (dof = NC node + comp), one 16-byte load for NC = 2.  NC = 1 is the plain scalar path (vec_t<1> = double).
+template <int NC>
+struct VN {
+    double c[NC];
+};
+template <int NC>
+using vec_t = typename std::conditional<NC == 1, double, VN<NC>>::type;
+
+template <int NC>
+__device__ __forceinline__ VN<NC> operator+(VN<NC> a, const VN<NC> &b)
+{
+#pragma unroll
+    for (int k = 0; k < NC; ++k) a.c[k] = a.c[k] + b.c[k];
+    return a;
+}
+template <int NC>
+__device__ __forceinline__ VN<NC> operator-(VN<NC> a, const VN<NC> &b)
+{
+#pragma unroll
+    for (int k = 0; k < NC; ++k) a.c[k] = a.c[k] - b.c[k];
+    return a;
+}
+template <int NC>
+__device__ __forceinline__ VN<NC> operator*(double s, VN<NC> a)
+{
+#pragma unroll
+    for (int k = 0; k < NC; ++k) a.c[k] = s * a.c[k];
+    return a;
+}
+__device__ __forceinline__ double vfma(double a, double x, double acc) { return fma(a, x, acc); }
+template <int NC>
+__device__ __forceinline__ VN<NC> vfma(double a, const VN<NC> &x, VN<NC> acc)
+{
+#pragma unroll
+    for (int k = 0; k < NC; ++k) acc.c[k] = fma(a, x.c[k], acc.c[k]);
+    return acc;
+}
+__device__ __forceinline__ double vshfl_add(double v, int o, int w) { return v + __shfl_xor_sync(0xffffffffu, v, o, w); }
+template <int NC>
+__device__ __forceinline__ VN<NC> vshfl_add(VN<NC> v, int o, int w)
+{
+#pragma unroll
+    for (int k = 0; k < NC; ++k) v.c[k] = v.c[k] + __shfl_xor_sync(0xffffffffu, v.c[k], o, w);
+    return v;
+}
+// the NC values of node c (a plain load: vectors are written by the chain).  16-byte aligned for NC = 2: the vectors
+// start 16-byte aligned and have an even number of entries on one GPU.
+template <int NC>
+__device__ __forceinline__ vec_t<NC> ld_node(const double *x, int c)
+{
+    if constexpr (NC == 1) {
+        return x[c];
+    } else if constexpr (NC == 2) {
+        const double2 v = *reinterpret_cast<const double2 *>(x + 2 * c);
+        VN<2> r;
+        r.c[0] = v.x;
+        r.c[1] = v.y;
+        return r;
+    } else {
+        VN<NC> r;
+#pragma unroll
+        for (int k = 0; k < NC; ++k) r.c[k] = x[NC * c + k];
+        return r;
+    }
+}
+__device__ __forceinline__ void st_node(double *out, int row, double v) { out[row] = v; }
+template <int NC>
+__device__ __forceinline__ void st_node(double *out, int row, const VN<NC> &v)
+{
+    if constexpr (NC == 2) {
+        *reinterpret_cast<double2 *>(out + 2 * row) = make_double2(v.c[0], v.c[1]);
+    } else {
+#pragma unroll
+        for (int k = 0; k < NC; ++k) out[NC * row + k] = v.c[k];
+    }
+}
+// a gathered vector of NC components (NC > 1: one GPU, so no ghost entries)
+template <int NC>
+__device__ __forceinline__ vec_t<NC> gat(const DVec &v, int c, unsigned seq_hi, const HaloCtx &ctx)
+{
+    if constexpr (NC == 1) return dvec_get(v, c, seq_hi, ctx);
+    else return ld_node<NC>(v.x, c);
+}
+
 // READ-ONLY LOADS.  Vectors that a kernel of the chain writes (iterates, right-hand sides, residuals) are read with
 // PLAIN loads in this file, never with __ldg / through a const __restrict__ parameter: ptxas orders a plain ld.global
 // against griddepcontrol.wait but moves a non-coherent one (LDG.CONSTANT) freely -- with the wait no longer the first
@@ -298,7 +384,7 @@ __device__ __forceinline__ double dvec_get(const DVec &v, int c, unsigned seq_hi
 // gathers x[row + delta_k] (coalesced); the other slices take the per-entry DICT16 path.
 // g: gather of a column that may be a ghost; g_own: gather of a column known to be owned (no ghost test)
 template <typename G, typename G0, typename PRE>
-__device__ __forceinline__ double sell_row_dot_stencil(const MatView &A, int row, G g, G0 g_own, PRE pre)
+__device__ __forceinline__ auto sell_row_dot_stencil(const MatView &A, int row, G g, G0 g_own, PRE pre)
 {
     const int s = row >> 5, lane = row & 31;
     const int4 s0 = pre_ld(A.sp4 + s);
@@ -310,21 +396,22 @@ __device__ __forceinline__ double sell_row_dot_stencil(const MatView &A, int row
     const bool spec = A.ps_w > 0 && first + A.ps_dmin >= 0 && first + 31 + A.ps_dmax < A.n_own;
     pdl_wait();
     pre();
-    double acc = 0.0;
+    using R = decltype(g(0));
+    R acc{};
     if (spec) {
-        double xv[8];
+        R xv[8];
 #pragma unroll
-        for (int j = 0; j < 8; ++j) xv[j] = (j < A.ps_w) ? g_own(row + A.ps_delta[j]) : 0.0;
+        for (int j = 0; j < 8; ++j) xv[j] = (j < A.ps_w) ? g_own(row + A.ps_delta[j]) : R{};
         if (s0.z == A.ps_off) {
 #pragma unroll
             for (int j = 0; j < 8; ++j)
-                if (j < A.ps_w) acc = fma(A.ps_v[j], xv[j], acc);
+                if (j < A.ps_w) acc = vfma(A.ps_v[j], xv[j], acc);
             if (A.ps_w > 8) {      // second half (a P1 tetrahedron stencil has 15 entries)
 #pragma unroll
-                for (int j = 0; j < 8; ++j) xv[j] = (8 + j < A.ps_w) ? g_own(row + A.ps_delta[8 + j]) : 0.0;
+                for (int j = 0; j < 8; ++j) xv[j] = (8 + j < A.ps_w) ? g_own(row + A.ps_delta[8 + j]) : R{};
 #pragma unroll
                 for (int j = 0; j < 8; ++j)
-                    if (8 + j < A.ps_w) acc = fma(A.ps_v[8 + j], xv[j], acc);
+                    if (8 + j < A.ps_w) acc = vfma(A.ps_v[8 + j], xv[j], acc);
             }
             return acc;
         }
@@ -333,12 +420,12 @@ __device__ __forceinline__ double sell_row_dot_stencil(const MatView &A, int row
 #pragma unroll
         for (int h0 = 0; h0 < SF_PS; h0 += 8) {
             if (h0 < A.ps_w) {
-                double xv[8];
+                R xv[8];
 #pragma unroll
-                for (int j = 0; j < 8; ++j) xv[j] = (h0 + j < A.ps_w) ? g(row + A.ps_delta[h0 + j]) : 0.0;
+                for (int j = 0; j < 8; ++j) xv[j] = (h0 + j < A.ps_w) ? g(row + A.ps_delta[h0 + j]) : R{};
 #pragma unroll
                 for (int j = 0; j < 8; ++j)
-                    if (h0 + j < A.ps_w) acc = fma(A.ps_v[h0 + j], xv[j], acc);
+                    if (h0 + j < A.ps_w) acc = vfma(A.ps_v[h0 + j], xv[j], acc);
             }
         }
         return acc;
@@ -352,12 +439,12 @@ __device__ __forceinline__ double sell_row_dot_stencil(const MatView &A, int row
 #pragma unroll
             for (int j = 0; j < SC; ++j)
                 if (k0 + j < s0.y) d[j] = __ldg(&st[k0 + j].delta);
-            double xv[SC];
+            R xv[SC];
 #pragma unroll
-            for (int j = 0; j < SC; ++j) xv[j] = (k0 + j < s0.y) ? g(row + d[j]) : 0.0;
+            for (int j = 0; j < SC; ++j) xv[j] = (k0 + j < s0.y) ? g(row + d[j]) : R{};
 #pragma unroll
             for (int j = 0; j < SC; ++j)
-                if (k0 + j < s0.y) acc = fma(__ldg(&st[k0 + j].v), xv[j], acc);
+                if (k0 + j < s0.y) acc = vfma(__ldg(&st[k0 + j].v), xv[j], acc);
         }
         return acc;
     }
@@ -367,7 +454,7 @@ __device__ __forceinline__ double sell_row_dot_stencil(const MatView &A, int row
 #pragma unroll 1
     for (int p = s0.x + lane; p < end; p += 32) {
         const DictEnt e = sf_dict(A.dict, __ldg(code + p));
-        acc = fma(e.v, g(row + e.delta), acc);
+        acc = vfma(e.v, g(row + e.delta), acc);
     }
     return acc;
 }
@@ -376,13 +463,14 @@ __device__ __forceinline__ double sell_row_dot_stencil(const MatView &A, int row
 // entries are fetched in chunks of SC with all stream loads issued before the dependent gathers
 // (memory-level parallelism instead of a serial load -> gather -> fma chain per entry).
 template <int FMT, bool STREAM, typename G, typename G0, typename PRE>
-__device__ __forceinline__ double sell_row_dot(const MatView &A, int row, G g, G0 g_own, PRE pre)
+__device__ __forceinline__ auto sell_row_dot(const MatView &A, int row, G g, G0 g_own, PRE pre)
 {
     if (FMT == FMT_STENCIL) return sell_row_dot_stencil(A, row, g, g_own, pre);
     const int s = row >> 5, lane = row & 31;
     const int2 s0 = pre_ld(A.sp + s);
     const int end = pre_ld(reinterpret_cast<const int *>(A.sp + s + 1));
-    double acc = 0.0;
+    using R = decltype(g(0));
+    R acc{};
     // chunk 0: its stream loads are issued before the wait for the predecessor grid
     auto chunk = [&](int p0, auto first) {
         constexpr bool PRE = decltype(first)::value;
@@ -408,11 +496,11 @@ __device__ __forceinline__ double sell_row_dot(const MatView &A, int row, G g, G
                 v[j] = 0.0;
             }
         }
-        double xv[SC];
+        R xv[SC];
 #pragma unroll
         for (int j = 0; j < SC; ++j) xv[j] = g(c[j]);
 #pragma unroll
-        for (int j = 0; j < SC; ++j) acc = fma(v[j], xv[j], acc);
+        for (int j = 0; j < SC; ++j) acc = vfma(v[j], xv[j], acc);
     };
     int p0 = s0.x + lane;
     chunk(p0, std::true_type());      // (a slice without entries loads nothing and only waits)
@@ -422,7 +510,7 @@ __device__ __forceinline__ double sell_row_dot(const MatView &A, int row, G g, G
 
 // format known only at run time (kernels that are not hot enough for one instantiation per format)
 template <typename G>
-__device__ __forceinline__ double sell_row_dot_rt(const MatView &A, int row, G g)
+__device__ __forceinline__ auto sell_row_dot_rt(const MatView &A, int row, G g)
 {
     auto none = [] {};
     switch (A.fmt) {
@@ -440,11 +528,12 @@ __device__ __forceinline__ double sell_row_dot_rt(const MatView &A, int row, G g
 // and of R A are long: a serial load -> gather chain per entry is what these latency-bound kernels cannot afford).
 constexpr int CU = 4;
 template <int T, int FMT, bool STREAM, typename G, typename PRE>
-__device__ __forceinline__ double csrv_row_dot_f(const MatView &A, int row, int sub, G g, PRE pre)
+__device__ __forceinline__ auto csrv_row_dot_f(const MatView &A, int row, int sub, G g, PRE pre)
 {
     const int beg = pre_ld(A.ptr + row), end = pre_ld(A.ptr + row + 1);
     const int base = (FMT == FMT_F64) ? 0 : pre_ld(A.rbase + row);
-    double acc = 0.0;
+    using R = decltype(g(0));
+    R acc{};
     auto chunk = [&](int p0, auto first) {
         constexpr bool PRE = decltype(first)::value;
         SfRaw raw[CU];
@@ -466,22 +555,22 @@ __device__ __forceinline__ double csrv_row_dot_f(const MatView &A, int row, int 
                 v[j] = 0.0;
             }
         }
-        double xv[CU];
+        R xv[CU];
 #pragma unroll
         for (int j = 0; j < CU; ++j) xv[j] = g(c[j]);
 #pragma unroll
-        for (int j = 0; j < CU; ++j) acc = fma(v[j], xv[j], acc);
+        for (int j = 0; j < CU; ++j) acc = vfma(v[j], xv[j], acc);
     };
     int p0 = beg + sub;
     chunk(p0, std::true_type());      // (a lane without entries of its own loads nothing and only waits)
     for (p0 += CU * T; p0 < end; p0 += CU * T) chunk(p0, std::false_type());
 #pragma unroll
-    for (int o = T / 2; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o, T);
+    for (int o = T / 2; o > 0; o >>= 1) acc = vshfl_add(acc, o, T);
     return acc;
 }
 
 template <int T, bool STREAM, typename G, typename PRE>
-__device__ __forceinline__ double csrv_row_dot(const MatView &A, int row, int sub, G g, PRE pre)
+__device__ __forceinline__ auto csrv_row_dot(const MatView &A, int row, int sub, G g, PRE pre)
 {
     if (A.fmt == FMT_F64) return csrv_row_dot_f<T, FMT_F64, STREAM>(A, row, sub, g, pre);
     if (A.fmt == FMT_D16) return csrv_row_dot_f<T, FMT_D16, STREAM>(A, row, sub, g, pre);
@@ -491,13 +580,17 @@ __device__ __forceinline__ double csrv_row_dot(const MatView &A, int row, int su
 // Row assignment shared by every kernel: the push CTAs (halo.cuh) come first and compute the listed boundary
 // rows, one chunk of <= 32 rows per warp, storing them locally and into the ghost slots of the ranks that gather
 // them; the regular CTAs compute ST / T consecutive rows each.  f(row) is evaluated by all T lanes of a row's
-// group and returns the value to store in out[row].
+// group and returns the value to store in out[row] (NC components: the NC values of out at row's node; such rows are
+// never pushed).
 template <int T, int BS = ST, typename F>
 __device__ __forceinline__ void run_rows(int n_rows, const HaloPush &push, unsigned seq_hi, double *out, F f)
 {
+    using R = decltype(f(0));
+    constexpr bool SCALAR = std::is_same<R, double>::value;
     constexpr int RPC = BS / T;
+    const int n_pc = SCALAR ? (push.n_chunks + BS / 32 - 1) / (BS / 32) : 0;
+    if constexpr (SCALAR) {
     const int lane = threadIdx.x & 31;
-    const int n_pc = (push.n_chunks + BS / 32 - 1) / (BS / 32);
     if ((int)blockIdx.x < n_pc) {
         const int ci = blockIdx.x * (BS / 32) + (threadIdx.x >> 5);
         if (ci >= push.n_chunks) {
@@ -526,15 +619,16 @@ __device__ __forceinline__ void run_rows(int n_rows, const HaloPush &push, unsig
         pdl_wait();
         return;
     }
+    }
     const int r0 = ((int)blockIdx.x - n_pc) * RPC;
     const int row = r0 + (int)threadIdx.x / T;
     if (T == 1) {
-        if (row < n_rows) out[row] = f(row);
+        if (row < n_rows) st_node(out, row, f(row));
         else pdl_wait();      // no thread leaves before the predecessor is complete: grids finish in launch order
     } else {
         const bool live = row < n_rows;
-        const double v = f(live ? row : n_rows - 1);
-        if (live && (threadIdx.x % T) == 0) out[row] = v;
+        const R v = f(live ? row : n_rows - 1);
+        if (live && (threadIdx.x % T) == 0) st_node(out, row, v);
     }
 }
 
@@ -544,6 +638,13 @@ __device__ __forceinline__ double apply_mode(int mode, double ax, double bi)
     if (mode == SELL_ASSIGN) return ax;
     if (mode == SELL_RESIDUAL) return bi - ax;
     return bi + ax;      // SELL_BPLUS
+}
+template <int NC>
+__device__ __forceinline__ VN<NC> apply_mode(int mode, const VN<NC> &ax, const VN<NC> &bi)
+{
+    if (mode == SELL_ASSIGN) return ax;
+    if (mode == SELL_RESIDUAL) return bi - ax;
+    return bi + ax;
 }
 
 // Start of every kernel of this file: let the successor be scheduled and read the epoch bits of the exchange's
@@ -560,37 +661,37 @@ __device__ __forceinline__ unsigned kernel_prologue(const HaloCtx &ctx)
 
 // ---------------------------------------------------------------- SELL kernels
 // GH: the gathered vector has ghost entries (several GPUs); without them the gather is a plain read-only load
-template <int FMT, bool STREAM, bool GH, int BS>
+template <int FMT, bool STREAM, bool GH, int BS, int NC>
 __global__ void __launch_bounds__(BS) sell_spmv_kernel(const MatView A, const DVec x, const HaloCtx ctx, const double *b,
                                                       double *y, int mode, double sign, const HaloPush push)
 {
     const unsigned hi = kernel_prologue(ctx);
     run_rows<1, BS>(A.n_rows, push, hi, y, [&](int row) {
-        double bi = 0.0;
-        const double ax = sign * sell_row_dot<FMT, STREAM>(
-                                     A, row, [&](int c) { return GH ? dvec_get(x, c, hi, ctx) : x.x[c]; },
-                                     [&](int c) { return x.x[c]; },
-                                     [&] { if (mode != SELL_ASSIGN) bi = b[row]; });
+        vec_t<NC> bi{};
+        const vec_t<NC> ax = sign * sell_row_dot<FMT, STREAM>(
+                                     A, row, [&](int c) { if constexpr (GH) return dvec_get(x, c, hi, ctx); else return ld_node<NC>(x.x, c); },
+                                     [&](int c) { return ld_node<NC>(x.x, c); },
+                                     [&] { if (mode != SELL_ASSIGN) bi = ld_node<NC>(b, row); });
         return apply_mode(mode, ax, bi);
     });
 }
 
 // one Chebyshev step; the loads of the row's own entries (b, p_cur, p_prev) travel with the gathers
 #define CHEB_ROW_UPDATE(DOT)                                                                              \
-    const double di = pre_ld(dinv + row);      /* constant: before the wait */                             \
-    double bi = 0.0, pc = 0.0, pp = 0.0;                                                                  \
+    const double di = pre_ld(dinv + row);      /* constant: before the wait; one per node */               \
+    vec_t<NC> bi{}, pc{}, pp{};                                                                           \
     auto pre = [&] {                                                                                      \
-        bi = b[row];                                                                                      \
-        pc = p_cur.x[row];                                                                                \
-        if (prev_scale == 0.0 && a != 0.0) pp = p_prev[row];                                              \
+        bi = ld_node<NC>(b, row);                                                                         \
+        pc = ld_node<NC>(p_cur.x, row);                                                                   \
+        if (prev_scale == 0.0 && a != 0.0) pp = ld_node<NC>(p_prev, row);                                 \
     };                                                                                                    \
-    const double ax = DOT;                                                                                \
-    double r = bq * pc + c * di * (bi - ax);                                                              \
-    if (prev_scale != 0.0) r = fma(a, prev_scale * di * bi, r);                                           \
-    else if (a != 0.0) r = fma(a, pp, r);                                                                 \
+    const vec_t<NC> ax = DOT;                                                                             \
+    vec_t<NC> r = bq * pc + c * di * (bi - ax);                                                           \
+    if (prev_scale != 0.0) r = vfma(a, prev_scale * di * bi, r);                                          \
+    else if (a != 0.0) r = vfma(a, pp, r);                                                                \
     return r
 
-template <int FMT, bool STREAM, bool GH, int BS>
+template <int FMT, bool STREAM, bool GH, int BS, int NC>
 __global__ void __launch_bounds__(BS) sell_cheb_kernel(const MatView A, const double *__restrict__ dinv,
                                                       const double *b, const double *p_prev, const DVec p_cur,
                                                       const HaloCtx ctx, double *out, double a, double bq, double c,
@@ -599,43 +700,48 @@ __global__ void __launch_bounds__(BS) sell_cheb_kernel(const MatView A, const do
     const unsigned hi = kernel_prologue(ctx);
     run_rows<1, BS>(A.n_rows, push, hi, out, [&](int row) {
         CHEB_ROW_UPDATE((sell_row_dot<FMT, STREAM>(
-            A, row, [&](int cc) { return GH ? dvec_get(p_cur, cc, hi, ctx) : p_cur.x[cc]; },
-            [&](int cc) { return p_cur.x[cc]; }, pre)));
+            A, row, [&](int cc) { if constexpr (GH) return dvec_get(p_cur, cc, hi, ctx); else return ld_node<NC>(p_cur.x, cc); },
+            [&](int cc) { return ld_node<NC>(p_cur.x, cc); }, pre)));
     });
 }
 
-template <int FMT, bool STREAM, bool GH, int BS>
+template <int FMT, bool STREAM, bool GH, int BS, int NC>
 __global__ void __launch_bounds__(BS) sell_first2_kernel(const MatView A, const DVec dinv, const DVec b, const HaloCtx ctx,
                                                         double *out, double s, double wgt, const HaloPush push)
 {
     const unsigned hi = kernel_prologue(ctx);
     run_rows<1, BS>(A.n_rows, push, hi, out, [&](int row) {
         const double di = pre_ld(dinv.x + row);
-        double bi = 0.0;
-        const double ax = sell_row_dot<FMT, STREAM>(
+        vec_t<NC> bi{};
+        const vec_t<NC> ax = sell_row_dot<FMT, STREAM>(
             A, row,
-            [&](int c) { return GH ? s * dvec_get(dinv, c, hi, ctx) * dvec_get(b, c, hi, ctx) : s * __ldg(dinv.x + c) * b.x[c]; },
-            [&](int c) { return s * __ldg(dinv.x + c) * b.x[c]; }, [&] { bi = b.x[row]; });
-        const double p1 = s * di * bi;
+            [&](int c) {
+                if constexpr (GH) return s * dvec_get(dinv, c, hi, ctx) * dvec_get(b, c, hi, ctx);
+                else return s * __ldg(dinv.x + c) * ld_node<NC>(b.x, c);
+            },
+            [&](int c) { return s * __ldg(dinv.x + c) * ld_node<NC>(b.x, c); }, [&] { bi = ld_node<NC>(b.x, row); });
+        const vec_t<NC> p1 = s * di * bi;
         return wgt * p1 + (wgt * s) * di * (bi - ax);
     });
 }
 
+template <int NC>
 __global__ void __launch_bounds__(ST) sell_spmv2_kernel(const MatView A1, const MatView A2, const DVec x1, const DVec x2,
                                                        const DVec x3, double *y, double alpha, double beta,
                                                        const HaloCtx ctx, const HaloPush push)
 {
     const unsigned hi = kernel_prologue(ctx);
     run_rows<1>(A1.n_rows, push, hi, y, [&](int row) {
-        double acc1;
-        if (x2.x) acc1 = sell_row_dot_rt(A1, row, [&](int c) { return dvec_get(x1, c, hi, ctx) + dvec_get(x2, c, hi, ctx); });
-        else acc1 = sell_row_dot_rt(A1, row, [&](int c) { return dvec_get(x1, c, hi, ctx); });
-        double acc2 = 0.0;
-        if (x3.x) acc2 = sell_row_dot_rt(A2, row, [&](int c) { return dvec_get(x3, c, hi, ctx); });
+        vec_t<NC> acc1;
+        if (x2.x) acc1 = sell_row_dot_rt(A1, row, [&](int c) { return gat<NC>(x1, c, hi, ctx) + gat<NC>(x2, c, hi, ctx); });
+        else acc1 = sell_row_dot_rt(A1, row, [&](int c) { return gat<NC>(x1, c, hi, ctx); });
+        vec_t<NC> acc2{};
+        if (x3.x) acc2 = sell_row_dot_rt(A2, row, [&](int c) { return gat<NC>(x3, c, hi, ctx); });
         return alpha * acc1 + beta * acc2;
     });
 }
 
+template <int NC>
 __global__ void __launch_bounds__(ST) dinv_scale_kernel(const double *__restrict__ dinv, const double *b,
                                                        double *out, double c, int n, const HaloCtx ctx,
                                                        const HaloPush push)
@@ -644,7 +750,7 @@ __global__ void __launch_bounds__(ST) dinv_scale_kernel(const double *__restrict
     run_rows<1>(n, push, hi, out, [&](int row) {
         const double di = pre_ld(dinv + row);
         pdl_wait();
-        return c * di * b[row];
+        return c * di * ld_node<NC>(b, row);
     });
 }
 
@@ -655,15 +761,17 @@ __global__ void __launch_bounds__(ST) dinv_scale_kernel(const double *__restrict
 // rows with 8-byte loads, four per thread and iteration.
 constexpr int GR = 4;
 constexpr int GU = 2;
+template <int NC>
 __global__ void __launch_bounds__(ST) dense_gemv_kernel(const double *__restrict__ A, const double *b,
                                                        double *y, int n, int lda)
 {
+    using R = vec_t<NC>;
     pdl_trigger();
-    __shared__ double part[GR][ST / 32];
+    __shared__ R part[GR][ST / 32];
     const int r0 = blockIdx.x * GR;
-    double acc[GR];
+    R acc[GR];
 #pragma unroll
-    for (int q = 0; q < GR; ++q) acc[q] = 0.0;
+    for (int q = 0; q < GR; ++q) acc[q] = R{};
     const int n2 = n >> 1;      // complete pairs; an odd last column is handled below (the padding column is zero)
     const bool b_aligned = (reinterpret_cast<uintptr_t>(b) & 15) == 0;
     const double2 *rowp[GR];
@@ -682,59 +790,67 @@ __global__ void __launch_bounds__(ST) dense_gemv_kernel(const double *__restrict
             pdl_wait();
             waited = true;
         }
-        double2 bv[GU];
+        R bx[GU], by[GU];      // b at the columns 2j and 2j + 1
 #pragma unroll
         for (int u = 0; u < GU; ++u) {
             const int j = j0 + u * ST;
-            if (j >= n2) bv[u] = make_double2(0.0, 0.0);
-            else if (b_aligned) bv[u] = reinterpret_cast<const double2 *>(b)[j];
-            else bv[u] = make_double2(b[2 * j], b[2 * j + 1]);
+            if (j >= n2) {
+                bx[u] = R{};
+                by[u] = R{};
+            } else if constexpr (NC == 1) {
+                const double2 t = b_aligned ? reinterpret_cast<const double2 *>(b)[j] : make_double2(b[2 * j], b[2 * j + 1]);
+                bx[u] = t.x;
+                by[u] = t.y;
+            } else {
+                bx[u] = ld_node<NC>(b, 2 * j);
+                by[u] = ld_node<NC>(b, 2 * j + 1);
+            }
         }
 #pragma unroll
         for (int u = 0; u < GU; ++u)
 #pragma unroll
-            for (int q = 0; q < GR; ++q) acc[q] = fma(av[u][q].y, bv[u].y, fma(av[u][q].x, bv[u].x, acc[q]));
+            for (int q = 0; q < GR; ++q) acc[q] = vfma(av[u][q].y, by[u], vfma(av[u][q].x, bx[u], acc[q]));
     }
     if (!waited) pdl_wait();
     if ((n & 1) && threadIdx.x == 0) {
-        const double bl = b[n - 1];
+        const R bl = ld_node<NC>(b, n - 1);
 #pragma unroll
-        for (int q = 0; q < GR; ++q) acc[q] = fma(__ldg(A + (size_t)min(r0 + q, n - 1) * lda + n - 1), bl, acc[q]);
+        for (int q = 0; q < GR; ++q) acc[q] = vfma(__ldg(A + (size_t)min(r0 + q, n - 1) * lda + n - 1), bl, acc[q]);
     }
 #pragma unroll
     for (int q = 0; q < GR; ++q) {
-        double s = acc[q];
+        R s = acc[q];
 #pragma unroll
-        for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+        for (int o = 16; o > 0; o >>= 1) s = vshfl_add(s, o, 32);
         if ((threadIdx.x & 31) == 0) part[q][threadIdx.x >> 5] = s;
     }
     __syncthreads();
     if (threadIdx.x < GR && r0 + threadIdx.x < n)
     {
-        double s = 0.0;
+        R s{};
 #pragma unroll
         for (int w = 0; w < ST / 32; w += 4)      // fixed order: pairs first
-            s += (part[threadIdx.x][w] + part[threadIdx.x][w + 1]) + (part[threadIdx.x][w + 2] + part[threadIdx.x][w + 3]);
-        y[r0 + threadIdx.x] = s;
+            s = s + ((part[threadIdx.x][w] + part[threadIdx.x][w + 1]) + (part[threadIdx.x][w + 2] + part[threadIdx.x][w + 3]));
+        st_node(y, r0 + threadIdx.x, s);
     }
 }
 
 // ---------------------------------------------------------------- CSR-vector kernels
-template <int T, bool STREAM>
+template <int T, bool STREAM, int NC>
 __global__ void __launch_bounds__(ST) csrv_spmv_kernel(const MatView A, const DVec x, const HaloCtx ctx, const double *b,
                                                       double *y, int mode, double sign, const HaloPush push)
 {
     const unsigned hi = kernel_prologue(ctx);
     const int sub = threadIdx.x % T;
     run_rows<T>(A.n_rows, push, hi, y, [&](int row) {
-        double bi = 0.0;
-        const double ax = sign * csrv_row_dot<T, STREAM>(A, row, sub, [&](int c) { return dvec_get(x, c, hi, ctx); },
-                                                         [&] { if (mode != SELL_ASSIGN) bi = b[row]; });
+        vec_t<NC> bi{};
+        const vec_t<NC> ax = sign * csrv_row_dot<T, STREAM>(A, row, sub, [&](int c) { return gat<NC>(x, c, hi, ctx); },
+                                                            [&] { if (mode != SELL_ASSIGN) bi = ld_node<NC>(b, row); });
         return apply_mode(mode, ax, bi);
     });
 }
 
-template <int T>
+template <int T, int NC>
 __global__ void __launch_bounds__(ST) csrv_cheb_kernel(const MatView A, const double *__restrict__ dinv,
                                                       const double *b, const double *p_prev, const DVec p_cur,
                                                       const HaloCtx ctx, double *out, double a, double bq, double c,
@@ -743,11 +859,11 @@ __global__ void __launch_bounds__(ST) csrv_cheb_kernel(const MatView A, const do
     const unsigned hi = kernel_prologue(ctx);
     const int sub = threadIdx.x % T;
     run_rows<T>(A.n_rows, push, hi, out, [&](int row) {
-        CHEB_ROW_UPDATE((csrv_row_dot<T, false>(A, row, sub, [&](int cc) { return dvec_get(p_cur, cc, hi, ctx); }, pre)));
+        CHEB_ROW_UPDATE((csrv_row_dot<T, false>(A, row, sub, [&](int cc) { return gat<NC>(p_cur, cc, hi, ctx); }, pre)));
     });
 }
 
-template <int T>
+template <int T, int NC>
 __global__ void __launch_bounds__(ST) csrv_first2_kernel(const MatView A, const DVec dinv, const DVec b, const HaloCtx ctx,
                                                         double *out, double s, double wgt, const HaloPush push)
 {
@@ -755,10 +871,10 @@ __global__ void __launch_bounds__(ST) csrv_first2_kernel(const MatView A, const 
     const int sub = threadIdx.x % T;
     run_rows<T>(A.n_rows, push, hi, out, [&](int row) {
         const double di = pre_ld(dinv.x + row);
-        double bi = 0.0;
-        const double ax = csrv_row_dot<T, false>(A, row, sub, [&](int c) { return s * dvec_get(dinv, c, hi, ctx) * dvec_get(b, c, hi, ctx); },
-                                                 [&] { bi = b.x[row]; });
-        const double p1 = s * di * bi;
+        vec_t<NC> bi{};
+        const vec_t<NC> ax = csrv_row_dot<T, false>(A, row, sub, [&](int c) { return s * dvec_get(dinv, c, hi, ctx) * gat<NC>(b, c, hi, ctx); },
+                                                    [&] { bi = ld_node<NC>(b.x, row); });
+        const vec_t<NC> p1 = s * di * bi;
         return wgt * p1 + (wgt * s) * di * (bi - ax);
     });
 }
@@ -775,6 +891,11 @@ DVec dvec(const GVec &g, const MatView &A)
 }
 
 bool has_ghosts(const GVec &g) { return g.ghost != nullptr || g.ll != nullptr; }
+
+// components run on one GPU only: no ghost entries, no pushed rows
+#define CHECK_NC(A, GHOSTS, what)                                                                           \
+    CTL_CHECK((A).nc == 1 || (!(GHOSTS) && push.n_chunks == 0 && !push.all_rows), CTL_ERR_STATE,            \
+              what ": matrices with several components run on one GPU only")
 
 // push CTAs first; a replicating exchange pushes every row, so the regular CTAs are not launched at all
 int grid_for(int n_rows, int T, const HaloPush &push, int bs = ST)
@@ -799,11 +920,19 @@ int big_block_rows()
     return v;
 }
 
+// components (nc__ > 1) come without ghosts
+#define SELL_LAUNCH_NC(KERNEL, FMT, STREAM, NC, ...)                                                        \
+    do {                                                                                                    \
+        if (big__) pdl_launch(h, grid__, 256, KERNEL<FMT, STREAM, false, 256, NC>, __VA_ARGS__);            \
+        else pdl_launch(h, grid__, ST, KERNEL<FMT, STREAM, false, ST, NC>, __VA_ARGS__);                    \
+    } while (0)
+
 #define SELL_LAUNCH_GH(KERNEL, FMT, STREAM, ...)                                                            \
     do {                                                                                                    \
-        if (gh__) pdl_launch(h, grid__, ST, KERNEL<FMT, STREAM, true, ST>, __VA_ARGS__);                    \
-        else if (big__) pdl_launch(h, grid__, 256, KERNEL<FMT, STREAM, false, 256>, __VA_ARGS__);           \
-        else pdl_launch(h, grid__, ST, KERNEL<FMT, STREAM, false, ST>, __VA_ARGS__);                        \
+        if (nc__ == 2) SELL_LAUNCH_NC(KERNEL, FMT, STREAM, 2, __VA_ARGS__);                                 \
+        else if (nc__ == 3) SELL_LAUNCH_NC(KERNEL, FMT, STREAM, 3, __VA_ARGS__);                            \
+        else if (gh__) pdl_launch(h, grid__, ST, KERNEL<FMT, STREAM, true, ST, 1>, __VA_ARGS__);            \
+        else SELL_LAUNCH_NC(KERNEL, FMT, STREAM, 1, __VA_ARGS__);                                           \
     } while (0)
 
 #define SELL_LAUNCH_ST(KERNEL, FMT, ...)                                                                    \
@@ -816,6 +945,7 @@ int big_block_rows()
 #define SELL_DISPATCH(KERNEL, A, GHOSTS, ...)                                                               \
     do {                                                                                                    \
         const bool st__ = (A).stream, gh__ = (GHOSTS);                                                      \
+        const int nc__ = (A).nc;                                                                            \
         const bool big__ = !gh__ && push.n_chunks == 0 && (A).pat->n_rows >= big_block_rows() &&            \
                            (A).pat->nnz <= 10ll * (A).pat->n_rows;                                          \
         const int grid__ = grid_for((A).pat->n_rows, 1, push, big__ ? 256 : ST);                            \
@@ -830,13 +960,20 @@ int big_block_rows()
         }                                                                                                   \
     } while (0)
 
+#define CSRV_LAUNCH_NC(KERNEL, A, NC, ...)                                                                  \
+    do {                                                                                                    \
+        if ((A).lanes == 4) pdl_launch(h, grid__, ST, KERNEL<4, NC>, __VA_ARGS__);                          \
+        else if ((A).lanes == 8) pdl_launch(h, grid__, ST, KERNEL<8, NC>, __VA_ARGS__);                     \
+        else pdl_launch(h, grid__, ST, KERNEL<16, NC>, __VA_ARGS__);                                        \
+    } while (0)
+
 #define CSRV_DISPATCH(KERNEL, A, ...)                                                                       \
     do {                                                                                                    \
         const int grid__ = grid_for((A).pat->n_rows, (A).lanes, push);                                      \
         if (grid__ == 0) return CTL_OK;                                                                     \
-        if ((A).lanes == 4) pdl_launch(h, grid__, ST, KERNEL<4>, __VA_ARGS__);                              \
-        else if ((A).lanes == 8) pdl_launch(h, grid__, ST, KERNEL<8>, __VA_ARGS__);                         \
-        else pdl_launch(h, grid__, ST, KERNEL<16>, __VA_ARGS__);                                            \
+        if ((A).nc == 2) CSRV_LAUNCH_NC(KERNEL, A, 2, __VA_ARGS__);                                         \
+        else if ((A).nc == 3) CSRV_LAUNCH_NC(KERNEL, A, 3, __VA_ARGS__);                                    \
+        else CSRV_LAUNCH_NC(KERNEL, A, 1, __VA_ARGS__);                                                     \
     } while (0)
 
 }  // namespace
@@ -854,21 +991,29 @@ int sell_spmv(ctl_handle_s *h, const SellMat &A, const GVec &x, double *y, const
     }
     CTL_CHECK(kmode == SELL_ASSIGN || b != nullptr, CTL_ERR_ARG, "sell_spmv: this mode needs b");
     CTL_CHECK(push.n_chunks == 0 || b != y, CTL_ERR_STATE, "sell_spmv: an in-place product cannot push its boundary rows");
+    CHECK_NC(A, has_ghosts(x), "sell_spmv");
     const MatView V = A.view();
     const DVec dx = dvec(x, V);
     const HaloCtx ctx = halo_ctx(h);
     if (A.lanes) {
         const int grid = grid_for(A.pat->n_rows, A.lanes, push);
         if (grid == 0) return CTL_OK;
+#define CSRV_SPMV_NC(T, NC)                                                                                          \
+    do {                                                                                                             \
+        if (A.stream) pdl_launch(h, grid, ST, csrv_spmv_kernel<T, true, NC>, V, dx, ctx, b, y, kmode, sign, push);   \
+        else pdl_launch(h, grid, ST, csrv_spmv_kernel<T, false, NC>, V, dx, ctx, b, y, kmode, sign, push);           \
+    } while (0)
 #define CSRV_SPMV(T)                                                                                                 \
     do {                                                                                                             \
-        if (A.stream) pdl_launch(h, grid, ST, csrv_spmv_kernel<T, true>, V, dx, ctx, b, y, kmode, sign, push);       \
-        else pdl_launch(h, grid, ST, csrv_spmv_kernel<T, false>, V, dx, ctx, b, y, kmode, sign, push);               \
+        if (A.nc == 2) CSRV_SPMV_NC(T, 2);                                                                           \
+        else if (A.nc == 3) CSRV_SPMV_NC(T, 3);                                                                      \
+        else CSRV_SPMV_NC(T, 1);                                                                                     \
     } while (0)
         if (A.lanes == 4) CSRV_SPMV(4);
         else if (A.lanes == 8) CSRV_SPMV(8);
         else CSRV_SPMV(16);
 #undef CSRV_SPMV
+#undef CSRV_SPMV_NC
     } else {
         SELL_DISPATCH(sell_spmv_kernel, A, has_ghosts(x), V, dx, ctx, b, y, kmode, sign, push);
     }
@@ -882,6 +1027,7 @@ int sell_cheb_step(ctl_handle_s *h, const SellMat &A, const double *dinv, const 
 {
     CTL_CHECK(push.n_chunks == 0 || (out != p_prev && out != p_cur.x), CTL_ERR_STATE,
               "sell_cheb_step: a pushing step must not overwrite its inputs");
+    CHECK_NC(A, has_ghosts(p_cur), "sell_cheb_step");
     const MatView V = A.view();
     const DVec dx = dvec(p_cur, V);
     const HaloCtx ctx = halo_ctx(h);
@@ -895,6 +1041,7 @@ int sell_cheb_step(ctl_handle_s *h, const SellMat &A, const double *dinv, const 
 int sell_cheb_first2(ctl_handle_s *h, const SellMat &A, const GVec &dinv, const GVec &b, double *out, double s, double w,
                      const HaloPush &push)
 {
+    CHECK_NC(A, has_ghosts(b) || has_ghosts(dinv), "sell_cheb_first2");
     const MatView V = A.view();
     const DVec dd = dvec(dinv, V), db = dvec(b, V);
     const HaloCtx ctx = halo_ctx(h);
@@ -905,21 +1052,28 @@ int sell_cheb_first2(ctl_handle_s *h, const SellMat &A, const GVec &dinv, const 
     return CTL_OK;
 }
 
-int vec_dinv_scale(ctl_handle_s *h, const double *dinv, const double *b, double *out, double c, int n, const HaloPush &push)
+int vec_dinv_scale(ctl_handle_s *h, const double *dinv, const double *b, double *out, double c, int n, const HaloPush &push,
+                   int nc)
 {
+    CTL_CHECK(nc == 1 || (push.n_chunks == 0 && !push.all_rows), CTL_ERR_STATE,
+              "vec_dinv_scale: vectors with several components run on one GPU only");
     const int grid = grid_for(n, 1, push);
     if (grid == 0) return CTL_OK;
-    pdl_launch(h, grid, ST, dinv_scale_kernel, dinv, b, out, c, n, halo_ctx(h), push);
+    if (nc == 2) pdl_launch(h, grid, ST, dinv_scale_kernel<2>, dinv, b, out, c, n, halo_ctx(h), push);
+    else if (nc == 3) pdl_launch(h, grid, ST, dinv_scale_kernel<3>, dinv, b, out, c, n, halo_ctx(h), push);
+    else pdl_launch(h, grid, ST, dinv_scale_kernel<1>, dinv, b, out, c, n, halo_ctx(h), push);
     h->launches++;
     CTL_CUDA(cudaGetLastError());
     return CTL_OK;
 }
 
-int dense_gemv(ctl_handle_s *h, const double *Ainv, const double *b, double *y, int n, int lda)
+int dense_gemv(ctl_handle_s *h, const double *Ainv, const double *b, double *y, int n, int lda, int nc)
 {
     CTL_CHECK(lda >= n && (lda & 1) == 0, CTL_ERR_ARG, "dense_gemv: the row stride must be even and >= n");
     if (n == 0) return CTL_OK;
-    pdl_launch(h, ceil_div(n, GR), ST, dense_gemv_kernel, Ainv, b, y, n, lda);
+    if (nc == 2) pdl_launch(h, ceil_div(n, GR), ST, dense_gemv_kernel<2>, Ainv, b, y, n, lda);
+    else if (nc == 3) pdl_launch(h, ceil_div(n, GR), ST, dense_gemv_kernel<3>, Ainv, b, y, n, lda);
+    else pdl_launch(h, ceil_div(n, GR), ST, dense_gemv_kernel<1>, Ainv, b, y, n, lda);
     h->launches++;
     CTL_CUDA(cudaGetLastError());
     return CTL_OK;
@@ -929,10 +1083,16 @@ int sell_spmv2(ctl_handle_s *h, const SellMat &A1, const SellMat &A2, const GVec
                double *y, double alpha, double beta, const HaloPush &push)
 {
     CTL_CHECK(A1.lanes == 0 && A2.lanes == 0, CTL_ERR_STATE, "sell_spmv2: SELL matrices only");
+    CTL_CHECK(A1.nc == A2.nc, CTL_ERR_STATE, "sell_spmv2: both matrices need the same number of components");
+    CHECK_NC(A1, has_ghosts(x1) || has_ghosts(x2) || has_ghosts(x3), "sell_spmv2");
     const int grid = grid_for(A1.pat->n_rows, 1, push);
     if (grid == 0) return CTL_OK;
     const MatView V1 = A1.view(), V2 = A2.view();
-    pdl_launch(h, grid, ST, sell_spmv2_kernel, V1, V2, dvec(x1, V1), dvec(x2, V1), dvec(x3, V2), y, alpha, beta, halo_ctx(h), push);
+    const DVec d1 = dvec(x1, V1), d2 = dvec(x2, V1), d3 = dvec(x3, V2);
+    const HaloCtx ctx = halo_ctx(h);
+    if (A1.nc == 2) pdl_launch(h, grid, ST, sell_spmv2_kernel<2>, V1, V2, d1, d2, d3, y, alpha, beta, ctx, push);
+    else if (A1.nc == 3) pdl_launch(h, grid, ST, sell_spmv2_kernel<3>, V1, V2, d1, d2, d3, y, alpha, beta, ctx, push);
+    else pdl_launch(h, grid, ST, sell_spmv2_kernel<1>, V1, V2, d1, d2, d3, y, alpha, beta, ctx, push);
     h->launches++;
     CTL_CUDA(cudaGetLastError());
     return CTL_OK;

@@ -30,6 +30,8 @@ struct SellMat {
     int fmt = FMT_F64;
     bool stream = false;               // matrix larger than the L2 share it can keep: evict-first loads
     int n_own = 0;                     // gathered columns >= n_own come from the ghost array (0: all owned)
+    int nc = 1;                        // components: the scalar matrix S acts on nc interleaved vectors, dof = nc * row
+                                       // + comp (I_nc (x) S, one GPU only); vectors have nc * n_rows entries
     int64_t bytes_per_pass = 0;        // matrix stream bytes of one product (byte model)
     // SELL value arrays (owned)
     double *vals = nullptr;
@@ -98,11 +100,11 @@ int sell_cheb_step(ctl_handle_s *h, const SellMat &A, const double *dinv, const 
 // columns, out = w p1 + w s dinv .* (b - A p1)   (dinv and b are gathered: both need their ghost entries)
 int sell_cheb_first2(ctl_handle_s *h, const SellMat &A, const GVec &dinv, const GVec &b, double *out, double s, double w,
                      const HaloPush &push = HaloPush());
-// out = c * dinv .* b   (first step from a zero guess)
+// out = c * dinv .* b   (first step from a zero guess); n rows of nc interleaved components, dinv per row
 int vec_dinv_scale(ctl_handle_s *h, const double *dinv, const double *b, double *out, double c, int n,
-                   const HaloPush &push = HaloPush());
-// y = Ainv b, dense row-major n x n with row stride lda (even)
-int dense_gemv(ctl_handle_s *h, const double *Ainv, const double *b, double *y, int n, int lda);
+                   const HaloPush &push = HaloPush(), int nc = 1);
+// y = Ainv b, dense row-major n x n with row stride lda (even); b and y hold nc interleaved components per row
+int dense_gemv(ctl_handle_s *h, const double *Ainv, const double *b, double *y, int n, int lda, int nc = 1);
 // two-matrix product on one shared row set (backward-sweep right-hand side, pc.cu):
 //   y = alpha * A1 (x1 + x2) + beta * A2 x3      (x2, x3 may be null)
 int sell_spmv2(ctl_handle_s *h, const SellMat &A1, const SellMat &A2, const GVec &x1, const GVec &x2, const GVec &x3,

@@ -24,13 +24,16 @@ __all__ = ["StokesSystem"]
 
 class StokesSystem:
     def __init__(self, M_v, K_v, B, M_p, K_p, *, n_t, beta, CN, time_interval=(0.0, 1.0), bc_dofs_v=(),
-                 epsilon=1e-3, device=None, D_p=None):
+                 epsilon=1e-3, device=None, D_p=None, velocity_block_size=1):
         """``K_v``: the forward matrix on the velocity space (one matrix or n_t matrices ``D_v_i``).  ``K_p``: the
         pressure Laplacian ``solver_K_p`` inverts (control/control.py:3746, 4300-4309).  ``D_p``: the forward
         form on the PRESSURE space (``D_p_i``, control/control.py:3787-3789; one matrix or n_t matrices) of the
-        pressure-space KKT multiply; default ``K_p`` (the Stokes forward operator)."""
+        pressure-space KKT multiply; default ``K_p`` (the Stokes forward operator).  ``velocity_block_size``: block
+        size of the velocity space (2 for a 2-D ``VectorFunctionSpace``): the velocity sweeps then run on the scalar
+        block of ``I_2 (x) S`` (``MultiBlockSystem(block_size=)``)."""
         self.velocity = MultiBlockSystem(M_v, K_v, n_t=n_t, beta=beta, CN=CN, time_interval=time_interval,
-                                         bc_dofs=bc_dofs_v, epsilon=epsilon, device=device)
+                                         bc_dofs=bc_dofs_v, epsilon=epsilon, device=device,
+                                         block_size=velocity_block_size)
         self.pressure = MultiBlockSystem(M_p, K_p if D_p is None else D_p, n_t=n_t, beta=beta, CN=CN,
                                          time_interval=time_interval, bc_dofs=(), epsilon=epsilon,
                                          device=self.velocity.device.index, stream=self.velocity.stream)

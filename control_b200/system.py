@@ -81,7 +81,15 @@ def _as_host_f64(x):
 
 class MultiBlockSystem:
     def __init__(self, M, K, *, n_t, beta, CN, time_interval=(0.0, 1.0), bc_dofs=(),
-                 epsilon=1e-3, device=None, rank=0, world=1, stream=None):
+                 epsilon=1e-3, device=None, rank=0, world=1, stream=None, block_size=1):
+        """``block_size``: PETSc's Mat block size of the space (``M.petscmat.getBlockSize()``), dofs interleaved as
+        ``bs * node + comp``.  With 2 or 3, the preconditioner runs its time sweeps on the scalar block ``S`` of
+        matrices ``I_bs (x) S`` (``ctl_set_block_size``; ``pc_block_size`` tells whether they had that structure)."""
+        block_size = int(block_size)
+        if block_size not in (1, 2, 3):
+            raise ValueError(f"block_size must be 1, 2 or 3, not {block_size}")
+        if block_size > 1 and world > 1:
+            raise ValueError("block_size > 1 runs on one GPU: block-scalar sweeps are not available with world > 1")
         self._lib = L.load()
         self._h = C.c_void_p()
         if not torch.cuda.is_available():
@@ -115,6 +123,9 @@ class MultiBlockSystem:
         self._check(self._lib.ctl_set_values(self._h, L.CTL_MAT_M, -1, m_data.ctypes.data))
         self.bc_dofs = np.ascontiguousarray(bc_dofs, dtype=np.int32)
         self._check(self._lib.ctl_set_bc(self._h, self.bc_dofs.ctypes.data, self.bc_dofs.size))
+        self.block_size = block_size
+        if block_size != 1:
+            self._check(self._lib.ctl_set_block_size(self._h, block_size))
         self._pc_ready = False
         self._cb_keepalive = None
         self.set_K(K)
@@ -283,6 +294,12 @@ class MultiBlockSystem:
         self._check(self._lib.ctl_pc_setup(self._h, C.byref(o)))
         self._pc_ready = True
         self._pc_opts = o
+
+    @property
+    def pc_block_size(self):
+        """Block size the preconditioner's time sweeps run with: ``block_size`` when every sweep matrix is
+        ``I_bs (x) S``, 1 when one is not (or ``block_size`` is 1); -1 before ``setup_preconditioner``."""
+        return int(self._lib.ctl_pc_block_size(self._h))
 
     def pc_apply(self, b_dev, u_dev=None, layout=L.CTL_LAYOUT_BLOCK_MAJOR, raw=False):
         """``Preconditioner.apply`` (raw=False) or the bare ``pc_fn`` (raw=True)."""

@@ -146,6 +146,17 @@ int ctl_set_values(ctl_handle h, int which, int level, const double *values_host
 /* homogeneous Dirichlet dofs: DirichletBCNullspace(bcs_v)
  * (preconditioner/preconditioner.py:158-197; control/control.py:2851-2862) */
 int ctl_set_bc(ctl_handle h, const int32_t *dofs_host, int32_t count);
+/* block size of a vector-valued space: PETSc's Mat block size with interleaved numbering, dof = bs node + comp
+ * (Firedrake's VectorFunctionSpace).  bs = 1 (the default) is the scalar path.  With bs > 1, ctl_pc_setup checks
+ * whether EVERY matrix of the time sweeps -- M, each distinct diagonal block and its AMG hierarchy, the
+ * Multigrid=True mass hierarchy, each off-diagonal block -- is I_bs (x) S: no entry couples two components and the
+ * bs component blocks are bitwise equal (absent entries and stored zeros count as 0; a Dirichlet list that is not
+ * node-closed breaks it).  If so, the sweeps are set up and run on the scalar S, each product acting on bs
+ * interleaved components (every AMG hierarchy is that of S with coarse_max replaced by ceil(coarse_max / bs));
+ * otherwise the handle takes the bs = 1 path.  The KKT apply and the batched parts of the preconditioner do not
+ * change.  CTL_ERR_ARG unless bs is 1, 2 or 3 and divides n, and for bs > 1 with world > 1 (block-scalar sweeps
+ * run on one GPU).  Drops a preconditioner that is already set up (call ctl_pc_setup again). */
+int ctl_set_block_size(ctl_handle h, int32_t bs);
 /* finish setup (uploads, eliminations); must precede apply/solve */
 int ctl_assemble(ctl_handle h);
 
@@ -166,6 +177,9 @@ int ctl_kkt_apply(ctl_handle h, const double *x, double *y, int layout);
  *      wrapped as Preconditioner.apply (preconditioner/preconditioner.py:562-656). */
 int ctl_pc_default_options(ctl_pc_options *opts);
 int ctl_pc_setup(ctl_handle h, const ctl_pc_options *opts);
+/* block size the preconditioner that is set up runs its sweeps with (1 when the matrices lack the structure
+ * ctl_set_block_size asks for); -1 before ctl_pc_setup */
+int32_t ctl_pc_block_size(ctl_handle h);
 int ctl_pc_apply(ctl_handle h, const double *b, double *u, int layout);
 /* the raw pc_fn(u_0, u_1, b_0, b_1) without the nullspace wrapping (what a user would
  * pass back through `P=`) */
@@ -226,7 +240,10 @@ int ctl_build_rhs(ctl_handle h, const double *v_hat, const double *f_nodal, cons
  *      has Dirichlet dofs.  With no Dirichlet dofs the call does nothing.  Asynchronous on the handle's stream. */
 int ctl_lift_bc(ctl_handle h, const double *g, double *b, int layout);
 
-/* ---- AMG introspection (tests compare the hierarchy with the oracle's) */
+/* ---- AMG introspection (tests compare the hierarchy with the oracle's).  A block hierarchy (ctl_pc_block_size > 1)
+ *      is that of the scalar S: level sizes, matrices and aggregates describe the scalar levels; ctl_amg_solve takes
+ *      n-vectors in the interleaved layout (16-byte aligned for bs = 2) and solves every component; ctl_time_amg counts
+ *      the matrix bytes once and the vector bytes bs times (the Jacobi diagonal, one entry per node, once). */
 int32_t ctl_amg_num_hierarchies(ctl_handle h);
 int32_t ctl_amg_num_levels(ctl_handle h, int32_t hierarchy);
 int ctl_amg_level_size(ctl_handle h, int32_t hierarchy, int32_t level, int32_t *n,

@@ -26,6 +26,8 @@ def main():
     ap.add_argument("--inner_its", type=int, default=5)
     ap.add_argument("--amg", default="", help="comma list key=value: velocity AMG options")
     ap.add_argument("--amg_p", default="", help="comma list key=value: K_p AMG options")
+    ap.add_argument("--block-size", type=int, default=1,
+                    help="velocity block size: 2 runs the velocity sweeps on the scalar block of I_2 (x) S")
     args = ap.parse_args()
     from synthetic import problems
     from control_b200.control import build_rhs
@@ -37,7 +39,7 @@ def main():
           flush=True)
     t = time.time()
     s = StokesSystem(th["M_v"], th["K_v"], th["B"], th["M_p"], th["K_p"], n_t=q["n_t"], beta=q["beta"], CN=not args.be,
-                     time_interval=q["time_interval"], bc_dofs_v=q["bdofs"])
+                     time_interval=q["time_interval"], bc_dofs_v=q["bdofs"], velocity_block_size=args.block_size)
     print(f"system created in {time.time() - t:.1f}s", flush=True)
     t = time.time()
     def parse(txt):
@@ -48,7 +50,7 @@ def main():
         return out
     s.setup_preconditioner(lambda_v_bounds=q["lambda_v_bounds"], lambda_p_bounds=q["lambda_p_bounds"],
                            inner_its=args.inner_its, amg=parse(args.amg), amg_p=parse(args.amg_p))
-    print(f"pc setup in {time.time() - t:.1f}s", flush=True)
+    print(f"pc setup in {time.time() - t:.1f}s, velocity sweeps with block size {s.velocity.pc_block_size}", flush=True)
     N = s.N
     b00, b01 = build_rhs(q["M"], q["K"], q["tau"], q["n_t"], not args.be, q["bdofs"], q["v_d"], q["f"], np.zeros(s.n_v))
     b = s.to_device(np.concatenate([b00, b01]), np.zeros((2 * N, s.n_p)))
