@@ -280,13 +280,15 @@ static void dense_inverse(const HostCSR &A, const std::vector<double> &shift, st
     }
 }
 
+int setup_threads(int fallback)
+{
+    if (const char *e = getenv("CTL_SETUP_THREADS")) return atoi(e);
+    return fallback;
+}
+
 void amg_setup_host(const HostCSR &A0, const AmgParams &p, std::vector<AmgLevelHost> &levels, int threads)
 {
-    if (threads <= 0) {
-        threads = (int)std::thread::hardware_concurrency();
-        if (const char *e = getenv("CTL_SETUP_THREADS")) threads = atoi(e);
-        threads = std::max(1, std::min(threads, 32));
-    }
+    if (threads <= 0) threads = std::max(1, std::min(setup_threads((int)std::thread::hardware_concurrency()), 32));
     levels.clear();
     levels.reserve((size_t)std::max(1, p.max_levels));      // references to a level stay valid while the next is built
     HostCSR next = A0;                                       // the one copy: the caller keeps its matrix

@@ -39,8 +39,12 @@ struct AmgLevelHost {
     bool has_inverse() const { return !Ainv.empty() || coarse_inverse != 0; }
 };
 
+// host threads of the preconditioner set-up: the environment variable CTL_SETUP_THREADS when it is set (a limit for
+// shared hosts), `fallback` otherwise
+int setup_threads(int fallback);
+
 // A must have sorted column indices.  Returns the levels, finest first.
-// threads: host threads for the row-parallel phases (0 = all hardware threads, CTL_SETUP_THREADS); the
+// threads: host threads for the row-parallel phases (0 = all hardware threads, up to 32, or setup_threads); the
 // result does not depend on it
 void amg_setup_host(const HostCSR &A, const AmgParams &p, std::vector<AmgLevelHost> &levels, int threads = 0);
 

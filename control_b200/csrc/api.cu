@@ -100,7 +100,6 @@ int ctl_create(const ctl_config *cfg, ctl_handle *out)
         h->own_stream = true;
     }
     h->h_bcmask.assign(cfg->n, 0);
-    if (const char *e = getenv("CTL_NO_PDL")) h->use_pdl = !(e[0] == '1');
     *out = h;
     return CTL_OK;
 }
@@ -254,7 +253,6 @@ static int build_local_pattern(ctl_handle_s *h)
         L.indptr[r + 1] = (int)p;
         h->max_row_len = std::max(h->max_row_len, ip[g + 1] - ip[g]);
     }
-    if (const char *e = getenv("CTL_KKT_UNSTAGED")) h->force_unstaged = (e[0] == '1');
     {   // gather chunk with the fewest padding slots over all rows (ties: the larger chunk)
         const int cand[4] = {4, 5, 7, 8};
         long best = -1;
@@ -268,10 +266,6 @@ static int build_local_pattern(ctl_handle_s *h)
                 best = slots;
                 h->gather_chunk = c;
             }
-        }
-        if (const char *e = getenv("CTL_KKT_CHUNK")) {      // experiment: only the instantiated chunk sizes
-            const int c = atoi(e);
-            if (c == 4 || c == 5 || c == 7 || c == 8) h->gather_chunk = c;
         }
     }
     // note: local column order within a row is no longer sorted when ghosts precede owned

@@ -60,7 +60,6 @@ struct ctl_handle_s {
     std::string err;
     int64_t launches = 0;
     bool assembled = false;
-    bool use_pdl = true;       // programmatic dependent launch for the chains of small sweep kernels (CTL_NO_PDL=1 disables)
     int block_size = 1;        // ctl_set_block_size: interleaved components of the space, dof = block_size node + comp
 
     // host copies of what the caller handed over (global numbering)
@@ -87,7 +86,6 @@ struct ctl_handle_s {
     bool per_level = false;
     int max_row_len = 0;        // longest local row (sizes the shared-memory staging)
     int gather_chunk = 4;       // entries per gather pass of the staged KKT apply (4, 5, 7 or 8: least padding)
-    bool force_unstaged = false;   // CTL_KKT_UNSTAGED=1: launch the unstaged kernel (the fallback for very long rows)
     bool k_symmetric = false;
     uint8_t *d_bcmask = nullptr;   // local rows (owned + ghost)
     int *d_bc_rows_all = nullptr;  // list of constrained owned rows
@@ -165,7 +163,7 @@ inline void pdl_launch(ctl_handle_s *h, int grid, int block, void (*kernel)(KArg
     at.id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at.val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = &at;
-    cfg.numAttrs = h->use_pdl ? 1 : 0;
+    cfg.numAttrs = 1;
     cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 #endif

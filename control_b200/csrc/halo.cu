@@ -312,7 +312,6 @@ int amg_build_distributed(ctl_handle_s *h, const AmgParams &p, const std::shared
     // distributed); a level pays once its products are stream bound (3-D: 18.5 M entries on the first level of C3).
     int64_t rep_nnz = 2000000;
     if (const char *e = getenv("CTL_AMG_REP_NNZ")) rep_nnz = std::max(1ll, atoll(e));
-    if (const char *e = getenv("CTL_AMG_REP_MIN")) rep_nnz = std::max(1ll, atoll(e));      // (older name, tests)
     DistHierarchy D;
     amg_distribute_host(world, me, H.host, rep_nnz, st.mesh_space->g, D);
     CTL_CHECK(D.part[0][me] == h->row_begin && D.part[0][me + 1] - D.part[0][me] == h->n_loc, CTL_ERR_STATE,

@@ -573,7 +573,7 @@ int ctl_kkt_apply_tf(ctl_handle_s *h, const double *x_tf, double *y_tf)
     int rows_per_cta = std::min(64, (STAGE_CAP / max_len) / 8 * 8);
     // the staged kernel addresses gathered rows with 31-bit byte offsets
     const bool fits = (size_t)std::max(h->n_loc, h->n_halo) * h->ld * 8 < 0x7fffffffull;
-    const bool staged = rows_per_cta >= 8 && !h->force_unstaged && fits;
+    const bool staged = rows_per_cta >= 8 && fits;
     const bool halo = h->n_halo > 0;
     if (h->ld > 64) {
         CTL_CHECK(rows_per_cta >= 8, CTL_ERR_ARG, "ctl_kkt_apply: rows too long for the wide (N > 64) kernel");

@@ -231,7 +231,6 @@ static int enqueue_sweeps(ctl_handle_s *h, PcState &st)
 
 static int run_sweeps(ctl_handle_s *h, PcState &st)
 {
-    if (!st.use_graph) return enqueue_sweeps(h, st);
     if (!st.sweep_graph) {
         const int64_t before = h->launches;
         cudaGraph_t graph = nullptr;
@@ -468,7 +467,6 @@ int ctl_pc_setup(ctl_handle h, const ctl_pc_options *opts)
     st.amg.cycles = opts->amg_cycles;
     st.amg.acc_lo = opts->amg_acc_lo;
     st.amg.acc_hi = opts->amg_acc_hi;
-    if (const char *e = getenv("CTL_NO_GRAPH")) st.use_graph = !(e[0] == '1');
 
     const int N = h->N, nl = h->n_loc, rb = h->row_begin;
     const bool cn = h->cfg.CN != 0;
@@ -610,8 +608,7 @@ int ctl_pc_setup(ctl_handle h, const ctl_pc_options *opts)
                 if (!has_block_structure(h, bsz, v)) ok = false;
             }
         };
-        int n_threads = std::max(1, (int)std::thread::hardware_concurrency());
-        if (const char *e = getenv("CTL_SETUP_THREADS")) n_threads = std::max(1, atoi(e));
+        int n_threads = std::max(1, setup_threads(std::max(1, (int)std::thread::hardware_concurrency())));
         n_threads = std::min(std::min(n_threads, n_tasks), 32);
         std::vector<std::thread> pool;
         for (int t = 1; t < n_threads; ++t) pool.emplace_back(check);
@@ -647,8 +644,7 @@ int ctl_pc_setup(ctl_handle h, const ctl_pc_options *opts)
         std::vector<std::vector<double>> off_values(n_off);
         // one process per GPU on one host: every rank sets the same hierarchies up, so each takes its share of the
         // cores (8 ranks x all 16 cores oversubscribed the box: 10-13 s of set-up at 8 GPUs against 2 s at one)
-        int n_threads = std::max(1, (int)std::thread::hardware_concurrency() / std::max(1, h->cfg.world));
-        if (const char *e = getenv("CTL_SETUP_THREADS")) n_threads = atoi(e);
+        int n_threads = setup_threads(std::max(1, (int)std::thread::hardware_concurrency() / std::max(1, h->cfg.world)));
         const int hw_threads = std::max(1, std::min(n_threads, 32));
         n_threads = std::max(1, std::min(std::min(n_threads, nh + n_off), 32));
         std::atomic<int> next{0};

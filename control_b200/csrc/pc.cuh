@@ -43,6 +43,5 @@ struct PcState {
     std::shared_ptr<HaloSpace> mesh_space;  // who gathers what through the mesh pattern
     HaloPlan *px0 = nullptr, *pb0 = nullptr;   // level-0 iterates / right-hand sides (shared by all hierarchies)
     cudaGraphExec_t sweep_graph = nullptr;
-    bool use_graph = true;
     int64_t sweep_launches = 0;             // kernels inside one sweep graph
 };

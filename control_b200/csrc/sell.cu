@@ -4,8 +4,6 @@
 // vector stream (HBM, or L2 once the compressed matrix stays resident) and by launch latency on the coarse levels;
 // nothing is a dense contraction.
 #include <algorithm>
-#include <cstdlib>
-#include <cstring>
 #include <type_traits>
 
 #include "sell.cuh"
@@ -71,67 +69,23 @@ MatView SellMat::view() const
     return v;
 }
 
-int sell_max_fmt()
-{
-    static int v = -1;
-    if (v < 0) {
-        v = FMT_STENCIL;
-        if (const char *e = getenv("CTL_SELL_FMT")) {      // experiment / tests: cap the automatic choice
-            if (!strcmp(e, "f64")) v = FMT_F64;
-            else if (!strcmp(e, "d16")) v = FMT_D16;
-            else if (!strcmp(e, "pk")) v = FMT_PK;
-            else if (!strcmp(e, "dict16")) v = FMT_DICT16;
-            else if (!strcmp(e, "dict8")) v = FMT_DICT8;
-        }
-    }
-    return v;
-}
+// cap of the automatic format choice for the mesh matrices (fine level, off-diagonal blocks): every exact format
+constexpr int FMT_MAX_FINE = FMT_STENCIL;
 
 // cap for the matrices that own their pattern (coarse AMG operators, transfers) while they are small enough to
-// stay in L2: CTL_SELL_FMT_COARSE.  Larger ones (3-D: the first Galerkin level of C3 has 18.5 M entries, 222 MB
-// plain) are bound by their stream and take the most compact exact format like the fine level.
-static int64_t coarse_plain_limit()
-{
-    static int64_t v = -1;
-    if (v < 0) {
-        v = 64ll << 20;
-        if (const char *e = getenv("CTL_COARSE_PLAIN_MB")) v = (int64_t)atoi(e) << 20;
-    }
-    return v;
-}
+// stay in L2.  Measured at C2 (round 2, profiles/r02_inner_solve_variants.txt): on the Galerkin levels and the
+// transfer operators the dictionary formats cost more instructions than their bytes save (everything there is
+// L2-resident and latency bound): inner solve 0.81 ms (dictionaries) / 0.73 (16-bit offsets) / 0.67 (plain)
+constexpr int FMT_MAX_COARSE = FMT_F64;
 
-static int sell_max_fmt_coarse()
-{
-    static int v = -1;
-    if (v < 0) {
-        // measured at C2 (round 2, profiles/r02_inner_solve_variants.txt): on the Galerkin levels and the transfer
-        // operators the dictionary formats cost more instructions than their bytes save (everything there is
-        // L2-resident and latency bound): inner solve 0.81 ms (dictionaries) / 0.73 (16-bit offsets) / 0.67 (plain)
-        v = FMT_F64;
-        if (const char *e = getenv("CTL_SELL_FMT_COARSE")) {
-            if (!strcmp(e, "f64")) v = FMT_F64;
-            else if (!strcmp(e, "d16")) v = FMT_D16;
-            else if (!strcmp(e, "pk")) v = FMT_PK;
-            else if (!strcmp(e, "dict16")) v = FMT_DICT16;
-            else if (!strcmp(e, "dict8")) v = FMT_DICT8;
-            else if (!strcmp(e, "stencil")) v = FMT_STENCIL;
-        }
-        v = std::min(v, sell_max_fmt());
-    }
-    return v;
-}
+// ... "small enough": a plain (12 B per entry) stream up to this size.  Larger ones (3-D: the first Galerkin level of
+// C3 has 18.5 M entries, 222 MB plain) are bound by their stream and take the most compact exact format like the
+// fine level.
+constexpr int64_t COARSE_PLAIN_BYTES = 64ll << 20;
 
 // matrices whose stream exceeds this many bytes are read evict-first: they cannot stay in L2 next to the
 // vectors of their level, and must not flush the coarse levels out of it
-static int64_t stream_threshold()
-{
-    static int64_t v = -1;
-    if (v < 0) {
-        v = 40ll << 20;
-        if (const char *e = getenv("CTL_STREAM_MB")) v = (int64_t)atoi(e) << 20;
-    }
-    return v;
-}
+constexpr int64_t STREAM_BYTES = 40ll << 20;
 
 template <typename T>
 static int upload_vec(ctl_handle_s *h, T **dst, const std::vector<T> &src)
@@ -156,7 +110,6 @@ int sell_build_pattern(ctl_handle_s *h, const HostCSR &A, std::shared_ptr<SellPa
     a.indptr = A.indptr.data();
     a.indices = A.indices.data();
     sf_sell_layout(a, p->host);
-    if (sell_max_fmt() < FMT_D16) p->host.dcol.clear();
     p->n_rows = A.n_rows;
     p->n_cols = A.n_cols;
     p->n_slices = p->host.n_slices;
@@ -174,7 +127,7 @@ static int sell_set_values_cap(ctl_handle_s *h, const std::shared_ptr<SellPatter
 
 int sell_set_values(ctl_handle_s *h, const std::shared_ptr<SellPattern> &pat, const double *csr_values, SellMat &out)
 {
-    return sell_set_values_cap(h, pat, csr_values, out, sell_max_fmt());
+    return sell_set_values_cap(h, pat, csr_values, out, FMT_MAX_FINE);
 }
 
 static int sell_set_values_cap(ctl_handle_s *h, const std::shared_ptr<SellPattern> &pat, const double *csr_values, SellMat &out,
@@ -186,7 +139,7 @@ static int sell_set_values_cap(ctl_handle_s *h, const std::shared_ptr<SellPatter
     out.fmt = V.fmt;
     out.lanes = 0;
     out.bytes_per_pass = V.bytes_per_pass;
-    out.stream = V.bytes_per_pass > stream_threshold();
+    out.stream = V.bytes_per_pass > STREAM_BYTES;
     CTL_TRY(upload_vec(h, &out.vals, V.vals));
     CTL_TRY(upload_vec(h, &out.vcode, V.vcode));
     CTL_TRY(upload_vec(h, &out.vdict, V.vdict));
@@ -206,21 +159,20 @@ int sell_from_csr(ctl_handle_s *h, const HostCSR &A, SellMat &out, int force_lan
     const double mean = A.n_rows ? (double)A.nnz() / A.n_rows : 0.0;
     // SELL-32 (one row per thread, coalesced) up to a mean row length of 24: measured at C2 against the
     // CSR-vector kernels, inner solve 0.842 ms (threshold 10) -> 0.792 (14) -> 0.774 (20-24) -> 0.779 (40)
-    double sell_max_mean = 24.0;
-    if (const char *e = getenv("CTL_SELL_MAX_MEAN")) sell_max_mean = atof(e);      // experiment
+    constexpr double SELL_MAX_MEAN = 24.0;
     // ... but only for levels with enough rows to fill the GPU with one row per thread: below ~50 k rows
     // the CSR-vector kernels (several threads per row) win (19 k-row level as SELL: 0.833 ms per solve)
-    int sell_min_rows = 50000;
-    if (const char *e = getenv("CTL_SELL_MIN_ROWS")) sell_min_rows = atoi(e);      // experiment
+    constexpr int SELL_MIN_ROWS = 50000;
     const bool mesh_like = mean <= 10.0;          // fine-mesh stencils (short rows): always SELL
     // ... and so is a level with long rows once it has enough of them (3-D: the first Galerkin level of C3, 248 k rows
     // of 75 entries): one thread per row streams coalesced indices and values (16-bit offsets: 10 B per entry),
     // where the lane-per-entry CSR kernel took 91 us per product for the same 18.5 M entries
     const bool many_rows = A.n_rows >= 100000;
-    if (force_lanes == 0 && (mesh_like || many_rows || (mean <= sell_max_mean && A.n_rows >= sell_min_rows))) {
+    const int max_fmt = 12 * A.nnz() > COARSE_PLAIN_BYTES ? FMT_MAX_FINE : FMT_MAX_COARSE;
+    if (force_lanes == 0 && (mesh_like || many_rows || (mean <= SELL_MAX_MEAN && A.n_rows >= SELL_MIN_ROWS))) {
         std::shared_ptr<SellPattern> pat;
         CTL_TRY(sell_build_pattern(h, A, pat));
-        return sell_set_values_cap(h, pat, A.values.data(), out, 12 * A.nnz() > coarse_plain_limit() ? sell_max_fmt() : sell_max_fmt_coarse());
+        return sell_set_values_cap(h, pat, A.values.data(), out, max_fmt);
     }
     auto pat = std::make_shared<SellPattern>();     // sizes only; no SELL arrays
     pat->n_rows = A.n_rows;
@@ -231,10 +183,6 @@ int sell_from_csr(ctl_handle_s *h, const HostCSR &A, SellMat &out, int force_lan
     // for the 13-entry rows of level 1 = 0.918 ms, 16 lanes = 1.189 ms, 4 lanes = 0.843 ms: the narrow
     // groups keep four times as many rows in flight, which is what these latency-bound kernels need.
     out.lanes = mean <= 16.0 ? 4 : (mean <= 48.0 ? 8 : 16);
-    if (const char *e = getenv("CTL_CSR_LANES_SHIFT")) {          // experiment: wider / narrower row groups
-        const int sh = atoi(e);
-        out.lanes = std::max(4, std::min(16, sh >= 0 ? out.lanes << sh : out.lanes >> (-sh)));
-    }
     if (force_lanes) out.lanes = force_lanes;
     SfCsr a;
     a.n_rows = A.n_rows;
@@ -242,10 +190,10 @@ int sell_from_csr(ctl_handle_s *h, const HostCSR &A, SellMat &out, int force_lan
     a.indptr = A.indptr.data();
     a.indices = A.indices.data();
     SfCsrvData D;
-    sf_csrv_data(a, A.values.data(), std::min(12 * A.nnz() > coarse_plain_limit() ? sell_max_fmt() : sell_max_fmt_coarse(), (int)FMT_PK), D);
+    sf_csrv_data(a, A.values.data(), std::min(max_fmt, (int)FMT_PK), D);
     out.fmt = D.fmt;
     out.bytes_per_pass = D.bytes_per_pass;
-    out.stream = D.bytes_per_pass > stream_threshold();
+    out.stream = D.bytes_per_pass > STREAM_BYTES;
     CTL_TRY(upload_vec(h, &out.csr_ptr, A.indptr));
     CTL_TRY(upload_vec(h, &out.csr_cols, A.indices));
     CTL_TRY(upload_vec(h, &out.csr_rbase, D.rbase));
@@ -262,7 +210,7 @@ int sell_from_csr(ctl_handle_s *h, const HostCSR &A, SellMat &out, int force_lan
 namespace {
 
 constexpr int ST = 128;      // threads per CTA of the kernels in this file (the one-row-per-thread kernels of a large
-                             // level run 256: big_block_rows)
+                             // level run 256: BIG_BLOCK_ROWS)
 constexpr int SC = 8;        // SELL entries fetched per thread before the first dependent gather
 
 // ---- a gathered vector on the device: owned entries, and the ghosts either plainly stored (completed earlier) or
@@ -893,9 +841,12 @@ DVec dvec(const GVec &g, const MatView &A)
 bool has_ghosts(const GVec &g) { return g.ghost != nullptr || g.ll != nullptr; }
 
 // components run on one GPU only: no ghost entries, no pushed rows
-#define CHECK_NC(A, GHOSTS, what)                                                                           \
-    CTL_CHECK((A).nc == 1 || (!(GHOSTS) && push.n_chunks == 0 && !push.all_rows), CTL_ERR_STATE,            \
-              what ": matrices with several components run on one GPU only")
+int check_nc(ctl_handle_s *h, const SellMat &A, bool ghosts, const HaloPush &push, const char *what)
+{
+    CTL_CHECK(A.nc == 1 || (!ghosts && push.n_chunks == 0 && !push.all_rows), CTL_ERR_STATE,
+              std::string(what) + ": matrices with several components run on one GPU only");
+    return CTL_OK;
+}
 
 // push CTAs first; a replicating exchange pushes every row, so the regular CTAs are not launched at all
 int grid_for(int n_rows, int T, const HaloPush &push, int bs = ST)
@@ -909,72 +860,85 @@ int grid_for(int n_rows, int T, const HaloPush &push, int bs = ST)
 // of twice the size take 11-15 % off them (smoother step 11.95 -> 10.63 us, residual 11.76 -> 10.02 us, measured with
 // an all-256 build: profiles/r02_inner_solve_variants.txt); the small levels lose with fewer, larger CTAs and keep 128,
 // and so do long rows (the 15-point stencil of C3: its level-0 smoother went from 53 to 58 us with 256-thread CTAs).
-int big_block_rows()
+constexpr int BIG_BLOCK_ROWS = 400000;
+
+// ---- launch dispatch: the run-time choices become the compile-time parameters of the kernel templates
+template <int V>
+using int_c = std::integral_constant<int, V>;
+template <bool V>
+using bool_c = std::integral_constant<bool, V>;
+
+// f(NC) for the component counts of the block-scalar sweeps
+template <typename F>
+void with_nc(int nc, F f)
 {
-    static int v = -1;
-    if (v < 0) {
-        v = 400000;
-        if (const char *e = getenv("CTL_BIG_BLOCK_ROWS")) v = atoi(e);      // experiment; 0 = never
-        if (v <= 0) v = 2147483647;
-    }
-    return v;
+    if (nc == 2) f(int_c<2>());
+    else if (nc == 3) f(int_c<3>());
+    else f(int_c<1>());
 }
 
-// components (nc__ > 1) come without ghosts
-#define SELL_LAUNCH_NC(KERNEL, FMT, STREAM, NC, ...)                                                        \
-    do {                                                                                                    \
-        if (big__) pdl_launch(h, grid__, 256, KERNEL<FMT, STREAM, false, 256, NC>, __VA_ARGS__);            \
-        else pdl_launch(h, grid__, ST, KERNEL<FMT, STREAM, false, ST, NC>, __VA_ARGS__);                    \
-    } while (0)
+// f(T) for the lanes per row of a CSR-vector matrix
+template <typename F>
+void with_lanes(int lanes, F f)
+{
+    if (lanes == 4) f(int_c<4>());
+    else if (lanes == 8) f(int_c<8>());
+    else f(int_c<16>());
+}
 
-#define SELL_LAUNCH_GH(KERNEL, FMT, STREAM, ...)                                                            \
-    do {                                                                                                    \
-        if (nc__ == 2) SELL_LAUNCH_NC(KERNEL, FMT, STREAM, 2, __VA_ARGS__);                                 \
-        else if (nc__ == 3) SELL_LAUNCH_NC(KERNEL, FMT, STREAM, 3, __VA_ARGS__);                            \
-        else if (gh__) pdl_launch(h, grid__, ST, KERNEL<FMT, STREAM, true, ST, 1>, __VA_ARGS__);            \
-        else SELL_LAUNCH_NC(KERNEL, FMT, STREAM, 1, __VA_ARGS__);                                           \
-    } while (0)
+// A SELL kernel of A: f(grid, FMT, STREAM, GH, BS, NC), the last five compile-time.  Only the combinations that occur
+// are instantiated: evict-first streaming only in the formats that read a plain value array (F64, D16, PK); ghosts
+// (GH: a gathered vector has ghost entries) only with one component in CTAs of ST threads; CTAs of 256 threads only
+// on one GPU without pushed rows.  Returns false and launches nothing when the grid is empty.
+template <typename F>
+bool sell_dispatch(const SellMat &A, bool ghosts, const HaloPush &push, F f)
+{
+    const bool big = !ghosts && push.n_chunks == 0 && A.pat->n_rows >= BIG_BLOCK_ROWS && A.pat->nnz <= 10ll * A.pat->n_rows;
+    const int grid = grid_for(A.pat->n_rows, 1, push, big ? 256 : ST);
+    if (grid == 0) return false;
+    auto launch = [&](auto fmt, auto stream) {
+        with_nc(A.nc, [&](auto nc) {
+            if constexpr (decltype(nc)::value == 1) {
+                if (ghosts) {
+                    f(grid, fmt, stream, bool_c<true>(), int_c<ST>(), nc);
+                    return;
+                }
+            }
+            if (big) f(grid, fmt, stream, bool_c<false>(), int_c<256>(), nc);
+            else f(grid, fmt, stream, bool_c<false>(), int_c<ST>(), nc);
+        });
+    };
+    auto with_stream = [&](auto fmt) {
+        constexpr int FMT = decltype(fmt)::value;
+        if constexpr (FMT == FMT_F64 || FMT == FMT_D16 || FMT == FMT_PK) {
+            if (A.stream) {
+                launch(fmt, bool_c<true>());
+                return;
+            }
+        }
+        launch(fmt, bool_c<false>());
+    };
+    switch (A.fmt) {
+    case FMT_F64: with_stream(int_c<FMT_F64>()); break;
+    case FMT_D16: with_stream(int_c<FMT_D16>()); break;
+    case FMT_PK: with_stream(int_c<FMT_PK>()); break;
+    case FMT_DICT16: with_stream(int_c<FMT_DICT16>()); break;
+    case FMT_STENCIL: with_stream(int_c<FMT_STENCIL>()); break;
+    default: with_stream(int_c<FMT_DICT8>()); break;
+    }
+    return true;
+}
 
-#define SELL_LAUNCH_ST(KERNEL, FMT, ...)                                                                    \
-    do {                                                                                                    \
-        if (st__) SELL_LAUNCH_GH(KERNEL, FMT, true, __VA_ARGS__);                                           \
-        else SELL_LAUNCH_GH(KERNEL, FMT, false, __VA_ARGS__);                                               \
-    } while (0)
-
-// gh__: a gathered vector comes with ghost entries
-#define SELL_DISPATCH(KERNEL, A, GHOSTS, ...)                                                               \
-    do {                                                                                                    \
-        const bool st__ = (A).stream, gh__ = (GHOSTS);                                                      \
-        const int nc__ = (A).nc;                                                                            \
-        const bool big__ = !gh__ && push.n_chunks == 0 && (A).pat->n_rows >= big_block_rows() &&            \
-                           (A).pat->nnz <= 10ll * (A).pat->n_rows;                                          \
-        const int grid__ = grid_for((A).pat->n_rows, 1, push, big__ ? 256 : ST);                            \
-        if (grid__ == 0) return CTL_OK;                                                                     \
-        switch ((A).fmt) {                                                                                  \
-        case FMT_F64: SELL_LAUNCH_ST(KERNEL, FMT_F64, __VA_ARGS__); break;                                  \
-        case FMT_D16: SELL_LAUNCH_ST(KERNEL, FMT_D16, __VA_ARGS__); break;                                  \
-        case FMT_PK: SELL_LAUNCH_ST(KERNEL, FMT_PK, __VA_ARGS__); break;                                    \
-        case FMT_DICT16: SELL_LAUNCH_GH(KERNEL, FMT_DICT16, false, __VA_ARGS__); break;                     \
-        case FMT_STENCIL: SELL_LAUNCH_GH(KERNEL, FMT_STENCIL, false, __VA_ARGS__); break;                   \
-        default: SELL_LAUNCH_GH(KERNEL, FMT_DICT8, false, __VA_ARGS__); break;                              \
-        }                                                                                                   \
-    } while (0)
-
-#define CSRV_LAUNCH_NC(KERNEL, A, NC, ...)                                                                  \
-    do {                                                                                                    \
-        if ((A).lanes == 4) pdl_launch(h, grid__, ST, KERNEL<4, NC>, __VA_ARGS__);                          \
-        else if ((A).lanes == 8) pdl_launch(h, grid__, ST, KERNEL<8, NC>, __VA_ARGS__);                     \
-        else pdl_launch(h, grid__, ST, KERNEL<16, NC>, __VA_ARGS__);                                        \
-    } while (0)
-
-#define CSRV_DISPATCH(KERNEL, A, ...)                                                                       \
-    do {                                                                                                    \
-        const int grid__ = grid_for((A).pat->n_rows, (A).lanes, push);                                      \
-        if (grid__ == 0) return CTL_OK;                                                                     \
-        if ((A).nc == 2) CSRV_LAUNCH_NC(KERNEL, A, 2, __VA_ARGS__);                                         \
-        else if ((A).nc == 3) CSRV_LAUNCH_NC(KERNEL, A, 3, __VA_ARGS__);                                    \
-        else CSRV_LAUNCH_NC(KERNEL, A, 1, __VA_ARGS__);                                                     \
-    } while (0)
+// A CSR-vector kernel of A (CTAs of ST threads): f(grid, T, NC), the last two compile-time.  Returns false and launches
+// nothing when the grid is empty.
+template <typename F>
+bool csrv_dispatch(const SellMat &A, const HaloPush &push, F f)
+{
+    const int grid = grid_for(A.pat->n_rows, A.lanes, push);
+    if (grid == 0) return false;
+    with_lanes(A.lanes, [&](auto T) { with_nc(A.nc, [&](auto nc) { f(grid, T, nc); }); });
+    return true;
+}
 
 }  // namespace
 
@@ -991,32 +955,22 @@ int sell_spmv(ctl_handle_s *h, const SellMat &A, const GVec &x, double *y, const
     }
     CTL_CHECK(kmode == SELL_ASSIGN || b != nullptr, CTL_ERR_ARG, "sell_spmv: this mode needs b");
     CTL_CHECK(push.n_chunks == 0 || b != y, CTL_ERR_STATE, "sell_spmv: an in-place product cannot push its boundary rows");
-    CHECK_NC(A, has_ghosts(x), "sell_spmv");
+    CTL_TRY(check_nc(h, A, has_ghosts(x), push, "sell_spmv"));
     const MatView V = A.view();
     const DVec dx = dvec(x, V);
     const HaloCtx ctx = halo_ctx(h);
+    bool launched;
     if (A.lanes) {
-        const int grid = grid_for(A.pat->n_rows, A.lanes, push);
-        if (grid == 0) return CTL_OK;
-#define CSRV_SPMV_NC(T, NC)                                                                                          \
-    do {                                                                                                             \
-        if (A.stream) pdl_launch(h, grid, ST, csrv_spmv_kernel<T, true, NC>, V, dx, ctx, b, y, kmode, sign, push);   \
-        else pdl_launch(h, grid, ST, csrv_spmv_kernel<T, false, NC>, V, dx, ctx, b, y, kmode, sign, push);           \
-    } while (0)
-#define CSRV_SPMV(T)                                                                                                 \
-    do {                                                                                                             \
-        if (A.nc == 2) CSRV_SPMV_NC(T, 2);                                                                           \
-        else if (A.nc == 3) CSRV_SPMV_NC(T, 3);                                                                      \
-        else CSRV_SPMV_NC(T, 1);                                                                                     \
-    } while (0)
-        if (A.lanes == 4) CSRV_SPMV(4);
-        else if (A.lanes == 8) CSRV_SPMV(8);
-        else CSRV_SPMV(16);
-#undef CSRV_SPMV
-#undef CSRV_SPMV_NC
+        launched = csrv_dispatch(A, push, [&](int grid, auto T, auto NC) {
+            if (A.stream) pdl_launch(h, grid, ST, csrv_spmv_kernel<T, true, NC>, V, dx, ctx, b, y, kmode, sign, push);
+            else pdl_launch(h, grid, ST, csrv_spmv_kernel<T, false, NC>, V, dx, ctx, b, y, kmode, sign, push);
+        });
     } else {
-        SELL_DISPATCH(sell_spmv_kernel, A, has_ghosts(x), V, dx, ctx, b, y, kmode, sign, push);
+        launched = sell_dispatch(A, has_ghosts(x), push, [&](int grid, auto F, auto S, auto G, auto B, auto NC) {
+            pdl_launch(h, grid, B, sell_spmv_kernel<F, S, G, B, NC>, V, dx, ctx, b, y, kmode, sign, push);
+        });
     }
+    if (!launched) return CTL_OK;
     h->launches++;
     CTL_CUDA(cudaGetLastError());
     return CTL_OK;
@@ -1027,12 +981,22 @@ int sell_cheb_step(ctl_handle_s *h, const SellMat &A, const double *dinv, const 
 {
     CTL_CHECK(push.n_chunks == 0 || (out != p_prev && out != p_cur.x), CTL_ERR_STATE,
               "sell_cheb_step: a pushing step must not overwrite its inputs");
-    CHECK_NC(A, has_ghosts(p_cur), "sell_cheb_step");
+    CTL_TRY(check_nc(h, A, has_ghosts(p_cur), push, "sell_cheb_step"));
     const MatView V = A.view();
     const DVec dx = dvec(p_cur, V);
     const HaloCtx ctx = halo_ctx(h);
-    if (A.lanes) CSRV_DISPATCH(csrv_cheb_kernel, A, V, dinv, b, p_prev, dx, ctx, out, a, bq, c, prev_scale, push);
-    else SELL_DISPATCH(sell_cheb_kernel, A, has_ghosts(p_cur), V, dinv, b, p_prev, dx, ctx, out, a, bq, c, prev_scale, push);
+    bool launched;
+    if (A.lanes) {
+        launched = csrv_dispatch(A, push, [&](int grid, auto T, auto NC) {
+            pdl_launch(h, grid, ST, csrv_cheb_kernel<T, NC>, V, dinv, b, p_prev, dx, ctx, out, a, bq, c, prev_scale, push);
+        });
+    } else {
+        launched = sell_dispatch(A, has_ghosts(p_cur), push, [&](int grid, auto F, auto S, auto G, auto B, auto NC) {
+            pdl_launch(h, grid, B, sell_cheb_kernel<F, S, G, B, NC>, V, dinv, b, p_prev, dx, ctx, out, a, bq, c, prev_scale,
+                       push);
+        });
+    }
+    if (!launched) return CTL_OK;
     h->launches++;
     CTL_CUDA(cudaGetLastError());
     return CTL_OK;
@@ -1041,12 +1005,22 @@ int sell_cheb_step(ctl_handle_s *h, const SellMat &A, const double *dinv, const 
 int sell_cheb_first2(ctl_handle_s *h, const SellMat &A, const GVec &dinv, const GVec &b, double *out, double s, double w,
                      const HaloPush &push)
 {
-    CHECK_NC(A, has_ghosts(b) || has_ghosts(dinv), "sell_cheb_first2");
+    const bool ghosts = has_ghosts(b) || has_ghosts(dinv);
+    CTL_TRY(check_nc(h, A, ghosts, push, "sell_cheb_first2"));
     const MatView V = A.view();
     const DVec dd = dvec(dinv, V), db = dvec(b, V);
     const HaloCtx ctx = halo_ctx(h);
-    if (A.lanes) CSRV_DISPATCH(csrv_first2_kernel, A, V, dd, db, ctx, out, s, w, push);
-    else SELL_DISPATCH(sell_first2_kernel, A, has_ghosts(b) || has_ghosts(dinv), V, dd, db, ctx, out, s, w, push);
+    bool launched;
+    if (A.lanes) {
+        launched = csrv_dispatch(A, push, [&](int grid, auto T, auto NC) {
+            pdl_launch(h, grid, ST, csrv_first2_kernel<T, NC>, V, dd, db, ctx, out, s, w, push);
+        });
+    } else {
+        launched = sell_dispatch(A, ghosts, push, [&](int grid, auto F, auto S, auto G, auto B, auto NC) {
+            pdl_launch(h, grid, B, sell_first2_kernel<F, S, G, B, NC>, V, dd, db, ctx, out, s, w, push);
+        });
+    }
+    if (!launched) return CTL_OK;
     h->launches++;
     CTL_CUDA(cudaGetLastError());
     return CTL_OK;
@@ -1059,9 +1033,7 @@ int vec_dinv_scale(ctl_handle_s *h, const double *dinv, const double *b, double 
               "vec_dinv_scale: vectors with several components run on one GPU only");
     const int grid = grid_for(n, 1, push);
     if (grid == 0) return CTL_OK;
-    if (nc == 2) pdl_launch(h, grid, ST, dinv_scale_kernel<2>, dinv, b, out, c, n, halo_ctx(h), push);
-    else if (nc == 3) pdl_launch(h, grid, ST, dinv_scale_kernel<3>, dinv, b, out, c, n, halo_ctx(h), push);
-    else pdl_launch(h, grid, ST, dinv_scale_kernel<1>, dinv, b, out, c, n, halo_ctx(h), push);
+    with_nc(nc, [&](auto NC) { pdl_launch(h, grid, ST, dinv_scale_kernel<NC>, dinv, b, out, c, n, halo_ctx(h), push); });
     h->launches++;
     CTL_CUDA(cudaGetLastError());
     return CTL_OK;
@@ -1071,9 +1043,7 @@ int dense_gemv(ctl_handle_s *h, const double *Ainv, const double *b, double *y, 
 {
     CTL_CHECK(lda >= n && (lda & 1) == 0, CTL_ERR_ARG, "dense_gemv: the row stride must be even and >= n");
     if (n == 0) return CTL_OK;
-    if (nc == 2) pdl_launch(h, ceil_div(n, GR), ST, dense_gemv_kernel<2>, Ainv, b, y, n, lda);
-    else if (nc == 3) pdl_launch(h, ceil_div(n, GR), ST, dense_gemv_kernel<3>, Ainv, b, y, n, lda);
-    else pdl_launch(h, ceil_div(n, GR), ST, dense_gemv_kernel<1>, Ainv, b, y, n, lda);
+    with_nc(nc, [&](auto NC) { pdl_launch(h, ceil_div(n, GR), ST, dense_gemv_kernel<NC>, Ainv, b, y, n, lda); });
     h->launches++;
     CTL_CUDA(cudaGetLastError());
     return CTL_OK;
@@ -1084,15 +1054,15 @@ int sell_spmv2(ctl_handle_s *h, const SellMat &A1, const SellMat &A2, const GVec
 {
     CTL_CHECK(A1.lanes == 0 && A2.lanes == 0, CTL_ERR_STATE, "sell_spmv2: SELL matrices only");
     CTL_CHECK(A1.nc == A2.nc, CTL_ERR_STATE, "sell_spmv2: both matrices need the same number of components");
-    CHECK_NC(A1, has_ghosts(x1) || has_ghosts(x2) || has_ghosts(x3), "sell_spmv2");
+    CTL_TRY(check_nc(h, A1, has_ghosts(x1) || has_ghosts(x2) || has_ghosts(x3), push, "sell_spmv2"));
     const int grid = grid_for(A1.pat->n_rows, 1, push);
     if (grid == 0) return CTL_OK;
     const MatView V1 = A1.view(), V2 = A2.view();
     const DVec d1 = dvec(x1, V1), d2 = dvec(x2, V1), d3 = dvec(x3, V2);
     const HaloCtx ctx = halo_ctx(h);
-    if (A1.nc == 2) pdl_launch(h, grid, ST, sell_spmv2_kernel<2>, V1, V2, d1, d2, d3, y, alpha, beta, ctx, push);
-    else if (A1.nc == 3) pdl_launch(h, grid, ST, sell_spmv2_kernel<3>, V1, V2, d1, d2, d3, y, alpha, beta, ctx, push);
-    else pdl_launch(h, grid, ST, sell_spmv2_kernel<1>, V1, V2, d1, d2, d3, y, alpha, beta, ctx, push);
+    with_nc(A1.nc, [&](auto NC) {
+        pdl_launch(h, grid, ST, sell_spmv2_kernel<NC>, V1, V2, d1, d2, d3, y, alpha, beta, ctx, push);
+    });
     h->launches++;
     CTL_CUDA(cudaGetLastError());
     return CTL_OK;

@@ -54,9 +54,6 @@ struct SellMat {
     MatView view() const;
 };
 
-// largest format the automatic choice may pick (CTL_SELL_FMT=f64|d16|pk|dict16|dict8|stencil, default stencil)
-int sell_max_fmt();
-
 // build the pattern from a host CSR (column indices need not be sorted)
 int sell_build_pattern(ctl_handle_s *h, const HostCSR &A, std::shared_ptr<SellPattern> &out);
 // lay one value set (CSR order, host) out on a pattern, in the most compact exact format

@@ -1,5 +1,5 @@
-"""Time of one AMG inner solve at config C2 (warm, back to back) and of the level-0 kernels -- for A/B experiments via
-env (CTL_SELL_FMT, CTL_AMG_RR, CTL_STREAM_MB, ...; the switches are read when the library sets the preconditioner up)."""
+"""Time of one AMG inner solve at config C2 (warm, back to back) and of the level-0 kernels -- for A/B experiments
+between builds, or between the keyword arguments of setup_preconditioner (argv[2], JSON)."""
 import json, os, sys, time
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)

@@ -25,7 +25,7 @@ def main():
     rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
     torch.cuda.set_device(int(os.environ["LOCAL_RANK"]))
     dist.init_process_group("nccl", device_id=torch.device("cuda", int(os.environ["LOCAL_RANK"])))
-    # a small dense coarsest level, so that the hierarchy has several levels at this size; MP_NX / CTL_AMG_REP_MIN
+    # a small dense coarsest level, so that the hierarchy has several levels at this size; MP_NX / CTL_AMG_REP_NNZ
     # choose how many of them are distributed (halo.cu)
     amg = dict(coarse_max=int(os.environ.get("MP_COARSE_MAX", "30")))
     nx = int(os.environ.get("MP_NX", "40"))

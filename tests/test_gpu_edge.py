@@ -38,6 +38,36 @@ def test_two_time_levels(CN):
     s.close()
 
 
+
+@pytest.mark.parametrize("CN", [True, False])
+def test_kkt_apply_with_rows_too_long_to_stage(CN):
+    """One extra dof coupled to every dof of a 12 x 12 P1 mesh (a symmetric dense row and column of M and K): its row
+    has 170 entries, more than the 128 per row that the staged KKT kernel can hold (kkt_apply.cu: STAGE_CAP entries
+    for at least 8 rows per CTA), so the apply runs the unstaged kernel."""
+    import scipy.sparse as sp
+    from control_b200 import MultiBlockSystem
+    q = kat.heat_problem(12, 6, CN)
+    n0 = q["M"].shape[0]
+    assert n0 + 1 > 128
+    rng = np.random.default_rng(5)
+
+    def bordered(A, scale):
+        c = sp.csr_matrix(scale * rng.uniform(0.5, 1.0, (n0, 1)))
+        B = sp.bmat([[sp.csr_matrix(A), c], [c.T, sp.csr_matrix([[scale * n0]])]], format="csr")
+        B.sort_indices()
+        return B
+
+    M, K, bd = bordered(q["M"], 1e-3), bordered(q["K"], 1e-1), q["bdofs"]
+    s = MultiBlockSystem(M, K, n_t=q["n_t"], beta=q["beta"], CN=CN, time_interval=q["time_interval"], bc_dofs=bd)
+    assert s.N <= 64                                       # the narrow kernels (one block of ld <= 64 columns)
+    x0 = rng.standard_normal((s.N, s.n))
+    x1 = rng.standard_normal((s.N, s.n))
+    y0, y1 = kkt.kkt_apply_fused(M, K, s.tau, q["beta"], q["n_t"], CN, bd, x0, x1)
+    g0, g1 = s.to_host_blocks(s.apply(s.to_device(x0, x1)))
+    err = max(np.abs(g0 - y0).max(), np.abs(g1 - y1).max()) / max(np.abs(y0).max(), np.abs(y1).max())
+    assert err < 1e-13, err
+    s.close()
+
 def test_no_constrained_dofs():
     q = kat.heat_problem(8, 5, True, beta=1e-2)
     q["bdofs"] = np.zeros(0, dtype=np.int32)
