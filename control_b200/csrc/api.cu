@@ -5,6 +5,7 @@
 #include <cstring>
 
 #include "common.cuh"
+#include "vec_ops.cuh"
 
 static thread_local std::string g_create_error;
 
@@ -39,22 +40,6 @@ template int ctl_upload<int>(ctl_handle_s *, int **, const int *, size_t);
 template int ctl_upload<double>(ctl_handle_s *, double **, const double *, size_t);
 template int ctl_upload<uint8_t>(ctl_handle_s *, uint8_t **, const uint8_t *, size_t);
 
-int ctl_scratch_get(ctl_handle_s *h, double **out)
-{
-    if (!h->pool.empty()) {
-        *out = h->pool.back();
-        h->pool.pop_back();
-        return CTL_OK;
-    }
-    CTL_CUDA(cudaMalloc((void **)out, (size_t)std::max<int64_t>(h->vec_len(), 1) * sizeof(double)));
-    return CTL_OK;
-}
-
-void ctl_scratch_put(ctl_handle_s *h, double *p)
-{
-    if (p) h->pool.push_back(p);
-}
-
 extern "C" {
 
 const char *ctl_version(void) { return "ctl_b200 0.1 (sm_100a)"; }
@@ -88,6 +73,7 @@ int ctl_create(const ctl_config *cfg, ctl_handle *out)
     h->ld = ld;
     h->n = cfg->n;
     split_ownership(cfg->n, cfg->world, cfg->rank, &h->row_begin, &h->n_loc);
+    h->pool.init(h, std::max<int64_t>(h->vec_len(), 1));
     if (cfg->stream) {
         h->stream = (cudaStream_t)cfg->stream;
     } else {
@@ -110,10 +96,8 @@ int ctl_destroy(ctl_handle h)
     cudaSetDevice(h->cfg.device);
     cudaStreamSynchronize(h->stream);
     ctl_pc_free(h);
-    ctl_krylov_free(h);
     ctl_comm_free(h);
     ctl_lift_invalidate(h);
-    for (double *p : h->pool) cudaFree(p);
     cudaFree(h->d_indptr);
     cudaFree(h->d_indices);
     cudaFree(h->d_M);
@@ -386,33 +370,23 @@ int ctl_kkt_apply(ctl_handle h, const double *x, double *y, int layout)
     CTL_CHECK(h && x && y, CTL_ERR_ARG, "ctl_kkt_apply: null argument");
     CTL_CUDA(cudaSetDevice(h->cfg.device));
     if (layout == CTL_LAYOUT_TIME_FASTEST) return ctl_kkt_apply_tf(h, x, y);
-    double *xt = nullptr, *yt = nullptr;
-    CTL_TRY(ctl_scratch_get(h, &xt));
-    CTL_TRY(ctl_scratch_get(h, &yt));
-    int rc = ctl_to_tf(h, x, xt);
-    if (rc == CTL_OK) rc = ctl_kkt_apply_tf(h, xt, yt);
-    if (rc == CTL_OK) rc = ctl_to_bm(h, yt, y);
-    ctl_scratch_put(h, xt);
-    ctl_scratch_put(h, yt);
-    return rc;
+    return with_tf(h, layout, {x, nullptr}, y,
+                   [&](const double *xt, double *yt) { return ctl_kkt_apply_tf(h, xt, yt); });
 }
 
 int ctl_time_kkt_apply(ctl_handle h, const double *x_tf, double *y_tf, int reps, float *ms)
 {
     CTL_CHECK(h && x_tf && y_tf && ms && reps > 0, CTL_ERR_ARG, "ctl_time_kkt_apply: bad argument");
     CTL_CUDA(cudaSetDevice(h->cfg.device));
-    cudaEvent_t e0, e1;
-    CTL_CUDA(cudaEventCreate(&e0));
-    CTL_CUDA(cudaEventCreate(&e1));
-    CTL_CUDA(cudaEventRecord(e0, h->stream));
+    EventPair ev;
+    CTL_TRY(ev.create(h));
+    CTL_CUDA(cudaEventRecord(ev.begin, h->stream));
     int rc = CTL_OK;
     for (int i = 0; i < reps && rc == CTL_OK; ++i) rc = ctl_kkt_apply_tf(h, x_tf, y_tf);
-    CTL_CUDA(cudaEventRecord(e1, h->stream));
-    CTL_CUDA(cudaEventSynchronize(e1));
+    CTL_CUDA(cudaEventRecord(ev.end, h->stream));
+    CTL_CUDA(cudaEventSynchronize(ev.end));
     float t = 0;
-    CTL_CUDA(cudaEventElapsedTime(&t, e0, e1));
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
+    CTL_CUDA(cudaEventElapsedTime(&t, ev.begin, ev.end));
     *ms = t / reps;
     return rc;
 }

@@ -3,9 +3,11 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <array>
 #include <cstdio>
 #include <memory>
 #include <string>
+#include <tuple>
 #include <vector>
 
 #include "../../include/ctl_b200.h"
@@ -45,6 +47,113 @@ struct HostCSR {
     std::vector<double> values;
     int64_t nnz() const { return (int64_t)indices.size(); }
 };
+
+// ---------------------------------------------------------------- scoped device resources
+// Each type below releases what it holds when it goes out of scope.  Outside this header no code destroys an event
+// or touches a pool's free list (tests/test_source_rules.py).
+class Scratch;
+
+// Device vectors of one fixed length, reused last in, first out, and freed with the pool
+class ScratchPool {
+  public:
+    ScratchPool() = default;
+    ScratchPool(const ScratchPool &) = delete;
+    ScratchPool &operator=(const ScratchPool &) = delete;
+    ~ScratchPool()
+    {
+        for (double *p : free_) cudaFree(p);
+    }
+    void init(ctl_handle_s *h, int64_t len)   // h takes the error text of a failed allocation
+    {
+        h_ = h;
+        len_ = len;
+    }
+    int take(Scratch *out);                   // *out (empty) holds one vector until it goes out of scope
+
+  private:
+    friend class Scratch;
+    ctl_handle_s *h_ = nullptr;
+    int64_t len_ = 0;
+    std::vector<double *> free_;
+};
+
+// The lease of one vector of a ScratchPool: converts to the vector and gives it back when it goes out of scope
+class Scratch {
+  public:
+    Scratch() = default;
+    Scratch(Scratch &&o) noexcept : pool_(o.pool_), p_(o.p_) { o.p_ = nullptr; }
+    ~Scratch()
+    {
+        if (p_) pool_->free_.push_back(p_);
+    }
+    operator double *() const { return p_; }
+
+  private:
+    friend class ScratchPool;
+    ScratchPool *pool_ = nullptr;
+    double *p_ = nullptr;
+};
+
+inline int ScratchPool::take(Scratch *out)
+{
+    ctl_handle_s *h = h_;
+    if (free_.empty()) {
+        double *p = nullptr;
+        CTL_CUDA(cudaMalloc((void **)&p, (size_t)len_ * sizeof(double)));
+        free_.push_back(p);
+    }
+    out->pool_ = this;
+    out->p_ = free_.back();
+    free_.pop_back();
+    return CTL_OK;
+}
+
+// Two events around a timed region, destroyed with the pair
+struct EventPair {
+    cudaEvent_t begin = nullptr, end = nullptr;
+    EventPair() = default;
+    EventPair(EventPair &&o) noexcept : begin(o.begin), end(o.end) { o.begin = o.end = nullptr; }
+    ~EventPair()
+    {
+        if (begin) cudaEventDestroy(begin);
+        if (end) cudaEventDestroy(end);
+    }
+    int create(ctl_handle_s *h)
+    {
+        CTL_CUDA(cudaEventCreate(&begin));
+        CTL_CUDA(cudaEventCreate(&end));
+        return CTL_OK;
+    }
+};
+
+// A device array for the temporaries of one call, freed when it goes out of scope
+template <typename T>
+struct DeviceArray {
+    T *p = nullptr;
+    DeviceArray() = default;
+    DeviceArray(const DeviceArray &) = delete;
+    DeviceArray &operator=(const DeviceArray &) = delete;
+    ~DeviceArray() { cudaFree(p); }
+    cudaError_t alloc(size_t count) { return cudaMalloc((void **)&p, count * sizeof(T)); }
+    operator T *() const { return p; }
+};
+
+// Runs fn on internal-layout copies of an entry point's device vectors, one vector of `pool` each: fn's i-th
+// argument holds to_internal(in[i]) (nothing for a null in[i]), and when fn succeeds the last one is written to `out`
+// (if set) with to_caller.  Each system passes its own layout conversions.
+template <size_t K, class In, class Out, class F>
+int with_internal(ScratchPool &pool, const double *const (&in)[K], double *out, In to_internal, Out to_caller, F fn)
+{
+    Scratch t[K];
+    for (Scratch &s : t) CTL_TRY(pool.take(&s));
+    std::array<double *, K> p;
+    for (size_t i = 0; i < K; ++i) {
+        p[i] = t[i];
+        if (in[i]) CTL_TRY(to_internal(in[i], p[i]));
+    }
+    CTL_TRY(std::apply(fn, p));
+    return out ? to_caller(p[K - 1], out) : CTL_OK;
+}
 
 // ---------------------------------------------------------------- the handle
 struct ctl_handle_s {
@@ -95,8 +204,8 @@ struct ctl_handle_s {
     // reduction workspace (vec_ops.cu)
     double *d_red = nullptr, *h_red = nullptr;
 
-    // scratch vectors (time-fastest, 2 * n_loc * ld doubles each)
-    std::vector<double *> pool;
+    // scratch vectors (time-fastest, 2 * n_loc * ld doubles each, at least one)
+    ScratchPool pool;
 
     // preconditioner, Krylov workspace, communicator: defined in their own units
     std::shared_ptr<struct PcState> pc;
@@ -125,7 +234,6 @@ int ctl_solve_tf(ctl_handle_s *h, const double *b_tf, double *u_tf, const ctl_kr
 
 // unit-private state teardown / invalidation
 void ctl_pc_free(ctl_handle_s *h);        // pc.cu
-void ctl_krylov_free(ctl_handle_s *h);    // krylov.cu
 void ctl_comm_free(ctl_handle_s *h);      // comm.cu
 int ctl_pc_invalidate(ctl_handle_s *h);   // pc.cu: matrices changed, rebuild on next setup
 void ctl_lift_invalidate(ctl_handle_s *h);   // lift.cu: M, K or the Dirichlet dofs changed
@@ -139,10 +247,6 @@ int ctl_halo_exchange(ctl_handle_s *h, const double *x_tf);            // both p
 int ctl_halo_exchange_panel(ctl_handle_s *h, const double *panel_tf);  // one panel -> d_halo[0]
 int ctl_allreduce_sum(ctl_handle_s *h, double *dev, int count);
 int ctl_comm_check(ctl_handle_s *h);                                   // peer-to-peer exchange timed out?
-
-// scratch management
-int ctl_scratch_get(ctl_handle_s *h, double **out);            // one full vector
-void ctl_scratch_put(ctl_handle_s *h, double *p);
 
 template <typename T>
 int ctl_upload(ctl_handle_s *h, T **dst, const T *src, size_t count);

@@ -11,63 +11,17 @@
 
 #include "krylov.cuh"
 
-void ctl_krylov_free(ctl_handle_s *h)
-{
-    if (!h->ks) return;
-    for (double *p : h->ks->basis) cudaFree(p);
-    for (cudaEvent_t e : h->ks->events) cudaEventDestroy(e);
-    h->ks.reset();
-}
-
-namespace {
-struct HeatSolver : Solver {
-    using Solver::Solver;
-    ~HeatSolver() override { release(); }
-};
-}  // namespace
-
 int ctl_solve_tf(ctl_handle_s *h, const double *b_tf, double *u_tf, const ctl_krylov_options *opts,
                     ctl_solve_result *result)
 {
     if (!h->ks) h->ks = std::make_shared<KrylovState>();
-    h->ks->next_event = 0;
-    h->ks->spans.clear();
-    memset(result, 0, sizeof(*result));
     CTL_CHECK(opts->ksp_type >= CTL_KSP_GMRES && opts->ksp_type <= CTL_KSP_MINRES, CTL_ERR_ARG,
               "ctl_solve: unknown ksp_type");
     CTL_CHECK(opts->pc >= CTL_PC_NONE && opts->pc <= CTL_PC_CALLBACK, CTL_ERR_ARG, "ctl_solve: unknown pc kind");
     if (opts->pc == CTL_PC_BUILTIN)
         CTL_CHECK(h->pc && h->pc->ready, CTL_ERR_STATE, "ctl_solve: call ctl_pc_setup first");
-    cudaEvent_t e0, e1;
-    CTL_CUDA(cudaEventCreate(&e0));
-    CTL_CUDA(cudaEventCreate(&e1));
-    CTL_CUDA(cudaEventRecord(e0, h->stream));
-    int rc;
-    {
-        HeatSolver S(h, *opts, *result, *h->ks, h->vec_len());
-        double *b = nullptr;
-        rc = S.get(&b);
-        // correct_soln / correct_rhs (preconditioner/preconditioner.py:658-704)
-        if (rc == CTL_OK) rc = vec_copy(h, b, b_tf, S.len);
-        if (rc == CTL_OK) rc = S.project(b, nullptr);
-        if (rc == CTL_OK) rc = S.project(u_tf, nullptr);
-        if (rc == CTL_OK) rc = (opts->ksp_type == CTL_KSP_MINRES) ? S.minres(b, u_tf) : S.gmres(b, u_tf);
-        if (rc == CTL_OK) rc = S.project(u_tf, nullptr);                   // 761-766
-        if (rc == CTL_OK) rc = ctl_comm_check(h);
-    }
-    cudaEventRecord(e1, h->stream);
-    cudaEventSynchronize(e1);
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, e0, e1);
-    result->seconds_total = ms * 1e-3;
-    for (auto &sp : h->ks->spans) {
-        float t = 0.f;
-        if (cudaEventElapsedTime(&t, h->ks->events[sp.first], h->ks->events[sp.first + 1]) == cudaSuccess)
-            (sp.second == 0 ? result->seconds_mult : result->seconds_pc) += t * 1e-3;
-    }
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
-    return rc;
+    Solver K(h, *opts, *result, *h->ks, h->pool, h->vec_len(), "ctl_solve", h->pc_cb, h->pc_cb_user);
+    return krylov_solve(K, b_tf, u_tf);
 }
 
 extern "C" {
@@ -92,16 +46,8 @@ int ctl_solve(ctl_handle h, const double *b, double *u, int layout, const ctl_kr
     CTL_CHECK(h->assembled, CTL_ERR_STATE, "ctl_solve: ctl_assemble has not been called");
     CTL_CUDA(cudaSetDevice(h->cfg.device));
     if (layout == CTL_LAYOUT_TIME_FASTEST) return ctl_solve_tf(h, b, u, opts, result);
-    double *bt = nullptr, *ut = nullptr;
-    CTL_TRY(ctl_scratch_get(h, &bt));
-    CTL_TRY(ctl_scratch_get(h, &ut));
-    int rc = ctl_to_tf(h, b, bt);
-    if (rc == CTL_OK) rc = ctl_to_tf(h, u, ut);
-    if (rc == CTL_OK) rc = ctl_solve_tf(h, bt, ut, opts, result);
-    if (rc == CTL_OK) rc = ctl_to_bm(h, ut, u);
-    ctl_scratch_put(h, bt);
-    ctl_scratch_put(h, ut);
-    return rc;
+    return with_tf(h, layout, {b, u}, u,
+                   [&](const double *bt, double *ut) { return ctl_solve_tf(h, bt, ut, opts, result); });
 }
 
 int ctl_solve_host(ctl_handle h, const double *b_host, double *u_host, const ctl_krylov_options *opts,
@@ -110,26 +56,21 @@ int ctl_solve_host(ctl_handle h, const double *b_host, double *u_host, const ctl
     CTL_CHECK(h && b_host && u_host && opts && result, CTL_ERR_ARG, "ctl_solve_host: null argument");
     CTL_CUDA(cudaSetDevice(h->cfg.device));
     const size_t bytes = (size_t)ctl_vec_len(h, CTL_LAYOUT_BLOCK_MAJOR) * sizeof(double);
-    double *b = nullptr, *u = nullptr;     // scratch vectors are at least block-major sized
-    CTL_TRY(ctl_scratch_get(h, &b));
-    CTL_TRY(ctl_scratch_get(h, &u));
-    int rc = CTL_OK;
+    Scratch b, u;     // scratch vectors are at least block-major sized
+    CTL_TRY(h->pool.take(&b));
+    CTL_TRY(h->pool.take(&u));
     if (cudaMemcpyAsync(b, b_host, bytes, cudaMemcpyHostToDevice, h->stream) != cudaSuccess ||
         cudaMemcpyAsync(u, u_host, bytes, cudaMemcpyHostToDevice, h->stream) != cudaSuccess) {
         ctl_set_error(h, "ctl_solve_host: host to device copy failed");
-        rc = CTL_ERR_CUDA;
+        return CTL_ERR_CUDA;
     }
-    if (rc == CTL_OK) rc = ctl_solve(h, b, u, CTL_LAYOUT_BLOCK_MAJOR, opts, result);
-    if (rc == CTL_OK) {
-        if (cudaMemcpyAsync(u_host, u, bytes, cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
-            cudaStreamSynchronize(h->stream) != cudaSuccess) {
-            ctl_set_error(h, "ctl_solve_host: device to host copy failed");
-            rc = CTL_ERR_CUDA;
-        }
+    CTL_TRY(ctl_solve(h, b, u, CTL_LAYOUT_BLOCK_MAJOR, opts, result));
+    if (cudaMemcpyAsync(u_host, u, bytes, cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
+        cudaStreamSynchronize(h->stream) != cudaSuccess) {
+        ctl_set_error(h, "ctl_solve_host: device to host copy failed");
+        return CTL_ERR_CUDA;
     }
-    ctl_scratch_put(h, b);
-    ctl_scratch_put(h, u);
-    return rc;
+    return CTL_OK;
 }
 
 int ctl_kkt_residual_norm(ctl_handle h, const double *b, const double *x, int layout, double *out)
@@ -137,31 +78,17 @@ int ctl_kkt_residual_norm(ctl_handle h, const double *b, const double *x, int la
     CTL_CHECK(h && b && x && out, CTL_ERR_ARG, "ctl_kkt_residual_norm: null argument");
     CTL_CHECK(h->assembled, CTL_ERR_STATE, "ctl_kkt_residual_norm: ctl_assemble has not been called");
     CTL_CUDA(cudaSetDevice(h->cfg.device));
-    double *bt = nullptr, *xt = nullptr, *r = nullptr;
-    CTL_TRY(ctl_scratch_get(h, &bt));
-    CTL_TRY(ctl_scratch_get(h, &xt));
-    CTL_TRY(ctl_scratch_get(h, &r));
     const int64_t len = h->vec_len();
-    int rc;
-    if (layout == CTL_LAYOUT_TIME_FASTEST) {
-        rc = vec_copy(h, bt, b, len);
-        if (rc == CTL_OK) rc = vec_copy(h, xt, x, len);
-    } else {
-        rc = ctl_to_tf(h, b, bt);
-        if (rc == CTL_OK) rc = ctl_to_tf(h, x, xt);
-    }
-    if (rc == CTL_OK && h->d_bc_rows_all) {
-        const size_t panel = (size_t)h->n_loc * h->ld;
-        rc = pcb_bc_fixup(h, h->d_bc_rows_all, h->n_bc_all, nullptr, bt);
-        if (rc == CTL_OK) rc = pcb_bc_fixup(h, h->d_bc_rows_all, h->n_bc_all, nullptr, bt + panel);
-    }
-    if (rc == CTL_OK) rc = ctl_kkt_apply_tf(h, xt, r);
-    if (rc == CTL_OK) rc = vec_lincomb(h, r, 1.0, bt, -1.0, r, 0.0, nullptr, nullptr, len);
-    if (rc == CTL_OK) rc = vec_norm_host(h, r, len, out);
-    ctl_scratch_put(h, bt);
-    ctl_scratch_put(h, xt);
-    ctl_scratch_put(h, r);
-    return rc;
+    return with_tf(h, layout, {b, x, nullptr}, nullptr, [&](double *bt, const double *xt, double *r) {
+        if (h->d_bc_rows_all) {
+            const size_t panel = (size_t)h->n_loc * h->ld;
+            CTL_TRY(pcb_bc_fixup(h, h->d_bc_rows_all, h->n_bc_all, nullptr, bt));
+            CTL_TRY(pcb_bc_fixup(h, h->d_bc_rows_all, h->n_bc_all, nullptr, bt + panel));
+        }
+        CTL_TRY(ctl_kkt_apply_tf(h, xt, r));
+        CTL_TRY(vec_lincomb(h, r, 1.0, bt, -1.0, r, 0.0, nullptr, nullptr, len));
+        return vec_norm_host(h, r, len, out);
+    });
 }
 
 // Residual of the outer Picard / Gauss-Newton loop on device vectors.  non_linear_res_eval (control/control.py:
@@ -175,36 +102,22 @@ int ctl_nonlinear_residual(ctl_handle h, const double *b, const double *x, doubl
     CTL_CHECK(h && b && x && r_out && norm_host, CTL_ERR_ARG, "ctl_nonlinear_residual: null argument");
     CTL_CHECK(h->assembled, CTL_ERR_STATE, "ctl_nonlinear_residual: ctl_assemble has not been called");
     CTL_CUDA(cudaSetDevice(h->cfg.device));
-    double *bt = nullptr, *xt = nullptr, *r = nullptr;
-    CTL_TRY(ctl_scratch_get(h, &bt));
-    CTL_TRY(ctl_scratch_get(h, &xt));
-    CTL_TRY(ctl_scratch_get(h, &r));
     const int64_t len = h->vec_len();
     const size_t panel = (size_t)h->n_loc * h->ld;
-    int rc;
-    if (layout == CTL_LAYOUT_TIME_FASTEST) {
-        rc = vec_copy(h, bt, b, len);
-        if (rc == CTL_OK) rc = vec_copy(h, xt, x, len);
-    } else {
-        rc = ctl_to_tf(h, b, bt);
-        if (rc == CTL_OK) rc = ctl_to_tf(h, x, xt);
-    }
-    if (rc == CTL_OK) rc = ctl_kkt_apply_tf(h, xt, r);
-    if (rc == CTL_OK) rc = vec_lincomb(h, r, 1.0, bt, -1.0, r, 0.0, nullptr, nullptr, len);
-    if (rc == CTL_OK && h->d_bc_rows_all) {      // rows of constrained dofs carry no residual (2816-2817)
-        rc = pcb_bc_fixup(h, h->d_bc_rows_all, h->n_bc_all, nullptr, r);
-        if (rc == CTL_OK) rc = pcb_bc_fixup(h, h->d_bc_rows_all, h->n_bc_all, nullptr, r + panel);
-    }
-    if (rc == CTL_OK) rc = (layout == CTL_LAYOUT_TIME_FASTEST) ? vec_copy(h, r_out, r, len) : ctl_to_bm(h, r, r_out);
-    if (rc == CTL_OK && h->cfg.CN) {
-        rc = ctl_panel_tinv(h, r, 1, h->n_loc);
-        if (rc == CTL_OK) rc = ctl_panel_tinv(h, r + panel, 2, h->n_loc);
-    }
-    if (rc == CTL_OK) rc = vec_norm_host(h, r, len, norm_host);
-    ctl_scratch_put(h, bt);
-    ctl_scratch_put(h, xt);
-    ctl_scratch_put(h, r);
-    return rc;
+    return with_tf(h, layout, {b, x, nullptr}, nullptr, [&](const double *bt, const double *xt, double *r) {
+        CTL_TRY(ctl_kkt_apply_tf(h, xt, r));
+        CTL_TRY(vec_lincomb(h, r, 1.0, bt, -1.0, r, 0.0, nullptr, nullptr, len));
+        if (h->d_bc_rows_all) {      // rows of constrained dofs carry no residual (2816-2817)
+            CTL_TRY(pcb_bc_fixup(h, h->d_bc_rows_all, h->n_bc_all, nullptr, r));
+            CTL_TRY(pcb_bc_fixup(h, h->d_bc_rows_all, h->n_bc_all, nullptr, r + panel));
+        }
+        CTL_TRY((layout == CTL_LAYOUT_TIME_FASTEST) ? vec_copy(h, r_out, r, len) : ctl_to_bm(h, r, r_out));
+        if (h->cfg.CN) {
+            CTL_TRY(ctl_panel_tinv(h, r, 1, h->n_loc));
+            CTL_TRY(ctl_panel_tinv(h, r + panel, 2, h->n_loc));
+        }
+        return vec_norm_host(h, r, len, norm_host);
+    });
 }
 
 // J_h (SURVEY.md section 8c), evaluated on the host from the mass matrix the caller handed over

@@ -11,9 +11,16 @@
 
 struct KrylovState {
     std::vector<double *> basis;      // V_0..V_m then Z_0..Z_{m-1}
-    std::vector<cudaEvent_t> events;
+    std::vector<EventPair> events;    // one pair per timed operator / pc application of a solve
     size_t next_event = 0;
-    std::vector<std::pair<size_t, int>> spans;   // (event index, 0 = mult / 1 = pc)
+    std::vector<std::pair<size_t, int>> spans;   // (event pair, 0 = mult / 1 = pc)
+    KrylovState() = default;
+    KrylovState(const KrylovState &) = delete;
+    KrylovState &operator=(const KrylovState &) = delete;
+    ~KrylovState()
+    {
+        for (double *p : basis) cudaFree(p);
+    }
 };
 
 namespace {
@@ -36,52 +43,41 @@ struct Solver {
     const ctl_krylov_options &o;
     ctl_solve_result &res;
     KrylovState &ks;
+    ScratchPool &pool;          // vectors of length len
     int64_t len;
-    std::vector<double *> scratch;
+    const char *name;           // entry point, for the error messages
+    ctl_pc_callback cb;         // pc = CTL_PC_CALLBACK: the user's pc_fn on block-major vectors
+    void *cb_user;
 
     // h carries the stream, the reduction workspace and the error string; the linear system
     // itself is behind the virtual hooks (defaults: the heat-type KKT system of the handle)
-    Solver(ctl_handle_s *h_, const ctl_krylov_options &o_, ctl_solve_result &r_, KrylovState &ks_, int64_t len_)
-        : h(h_), o(o_), res(r_), ks(ks_), len(len_) {}
+    Solver(ctl_handle_s *h_, const ctl_krylov_options &o_, ctl_solve_result &r_, KrylovState &ks_, ScratchPool &pool_,
+           int64_t len_, const char *name_, ctl_pc_callback cb_, void *cb_user_)
+        : h(h_), o(o_), res(r_), ks(ks_), pool(pool_), len(len_), name(name_), cb(cb_), cb_user(cb_user_) {}
 
     virtual ~Solver() {}
 
-    void release()           // derived classes call this from their destructor (virtual put)
-    {
-        for (double *p : scratch) put_vec(p);
-        scratch.clear();
-    }
-
-    virtual int get_vec(double **p) { return ctl_scratch_get(h, p); }
-    virtual void put_vec(double *p) { ctl_scratch_put(h, p); }
     virtual int apply_operator(const double *x, double *y) { return ctl_kkt_apply_tf(h, x, y); }
     virtual int apply_builtin_pc(const double *x, double *y) { return ctl_pc_apply_tf(h, x, y); }
-
-    int get(double **p)
-    {
-        CTL_TRY(get_vec(p));
-        scratch.push_back(*p);
-        return CTL_OK;
-    }
+    virtual int to_bm(const double *tf, double *bm) { return ctl_to_bm(h, tf, bm); }
+    virtual int to_tf(const double *bm, double *tf) { return ctl_to_tf(h, bm, tf); }
 
     int span_begin(int kind)
     {
-        if (ks.next_event + 2 > ks.events.size()) {
-            cudaEvent_t a, b;
-            CTL_CUDA(cudaEventCreate(&a));
-            CTL_CUDA(cudaEventCreate(&b));
-            ks.events.push_back(a);
-            ks.events.push_back(b);
+        if (ks.next_event == ks.events.size()) {
+            EventPair e;
+            CTL_TRY(e.create(h));
+            ks.events.push_back(std::move(e));
         }
         ks.spans.emplace_back(ks.next_event, kind);
-        CTL_CUDA(cudaEventRecord(ks.events[ks.next_event], h->stream));
+        CTL_CUDA(cudaEventRecord(ks.events[ks.next_event].begin, h->stream));
         return CTL_OK;
     }
 
     int span_end()
     {
-        CTL_CUDA(cudaEventRecord(ks.events[ks.next_event + 1], h->stream));
-        ks.next_event += 2;
+        CTL_CUDA(cudaEventRecord(ks.events[ks.next_event].end, h->stream));
+        ks.next_event++;
         return CTL_OK;
     }
 
@@ -108,32 +104,24 @@ struct Solver {
         return span_end();
     }
 
-    virtual int apply_callback_pc(const double *x, double *y)
+    // Preconditioner.apply around a user pc_fn (preconditioner/preconditioner.py:562-656): project the right-hand
+    // side, hand block-major device vectors of the system to the callback, restore the constrained entries
+    int apply_callback_pc(const double *x, double *y)
     {
-        {
-            CTL_CHECK(h->pc_cb, CTL_ERR_STATE, "ctl_solve: no preconditioner callback installed");
-            double *bm_b = nullptr, *bm_u = nullptr, *xc = nullptr;
-            CTL_TRY(ctl_scratch_get(h, &bm_b));
-            CTL_TRY(ctl_scratch_get(h, &bm_u));
-            CTL_TRY(ctl_scratch_get(h, &xc));
-            int rc = vec_copy(h, xc, x, len);
-            if (rc == CTL_OK) rc = project(xc, nullptr);                  // pc_pre_mult_corrected
-            if (rc == CTL_OK) rc = ctl_to_bm(h, xc, bm_b);
-            if (rc == CTL_OK) rc = vec_zero(h, bm_u, len);
-            if (rc == CTL_OK) {
-                cudaStreamSynchronize(h->stream);
-                if (h->pc_cb(h->pc_cb_user, bm_b, bm_u) != 0) {
-                    ctl_set_error(h, "preconditioner callback failed");
-                    rc = CTL_ERR_CALLBACK;
-                }
-            }
-            if (rc == CTL_OK) rc = ctl_to_tf(h, bm_u, y);
-            if (rc == CTL_OK) rc = project(y, x);                         // pc_post_mult_correct
-            ctl_scratch_put(h, bm_b);
-            ctl_scratch_put(h, bm_u);
-            ctl_scratch_put(h, xc);
-            return rc;
+        CTL_CHECK(cb, CTL_ERR_STATE, std::string(name) + ": no preconditioner callback installed");
+        Scratch bm_b, bm_u, xc;
+        for (Scratch *s : {&bm_b, &bm_u, &xc}) CTL_TRY(pool.take(s));
+        CTL_TRY(vec_copy(h, xc, x, len));
+        CTL_TRY(project(xc, nullptr));                  // pc_pre_mult_corrected
+        CTL_TRY(to_bm(xc, bm_b));
+        CTL_TRY(vec_zero(h, bm_u, len));
+        cudaStreamSynchronize(h->stream);
+        if (cb(cb_user, bm_b, bm_u) != 0) {
+            ctl_set_error(h, "preconditioner callback failed");
+            return CTL_ERR_CALLBACK;
         }
+        CTL_TRY(to_tf(bm_u, y));
+        return project(y, x);                           // pc_post_mult_correct
     }
 
     // constrained rows of both panels: v = wrap ? wrap : 0
@@ -173,8 +161,8 @@ struct Solver {
         CTL_TRY(ensure_basis((size_t)(m + 1) + (flexible ? m : 0)));
         double **V = ks.basis.data();
         double **Z = ks.basis.data() + (m + 1);
-        double *t = nullptr;
-        CTL_TRY(get(&t));
+        Scratch t;
+        CTL_TRY(pool.take(&t));
         double *partials, *scal;
         CTL_TRY(vec_workspace(h, &partials, &scal));
         double ref = 0.0;
@@ -267,8 +255,9 @@ struct Solver {
 
     int minres(const double *b, double *x)
     {
-        double *r1, *r2, *y, *v, *w, *w1, *w2;
-        for (double **p : {&r1, &r2, &y, &v, &w, &w1, &w2}) CTL_TRY(get(p));
+        Scratch vecs[7];
+        for (Scratch &s : vecs) CTL_TRY(pool.take(&s));
+        double *r1 = vecs[0], *r2 = vecs[1], *y = vecs[2], *v = vecs[3], *w = vecs[4], *w1 = vecs[5], *w2 = vecs[6];
         CTL_TRY(prec(b, y));
         double bb = 0.0;
         CTL_TRY(dot(b, y, &bb));
@@ -345,5 +334,42 @@ struct Solver {
         return CTL_OK;
     }
 };
+
+// MultiBlockSystem.solve of K's system on internal-layout vectors (u: initial guess in, solution out), timed with
+// device events: the whole solve into seconds_total, each operator / pc application into seconds_mult / seconds_pc
+int krylov_solve(Solver &K, const double *b_in, double *u)
+{
+    ctl_handle_s *h = K.h;
+    ctl_solve_result &res = K.res;
+    K.ks.next_event = 0;
+    K.ks.spans.clear();
+    memset(&res, 0, sizeof(res));
+    EventPair ev;
+    CTL_TRY(ev.create(h));
+    CTL_CUDA(cudaEventRecord(ev.begin, h->stream));
+    int rc;
+    {
+        Scratch b;
+        rc = K.pool.take(&b);
+        // correct_soln / correct_rhs (preconditioner/preconditioner.py:658-704)
+        if (rc == CTL_OK) rc = vec_copy(h, b, b_in, K.len);
+        if (rc == CTL_OK) rc = K.project(b, nullptr);
+        if (rc == CTL_OK) rc = K.project(u, nullptr);
+        if (rc == CTL_OK) rc = (K.o.ksp_type == CTL_KSP_MINRES) ? K.minres(b, u) : K.gmres(b, u);
+        if (rc == CTL_OK) rc = K.project(u, nullptr);                   // 761-766
+        if (rc == CTL_OK) rc = ctl_comm_check(h);
+    }
+    cudaEventRecord(ev.end, h->stream);
+    cudaEventSynchronize(ev.end);
+    float ms = 0.f;
+    cudaEventElapsedTime(&ms, ev.begin, ev.end);
+    res.seconds_total = ms * 1e-3;
+    for (auto &sp : K.ks.spans) {
+        float t = 0.f;
+        if (cudaEventElapsedTime(&t, K.ks.events[sp.first].begin, K.ks.events[sp.first].end) == cudaSuccess)
+            (sp.second == 0 ? res.seconds_mult : res.seconds_pc) += t * 1e-3;
+    }
+    return rc;
+}
 
 }  // namespace

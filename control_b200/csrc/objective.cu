@@ -98,24 +98,21 @@ static int extend_levels(ctl_handle_s *h, const double *x_loc, int L, double *ex
     CTL_CUDA(cudaMemcpy2DAsync(ext, (size_t)stride * sizeof(double), x_loc, (size_t)nl * sizeof(double),
                                (size_t)nl * sizeof(double), (size_t)L, cudaMemcpyDeviceToDevice, h->stream));
     if (nh == 0) return CTL_OK;
-    double *panel = nullptr;
-    CTL_TRY(ctl_scratch_get(h, &panel));
-    int rc = CTL_OK;
-    for (int l0 = 0; l0 < L && rc == CTL_OK; l0 += ld) {
+    Scratch panel;
+    CTL_TRY(h->pool.take(&panel));
+    for (int l0 = 0; l0 < L; l0 += ld) {
         const int cnt = std::min(ld, L - l0);
         levels_to_panel_kernel<<<ceil_div((int64_t)nl * ld, 256), 256, 0, h->stream>>>(x_loc, l0, cnt, nl, ld, panel);
         h->launches++;
-        rc = ctl_halo_exchange_panel(h, panel);
-        if (rc != CTL_OK) break;
+        CTL_TRY(ctl_halo_exchange_panel(h, panel));
         halo_to_levels_kernel<<<ceil_div((int64_t)nh * cnt, 256), 256, 0, h->stream>>>(h->d_halo, l0, cnt, nh, ld, nl, stride, ext);
         h->launches++;
         if (cudaGetLastError() != cudaSuccess) {
             ctl_set_error(h, "extend_levels: CUDA failure");
-            rc = CTL_ERR_CUDA;
+            return CTL_ERR_CUDA;
         }
     }
-    ctl_scratch_put(h, panel);
-    return rc;
+    return CTL_OK;
 }
 
 extern "C" int ctl_objective(ctl_handle h, const double *v, const double *zeta, const double *v_hat, double *out)
@@ -131,7 +128,7 @@ extern "C" int ctl_objective(ctl_handle h, const double *v, const double *zeta, 
         CTL_TRY(ctl_upload(h, &h->d_M_full, buf.data(), buf.size()));
     }
     const int blocks = ceil_div(n, QT);
-    double *partial = nullptr, *sums = nullptr, *ext = nullptr;
+    DeviceArray<double> partial, sums, ext;
     int rc = CTL_OK;
     cudaError_t e = cudaSuccess;
     std::vector<double> hs(2 * (size_t)n_t);
@@ -139,7 +136,7 @@ extern "C" int ctl_objective(ctl_handle h, const double *v, const double *zeta, 
         const double *pv = v, *pz = zeta, *ph = v_hat;
         if (h->n_halo > 0) {      // several ranks: ghost entries of the three arrays behind the owned ones
             const size_t one = (size_t)n_t * stride;
-            if ((e = cudaMalloc((void **)&ext, 3 * one * sizeof(double))) != cudaSuccess) break;
+            if ((e = ext.alloc(3 * one)) != cudaSuccess) break;
             if ((rc = extend_levels(h, v, n_t, ext)) != CTL_OK) break;
             if ((rc = extend_levels(h, zeta, n_t, ext + one)) != CTL_OK) break;
             if ((rc = extend_levels(h, v_hat, n_t, ext + 2 * one)) != CTL_OK) break;
@@ -147,8 +144,8 @@ extern "C" int ctl_objective(ctl_handle h, const double *v, const double *zeta, 
             pz = ext + one;
             ph = ext + 2 * one;
         }
-        if ((e = cudaMalloc((void **)&partial, sizeof(double) * 2 * (size_t)blocks * n_t)) != cudaSuccess) break;
-        if ((e = cudaMalloc((void **)&sums, sizeof(double) * 2 * n_t)) != cudaSuccess) break;
+        if ((e = partial.alloc(2 * (size_t)blocks * n_t)) != cudaSuccess) break;
+        if ((e = sums.alloc(2 * n_t)) != cudaSuccess) break;
         quadform_partial_kernel<<<dim3(blocks, n_t), QT, 0, h->stream>>>(h->d_indptr, h->d_indices, h->d_M_full, pv, pz, ph,
                                                                         partial, n, h->n_halo > 0 ? stride : n);
         quadform_finish_kernel<<<n_t, 32, 0, h->stream>>>(partial, sums, blocks);
@@ -157,9 +154,6 @@ extern "C" int ctl_objective(ctl_handle h, const double *v, const double *zeta, 
         e = cudaMemcpyAsync(hs.data(), sums, sizeof(double) * hs.size(), cudaMemcpyDeviceToHost, h->stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
     } while (0);
-    cudaFree(partial);
-    cudaFree(sums);
-    cudaFree(ext);
     if (e != cudaSuccess) {
         ctl_set_error(h, std::string("ctl_objective: ") + cudaGetErrorString(e));
         return CTL_ERR_CUDA;
@@ -242,27 +236,20 @@ extern "C" int ctl_build_rhs(ctl_handle h, const double *v_hat, const double *f_
         for (size_t p = 0; p < buf.size(); ++p) buf[p] = h->h_M[h->loc_entry[p]];
         CTL_TRY(ctl_upload(h, &h->d_M_full, buf.data(), buf.size()));
     }
-    double *ext = nullptr;
+    DeviceArray<double> ext;
     const double *pv = v_hat, *pf = f_nodal;
     if (h->n_halo > 0) {      // several ranks: this rank's rows of the nodal data + the ghost entries the products gather
         const size_t one = (size_t)n_t * stride;
-        CTL_CUDA(cudaMalloc((void **)&ext, 2 * one * sizeof(double)));
-        int rc0 = extend_levels(h, v_hat, n_t, ext);
-        if (rc0 == CTL_OK) rc0 = extend_levels(h, f_nodal, n_t, ext + one);
-        if (rc0 != CTL_OK) {
-            cudaFree(ext);
-            return rc0;
-        }
+        CTL_CUDA(ext.alloc(2 * one));
+        CTL_TRY(extend_levels(h, v_hat, n_t, ext));
+        CTL_TRY(extend_levels(h, f_nodal, n_t, ext + one));
         pv = ext;
         pf = ext + one;
     }
     const int blocks = ceil_div(n, QT);
     const size_t half = (size_t)N * n;
-    double *work = nullptr;                       // untransformed rows (CN) before T_1 / T_2
-    if (ctl_scratch_get(h, &work) != CTL_OK) {    // a scratch vector holds at least 2 N n doubles
-        cudaFree(ext);
-        return CTL_ERR_CUDA;
-    }
+    Scratch work;                           // untransformed rows (CN) before T_1 / T_2
+    CTL_TRY(h->pool.take(&work));           // a scratch vector holds at least 2 N n doubles
     double *r0 = cn ? work : b, *r1 = cn ? work + half : b + half;
     // M-weighted rows: CN h M (x_i + x_{i+1}), i < N;  BE tau M x_i, with b_0 row n_t - 1 = 0 and b_1 row 0 from v_0
     const double alpha = cn ? 0.5 * tau : tau;
@@ -297,8 +284,8 @@ extern "C" int ctl_build_rhs(ctl_handle h, const double *v_hat, const double *f_
                 c1[r] = -(tau * kv + mv);               // b_1[0]  = (tau K_0 + M) v_0
             }
         }
-        double *d_c = nullptr;
-        if (cudaMalloc((void **)&d_c, 2 * (size_t)n * sizeof(double)) != cudaSuccess) rc = CTL_ERR_CUDA;
+        DeviceArray<double> d_c;
+        if (d_c.alloc(2 * (size_t)n) != cudaSuccess) rc = CTL_ERR_CUDA;
         if (rc == CTL_OK) {
             cudaMemcpyAsync(d_c, c0.data(), (size_t)n * sizeof(double), cudaMemcpyHostToDevice, h->stream);
             cudaMemcpyAsync(d_c + n, c1.data(), (size_t)n * sizeof(double), cudaMemcpyHostToDevice, h->stream);
@@ -306,7 +293,6 @@ extern "C" int ctl_build_rhs(ctl_handle h, const double *v_hat, const double *f_
             block_sub_kernel<<<ceil_div(n, 256), 256, 0, h->stream>>>(r1, d_c + n, h->d_bcmask, n);
             h->launches += cn ? 2 : 1;
             cudaStreamSynchronize(h->stream);           // c0 / c1 are host temporaries
-            cudaFree(d_c);
         }
     }
     if (rc == CTL_OK && cn) {                           // b_0 = T_1 rows, b_1 = T_2 rows (3242-3243)
@@ -316,9 +302,7 @@ extern "C" int ctl_build_rhs(ctl_handle h, const double *v_hat, const double *f_
         h->launches += 2;
     }
     if (rc == CTL_OK && cudaGetLastError() != cudaSuccess) rc = CTL_ERR_CUDA;
-    if (rc == CTL_OK && ext && cudaStreamSynchronize(h->stream) != cudaSuccess) rc = CTL_ERR_CUDA;      // ext is freed below
+    if (rc == CTL_OK && ext && cudaStreamSynchronize(h->stream) != cudaSuccess) rc = CTL_ERR_CUDA;      // ext is freed on return
     if (rc != CTL_OK) ctl_set_error(h, "ctl_build_rhs: CUDA failure");
-    ctl_scratch_put(h, work);
-    cudaFree(ext);
     return rc;
 }

@@ -266,65 +266,55 @@ static int pc_fn_tf(ctl_handle_s *h, const double *b, double *u, bool wrap)
     double *u0 = u, *u1 = u + panel;
     const bool cn = h->cfg.CN != 0;
     const double tau = h->cfg.tau;
-    double *s1 = nullptr, *s2 = nullptr;
-    CTL_TRY(ctl_scratch_get(h, &s1));
-    CTL_TRY(ctl_scratch_get(h, &s2));
+    Scratch s1, s2;
+    CTL_TRY(h->pool.take(&s1));
+    CTL_TRY(h->pool.take(&s2));
     double *btil = s1, *pa = s1 + panel, *pb = s2, *rhs = s2 + panel;
-    int rc = CTL_OK;
-    do {
-        // ---- (1,1) block: control/control.py:1997-2014 (CN), 2193-2206 (BE)
-        const double *p_fin = nullptr;
-        if (st.opts.solver_0 == CTL_S0_CHEBYSHEV) {
-            double scale;
-            std::vector<double> om;
-            cheb_coefficients(st.opts.cheb_emin, st.opts.cheb_emax, st.opts.cheb_steps, &scale, om);
-            double *buf[2] = {pa, pb};
-            if ((rc = pcb_u0_first(h, b0, st.d_mass_dinv, btil, buf[1], scale)) != CTL_OK) break;
-            for (int k = 2; k <= st.opts.cheb_steps && rc == CTL_OK; ++k) {
-                const double w = om[k - 2];
-                if (h->n_halo > 0) rc = ctl_halo_exchange_panel(h, buf[(k - 1) & 1]);
-                if (rc != CTL_OK) break;
-                rc = pcb_cheb_step(h, st.d_mass_dinv, btil, k == 2 ? nullptr : buf[k & 1], buf[(k - 1) & 1],
-                                   buf[k & 1], k == 2 ? 0.0 : 1.0 - w, w, w * scale);
-            }
-            if (rc != CTL_OK) break;
-            p_fin = buf[st.opts.cheb_steps & 1];
-        } else if (st.opts.solver_0 == CTL_S0_JACOBI) {
-            if ((rc = pcb_u0_first(h, b0, st.d_mass_dinv, btil, pa, 1.0)) != CTL_OK) break;
-            p_fin = pa;
-        } else {
-            // Multigrid=True: AMG on assemble(M, bcs), column by column
-            if ((rc = pcb_u0_first(h, b0, st.d_mass_dinv, btil, pa, 1.0)) != CTL_OK) break;
-            if ((rc = pcb_panel_to_ts(h, btil, st.B, st.ts_stride)) != CTL_OK) break;
-            if ((rc = halo_epoch_begin(h)) != CTL_OK) break;
-            for (int i = 0; i < h->N && rc == CTL_OK; ++i)
-                rc = amg_solve(h, st.hier[st.h_mass], st.B + i * st.ts_stride, st.Uf + i * st.ts_stride);
-            if (rc != CTL_OK) break;
-            if ((rc = pcb_ts_to_panel(h, st.Uf, pa, st.ts_stride)) != CTL_OK) break;
-            p_fin = pa;
+    // ---- (1,1) block: control/control.py:1997-2014 (CN), 2193-2206 (BE)
+    const double *p_fin = nullptr;
+    if (st.opts.solver_0 == CTL_S0_CHEBYSHEV) {
+        double scale;
+        std::vector<double> om;
+        cheb_coefficients(st.opts.cheb_emin, st.opts.cheb_emax, st.opts.cheb_steps, &scale, om);
+        double *buf[2] = {pa, pb};
+        CTL_TRY(pcb_u0_first(h, b0, st.d_mass_dinv, btil, buf[1], scale));
+        for (int k = 2; k <= st.opts.cheb_steps; ++k) {
+            const double w = om[k - 2];
+            if (h->n_halo > 0) CTL_TRY(ctl_halo_exchange_panel(h, buf[(k - 1) & 1]));
+            CTL_TRY(pcb_cheb_step(h, st.d_mass_dinv, btil, k == 2 ? nullptr : buf[k & 1], buf[(k - 1) & 1], buf[k & 1],
+                                  k == 2 ? 0.0 : 1.0 - w, w, w * scale));
         }
-        const double sc = cn ? 2.0 / tau : 1.0 / tau;
-        const double sc_last = cn ? sc : 1.0 / (tau * h->cfg.epsilon);
-        if ((rc = pcb_u0_final(h, p_fin, wrap ? b0 : nullptr, u0, sc, sc_last)) != CTL_OK) break;
-        // ---- Schur block right-hand side: control/control.py:2016-2053 (CN), 2208-2237 (BE)
-        if (st.opts.mode == CTL_PCMODE_TRIANGULAR) {
-            // u0 has b's values on constrained rows when wrapping; the products must see
-            // zeros there: the value arrays have constrained COLUMNS eliminated, so they do
-            if (h->n_halo > 0 && (rc = ctl_halo_exchange_panel(h, u0)) != CTL_OK) break;
-            rc = pcb_schur_rhs(h, u0, b1, rhs);
-        } else {
-            rc = pcb_schur_rhs(h, nullptr, b1, rhs);
-        }
-        if (rc != CTL_OK) break;
-        if ((rc = pcb_panel_to_ts(h, rhs, st.B, st.ts_stride)) != CTL_OK) break;
-        // ---- forward / backward time sweeps
-        if ((rc = run_sweeps(h, st)) != CTL_OK) break;
-        if ((rc = pcb_ts_to_panel(h, st.Ub, u1, st.ts_stride)) != CTL_OK) break;
-        rc = pcb_bc_fixup(h, h->d_bc_rows_all, h->n_bc_all, wrap ? b1 : nullptr, u1);
-    } while (0);
-    ctl_scratch_put(h, s1);
-    ctl_scratch_put(h, s2);
-    return rc;
+        p_fin = buf[st.opts.cheb_steps & 1];
+    } else if (st.opts.solver_0 == CTL_S0_JACOBI) {
+        CTL_TRY(pcb_u0_first(h, b0, st.d_mass_dinv, btil, pa, 1.0));
+        p_fin = pa;
+    } else {
+        // Multigrid=True: AMG on assemble(M, bcs), column by column
+        CTL_TRY(pcb_u0_first(h, b0, st.d_mass_dinv, btil, pa, 1.0));
+        CTL_TRY(pcb_panel_to_ts(h, btil, st.B, st.ts_stride));
+        CTL_TRY(halo_epoch_begin(h));
+        for (int i = 0; i < h->N; ++i)
+            CTL_TRY(amg_solve(h, st.hier[st.h_mass], st.B + i * st.ts_stride, st.Uf + i * st.ts_stride));
+        CTL_TRY(pcb_ts_to_panel(h, st.Uf, pa, st.ts_stride));
+        p_fin = pa;
+    }
+    const double sc = cn ? 2.0 / tau : 1.0 / tau;
+    const double sc_last = cn ? sc : 1.0 / (tau * h->cfg.epsilon);
+    CTL_TRY(pcb_u0_final(h, p_fin, wrap ? b0 : nullptr, u0, sc, sc_last));
+    // ---- Schur block right-hand side: control/control.py:2016-2053 (CN), 2208-2237 (BE)
+    if (st.opts.mode == CTL_PCMODE_TRIANGULAR) {
+        // u0 has b's values on constrained rows when wrapping; the products must see
+        // zeros there: the value arrays have constrained COLUMNS eliminated, so they do
+        if (h->n_halo > 0) CTL_TRY(ctl_halo_exchange_panel(h, u0));
+        CTL_TRY(pcb_schur_rhs(h, u0, b1, rhs));
+    } else {
+        CTL_TRY(pcb_schur_rhs(h, nullptr, b1, rhs));
+    }
+    CTL_TRY(pcb_panel_to_ts(h, rhs, st.B, st.ts_stride));
+    // ---- forward / backward time sweeps
+    CTL_TRY(run_sweeps(h, st));
+    CTL_TRY(pcb_ts_to_panel(h, st.Ub, u1, st.ts_stride));
+    return pcb_bc_fixup(h, h->d_bc_rows_all, h->n_bc_all, wrap ? b1 : nullptr, u1);
 }
 
 int ctl_pc_apply_tf(ctl_handle_s *h, const double *b_tf, double *u_tf) { return pc_fn_tf(h, b_tf, u_tf, true); }
@@ -338,16 +328,9 @@ static int pc_entry(ctl_handle_s *h, const double *b, double *u, int layout, boo
         CTL_TRY(pc_fn_tf(h, b, u, wrap));
         return ctl_comm_check(h);
     }
-    double *bt = nullptr, *ut = nullptr;
-    CTL_TRY(ctl_scratch_get(h, &bt));
-    CTL_TRY(ctl_scratch_get(h, &ut));
-    int rc = ctl_to_tf(h, b, bt);
-    if (rc == CTL_OK) rc = pc_fn_tf(h, bt, ut, wrap);
-    if (rc == CTL_OK) rc = ctl_to_bm(h, ut, u);
-    ctl_scratch_put(h, bt);
-    ctl_scratch_put(h, ut);
-    if (rc == CTL_OK) rc = ctl_comm_check(h);
-    return rc;
+    CTL_TRY(with_tf(h, layout, {b, nullptr}, u,
+                    [&](const double *bt, double *ut) { return pc_fn_tf(h, bt, ut, wrap); }));
+    return ctl_comm_check(h);
 }
 
 extern "C" {
@@ -791,11 +774,11 @@ int ctl_time_amg(ctl_handle h, int32_t hi, int reps, int flush_l2, double *out)
     constexpr int kSetVecs = 5;
     const size_t set_bytes = (size_t)kSetVecs * nv * sizeof(double);
     const int n_sets = flush_l2 ? (int)std::max<size_t>(2, ((size_t)300 << 20) / set_bytes + 1) : 1;
-    double *sets = nullptr, *flush = nullptr;
+    DeviceArray<double> sets, flush;
     const size_t flush_bytes = 256u << 20;
-    CTL_CUDA(cudaMalloc((void **)&sets, (size_t)n_sets * set_bytes));
+    CTL_CUDA(sets.alloc((size_t)n_sets * kSetVecs * nv));
     CTL_CUDA(cudaMemset(sets, 0, (size_t)n_sets * set_bytes));
-    if (flush_l2) CTL_CUDA(cudaMalloc((void **)&flush, flush_bytes));
+    if (flush_l2) CTL_CUDA(flush.alloc(flush_bytes / sizeof(double)));
     auto vec = [&](int set, int k) { return sets + ((size_t)set * kSetVecs + k) * nv; };      // k: 0 dinv 1 b 2 x 3 p 4 out
     {
         std::vector<double> hb((size_t)n * nc);
@@ -807,9 +790,8 @@ int ctl_time_amg(ctl_handle h, int32_t hi, int reps, int flush_l2, double *out)
         }
     }
     double *b = vec(0, 1), *x = vec(0, 2);
-    cudaEvent_t e0, e1;
-    CTL_CUDA(cudaEventCreate(&e0));
-    CTL_CUDA(cudaEventCreate(&e1));
+    EventPair ev;
+    CTL_TRY(ev.create(h));
     // Each kernel is timed over `reps` launches between ONE pair of events: an event pair around a single 10 us
     // launch would add several microseconds of record / launch latency to it.  The whole inner solve (which = 2)
     // streams 2 GB per call; it is timed as (reps x [256 MB overwrite, solve]) minus (reps x [overwrite]).
@@ -818,7 +800,7 @@ int ctl_time_amg(ctl_handle h, int32_t hi, int reps, int flush_l2, double *out)
     int rc = CTL_OK;
     auto timed = [&](int which, bool with_kernel, float *ms) -> int {
         int r2 = which == 2 ? halo_epoch_begin(h) : CTL_OK;      // every rank times the same sequence
-        cudaEventRecord(e0, h->stream);
+        cudaEventRecord(ev.begin, h->stream);
         for (int r = 0; r < reps && r2 == CTL_OK; ++r) {
             if (which == 2 && flush) cudaMemsetAsync(flush, r & 0xff, flush_bytes, h->stream);
             if (!with_kernel) continue;
@@ -830,9 +812,9 @@ int ctl_time_amg(ctl_handle h, int32_t hi, int reps, int flush_l2, double *out)
             else r2 = amg_solve(h, H, b, x);
             launches_solve = h->launches - l0;
         }
-        cudaEventRecord(e1, h->stream);
-        cudaEventSynchronize(e1);
-        cudaEventElapsedTime(ms, e0, e1);
+        cudaEventRecord(ev.end, h->stream);
+        cudaEventSynchronize(ev.end);
+        cudaEventElapsedTime(ms, ev.begin, ev.end);
         return r2;
     };
     for (int which = 0; which < 3 && rc == CTL_OK; ++which) {
@@ -850,10 +832,6 @@ int ctl_time_amg(ctl_handle h, int32_t hi, int reps, int flush_l2, double *out)
     out[4] = acc[2] / reps;
     out[5] = (double)H.bytes_per_cycle * H.params.cycles;
     out[6] = (double)launches_solve;
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
-    cudaFree(sets);
-    cudaFree(flush);
     return rc;
 }
 

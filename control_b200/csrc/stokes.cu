@@ -48,7 +48,7 @@ struct ctl_stokes_s {
     int colsum_blocks = 0;
     double *d_res_part = nullptr; // per-block partial norms of ctl_stokes_nonlinear_residual, then the norm
     int res_blocks = 0;
-    std::vector<double *> pool;   // outer-length scratch vectors
+    ScratchPool pool;             // outer vectors (len() is never below the block-major length: ld >= N)
     KrylovState ks;
     ctl_pc_callback pc_cb = nullptr;   // user preconditioner P= of incompressible_linear_solve (control/control.py:4686-4689)
     void *pc_cb_user = nullptr;
@@ -350,20 +350,18 @@ int stokes_apply_tf(ctl_stokes_s *S, const double *x, double *y)
     const double *x0 = x, *x1 = x + hv->vec_len();
     double *y0 = y, *y1 = y + hv->vec_len();
     CTL_TRY(ctl_kkt_apply_tf(hv, x0, y0));                       // block_00 (constrained rows: y = x)
-    double *xc1 = nullptr;
-    CTL_TRY(ctl_scratch_get(hp, &xc1));
-    int rc = pressure_center(S, x1, nullptr, xc1);               // pre_mult_corrected_lhs
+    Scratch xc1;
+    CTL_TRY(hp->pool.take(&xc1));
+    CTL_TRY(pressure_center(S, x1, nullptr, xc1));               // pre_mult_corrected_lhs
     // block_01 = diag(tau B^T): rows [0, N) get T_1, rows [N, 2N) get T_2 (preconditioner.py:471-525)
-    for (int q = 0; q < 2 && rc == CTL_OK; ++q)
-        rc = panel_spmm(S, S->BT, xc1 + q * pp, nullptr, y0 + q * pv, tau, 1.0, cn ? (q == 0 ? T_ONE : T_TWO) : T_NONE,
-                        T_NONE, true);
+    for (int q = 0; q < 2; ++q)
+        CTL_TRY(panel_spmm(S, S->BT, xc1 + q * pp, nullptr, y0 + q * pv, tau, 1.0,
+                           cn ? (q == 0 ? T_ONE : T_TWO) : T_NONE, T_NONE, true));
     // block_10 = diag(tau B): rows [0, N) get T_2, rows [N, 2N) get T_1
-    for (int q = 0; q < 2 && rc == CTL_OK; ++q)
-        rc = panel_spmm(S, S->B, x0 + q * pv, nullptr, y1 + q * pp, tau, 1.0, cn ? (q == 0 ? T_TWO : T_ONE) : T_NONE,
-                        T_NONE, false);
-    if (rc == CTL_OK) rc = pressure_center(S, y1, x1, y1);        // post_mult_correct_lhs
-    ctl_scratch_put(hp, xc1);
-    return rc;
+    for (int q = 0; q < 2; ++q)
+        CTL_TRY(panel_spmm(S, S->B, x0 + q * pv, nullptr, y1 + q * pp, tau, 1.0,
+                           cn ? (q == 0 ? T_TWO : T_ONE) : T_NONE, T_NONE, false));
+    return pressure_center(S, y1, x1, y1);                       // post_mult_correct_lhs
 }
 
 // solver_M_p on one panel: Chebyshev/Jacobi with fixed bounds or one Jacobi sweep
@@ -400,91 +398,67 @@ int mass_p_solve(ctl_stokes_s *S, const double *c, double *u, double *tmp)
 
 // pc_fn(u_0, u_1, b_0, b_1) of control/control.py:4337-4513 (CN) / 4515-4687 (BE); wrap adds the
 // nullspace handling of Preconditioner.apply (preconditioner/preconditioner.py:562-656)
-int stokes_pc_tf(ctl_stokes_s *S, const double *b, double *u, bool wrap)
+int stokes_pc_run(ctl_stokes_s *S, const double *b, double *u, bool wrap)
 {
     ctl_handle_s *hv = S->hv, *hp = S->hp;
-    ctl_handle_s *h = hv;
-    CTL_CHECK(S->pc_ready, CTL_ERR_STATE, "Stokes preconditioner: call ctl_stokes_pc_setup first");
     const bool cn = hv->cfg.CN != 0;
     const double tau = hv->cfg.tau;
     const int N = hv->N, n_p = hp->n_loc;
     const size_t pv = (size_t)hv->n_loc * hv->ld, pp = (size_t)n_p * hp->ld;
     const double *b0 = b, *b1 = b + hv->vec_len();
     double *u0 = u, *u1 = u + hv->vec_len();
-    double *d1 = nullptr, *s1 = nullptr, *s2 = nullptr, *s3 = nullptr;
-    CTL_TRY(ctl_scratch_get(hp, &d1));
-    CTL_TRY(ctl_scratch_get(hp, &s1));
-    CTL_TRY(ctl_scratch_get(hp, &s2));
-    CTL_TRY(ctl_scratch_get(hp, &s3));
-    int rc = CTL_OK;
-    do {
-        const double *rhs1 = b1;
-        if (wrap) {                                                 // pc_pre_mult_corrected
-            if ((rc = pressure_center(S, b1, nullptr, d1)) != CTL_OK) break;
-            rhs1 = d1;
-        }
-        // ---- u_0: inner_its GMRES iterations on block_00 with the heat-type preconditioner, zero
-        //      initial guess (4355-4361); the solve projects its right-hand side itself
-        ctl_krylov_options io;
-        ctl_krylov_default_options(&io);
-        io.ksp_type = CTL_KSP_GMRES;
-        io.max_it = S->opts.inner_its;
-        io.rtol = 0.0;
-        io.atol = 0.0;
-        io.pc = CTL_PC_BUILTIN;
-        ctl_solve_result ir;
-        if ((rc = vec_zero(hv, u0, hv->vec_len())) != CTL_OK) break;
-        if ((rc = ctl_solve_tf(hv, b0, u0, &io, &ir)) != CTL_OK) break;
-        // ---- u_1 = T^-1 ((T (tau B u_0) - b_1) / tau^2)
-        for (int q = 0; q < 2 && rc == CTL_OK; ++q) {
-            const int t = cn ? (q == 0 ? T_TWO : T_ONE) : T_NONE;
-            rc = panel_spmm(S, S->B, u0 + q * pv, rhs1 + q * pp, s1 + q * pp, tau, 1.0 / (tau * tau), t, t, false);
-        }
-        if (rc != CTL_OK) break;
-        // ---- AMG cycles on K_p, one solve per time block
-        for (int q = 0; q < 2 && rc == CTL_OK; ++q)
-            rc = pcb_panel_to_ts(hp, s1 + q * pp, S->ts_b + (size_t)q * N * n_p, (size_t)n_p);
-        for (int j = 0; j < 2 * N && rc == CTL_OK; ++j)
-            rc = amg_solve(hp, S->Kp, S->ts_b + (size_t)j * n_p, S->ts_x + (size_t)j * n_p);
-        for (int q = 0; q < 2 && rc == CTL_OK; ++q)
-            rc = pcb_ts_to_panel(hp, S->ts_x + (size_t)q * N * n_p, s1 + q * pp, (size_t)n_p);
-        if (rc != CTL_OK) break;
-        // ---- multiply with the (untransformed) heat-type KKT blocks of the pressure space
-        if ((rc = ctl_kkt_apply_tf(hp, s1, s2)) != CTL_OK) break;
-        if (cn) {
-            if ((rc = panel_tinv(S, s2, T_ONE, n_p)) != CTL_OK) break;
-            if ((rc = panel_tinv(S, s2 + pp, T_TWO, n_p)) != CTL_OK) break;
-        }
-        // ---- pressure mass solves
-        for (int q = 0; q < 2 && rc == CTL_OK; ++q) rc = mass_p_solve(S, s2 + q * pp, u1 + q * pp, s3);
-        if (rc != CTL_OK) break;
-        if (wrap) {                                                 // pc_post_mult_correct
-            if ((rc = pcb_bc_fixup(hv, hv->d_bc_rows_all, hv->n_bc_all, b0, u0)) != CTL_OK) break;
-            if ((rc = pcb_bc_fixup(hv, hv->d_bc_rows_all, hv->n_bc_all, b0 + pv, u0 + pv)) != CTL_OK) break;
-            rc = pressure_center(S, u1, b1, u1);
-        }
-    } while (0);
-    hv->launches += hp->launches;      // one counter for the whole system
-    hp->launches = 0;
-    ctl_scratch_put(hp, d1);
-    ctl_scratch_put(hp, s1);
-    ctl_scratch_put(hp, s2);
-    ctl_scratch_put(hp, s3);
-    return rc;
+    Scratch d1, s1, s2, s3;
+    for (Scratch *s : {&d1, &s1, &s2, &s3}) CTL_TRY(hp->pool.take(s));
+    const double *rhs1 = b1;
+    if (wrap) {                                                 // pc_pre_mult_corrected
+        CTL_TRY(pressure_center(S, b1, nullptr, d1));
+        rhs1 = d1;
+    }
+    // ---- u_0: inner_its GMRES iterations on block_00 with the heat-type preconditioner, zero
+    //      initial guess (4355-4361); the solve projects its right-hand side itself
+    ctl_krylov_options io;
+    ctl_krylov_default_options(&io);
+    io.ksp_type = CTL_KSP_GMRES;
+    io.max_it = S->opts.inner_its;
+    io.rtol = 0.0;
+    io.atol = 0.0;
+    io.pc = CTL_PC_BUILTIN;
+    ctl_solve_result ir;
+    CTL_TRY(vec_zero(hv, u0, hv->vec_len()));
+    CTL_TRY(ctl_solve_tf(hv, b0, u0, &io, &ir));
+    // ---- u_1 = T^-1 ((T (tau B u_0) - b_1) / tau^2)
+    for (int q = 0; q < 2; ++q) {
+        const int t = cn ? (q == 0 ? T_TWO : T_ONE) : T_NONE;
+        CTL_TRY(panel_spmm(S, S->B, u0 + q * pv, rhs1 + q * pp, s1 + q * pp, tau, 1.0 / (tau * tau), t, t, false));
+    }
+    // ---- AMG cycles on K_p, one solve per time block
+    for (int q = 0; q < 2; ++q) CTL_TRY(pcb_panel_to_ts(hp, s1 + q * pp, S->ts_b + (size_t)q * N * n_p, (size_t)n_p));
+    for (int j = 0; j < 2 * N; ++j) CTL_TRY(amg_solve(hp, S->Kp, S->ts_b + (size_t)j * n_p, S->ts_x + (size_t)j * n_p));
+    for (int q = 0; q < 2; ++q) CTL_TRY(pcb_ts_to_panel(hp, S->ts_x + (size_t)q * N * n_p, s1 + q * pp, (size_t)n_p));
+    // ---- multiply with the (untransformed) heat-type KKT blocks of the pressure space
+    CTL_TRY(ctl_kkt_apply_tf(hp, s1, s2));
+    if (cn) {
+        CTL_TRY(panel_tinv(S, s2, T_ONE, n_p));
+        CTL_TRY(panel_tinv(S, s2 + pp, T_TWO, n_p));
+    }
+    // ---- pressure mass solves
+    for (int q = 0; q < 2; ++q) CTL_TRY(mass_p_solve(S, s2 + q * pp, u1 + q * pp, s3));
+    if (wrap) {                                                 // pc_post_mult_correct
+        CTL_TRY(pcb_bc_fixup(hv, hv->d_bc_rows_all, hv->n_bc_all, b0, u0));
+        CTL_TRY(pcb_bc_fixup(hv, hv->d_bc_rows_all, hv->n_bc_all, b0 + pv, u0 + pv));
+        CTL_TRY(pressure_center(S, u1, b1, u1));
+    }
+    return CTL_OK;
 }
 
-int outer_get(ctl_stokes_s *S, double **p)
+int stokes_pc_tf(ctl_stokes_s *S, const double *b, double *u, bool wrap)
 {
     ctl_handle_s *h = S->hv;
-    if (!S->pool.empty()) {
-        *p = S->pool.back();
-        S->pool.pop_back();
-        return CTL_OK;
-    }
-    // block-major and internal lengths differ; size for the larger
-    const int64_t bm = 2ll * h->N * ((int64_t)S->hv->n_loc + S->hp->n_loc);
-    CTL_CUDA(cudaMalloc((void **)p, (size_t)std::max(S->len(), bm) * sizeof(double)));
-    return CTL_OK;
+    CTL_CHECK(S->pc_ready, CTL_ERR_STATE, "Stokes preconditioner: call ctl_stokes_pc_setup first");
+    const int rc = stokes_pc_run(S, b, u, wrap);
+    S->hv->launches += S->hp->launches;      // one counter for the whole system
+    S->hp->launches = 0;
+    return rc;
 }
 
 int outer_to_tf(ctl_stokes_s *S, const double *bm, double *tf)
@@ -502,39 +476,11 @@ int outer_to_bm(ctl_stokes_s *S, const double *tf, double *bm)
 struct StokesSolver : Solver {
     ctl_stokes_s *S;
     StokesSolver(ctl_stokes_s *S_, const ctl_krylov_options &o_, ctl_solve_result &r_)
-        : Solver(S_->hv, o_, r_, S_->ks, S_->len()), S(S_) {}
-    ~StokesSolver() override { release(); }
-    int get_vec(double **p) override { return outer_get(S, p); }
-    void put_vec(double *p) override { S->pool.push_back(p); }
+        : Solver(S_->hv, o_, r_, S_->ks, S_->pool, S_->len(), "ctl_stokes_solve", S_->pc_cb, S_->pc_cb_user), S(S_) {}
     int apply_operator(const double *x, double *y) override { return stokes_apply_tf(S, x, y); }
     int apply_builtin_pc(const double *x, double *y) override { return stokes_pc_tf(S, x, y, true); }
-    // Preconditioner.apply around a user pc_fn (preconditioner/preconditioner.py:562-656): project the right-hand
-    // side, hand block-major device vectors of the outer system to the callback, restore the constrained entries
-    int apply_callback_pc(const double *x, double *y) override
-    {
-        CTL_CHECK(S->pc_cb, CTL_ERR_STATE, "ctl_stokes_solve: no preconditioner callback installed");
-        double *bm_b = nullptr, *bm_u = nullptr, *xc = nullptr;
-        CTL_TRY(outer_get(S, &bm_b));
-        CTL_TRY(outer_get(S, &bm_u));
-        CTL_TRY(outer_get(S, &xc));
-        int rc = vec_copy(h, xc, x, len);
-        if (rc == CTL_OK) rc = project(xc, nullptr);                  // pc_pre_mult_corrected
-        if (rc == CTL_OK) rc = outer_to_bm(S, xc, bm_b);
-        if (rc == CTL_OK) rc = vec_zero(h, bm_u, len);
-        if (rc == CTL_OK) {
-            cudaStreamSynchronize(h->stream);
-            if (S->pc_cb(S->pc_cb_user, bm_b, bm_u) != 0) {
-                ctl_set_error(h, "preconditioner callback failed");
-                rc = CTL_ERR_CALLBACK;
-            }
-        }
-        if (rc == CTL_OK) rc = outer_to_tf(S, bm_u, y);
-        if (rc == CTL_OK) rc = project(y, x);                         // pc_post_mult_correct
-        S->pool.push_back(bm_b);
-        S->pool.push_back(bm_u);
-        S->pool.push_back(xc);
-        return rc;
-    }
+    int to_bm(const double *tf, double *bm) override { return outer_to_bm(S, tf, bm); }
+    int to_tf(const double *bm, double *tf) override { return outer_to_tf(S, bm, tf); }
     // velocity blocks: Dirichlet rows; pressure blocks: constants (full_nullspace_0 / _1, 3628-3652)
     int project(double *v, const double *wrap) override
     {
@@ -544,22 +490,15 @@ struct StokesSolver : Solver {
     }
 };
 
-// run `fn` on internal-layout copies of block-major device vectors
-template <typename F>
-int with_tf(ctl_stokes_s *S, const double *b, double *u, bool u_in, F fn)
+// with_internal for the Stokes system: the caller's vectors are block-major
+template <size_t K, class F>
+int with_tf(ctl_stokes_s *S, const double *const (&in)[K], double *out, F fn)
 {
     ctl_handle_s *h = S->hv;
     CTL_CUDA(cudaSetDevice(h->cfg.device));
-    double *bt = nullptr, *ut = nullptr;
-    CTL_TRY(outer_get(S, &bt));
-    CTL_TRY(outer_get(S, &ut));
-    int rc = outer_to_tf(S, b, bt);
-    if (rc == CTL_OK && u_in) rc = outer_to_tf(S, u, ut);
-    if (rc == CTL_OK) rc = fn(bt, ut);
-    if (rc == CTL_OK) rc = outer_to_bm(S, ut, u);
-    S->pool.push_back(bt);
-    S->pool.push_back(ut);
-    return rc;
+    return with_internal(
+        S->pool, in, out, [S](const double *bm, double *tf) { return outer_to_tf(S, bm, tf); },
+        [S](const double *tf, double *bm) { return outer_to_bm(S, tf, bm); }, fn);
 }
 
 }  // namespace
@@ -602,6 +541,7 @@ int ctl_stokes_create(ctl_handle velocity, ctl_handle pressure, const int32_t *B
     ctl_stokes_s *S = new ctl_stokes_s();
     S->hv = velocity;
     S->hp = pressure;
+    S->pool.init(h, S->len());
     S->lift_div = lift_div;
     int rc = upload_csr(h, B, S->B);
     if (rc == CTL_OK) rc = upload_csr(h, BT, S->BT);
@@ -633,9 +573,6 @@ int ctl_stokes_destroy(ctl_stokes S)
     cudaFree(S->d_part);
     cudaFree(S->d_mean);
     cudaFree(S->d_res_part);
-    for (double *p : S->pool) cudaFree(p);
-    for (double *p : S->ks.basis) cudaFree(p);
-    for (cudaEvent_t e : S->ks.events) cudaEventDestroy(e);
     delete S;
     return CTL_OK;
 }
@@ -673,35 +610,23 @@ int ctl_stokes_nonlinear_residual(ctl_stokes S, const double *b, const double *x
     const int64_t lv = h->vec_len();
     double *partials = nullptr, *scalars = nullptr;
     CTL_TRY(vec_workspace(h, &partials, &scalars));                             // pinned staging of vec_read_scalars
-    double *bt = nullptr, *xt = nullptr, *yt = nullptr;
-    CTL_TRY(outer_get(S, &bt));
-    CTL_TRY(outer_get(S, &xt));
-    CTL_TRY(outer_get(S, &yt));
-    int rc = outer_to_tf(S, b, bt);
-    if (rc == CTL_OK) rc = outer_to_tf(S, x, xt);
-    if (rc == CTL_OK) rc = ctl_kkt_apply_tf(h, xt, yt);                          // block_00 with D_v at the iterate
-    for (int q = 0; q < 2 && rc == CTL_OK; ++q)                                   // + tau T(B^T x_p), raw x_p
-        rc = panel_spmm(S, S->BT, xt + lv + q * pp, nullptr, yt + q * pv, tau, 1.0,
-                        cn ? (q == 0 ? T_ONE : T_TWO) : T_NONE, T_NONE, true);
-    for (int q = 0; q < 2 && rc == CTL_OK; ++q)                                   // r_p = b_p - tau T(B x_v)
-        rc = panel_spmm(S, S->B, xt + q * pv, bt + lv + q * pp, yt + lv + q * pp, tau, -1.0,
-                        cn ? (q == 0 ? T_TWO : T_ONE) : T_NONE, T_NONE, false);
-    if (rc == CTL_OK) {
+    CTL_TRY(with_tf(S, {b, x, nullptr}, r, [&](const double *bt, const double *xt, double *yt) -> int {
+        CTL_TRY(ctl_kkt_apply_tf(h, xt, yt));                                    // block_00 with D_v at the iterate
+        for (int q = 0; q < 2; ++q)                                               // + tau T(B^T x_p), raw x_p
+            CTL_TRY(panel_spmm(S, S->BT, xt + lv + q * pp, nullptr, yt + q * pv, tau, 1.0,
+                               cn ? (q == 0 ? T_ONE : T_TWO) : T_NONE, T_NONE, true));
+        for (int q = 0; q < 2; ++q)                                               // r_p = b_p - tau T(B x_v)
+            CTL_TRY(panel_spmm(S, S->B, xt + q * pv, bt + lv + q * pp, yt + lv + q * pp, tau, -1.0,
+                               cn ? (q == 0 ? T_TWO : T_ONE) : T_NONE, T_NONE, false));
         DISPATCH_G(ld, (stokes_residual_kernel<GG, CC><<<S->res_blocks, 256, 0, h->stream>>>(
                            bt, yt, h->d_bcmask, S->d_res_part, n_v, n_p, h->N, ld, cn ? 1 : 0, 1.0 / (tau * tau))));
         residual_finish_kernel<<<1, 256, 0, h->stream>>>(S->d_res_part, S->res_blocks, S->d_res_part + S->res_blocks);
         h->launches += 2;
-        if (cudaGetLastError() != cudaSuccess) {
-            ctl_set_error(h, "ctl_stokes_nonlinear_residual: kernel launch failed");
-            rc = CTL_ERR_CUDA;
-        }
-    }
-    if (rc == CTL_OK) rc = outer_to_bm(S, yt, r);
-    if (rc == CTL_OK) rc = vec_read_scalars(h, S->d_res_part + S->res_blocks, 1, norm_host);
-    S->pool.push_back(bt);
-    S->pool.push_back(xt);
-    S->pool.push_back(yt);
-    return rc;
+        CTL_CHECK(cudaGetLastError() == cudaSuccess, CTL_ERR_CUDA,
+                  "ctl_stokes_nonlinear_residual: kernel launch failed");
+        return CTL_OK;
+    }));
+    return vec_read_scalars(h, S->d_res_part + S->res_blocks, 1, norm_host);
 }
 
 int64_t ctl_stokes_vec_len(ctl_stokes S) { return S ? 2ll * S->hv->N * ((int64_t)S->hv->n_loc + S->hp->n_loc) : 0; }
@@ -822,7 +747,7 @@ int ctl_stokes_apply(ctl_stokes S, const double *x, double *y)
     if (!S) return CTL_ERR_ARG;
     ctl_handle_s *h = S->hv;
     CTL_CHECK(x && y, CTL_ERR_ARG, "ctl_stokes_apply: null argument");
-    return with_tf(S, x, y, false, [&](const double *xt, double *yt) { return stokes_apply_tf(S, xt, yt); });
+    return with_tf(S, {x, nullptr}, y, [&](const double *xt, double *yt) { return stokes_apply_tf(S, xt, yt); });
 }
 
 int ctl_stokes_pc_apply(ctl_stokes S, const double *b, double *u)
@@ -830,7 +755,7 @@ int ctl_stokes_pc_apply(ctl_stokes S, const double *b, double *u)
     if (!S) return CTL_ERR_ARG;
     ctl_handle_s *h = S->hv;
     CTL_CHECK(b && u, CTL_ERR_ARG, "ctl_stokes_pc_apply: null argument");
-    return with_tf(S, b, u, false, [&](const double *bt, double *ut) { return stokes_pc_tf(S, bt, ut, true); });
+    return with_tf(S, {b, nullptr}, u, [&](const double *bt, double *ut) { return stokes_pc_tf(S, bt, ut, true); });
 }
 
 int ctl_stokes_pc_fn(ctl_stokes S, const double *b, double *u)
@@ -838,7 +763,7 @@ int ctl_stokes_pc_fn(ctl_stokes S, const double *b, double *u)
     if (!S) return CTL_ERR_ARG;
     ctl_handle_s *h = S->hv;
     CTL_CHECK(b && u, CTL_ERR_ARG, "ctl_stokes_pc_fn: null argument");
-    return with_tf(S, b, u, false, [&](const double *bt, double *ut) { return stokes_pc_tf(S, bt, ut, false); });
+    return with_tf(S, {b, nullptr}, u, [&](const double *bt, double *ut) { return stokes_pc_tf(S, bt, ut, false); });
 }
 
 int ctl_stokes_set_pc_callback(ctl_stokes S, ctl_pc_callback fn, void *user)
@@ -859,39 +784,9 @@ int ctl_stokes_solve(ctl_stokes S, const double *b, double *u, const ctl_krylov_
     CTL_CHECK(opts->pc >= CTL_PC_NONE && opts->pc <= CTL_PC_CALLBACK, CTL_ERR_ARG, "ctl_stokes_solve: unknown pc kind");
     if (opts->pc == CTL_PC_CALLBACK) CTL_CHECK(S->pc_cb, CTL_ERR_STATE, "ctl_stokes_solve: call ctl_stokes_set_pc_callback first");
     if (opts->pc == CTL_PC_BUILTIN) CTL_CHECK(S->pc_ready, CTL_ERR_STATE, "ctl_stokes_solve: call ctl_stokes_pc_setup first");
-    memset(result, 0, sizeof(*result));
-    S->ks.next_event = 0;
-    S->ks.spans.clear();
-    return with_tf(S, b, u, true, [&](const double *bt, double *ut) -> int {
-        cudaEvent_t e0, e1;
-        CTL_CUDA(cudaEventCreate(&e0));
-        CTL_CUDA(cudaEventCreate(&e1));
-        CTL_CUDA(cudaEventRecord(e0, h->stream));
-        int rc;
-        {
-            StokesSolver K(S, *opts, *result);
-            double *bp = nullptr;
-            rc = K.get(&bp);
-            // correct_soln / correct_rhs (preconditioner/preconditioner.py:658-704)
-            if (rc == CTL_OK) rc = vec_copy(h, bp, bt, K.len);
-            if (rc == CTL_OK) rc = K.project(bp, nullptr);
-            if (rc == CTL_OK) rc = K.project(ut, nullptr);
-            if (rc == CTL_OK) rc = (opts->ksp_type == CTL_KSP_MINRES) ? K.minres(bp, ut) : K.gmres(bp, ut);
-            if (rc == CTL_OK) rc = K.project(ut, nullptr);
-        }
-        cudaEventRecord(e1, h->stream);
-        cudaEventSynchronize(e1);
-        float ms = 0.f;
-        cudaEventElapsedTime(&ms, e0, e1);
-        result->seconds_total = ms * 1e-3;
-        for (auto &sp : S->ks.spans) {
-            float t = 0.f;
-            if (cudaEventElapsedTime(&t, S->ks.events[sp.first], S->ks.events[sp.first + 1]) == cudaSuccess)
-                (sp.second == 0 ? result->seconds_mult : result->seconds_pc) += t * 1e-3;
-        }
-        cudaEventDestroy(e0);
-        cudaEventDestroy(e1);
-        return rc;
+    return with_tf(S, {b, u}, u, [&](const double *bt, double *ut) {
+        StokesSolver K(S, *opts, *result);
+        return krylov_solve(K, bt, ut);
     });
 }
 
@@ -901,27 +796,26 @@ int ctl_stokes_time(ctl_stokes S, int reps, double *out)
     ctl_handle_s *h = S->hv, *hp = S->hp;
     CTL_CHECK(out && reps > 0, CTL_ERR_ARG, "ctl_stokes_time: bad argument");
     CTL_CUDA(cudaSetDevice(h->cfg.device));
-    double *xv = nullptr, *yv = nullptr, *xp = nullptr;
-    CTL_TRY(ctl_scratch_get(h, &xv));
-    CTL_TRY(ctl_scratch_get(h, &yv));
-    CTL_TRY(ctl_scratch_get(hp, &xp));
+    Scratch xv, yv, xp;
+    CTL_TRY(h->pool.take(&xv));
+    CTL_TRY(h->pool.take(&yv));
+    CTL_TRY(hp->pool.take(&xp));
     int rc = vec_zero(h, xv, h->vec_len());
     if (rc == CTL_OK) rc = vec_zero(h, yv, h->vec_len());
     if (rc == CTL_OK) rc = vec_zero(h, xp, hp->vec_len());
-    cudaEvent_t e0, e1;
-    CTL_CUDA(cudaEventCreate(&e0));
-    CTL_CUDA(cudaEventCreate(&e1));
+    EventPair ev;
+    CTL_TRY(ev.create(h));
     const double tau = h->cfg.tau;
     float ms[2] = {0.f, 0.f};
     for (int which = 0; which < 2 && rc == CTL_OK; ++which) {
         for (int pass = 0; pass < 2 && rc == CTL_OK; ++pass) {        // pass 0 warms up
-            cudaEventRecord(e0, h->stream);
+            cudaEventRecord(ev.begin, h->stream);
             for (int r = 0; r < reps && rc == CTL_OK; ++r)
                 rc = which == 0 ? panel_spmm(S, S->B, xv, nullptr, xp, tau, 1.0, T_TWO, T_NONE, false)
                                 : panel_spmm(S, S->BT, xp, nullptr, yv, tau, 1.0, T_ONE, T_NONE, true);
-            cudaEventRecord(e1, h->stream);
-            cudaEventSynchronize(e1);
-            cudaEventElapsedTime(&ms[which], e0, e1);
+            cudaEventRecord(ev.end, h->stream);
+            cudaEventSynchronize(ev.end);
+            cudaEventElapsedTime(&ms[which], ev.begin, ev.end);
         }
     }
     const double n_v = h->n_loc, n_p = hp->n_loc, N = h->N;
@@ -932,11 +826,6 @@ int ctl_stokes_time(ctl_stokes S, int reps, double *out)
     out[1] = 12.0 * nnz + 4.0 * (n_p + 1) + 8.0 * N * (n_v + n_p);
     out[2] = ms[1] / reps;
     out[3] = 12.0 * nnz + 4.0 * (n_v + 1) + 8.0 * N * (n_v + n_p) + 8.0 * N * n_v;
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
-    ctl_scratch_put(h, xv);
-    ctl_scratch_put(h, yv);
-    ctl_scratch_put(hp, xp);
     return rc;
 }
 

@@ -20,3 +20,15 @@ int vec_sqrt_dev(ctl_handle_s *h, const double *in, double *out, int k);
 int vec_read_scalars(ctl_handle_s *h, const double *dev, int k, double *host_out);
 int vec_dot_host(ctl_handle_s *h, const double *x, const double *y, int64_t len, double *out);
 int vec_norm_host(ctl_handle_s *h, const double *x, int64_t len, double *out);
+
+// with_internal for the heat-type handle: the caller's vectors are block-major, or time-fastest (copied)
+template <size_t K, class F>
+int with_tf(ctl_handle_s *h, int layout, const double *const (&in)[K], double *out, F fn)
+{
+    const bool tf = layout == CTL_LAYOUT_TIME_FASTEST;
+    const int64_t len = h->vec_len();
+    return with_internal(
+        h->pool, in, out,
+        [&](const double *src, double *dst) { return tf ? vec_copy(h, dst, src, len) : ctl_to_tf(h, src, dst); },
+        [&](const double *src, double *dst) { return tf ? vec_copy(h, dst, src, len) : ctl_to_bm(h, src, dst); }, fn);
+}

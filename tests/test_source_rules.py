@@ -67,3 +67,25 @@ def test_early_loads_precede_the_wait_in_the_sass():
         # and somewhere a plain load precedes a wait directly (the early matrix loads were kept in place)
         assert any(any(o.startswith("LDG") and "CONSTANT" not in o for o in ops[(waits[k - 1] if k else 0):w])
                    for k, w in enumerate(waits)), name
+
+
+CSRC = os.path.join(ROOT, "control_b200", "csrc")
+
+
+def test_device_resources_are_released_only_by_their_owning_types():
+    """Per-call device resources are scoped (csrc/common.cuh): scratch vectors are leased from a ScratchPool and given
+    back by the lease, events are destroyed by an EventPair.  No other file destroys an event or pushes to / pops from
+    a pool's free list by hand, and the retired get / put functions stay retired -- releasing by hand leaked on the
+    error paths."""
+    owner = "common.cuh"
+    names = sorted(f for f in os.listdir(CSRC) if f.endswith((".cu", ".cuh", ".cpp", ".h")))
+    assert owner in names
+    for name in names:
+        src = open(os.path.join(CSRC, name)).read()
+        for retired in ("ctl_scratch_get", "ctl_scratch_put", "outer_get"):
+            assert not re.search(rf"\b{retired}\b", src), f"{name}: {retired}"
+        if name == owner:
+            continue
+        assert "cudaEventDestroy" not in src, f"{name}: events are destroyed by EventPair ({owner})"
+        assert not re.search(r"\b(pool|free_)\s*\.\s*(push_back|pop_back)\b", src), \
+            f"{name}: scratch vectors are leased with ScratchPool::take ({owner})"
