@@ -16,7 +16,8 @@ README.md:57 and every test).
 """
 import numpy as np
 
-from .system import MultiBlockSystem
+from .outer_loop import picard
+from .system import MultiBlockSystem, fgmres_defaults, finish_ksp, gmres_defaults
 
 __all__ = ["Control", "build_rhs"]
 
@@ -217,15 +218,47 @@ class Control:
                              check_v_d=check_v_d, check_f=check_f, bc_values=self._dirichlet_data(),
                              K_levels=K_levels)
 
+        def _v_0(self):
+            return np.zeros(self._n) if self._initial_condition is None else np.asarray(self._initial_condition, float)
+
+        def _store_blocks(self, v, zeta, v_0, g):
+            """Store the solution blocks (N, n) of a linear solve as ``_v``, ``_zeta`` (control.py:3299-3312,
+            4705-4725): for CN level 0 of v is ``v_0`` (None: zero) and the last level of zeta is zero.  The
+            boundary conditions are re-applied as set_v / set_zeta do (1836-1856), with the Dirichlet data ``g``."""
+            if self._CN:
+                self._v = np.zeros((self._n_t, self._n))
+                self._zeta = np.zeros((self._n_t, self._n))
+                if v_0 is not None:
+                    self._v[0] = v_0
+                self._v[1:] = v
+                self._zeta[:-1] = zeta
+            else:
+                self._v, self._zeta = v.copy(), zeta.copy()
+            self._bc(self._zeta)
+            if g is not None:
+                self._v[:, self._bc_dofs] = g
+
+        def _loop_start(self):
+            """Starting point of a non-linear loop (control.py:3377-3400, 4960-4978): the iterate (v, zeta) -- the
+            current state with v_0 on level 0 for CN and the last zeta level zeroed, also stored as ``_v``, ``_zeta``
+            -- and v_0, f, v_d."""
+            v_0 = self._v_0()
+            v_old, zeta_old = self._v.copy(), self._zeta.copy()
+            if self._CN:
+                v_old[0] = v_0
+            zeta_old[-1] = 0.0
+            f = self.construct_f()
+            v_d = self.construct_v_d()
+            self._v, self._zeta = v_old.copy(), zeta_old.copy()
+            return v_old, zeta_old, v_0, f, v_d
+
         # ------------------------------------------------------------------ linear_solve
         def linear_solve(self, *, P=None, solver_parameters=None, Multigrid=False, lambda_v_bounds=None,
                          v_d=None, f=None, print_error=True, create_output=False, plots=False,
                          pc_mode="triangular", **amg):
             """control/control.py:2820-3375 (homogeneous Dirichlet data)."""
-            n_t, n, tau, CN = self._n_t, self._n, self.tau, self._CN
-            M = self._M
-            N = n_t - 1 if CN else n_t
-            v_0 = np.zeros(n) if self._initial_condition is None else np.asarray(self._initial_condition, float)
+            N = self._n_t - 1 if self._CN else self._n_t
+            v_0 = self._v_0()
             check_f, check_v_d = f is None, v_d is None
             if check_f:
                 f = self.construct_f()
@@ -236,9 +269,7 @@ class Control:
             b_0, b_1 = self._build_rhs(v_0, v_d, f, K0, check_v_d, check_f,
                                        K_levels=None if self._is_linear() else K)
             if solver_parameters is None:                       # control.py:3260-3266
-                solver_parameters = {"linear_solver": "gmres", "gmres_restart": 10, "maximum_iterations": 50,
-                                     "relative_tolerance": 1.0e-6, "absolute_tolerance": 0.0,
-                                     "monitor_convergence": print_error}
+                solver_parameters = gmres_defaults(print_error)
             system = self._ensure_system(K)
             if P is None:                                       # control.py:3245-3258
                 system.setup_preconditioner(lambda_v_bounds=lambda_v_bounds, Multigrid=Multigrid,
@@ -254,20 +285,7 @@ class Control:
                                          solver_parameters=solver_parameters, pc_fn=pc_fn)
             if system.world > 1:
                 v, zeta = system.allgather_blocks(v), system.allgather_blocks(zeta)
-            if CN:                                              # control.py:3299-3312
-                v_new = np.zeros((n_t, n))
-                zeta_new = np.zeros((n_t, n))
-                if check_f and check_v_d:
-                    v_new[0] = v_0
-                v_new[1:] = v
-                zeta_new[:-1] = zeta
-                self._v, self._zeta = v_new, zeta_new
-            else:
-                self._v, self._zeta = v, zeta
-            self._bc(self._zeta)                                # set_zeta re-applies bcs, control.py:1847-1856
-            g = self._dirichlet_data()
-            if g is not None:                                   # set_v re-applies the (inhomogeneous) bcs, 1836-1845
-                self._v[:, self._bc_dofs] = g
+            self._store_blocks(v, zeta, v_0 if check_f and check_v_d else None, self._dirichlet_data())
             return self.last_ksp
 
         # ------------------------------------------------------------------ Stokes control
@@ -280,6 +298,28 @@ class Control:
             needed when the forward operator is not the Stokes one (Navier-Stokes Picard iterations)."""
             self._space_p = space_p
 
+        def _stokes_forward(self, space_p, v):
+            """The forward matrices at the velocity state ``v`` on both spaces, ``D_v_i`` and ``D_p_i``
+            (control/control.py:3780-3789); (the forward matrix, None) for a linear operator."""
+            if self._is_linear():
+                return self._forward_matrix, None
+            fp = space_p.get("forward_matrix_p")
+            if fp is None:
+                raise ValueError("a non-linear forward operator needs space_p['forward_matrix_p']")
+            return self._K_levels(v), [fp(v[i], t, self._Gauss_Newton) for i, t in enumerate(self._times())]
+
+        def _stokes_system(self, space_p, K, D_p):
+            """The ``StokesSystem`` of this instance, created on first use, with the forward matrices K, D_p."""
+            from .stokes import StokesSystem
+            if getattr(self, "_stokes", None) is None:
+                self._stokes = StokesSystem(self._M, K, space_p["B"], space_p["M_p"], space_p["K_p"], n_t=self._n_t,
+                                            beta=self._beta, CN=self._CN, time_interval=self._time_interval,
+                                            bc_dofs_v=self._bc_dofs, device=self._dev["device"], D_p=D_p,
+                                            **self._block_kw("velocity_block_size"))
+            elif not self._is_linear():
+                self._stokes.set_forward(K, D_p)
+            return self._stokes
+
         def incompressible_linear_solve(self, nullspace_p=None, *, space_p=None, P=None, solver_parameters=None,
                                         Multigrid=False, lambda_v_bounds=None, lambda_p_bounds=None, v_d=None,
                                         f=None, div_v=None, div_zeta=None, print_error=True, create_output=False,
@@ -289,7 +329,6 @@ class Control:
             at the current ``_v`` per time level, with ``space_p["forward_matrix_p"]`` on the pressure space).  ``nullspace_p``: None or "constant" -- the pressure blocks
             carry ConstantNullspace as in every caller of the reference (test/test_control.py,
             README.md).  Sets ``_v``, ``_zeta``, ``_p``, ``_mu`` and returns the KSP information."""
-            from .stokes import StokesSystem
             if space_p is None:
                 space_p = getattr(self, "_space_p", None)
                 if space_p is None:
@@ -301,22 +340,14 @@ class Control:
             n_t, n, tau, CN = self._n_t, self._n, self.tau, self._CN
             N = n_t - 1 if CN else n_t
             n_p = space_p["M_p"].shape[0]
-            v_0 = np.zeros(n) if self._initial_condition is None else np.asarray(self._initial_condition, float)
+            v_0 = self._v_0()
             check_f, check_v_d = f is None, v_d is None
             if check_f:
                 f = self.construct_f()
             if check_v_d:
                 v_d = self.construct_v_d()
-            K = self._K_levels(self._v)                             # D_v_i at the current state, 3780-3785
-            D_p = None
-            if self._is_linear():
-                K0 = K
-            else:
-                K0 = self.construct_D_v(v_0, self._time_interval[0])
-                fp = space_p.get("forward_matrix_p")
-                if fp is None:
-                    raise ValueError("a non-linear forward operator needs space_p['forward_matrix_p']")
-                D_p = [fp(self._v[i], t, self._Gauss_Newton) for i, t in enumerate(self._times())]      # 3787-3789
+            K, D_p = self._stokes_forward(space_p, self._v)             # D_v_i, D_p_i at the current state, 3780-3789
+            K0 = K if self._is_linear() else self.construct_D_v(v_0, self._time_interval[0])
             b_0_0, b_0_1 = self._build_rhs(v_0, v_d, f, K0, check_v_d, check_f,
                                            K_levels=None if self._is_linear() else K)  # 3961-4243
             b_1_0 = np.zeros((N, n_p)) if div_v is None else np.array(div_v, dtype=float)      # 4107-4128, 4207-4228
@@ -332,17 +363,8 @@ class Control:
             b_0 = np.concatenate([b_0_0, b_0_1])
             b_1 = np.concatenate([b_1_0, b_1_1])
             if solver_parameters is None:                                                 # 4291-4297
-                solver_parameters = {"linear_solver": "fgmres", "fgmres_restart": 10, "maximum_iterations": 100,
-                                     "relative_tolerance": 1.0e-6, "absolute_tolerance": 0.0,
-                                     "monitor_convergence": print_error}
-            if getattr(self, "_stokes", None) is None:
-                self._stokes = StokesSystem(self._M, K, space_p["B"], space_p["M_p"], space_p["K_p"], n_t=n_t,
-                                            beta=self._beta, CN=CN, time_interval=self._time_interval,
-                                            bc_dofs_v=self._bc_dofs, device=self._dev["device"], D_p=D_p,
-                                            **self._block_kw("velocity_block_size"))
-            elif not self._is_linear():
-                self._stokes.set_forward(K, D_p)
-            system = self._stokes
+                solver_parameters = fgmres_defaults(print_error)
+            system = self._stokes_system(space_p, K, D_p)
             if P is None:                                           # control.py:4686-4689: pc_fn = P or the in-built one
                 system.setup_preconditioner(lambda_v_bounds=lambda_v_bounds, lambda_p_bounds=lambda_p_bounds, amg=amg,
                                             amg_p=amg_p, Multigrid=Multigrid)
@@ -350,23 +372,8 @@ class Control:
             u_1 = np.zeros((2 * N, n_p))
             self.last_ksp = system.solve(u_0, u_1, b_0, b_1, solver_parameters=solver_parameters,
                                          pc_fn="builtin" if P is None else P)
-            if solver_parameters.get("monitor_convergence", True):
-                for it, r_norm in enumerate(self.last_ksp.history):
-                    print(f"KSP: iteration {it:d}, residual norm {r_norm:.16e}")
-            if CN:                                                                        # 4705-4716
-                v_new = np.zeros((n_t, n))
-                zeta_new = np.zeros((n_t, n))
-                if check_f and check_v_d:
-                    v_new[0] = v_0
-                v_new[1:] = u_0[:N]
-                zeta_new[:-1] = u_0[N:]
-                self._v, self._zeta = v_new, zeta_new
-            else:                                                                         # 4717-4725
-                self._v, self._zeta = u_0[:N].copy(), u_0[N:].copy()
+            self._store_blocks(u_0[:N], u_0[N:], v_0 if check_f and check_v_d else None, g)     # 4705-4725
             self._p, self._mu = u_1[N:].copy(), u_1[:N].copy()
-            self._bc(self._zeta)
-            if g is not None:                                   # set_v re-applies the (inhomogeneous) bcs
-                self._v[:, self._bc_dofs] = g
             return self.last_ksp
 
         def incompressible_non_linear_solve(self, nullspace_p=None, *, space_p=None, P=None, solver_parameters=None,
@@ -392,22 +399,14 @@ class Control:
                     raise ValueError("Undefined space_p")               # 4904-4910
             else:
                 self.set_space_p(space_p)
-            n_t, n, tau, CN = self._n_t, self._n, self.tau, self._CN
+            n_t, tau, CN = self._n_t, self.tau, self._CN
             N = n_t - 1 if CN else n_t
             B = space_p["B"]
             n_p = space_p["M_p"].shape[0]
-            v_old = self._v.copy()
-            zeta_old = self._zeta.copy()
             p_old = np.array(getattr(self, "_p", np.zeros((N, n_p))), dtype=float)
             mu_old = np.array(getattr(self, "_mu", np.zeros((N, n_p))), dtype=float)
-            v_0 = np.zeros(n) if self._initial_condition is None else np.asarray(self._initial_condition, float)
-            if CN:
-                v_old[0] = v_0                                          # 4968-4969
-            zeta_old[n_t - 1] = 0.0
-            f = self.construct_f()
-            v_d = self.construct_v_d()
+            v_old, zeta_old, v_0, f, v_d = self._loop_start()                 # 4968-4969
             g = self._dirichlet_data()
-            self._v, self._zeta = v_old.copy(), zeta_old.copy()
             if device_loop:
                 if nullspace_p not in (None, "constant"):
                     raise ValueError("only the constant pressure nullspace is supported")
@@ -415,8 +414,10 @@ class Control:
                     space_p, v_old, zeta_old, p_old, mu_old, v_0, v_d, f, g, solver_parameters, Multigrid,
                     lambda_v_bounds, lambda_p_bounds, max_non_linear_iter, relative_non_linear_tol,
                     absolute_non_linear_tol, print_error_linear, print_error_non_linear, amg, amg_p)
+            r = None
 
-            def res_eval():                                             # 4979-5072
+            def residual():                                             # 4979-5072
+                nonlocal r
                 r00, r01 = self.non_linear_res_eval(v_old, zeta_old, v_0, v_d, f)
                 r00 -= tau * (B.T @ mu_old.T).T
                 r01 -= tau * (B.T @ p_old.T).T
@@ -424,19 +425,11 @@ class Control:
                 self._bc(r01)
                 r10 = -(B @ (v_old[1:] if CN else v_old).T).T
                 r11 = -(B @ (zeta_old[:-1] if CN else zeta_old).T).T
-                return r00, r01, r10, r11
+                r = r00, r01, r10, r11
+                return float(np.sqrt(sum((a ** 2).sum() for a in r)))
 
-            def norm(parts):
-                return float(np.sqrt(sum((a ** 2).sum() for a in parts)))
-
-            r = res_eval()
-            norm_0 = norm(r)
-            norm_k, k = norm_0, 0
-            self.non_linear_history = [norm_0]
-            self.inner_iterations = []
-            if print_error_non_linear:
-                print(f"Initial non-linear residual: {norm_0:.16e}")
-            while norm_k > relative_non_linear_tol * norm_0 and norm_k > absolute_non_linear_tol:
+            def step():
+                nonlocal v_old, zeta_old, p_old, mu_old
                 ksp = self.incompressible_linear_solve(nullspace_p, space_p=space_p, P=P,
                                                        solver_parameters=solver_parameters, Multigrid=Multigrid,
                                                        lambda_v_bounds=lambda_v_bounds, lambda_p_bounds=lambda_p_bounds,
@@ -452,15 +445,9 @@ class Control:
                 mu_old = mu_old + self._mu
                 self._v, self._zeta = v_old.copy(), zeta_old.copy()
                 self._p, self._mu = p_old.copy(), mu_old.copy()
-                r = res_eval()
-                norm_k = norm(r)
-                k += 1
-                self.non_linear_history.append(norm_k)
-                if print_error_non_linear:
-                    print(f"Non-linear solver: iteration {k:d}, non-linear residual norm {norm_k:.16e}")
-                if k + 1 > max_non_linear_iter:
-                    break
-            return k
+            self.non_linear_history, self.inner_iterations = [], []
+            return picard(residual, step, self.non_linear_history, max_iter=max_non_linear_iter,
+                          rel_tol=relative_non_linear_tol, abs_tol=absolute_non_linear_tol, verbose=print_error_non_linear)
 
         def _incompressible_non_linear_solve_device(self, space_p, v_old, zeta_old, p_old, mu_old, v_0, v_d, f, g,
                                                     solver_parameters, Multigrid, lambda_v_bounds, lambda_p_bounds,
@@ -473,40 +460,19 @@ class Control:
             (``set_forward``), a copy of b is lifted with g (``lift_bc_device``), and the residual is
             ``ctl_stokes_nonlinear_residual``: b - A_raw x with the RAW coupling products, as ``res_eval`` has them
             (no ConstantNullspace corrections), and the norm of its untransformed parts."""
-            from .stokes import StokesSystem
             n_t, tau, CN = self._n_t, self.tau, self._CN
             N = n_t - 1 if CN else n_t
             n_p = space_p["M_p"].shape[0]
-            times = self._times()
             bd = self._bc_dofs
             linear = self._is_linear()
-            fp = space_p.get("forward_matrix_p")
-            if not linear and fp is None:
-                raise ValueError("a non-linear forward operator needs space_p['forward_matrix_p']")
-
-            def forward(v):                                             # D_v_i, D_p_i at the state, 3780-3789
-                if linear:
-                    return self._forward_matrix, None
-                return ([self.construct_D_v(v[i], t) for i, t in enumerate(times)],
-                        [fp(v[i], t, self._Gauss_Newton) for i, t in enumerate(times)])
 
             def rhs(v_init):                                            # 3961-4243, homogeneous data
                 K0 = self._forward_matrix if linear else self.construct_D_v(v_init, self._time_interval[0])
                 b_0_0, b_0_1 = build_rhs(self._M, K0, tau, n_t, CN, bd, v_d, f, v_init)
                 return system.to_device(np.concatenate([b_0_0, b_0_1]), np.zeros((2 * N, n_p)))
             if solver_parameters is None:                               # 4291-4297
-                solver_parameters = {"linear_solver": "fgmres", "fgmres_restart": 10, "maximum_iterations": 100,
-                                     "relative_tolerance": 1.0e-6, "absolute_tolerance": 0.0,
-                                     "monitor_convergence": print_error_linear}
-            K, D_p = forward(v_old)
-            if getattr(self, "_stokes", None) is None:
-                self._stokes = StokesSystem(self._M, K, space_p["B"], space_p["M_p"], space_p["K_p"], n_t=n_t,
-                                            beta=self._beta, CN=CN, time_interval=self._time_interval,
-                                            bc_dofs_v=bd, device=self._dev["device"], D_p=D_p,
-                                            **self._block_kw("velocity_block_size"))
-            elif not linear:
-                self._stokes.set_forward(K, D_p)
-            system = self._stokes
+                solver_parameters = fgmres_defaults(print_error_linear)
+            system = self._stokes_system(space_p, *self._stokes_forward(space_p, v_old))
             if g is None:
                 b_dev = b_hom = rhs(v_0)
             else:
@@ -514,24 +480,19 @@ class Control:
             x_dev = system.to_device(np.concatenate([v_old[1:], zeta_old[:-1]] if CN else [v_old, zeta_old]),
                                      np.concatenate([mu_old, p_old]))
             r_dev = system.new_vector()
-            norm_0 = system.nonlinear_residual(b_dev, x_dev, r_dev)
-            norm_k, k = norm_0, 0
-            self.non_linear_history = [norm_0]
-            self.inner_iterations = []
-            if print_error_non_linear:
-                print(f"Initial non-linear residual: {norm_0:.16e}")
-            while norm_k > rel_tol * norm_0 and norm_k > abs_tol:
+
+            def residual():
+                return system.nonlinear_residual(b_dev, x_dev, r_dev)
+
+            def step():
+                nonlocal v_old, b_dev
                 system.setup_preconditioner(lambda_v_bounds=lambda_v_bounds, lambda_p_bounds=lambda_p_bounds, amg=amg,
                                             amg_p=amg_p, Multigrid=Multigrid)
                 d_dev = system.new_vector()
                 self.last_ksp = system.solve_device(r_dev, d_dev, solver_parameters=solver_parameters)
-                if not solver_parameters.get("preconditioner", False) and self.last_ksp.reason <= 0:
-                    raise RuntimeError("Solver failed to converge")
-                if solver_parameters.get("monitor_convergence", True):
-                    for it, r_norm in enumerate(self.last_ksp.history):
-                        print(f"KSP: iteration {it:d}, residual norm {r_norm:.16e}")
+                finish_ksp(self.last_ksp, solver_parameters)
                 self.inner_iterations.append(self.last_ksp.its)
-                x_dev += d_dev
+                x_dev.add_(d_dev)
                 v_blocks = system.velocity_state_to_host(x_dev)
                 if CN:
                     v_old[1:] = v_blocks
@@ -540,16 +501,12 @@ class Control:
                 if g is not None:                                       # 5127-5160
                     v_old[:, bd] = g
                 if not linear:
-                    system.set_forward(*forward(v_old))
+                    system.set_forward(*self._stokes_forward(space_p, v_old))
                 if g is not None:
                     b_dev = system.lift_bc_device(g, b_hom.clone())
-                norm_k = system.nonlinear_residual(b_dev, x_dev, r_dev)
-                k += 1
-                self.non_linear_history.append(norm_k)
-                if print_error_non_linear:
-                    print(f"Non-linear solver: iteration {k:d}, non-linear residual norm {norm_k:.16e}")
-                if k + 1 > max_non_linear_iter:
-                    break
+            self.non_linear_history, self.inner_iterations = [], []
+            k = picard(residual, step, self.non_linear_history, max_iter=max_non_linear_iter, rel_tol=rel_tol,
+                       abs_tol=abs_tol, verbose=print_error_non_linear)
             x_0, x_1 = system.to_host_blocks(x_dev)
             if CN:
                 v_old[1:], zeta_old[:-1] = x_0[:N], x_0[N:]
@@ -618,17 +575,8 @@ class Control:
                 raise ValueError("device_loop=True runs the in-built preconditioner; it does not take P=")
             if device_loop and self._dev["world"] > 1:
                 raise ValueError("device_loop=True runs on one rank")
-            n_t, n = self._n_t, self._n
             g = self._dirichlet_data()
-            v_old = self._v.copy()
-            zeta_old = self._zeta.copy()
-            v_0 = np.zeros(n) if self._initial_condition is None else np.asarray(self._initial_condition, float)
-            if self._CN:
-                v_old[0] = v_0
-            zeta_old[n_t - 1] = 0.0
-            f = self.construct_f()
-            v_d = self.construct_v_d()
-            self._v, self._zeta = v_old.copy(), zeta_old.copy()
+            v_old, zeta_old, v_0, f, v_d = self._loop_start()
             if device_loop is None:
                 device_loop = P is None and g is None and self._dev["world"] == 1 and not self._is_linear()
             if device_loop:
@@ -638,14 +586,15 @@ class Control:
                                                      lambda_v_bounds, max_non_linear_iter, relative_non_linear_tol,
                                                      absolute_non_linear_tol, print_error_linear,
                                                      print_error_non_linear, amg)
-            rhs_0, rhs_1 = self.non_linear_res_eval(v_old, zeta_old, v_0, v_d, f)
-            norm_0 = float(np.sqrt((rhs_0 ** 2).sum() + (rhs_1 ** 2).sum()))
-            norm_k = norm_0
-            k = 0
-            self.non_linear_history = [norm_0]
-            if print_error_non_linear:
-                print(f"Initial non-linear residual: {norm_0:.16e}")
-            while norm_k > relative_non_linear_tol * norm_0 and norm_k > absolute_non_linear_tol:
+            rhs_0 = rhs_1 = None
+
+            def residual():
+                nonlocal rhs_0, rhs_1
+                rhs_0, rhs_1 = self.non_linear_res_eval(v_old, zeta_old, v_0, v_d, f)
+                return float(np.sqrt((rhs_0 ** 2).sum() + (rhs_1 ** 2).sum()))
+
+            def step():
+                nonlocal v_old, zeta_old
                 self.linear_solve(P=P, solver_parameters=solver_parameters, Multigrid=Multigrid,
                                   lambda_v_bounds=lambda_v_bounds, v_d=rhs_0, f=rhs_1,
                                   print_error=print_error_linear, **amg)
@@ -655,16 +604,9 @@ class Control:
                 zeta_old = zeta_old + self._zeta
                 self._bc(zeta_old)
                 self._v, self._zeta = v_old.copy(), zeta_old.copy()
-                rhs_0, rhs_1 = self.non_linear_res_eval(v_old, zeta_old, v_0, v_d, f)
-                norm_k = float(np.sqrt((rhs_0 ** 2).sum() + (rhs_1 ** 2).sum()))
-                k += 1
-                self.non_linear_history.append(norm_k)
-                if print_error_non_linear:
-                    print(f"Non-linear solver: iteration {k:d}, non-linear residual norm {norm_k:.16e}")
-                if k + 1 > max_non_linear_iter:
-                    break
-            return k
-
+            self.non_linear_history = []
+            return picard(residual, step, self.non_linear_history, max_iter=max_non_linear_iter,
+                          rel_tol=relative_non_linear_tol, abs_tol=absolute_non_linear_tol, verbose=print_error_non_linear)
 
         def _non_linear_solve_device(self, v_old, zeta_old, v_0, v_d, f, solver_parameters, Multigrid, lambda_v_bounds,
                                      max_non_linear_iter, rel_tol, abs_tol, print_error_linear, print_error_non_linear,
@@ -676,7 +618,7 @@ class Control:
             tests/test_oracle.py::test_non_linear_residual_is_rhs_minus_operator), and the increment solve reads
             it where it lies.  Inhomogeneous Dirichlet data g (INTEGRATION.md section 6): the residual takes a copy
             of b lifted with the K_i of the iterate (``lift_bc_device``), and g is written into the iterate."""
-            n_t, n, CN = self._n_t, self._n, self._CN
+            n_t, CN = self._n_t, self._CN
             times = self._times()
             g = self._dirichlet_data()
             bd = self._bc_dofs
@@ -685,9 +627,7 @@ class Control:
                 K0 = self.construct_D_v(v_init, self._time_interval[0])
                 return system.to_device(*build_rhs(self._M, K0, self.tau, n_t, CN, bd, v_d, f, v_init))
             if solver_parameters is None:                       # control.py:3260-3266
-                solver_parameters = {"linear_solver": "gmres", "gmres_restart": 10, "maximum_iterations": 50,
-                                     "relative_tolerance": 1.0e-6, "absolute_tolerance": 0.0,
-                                     "monitor_convergence": print_error_linear}
+                solver_parameters = gmres_defaults(print_error_linear)
             system = self._ensure_system([self.construct_D_v(v_old[i], times[i]) for i in range(n_t)])
             if g is None:
                 b_dev = rhs(v_0)
@@ -695,21 +635,17 @@ class Control:
                 b_hom, b_dev = self._lifted_rhs_pair(system, rhs, v_old, v_0, g)
             x_dev = system.to_device(*((v_old[1:], zeta_old[:-1]) if CN else (v_old, zeta_old)))
             r_dev = system.new_vector()
-            norm_0 = system.nonlinear_residual(b_dev, x_dev, r_dev)
-            norm_k, k = norm_0, 0
-            self.non_linear_history = [norm_0]
-            if print_error_non_linear:
-                print(f"Initial non-linear residual: {norm_0:.16e}")
-            while norm_k > rel_tol * norm_0 and norm_k > abs_tol:
+
+            def residual():
+                return system.nonlinear_residual(b_dev, x_dev, r_dev)
+
+            def step():
+                nonlocal v_old, b_dev
                 system.setup_preconditioner(lambda_v_bounds=lambda_v_bounds, Multigrid=Multigrid, **amg)
                 d_dev = system.new_vector()
                 self.last_ksp = system.solve_device(r_dev, d_dev, solver_parameters=solver_parameters, pc="builtin")
-                if solver_parameters.get("monitor_convergence", True):
-                    for it, r_norm in enumerate(self.last_ksp.history):
-                        print(f"KSP: iteration {it:d}, residual norm {r_norm:.16e}")
-                if not solver_parameters.get("preconditioner", False) and self.last_ksp.reason <= 0:
-                    raise RuntimeError("Solver failed to converge")
-                x_dev += d_dev
+                finish_ksp(self.last_ksp, solver_parameters)
+                x_dev.add_(d_dev)
                 v_blocks = system.to_host_blocks(x_dev)[0]
                 if CN:
                     v_old[1:] = v_blocks
@@ -720,13 +656,9 @@ class Control:
                 system.set_K([self.construct_D_v(v_old[i], times[i]) for i in range(n_t)])
                 if g is not None:
                     b_dev = system.lift_bc_device(g, b_hom.clone())
-                norm_k = system.nonlinear_residual(b_dev, x_dev, r_dev)
-                k += 1
-                self.non_linear_history.append(norm_k)
-                if print_error_non_linear:
-                    print(f"Non-linear solver: iteration {k:d}, non-linear residual norm {norm_k:.16e}")
-                if k + 1 > max_non_linear_iter:
-                    break
+            self.non_linear_history = []
+            k = picard(residual, step, self.non_linear_history, max_iter=max_non_linear_iter, rel_tol=rel_tol,
+                       abs_tol=abs_tol, verbose=print_error_non_linear)
             x_0, x_1 = system.to_host_blocks(x_dev)
             if CN:
                 v_old[1:], zeta_old[:-1] = x_0, x_1

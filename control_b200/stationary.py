@@ -18,7 +18,8 @@ reference does in Firedrake (right-hand sides, lifting, residuals of the non-lin
 import numpy as np
 import scipy.sparse as sp
 
-from .system import MultiBlockSystem
+from .outer_loop import picard
+from .system import MultiBlockSystem, fgmres_defaults, gmres_defaults
 
 __all__ = ["Stationary"]
 
@@ -130,9 +131,7 @@ class Stationary:
         else:
             b_0 = np.array(v_d, dtype=float)
         if solver_parameters is None:                   # 562-568
-            solver_parameters = {"linear_solver": "gmres", "gmres_restart": 10, "maximum_iterations": 50,
-                                 "relative_tolerance": 1.0e-6, "absolute_tolerance": 0.0,
-                                 "monitor_convergence": print_error}
+            solver_parameters = gmres_defaults(print_error)
         system = self._ensure_system(D_v)
         if P is None:                                   # 541-545
             system.setup_preconditioner(lambda_v_bounds=lambda_v_bounds, Multigrid=Multigrid, **amg)
@@ -217,9 +216,7 @@ class Stationary:
             b_10 = np.array(div_v, dtype=float)
         b_11 = np.zeros(n_p) if div_zeta is None else np.array(div_zeta, dtype=float)
         if solver_parameters is None:                   # 1088-1094
-            solver_parameters = {"linear_solver": "fgmres", "fgmres_restart": 10, "maximum_iterations": 50,
-                                 "relative_tolerance": 1.0e-6, "absolute_tolerance": 0.0,
-                                 "monitor_convergence": print_error}
+            solver_parameters = fgmres_defaults(print_error, max_it=50)
         K_shift = self._shifted(D_v)
         D_p_shift = sp.csr_matrix((D_p.data - M_p.data, M_p.indices, M_p.indptr), shape=M_p.shape)
         if getattr(self, "_stokes", None) is None:
@@ -267,25 +264,20 @@ class Stationary:
         f = self._assembled_force()
         v_d = self._assembled_desired_state()
 
-        def res_eval():                                 # 1272-1319
+        r = None
+
+        def residual():                                 # 1272-1319
+            nonlocal r
             r00, r01 = self.non_linear_res_eval(v_d, f, v_old, zeta_old, self.construct_D_v(v_old))
             r00 = r00 - B.T @ mu_old
             r01 = r01 - B.T @ p_old
             self._bc(r00)
             self._bc(r01)
-            return r00, r01, -(B @ v_old), -(B @ zeta_old)
+            r = r00, r01, -(B @ v_old), -(B @ zeta_old)
+            return float(np.sqrt(sum(a @ a for a in r)))
 
-        def norm(parts):
-            return float(np.sqrt(sum(a @ a for a in parts)))
-
-        r = res_eval()
-        norm_0 = norm(r)
-        norm_k, k = norm_0, 0
-        self.non_linear_history = [norm_0]
-        self.inner_iterations = []
-        if print_error_non_linear:
-            print(f"Initial non-linear residual: {norm_0:.16e}")
-        while norm_k > relative_non_linear_tol * norm_0 and norm_k > absolute_non_linear_tol:
+        def step():
+            nonlocal v_old, zeta_old, p_old, mu_old
             ksp = self.incompressible_linear_solve(nullspace_p, space_p=space_p, P=P, solver_parameters=solver_parameters,
                                                    Multigrid=Multigrid, lambda_v_bounds=lambda_v_bounds,
                                                    lambda_p_bounds=lambda_p_bounds, v_d=r[0], f=r[1], div_v=r[2],
@@ -299,14 +291,9 @@ class Stationary:
             p_old = p_old + self._p
             mu_old = mu_old + self._mu
             self._v, self._zeta, self._p, self._mu = v_old.copy(), zeta_old.copy(), p_old.copy(), mu_old.copy()
-            r = res_eval()
-            norm_k = norm(r)
-            k += 1
-            self.non_linear_history.append(norm_k)
-            if print_error_non_linear:
-                print(f"Non-linear solver: iteration {k:d}, non-linear residual norm {norm_k:.16e}")
-            if k + 1 > max_non_linear_iter:
-                break
+        self.non_linear_history, self.inner_iterations = [], []
+        k = picard(residual, step, self.non_linear_history, max_iter=max_non_linear_iter,
+                   rel_tol=relative_non_linear_tol, abs_tol=absolute_non_linear_tol, verbose=print_error_non_linear)
         if print_error_non_linear:
             self.print_error()
         return k
@@ -330,14 +317,15 @@ class Stationary:
         zeta_old = self._zeta.copy()
         f = self._assembled_force()
         v_d = self._assembled_desired_state()
-        D_v = self.construct_D_v(v_old)
-        rhs_0, rhs_1 = self.non_linear_res_eval(v_d, f, v_old, zeta_old, D_v)
-        norm_0 = float(np.sqrt(rhs_0 @ rhs_0 + rhs_1 @ rhs_1))
-        norm_k, k = norm_0, 0
-        self.non_linear_history = [norm_0]
-        if print_error_non_linear:
-            print(f"Initial non-linear residual: {norm_0:.16e}")
-        while norm_k > relative_non_linear_tol * norm_0 and norm_k > absolute_non_linear_tol:
+        rhs_0 = rhs_1 = None
+
+        def residual():
+            nonlocal rhs_0, rhs_1
+            rhs_0, rhs_1 = self.non_linear_res_eval(v_d, f, v_old, zeta_old, self.construct_D_v(v_old))
+            return float(np.sqrt(rhs_0 @ rhs_0 + rhs_1 @ rhs_1))
+
+        def step():
+            nonlocal v_old, zeta_old
             self.linear_solve(P=P, solver_parameters=solver_parameters, Multigrid=Multigrid,
                               lambda_v_bounds=lambda_v_bounds, v_d=rhs_0, f=rhs_1, print_error=print_error_linear, **amg)
             v_old = v_old + self._v
@@ -346,15 +334,9 @@ class Stationary:
             zeta_old = zeta_old + self._zeta
             self._bc(zeta_old)
             self._v, self._zeta = v_old.copy(), zeta_old.copy()
-            D_v = self.construct_D_v(v_old)
-            rhs_0, rhs_1 = self.non_linear_res_eval(v_d, f, v_old, zeta_old, D_v)
-            norm_k = float(np.sqrt(rhs_0 @ rhs_0 + rhs_1 @ rhs_1))
-            k += 1
-            self.non_linear_history.append(norm_k)
-            if print_error_non_linear:
-                print(f"Non-linear solver: iteration {k:d}, non-linear residual norm {norm_k:.16e}")
-            if k + 1 > max_non_linear_iter:
-                break
+        self.non_linear_history = []
+        k = picard(residual, step, self.non_linear_history, max_iter=max_non_linear_iter,
+                   rel_tol=relative_non_linear_tol, abs_tol=absolute_non_linear_tol, verbose=print_error_non_linear)
         if print_error_non_linear:
             self.print_error()
         return k

@@ -18,7 +18,7 @@ import torch
 
 from . import _lib as L
 
-__all__ = ["MultiBlockSystem", "KSPInfo", "csr_arrays"]
+__all__ = ["MultiBlockSystem", "KSPInfo", "csr_arrays", "finish_ksp", "gmres_defaults", "fgmres_defaults"]
 
 _KSP_TYPES = {"gmres": L.CTL_KSP_GMRES, "fgmres": L.CTL_KSP_FGMRES, "minres": L.CTL_KSP_MINRES}
 
@@ -79,7 +79,198 @@ def _as_host_f64(x):
     return np.asarray(x)
 
 
-class MultiBlockSystem:
+def gmres_defaults(monitor):
+    """The heat-type drivers' ``solver_parameters`` when the caller gives none (control/control.py:562-568,
+    3260-3266)."""
+    return {"linear_solver": "gmres", "gmres_restart": 10, "maximum_iterations": 50, "relative_tolerance": 1.0e-6,
+            "absolute_tolerance": 0.0, "monitor_convergence": monitor}
+
+
+def fgmres_defaults(monitor, max_it=100):
+    """The Stokes-type drivers' ``solver_parameters`` when the caller gives none: ``max_it`` 100 for the instationary
+    ones (control/control.py:4291-4297), 50 for the stationary one (1088-1094)."""
+    return {"linear_solver": "fgmres", "fgmres_restart": 10, "maximum_iterations": max_it,
+            "relative_tolerance": 1.0e-6, "absolute_tolerance": 0.0, "monitor_convergence": monitor}
+
+
+def finish_ksp(info, solver_parameters):
+    """The end of the reference's ``MultiBlockSystem.solve`` (preconditioner/preconditioner.py:749-770): print the
+    residual history when ``monitor_convergence`` is set (the reference's default is True), and raise when the solve
+    did not converge unless ``preconditioner`` is set."""
+    if solver_parameters.get("monitor_convergence", True):
+        for it, r_norm in enumerate(info.history):
+            print(f"KSP: iteration {it:d}, residual norm {r_norm:.16e}")
+    if not solver_parameters.get("preconditioner", False) and info.reason <= 0:
+        raise RuntimeError("Solver failed to converge")
+
+
+class _DeviceSystem:
+    """What the heat-type and the Stokes systems share at the host boundary: ordered library calls, block-major
+    device vectors, the Krylov options and the host ``solve`` with the reference's ``pc_fn`` hook.  A subclass
+    supplies ``_lib``, ``device``, ``_stream``, ``_pc_ready``, its handle (``_handle``, ``_check``), ``vec_len``,
+    ``to_host_blocks``, ``pc_apply``, ``solve_device`` and the name of its callback setter (``_SET_CALLBACK``)."""
+
+    @property
+    def stream(self):
+        """The CUDA stream the library launches on (time it with events recorded here)."""
+        return self._stream
+
+    def _call(self, fn, *args):
+        """Library call ordered after the work already queued on torch's current stream,
+        and torch's later work ordered after the call."""
+        cur = torch.cuda.current_stream(self.device)
+        self._stream.wait_stream(cur)
+        rc = fn(self._handle, *args)
+        cur.wait_stream(self._stream)
+        self._check(rc)
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    # ------------------------------------------------------------------ device vectors
+    def new_vector(self, layout=L.CTL_LAYOUT_BLOCK_MAJOR):
+        """A zero device vector of ``vec_len(layout)`` entries."""
+        return torch.zeros(self.vec_len(layout), dtype=torch.float64, device=self.device)
+
+    def to_device(self, x_0, x_1=None):
+        """Block-major device vector from the two host block arrays of ``to_host_blocks`` or a flat array."""
+        if x_1 is None:
+            host = np.ascontiguousarray(_as_host_f64(x_0), dtype=np.float64).ravel()
+        else:
+            host = np.concatenate([np.asarray(_as_host_f64(x_0), dtype=np.float64).ravel(),
+                                   np.asarray(_as_host_f64(x_1), dtype=np.float64).ravel()])
+        if host.size != self.vec_len():
+            raise ValueError(f"vector has {host.size} entries, expected {self.vec_len()}")
+        return torch.from_numpy(host).to(self.device)
+
+    def _to_host_arrays(self, x_dev, x_0, x_1):
+        """Copy a block-major device vector into the caller's host block arrays in place."""
+        r0, r1 = self.to_host_blocks(x_dev)
+        np.copyto(_as_host_f64(x_0).reshape(r0.shape), r0)
+        np.copyto(_as_host_f64(x_1).reshape(r1.shape), r1)
+
+    def _check_vecs(self, what, *ts, count=None, layout=L.CTL_LAYOUT_BLOCK_MAJOR):
+        """Device vector arguments: contiguous float64 CUDA tensors of ``count`` (default ``vec_len(layout)``)
+        entries."""
+        n = self.vec_len(layout) if count is None else count
+        for t in ts:
+            if not isinstance(t, torch.Tensor) or t.numel() != n or t.dtype != torch.float64 or not t.is_cuda \
+                    or not t.is_contiguous():
+                raise ValueError(f"{what} needs contiguous float64 CUDA tensors of {n} entries")
+
+    # ------------------------------------------------------------------ solve
+    def _pc_kind(self, pc):
+        kind = {"none": L.CTL_PC_NONE, "builtin": L.CTL_PC_BUILTIN, "callback": L.CTL_PC_CALLBACK}[pc]
+        if kind == L.CTL_PC_BUILTIN and not self._pc_ready:
+            raise L.CtlError("call setup_preconditioner() first")
+        return kind
+
+    def _krylov_options(self, solver_parameters, pc):
+        kind = self._pc_kind(pc)
+        sp = solver_parameters or {}
+        o = L.ctl_krylov_options()
+        self._check(self._lib.ctl_krylov_default_options(C.byref(o)))
+        ksp_type = sp.get("linear_solver", "fgmres")              # preconditioner.py:733
+        if ksp_type not in _KSP_TYPES:
+            raise ValueError(f"unsupported linear_solver {ksp_type!r}")
+        o.ksp_type = _KSP_TYPES[ksp_type]
+        o.rtol = float(sp["relative_tolerance"])                  # required keys: 739-740
+        o.atol = float(sp["absolute_tolerance"])
+        if sp.get("divergence limit") is not None:
+            o.divtol = float(sp["divergence limit"])
+        o.max_it = int(sp.get("maximum_iterations", 1000))
+        if "gmres_restart" in sp:                                 # "fgmres_restart" is never read: 747-748
+            o.restart = int(sp["gmres_restart"])
+        # "pc_side" (735-736) and "norm_type" (744-746) are forwarded to PETSc by the reference.  krylov.cuh
+        # implements PETSc's defaults for each solver -- left + preconditioned norm for gmres / minres, right +
+        # unpreconditioned norm for fgmres -- so any other request is refused instead of silently ignored (a
+        # different side or norm changes the convergence test and the iteration count)
+        right = ksp_type == "fgmres"
+        side = sp.get("pc_side")
+        if side is not None and str(side).lower() not in (("right", "2", "pc_right") if right else ("left", "1", "pc_left")):
+            raise ValueError(f"pc_side={side!r} is not implemented for {ksp_type}: only PETSc's default side "
+                             f"({'right' if right else 'left'})")
+        norm = sp.get("norm_type")
+        if norm is not None and str(norm).lower() not in (
+                ("default", "-1", "unpreconditioned", "2", "norm_unpreconditioned") if right
+                else ("default", "-1", "preconditioned", "1", "norm_preconditioned")):
+            raise ValueError(f"norm_type={norm!r} is not implemented for {ksp_type}: only PETSc's default "
+                             f"({'unpreconditioned' if right else 'preconditioned'})")
+        o.pc = kind
+        return o
+
+    def _ksp(self, entry, b_dev, u_dev, solver_parameters, pc, *args):
+        """One Krylov solve through the C entry point ``entry(handle, b, u, *args, options, result)``."""
+        o = self._krylov_options(solver_parameters, pc)
+        res = L.ctl_solve_result()
+        self._call(entry, b_dev.data_ptr(), u_dev.data_ptr(), *args, C.byref(o), C.byref(res))
+        return KSPInfo(res)
+
+    def pc_fn(self):
+        """The in-built preconditioner as a ``P``-compatible callable ``pc_fn(u_0, u_1, b_0, b_1)`` on host block
+        arrays (control/control.py:3245-3258, 4686-4689)."""
+        def pc_fn(u_0, u_1, b_0, b_1):
+            self._to_host_arrays(self.pc_apply(self.to_device(b_0, b_1), raw=True), u_0, u_1)
+        return pc_fn
+
+    def _install_callback(self, pc_fn):
+        sys_ = self
+
+        def trampoline(_user, b_ptr, u_ptr):
+            try:
+                b = _wrap_device_ptr(b_ptr, sys_.vec_len(), sys_.device)
+                u = _wrap_device_ptr(u_ptr, sys_.vec_len(), sys_.device)
+                # the library synchronised its stream before calling back
+                b0, b1 = sys_.to_host_blocks(b)
+                u0 = np.zeros_like(b0)
+                u1 = np.zeros_like(b1)
+                pc_fn(u0, u1, b0, b1)
+                u.copy_(sys_.to_device(u0, u1))
+                torch.cuda.current_stream(sys_.device).synchronize()
+                return 0
+            except Exception:                                     # flag_errors, preconditioner.py:64-72
+                _error_flag[0] = True
+                import traceback
+                traceback.print_exc()
+                return 1
+        cb = L.PC_CALLBACK(trampoline)
+        self._cb_keepalive = cb
+        self._check(getattr(self._lib, self._SET_CALLBACK)(self._handle, cb, None))
+
+    def solve(self, u_0, u_1, b_0, b_1, *, solver_parameters=None, pc_fn=None):
+        """``MultiBlockSystem.solve`` (preconditioner/preconditioner.py:337-786) on the host block arrays of
+        ``to_host_blocks``: u_* carry the initial guess in and the solution out.
+
+        ``pc_fn``: None = identity (342-345); the string "builtin" = the in-built preconditioner running on the
+        device (set up with ``setup_preconditioner``); a callable ``pc_fn(u_0, u_1, b_0, b_1)`` = the reference's
+        user hook, called back every iteration on host block arrays: ``b_*`` projected and read-only, ``u_*`` zero,
+        filled in place (620-627)."""
+        _error_flag[0] = False
+        if pc_fn is None:
+            pc = "none"
+        elif isinstance(pc_fn, str) and pc_fn == "builtin":
+            pc = "builtin"
+        elif callable(pc_fn):
+            self._install_callback(pc_fn)
+            pc = "callback"
+        else:
+            raise ValueError(f"pc_fn must be None, 'builtin' or a callable P(u_0, u_1, b_0, b_1), not {pc_fn!r}")
+        b = self.to_device(b_0, b_1)
+        u = self.to_device(u_0, u_1)
+        info = self.solve_device(b, u, solver_parameters=solver_parameters, pc=pc)
+        self._to_host_arrays(u, u_0, u_1)
+        finish_ksp(info, solver_parameters or {})
+        if _error_flag[0]:                                        # 771-772
+            raise RuntimeError("Error encountered in PETSc solve")
+        return info
+
+
+class MultiBlockSystem(_DeviceSystem):
+    _SET_CALLBACK = "ctl_set_pc_callback"
+
     def __init__(self, M, K, *, n_t, beta, CN, time_interval=(0.0, 1.0), bc_dofs=(),
                  epsilon=1e-3, device=None, rank=0, world=1, stream=None, block_size=1):
         """``block_size``: PETSc's Mat block size of the space (``M.petscmat.getBlockSize()``), dofs interleaved as
@@ -131,33 +322,17 @@ class MultiBlockSystem:
         self.set_K(K)
 
     # ------------------------------------------------------------------ plumbing
+    @property
+    def _handle(self):
+        return self._h
+
     def _check(self, rc):
         L.check(self._h, rc)
-
-    @property
-    def stream(self):
-        """The CUDA stream the library launches on (time it with events recorded here)."""
-        return self._stream
-
-    def _call(self, fn, *args):
-        """Library call ordered after the work already queued on torch's current stream,
-        and torch's later work ordered after the call."""
-        cur = torch.cuda.current_stream(self.device)
-        self._stream.wait_stream(cur)
-        rc = fn(self._h, *args)
-        cur.wait_stream(self._stream)
-        self._check(rc)
 
     def close(self):
         if getattr(self, "_h", None) is not None and self._h:
             self._lib.ctl_destroy(self._h)
             self._h = C.c_void_p()
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
 
     def _same_pattern(self, A):
         indptr, indices, data = csr_arrays(A)
@@ -210,20 +385,6 @@ class MultiBlockSystem:
     # ------------------------------------------------------------------ device vectors
     def vec_len(self, layout=L.CTL_LAYOUT_BLOCK_MAJOR):
         return int(self._lib.ctl_vec_len(self._h, layout))
-
-    def new_vector(self, layout=L.CTL_LAYOUT_BLOCK_MAJOR):
-        return torch.zeros(self.vec_len(layout), dtype=torch.float64, device=self.device)
-
-    def to_device(self, x_0, x_1=None):
-        """Block-major device vector from host blocks (N, n_local) x 2 or a flat array."""
-        if x_1 is None:
-            host = np.ascontiguousarray(_as_host_f64(x_0), dtype=np.float64).ravel()
-        else:
-            host = np.concatenate([np.asarray(_as_host_f64(x_0), dtype=np.float64).ravel(),
-                                   np.asarray(_as_host_f64(x_1), dtype=np.float64).ravel()])
-        if host.size != self.vec_len():
-            raise ValueError(f"vector has {host.size} entries, expected {self.vec_len()}")
-        return torch.from_numpy(host).to(self.device)
 
     def to_host_blocks(self, x_dev):
         a = x_dev.detach().cpu().numpy()
@@ -309,130 +470,20 @@ class MultiBlockSystem:
         self._call(fn, b_dev.data_ptr(), u_dev.data_ptr(), layout)
         return u_dev
 
-    def pc_fn(self):
-        """The in-built preconditioner as a ``P``-compatible callable
-        ``pc_fn(u_0, u_1, b_0, b_1)`` on host block arrays (control/control.py:3245-3258)."""
-        def pc_fn(u_0, u_1, b_0, b_1):
-            u = self.pc_apply(self.to_device(b_0, b_1), raw=True)
-            r0, r1 = self.to_host_blocks(u)
-            np.copyto(_as_host_f64(u_0).reshape(r0.shape), r0)
-            np.copyto(_as_host_f64(u_1).reshape(r1.shape), r1)
-        return pc_fn
-
     # ------------------------------------------------------------------ solve
-    def _krylov_options(self, solver_parameters, pc_kind):
-        sp = solver_parameters
-        o = L.ctl_krylov_options()
-        self._check(self._lib.ctl_krylov_default_options(C.byref(o)))
-        ksp_type = sp.get("linear_solver", "fgmres")              # preconditioner.py:733
-        if ksp_type not in _KSP_TYPES:
-            raise ValueError(f"unsupported linear_solver {ksp_type!r}")
-        o.ksp_type = _KSP_TYPES[ksp_type]
-        o.rtol = float(sp["relative_tolerance"])                  # required keys: 739-740
-        o.atol = float(sp["absolute_tolerance"])
-        if sp.get("divergence limit") is not None:
-            o.divtol = float(sp["divergence limit"])
-        o.max_it = int(sp.get("maximum_iterations", 1000))
-        if "gmres_restart" in sp:                                 # "fgmres_restart" is never read: 747-748
-            o.restart = int(sp["gmres_restart"])
-        # "pc_side" (735-736) and "norm_type" (744-746) are forwarded to PETSc by the reference.  krylov.cuh
-        # implements PETSc's defaults for each solver -- left + preconditioned norm for gmres / minres, right +
-        # unpreconditioned norm for fgmres -- so any other request is refused instead of silently ignored (a
-        # different side or norm changes the convergence test and the iteration count)
-        right = ksp_type == "fgmres"
-        side = sp.get("pc_side")
-        if side is not None and str(side).lower() not in (("right", "2", "pc_right") if right else ("left", "1", "pc_left")):
-            raise ValueError(f"pc_side={side!r} is not implemented for {ksp_type}: only PETSc's default side "
-                             f"({'right' if right else 'left'})")
-        norm = sp.get("norm_type")
-        if norm is not None and str(norm).lower() not in (
-                ("default", "-1", "unpreconditioned", "2", "norm_unpreconditioned") if right
-                else ("default", "-1", "preconditioned", "1", "norm_preconditioned")):
-            raise ValueError(f"norm_type={norm!r} is not implemented for {ksp_type}: only PETSc's default "
-                             f"({'unpreconditioned' if right else 'preconditioned'})")
-        o.pc = pc_kind
-        return o
-
     def solve_device(self, b_dev, u_dev, *, solver_parameters, pc="builtin",
                      layout=L.CTL_LAYOUT_BLOCK_MAJOR):
         """KSP solve on device vectors; u_dev holds the initial guess and the solution."""
-        kind = {"none": L.CTL_PC_NONE, "builtin": L.CTL_PC_BUILTIN, "callback": L.CTL_PC_CALLBACK}[pc]
-        if kind == L.CTL_PC_BUILTIN and not self._pc_ready:
-            raise L.CtlError("call setup_preconditioner() first")
-        o = self._krylov_options(solver_parameters, kind)
-        res = L.ctl_solve_result()
-        self._call(self._lib.ctl_solve, b_dev.data_ptr(), u_dev.data_ptr(), layout, C.byref(o), C.byref(res))
-        return KSPInfo(res)
-
-    def _install_callback(self, pc_fn):
-        sys_ = self
-
-        def trampoline(_user, b_ptr, u_ptr):
-            try:
-                b = _wrap_device_ptr(b_ptr, sys_.vec_len(), sys_.device)
-                u = _wrap_device_ptr(u_ptr, sys_.vec_len(), sys_.device)
-                # the library synchronised its stream before calling back
-                b0, b1 = sys_.to_host_blocks(b)
-                u0 = np.zeros_like(b0)
-                u1 = np.zeros_like(b1)
-                pc_fn(u0, u1, b0, b1)
-                u.copy_(sys_.to_device(u0, u1))
-                torch.cuda.current_stream(sys_.device).synchronize()
-                return 0
-            except Exception:                                     # flag_errors, preconditioner.py:64-72
-                _error_flag[0] = True
-                import traceback
-                traceback.print_exc()
-                return 1
-        cb = L.PC_CALLBACK(trampoline)
-        self._cb_keepalive = cb
-        self._check(self._lib.ctl_set_pc_callback(self._h, cb, None))
-
-    def solve(self, u_0, u_1, b_0, b_1, *, solver_parameters=None, pc_fn=None):
-        """``MultiBlockSystem.solve`` (preconditioner/preconditioner.py:337-786) on host
-        block arrays of shape (N, n): u_* carry the initial guess in and the solution out.
-
-        ``pc_fn``: None = identity (342-345); the string "builtin" = the in-built
-        preconditioner running on the device (set up with ``setup_preconditioner``); any
-        callable ``pc_fn(u_0, u_1, b_0, b_1)`` = the reference's user hook, called back on
-        host arrays every iteration."""
-        if solver_parameters is None:
-            solver_parameters = {}
-        _error_flag[0] = False
-        if pc_fn is None:
-            pc = "none"
-        elif isinstance(pc_fn, str) and pc_fn == "builtin":
-            pc = "builtin"
-        else:
-            self._install_callback(pc_fn)
-            pc = "callback"
-        b = self.to_device(b_0, b_1)
-        u = self.to_device(u_0, u_1)
-        info = self.solve_device(b, u, solver_parameters=solver_parameters, pc=pc)
-        r0, r1 = self.to_host_blocks(u)
-        np.copyto(_as_host_f64(u_0).reshape(r0.shape), r0)
-        np.copyto(_as_host_f64(u_1).reshape(r1.shape), r1)
-        if solver_parameters.get("monitor_convergence", True):    # 749-754 (the reference's default is True)
-            for it, r_norm in enumerate(info.history):
-                print(f"KSP: iteration {it:d}, residual norm {r_norm:.16e}")
-        if not solver_parameters.get("preconditioner", False):    # 756, 768-770
-            if info.reason <= 0:
-                raise RuntimeError("Solver failed to converge")
-        if _error_flag[0]:                                        # 771-772
-            raise RuntimeError("Error encountered in PETSc solve")
-        return info
+        return self._ksp(self._lib.ctl_solve, b_dev, u_dev, solver_parameters, pc, layout)
 
     def solve_host(self, u_host, b_host, *, solver_parameters, pc="builtin"):
         """``ctl_solve_host``: the end-to-end C entry point.  ``b_host`` / ``u_host`` are flat
         block-major float64 numpy arrays (``u_host``: initial guess in, solution out); the
         library copies them to the device and back itself."""
-        kind = {"none": L.CTL_PC_NONE, "builtin": L.CTL_PC_BUILTIN, "callback": L.CTL_PC_CALLBACK}[pc]
-        if kind == L.CTL_PC_BUILTIN and not self._pc_ready:
-            raise L.CtlError("call setup_preconditioner() first")
+        o = self._krylov_options(solver_parameters, pc)
         if b_host.dtype != np.float64 or u_host.dtype != np.float64 or not b_host.flags.c_contiguous \
                 or not u_host.flags.c_contiguous or b_host.size != self.vec_len() or u_host.size != self.vec_len():
             raise ValueError("solve_host needs contiguous float64 arrays of vec_len() entries")
-        o = self._krylov_options(solver_parameters, kind)
         res = L.ctl_solve_result()
         self._call(self._lib.ctl_solve_host, b_host.ctypes.data, u_host.ctypes.data, C.byref(o), C.byref(res))
         return KSPInfo(res)
@@ -455,10 +506,7 @@ class MultiBlockSystem:
     def objective_device(self, v_dev, zeta_dev, v_hat_dev):
         """J_h from device arrays of n_t levels x n_local (level-major; this rank's rows), evaluated on the GPU;
         on several ranks every rank receives the global value."""
-        need = self.n_t * self.n_local
-        for t in (v_dev, zeta_dev, v_hat_dev):
-            if t.numel() != need or t.dtype != torch.float64 or not t.is_cuda or not t.is_contiguous():
-                raise ValueError("objective_device needs contiguous float64 CUDA tensors of n_t * n_local entries")
+        self._check_vecs("objective_device", v_dev, zeta_dev, v_hat_dev, count=self.n_t * self.n_local)
         out = C.c_double()
         self._call(self._lib.ctl_objective, v_dev.data_ptr(), zeta_dev.data_ptr(), v_hat_dev.data_ptr(), C.byref(out))
         return float(out.value)
@@ -468,10 +516,7 @@ class MultiBlockSystem:
         (n_t levels x n_local each: this rank's rows); ``v_0``: host initial condition (all n entries) or None
         (``ctl_build_rhs``).  ``bc_values``: None (homogeneous Dirichlet data) or the (n_t, len(bc_dofs))
         boundary values of the state, lifted in with ``lift_bc_device``."""
-        need = self.n_t * self.n_local
-        for t in (v_hat_dev, f_nodal_dev):
-            if t.numel() != need or t.dtype != torch.float64 or not t.is_cuda or not t.is_contiguous():
-                raise ValueError("build_rhs_device needs contiguous float64 CUDA tensors of n_t * n_local entries")
+        self._check_vecs("build_rhs_device", v_hat_dev, f_nodal_dev, count=self.n_t * self.n_local)
         if v_0 is not None and np.size(v_0) != self.n:
             raise ValueError("build_rhs_device: v_0 must hold all n entries")
         b = self.new_vector()
@@ -499,9 +544,7 @@ class MultiBlockSystem:
         values the system holds, T_1 / T_2 applied, constrained rows untouched.  ``g``: (n_t, len(bc_dofs)) host array
         or CUDA tensor, columns in the order of ``bc_dofs`` (what ``Control.Instationary._dirichlet_data`` returns);
         every rank passes all of it.  Returns ``b_dev``."""
-        if b_dev.numel() != self.vec_len(layout) or b_dev.dtype != torch.float64 or not b_dev.is_cuda \
-                or not b_dev.is_contiguous():
-            raise ValueError("lift_bc_device needs a contiguous float64 CUDA vector of vec_len(layout) entries")
+        self._check_vecs("lift_bc_device", b_dev, layout=layout)
         g_dev = self._bc_values_device(g)
         self._call(self._lib.ctl_lift_bc, g_dev.data_ptr(), b_dev.data_ptr(), layout)
         return b_dev

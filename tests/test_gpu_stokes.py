@@ -131,12 +131,13 @@ def test_stokes_solve_matches_oracle(CN):
     s.close()
 
 
-def test_stokes_user_preconditioner_hook():
+def test_stokes_user_preconditioner_hook(capsys):
     """``P=`` of ``incompressible_linear_solve`` (control/control.py:3592-3594, 4686-4689): a user callable
     ``pc_fn(u_0, u_1, b_0, b_1)`` on the blocks of the outer system, called through ctl_stokes_set_pc_callback.  Handing
     the in-built preconditioner back in as the user's P must reproduce the in-built solve (same count, same solution);
     the callable sees projected right-hand sides (Dirichlet rows zero, pressure blocks mean free) and zero u's; an
-    exception inside it surfaces as the reference's RuntimeError."""
+    exception inside it surfaces as the reference's RuntimeError, and the next solve starts afresh.  The solve prints
+    its residual history exactly when ``monitor_convergence`` is set."""
     q = _problem(6, 5, True)
     th, N = q["th"], q["N"]
     s = _system(q)
@@ -170,8 +171,13 @@ def test_stokes_user_preconditioner_hook():
         raise ValueError("user preconditioner failed")
     with pytest.raises(Exception):
         s.solve(np.zeros_like(xr0), np.zeros_like(xr1), b0, b1, solver_parameters=sp_, pc_fn=broken)
-    from control_b200 import system as sysm
-    sysm._error_flag[0] = False
+    capsys.readouterr()
+    info = s.solve(np.zeros_like(xr0), np.zeros_like(xr1), b0, b1, solver_parameters=dict(sp_, monitor_convergence=False))
+    assert info.reason > 0 and abs(info.its - ref.its) <= 1
+    assert capsys.readouterr().out == ""
+    info = s.solve(np.zeros_like(xr0), np.zeros_like(xr1), b0, b1, solver_parameters=dict(sp_, monitor_convergence=True))
+    assert len(info.history) > 1 and capsys.readouterr().out.splitlines() == \
+        [f"KSP: iteration {it:d}, residual norm {r:.16e}" for it, r in enumerate(info.history)]
     s.close()
 
 

@@ -304,3 +304,45 @@ def test_instationary_non_linear_loop_with_inhomogeneous_data_host_logic(fake_de
     assert np.array_equal(c._v[1:, q["bdofs"]], g[1:])
     if not gauss_newton:                                  # (the Gauss-Newton variant of the reference evaluates the
         assert ref["history"][-1] < 0.2 * ref["history"][0]   # residual with the Jacobian, DESIGN.md section 1 row a11)
+
+
+def _loop_lines(history):
+    return [f"Initial non-linear residual: {history[0]:.16e}"] + \
+        [f"Non-linear solver: iteration {k:d}, non-linear residual norm {h:.16e}" for k, h in enumerate(history[1:], 1)]
+
+
+def test_outer_loop_output(fake_device, capsys):
+    """What a heat and a Navier-Stokes loop print with ``print_error_non_linear``: the first residual norm, then one
+    line per outer iteration, formatted as the reference's loops (control/control.py:3377-3590, 4886-5219) format
+    them, and nothing else when the inner solves are quiet; ``max_non_linear_iter`` stops both after the second."""
+    Control = fake_device
+    quiet = dict(SP, monitor_convergence=False)
+    q = kat.heat_problem(6, 5, True, beta=1e-2)
+    Dv = fem.nonlinear_diffusion_p1_2d(6, 6, 2.0, 2.0)
+
+    def level(t):
+        return int(round(t / q["tau"]))
+    c = Control.Instationary(q["M"], lambda v, t, gn: Dv(v, gn), desired_state=lambda t: (q["v_d"][level(t)], q["v_hat"][level(t)]),
+                             force_f=lambda t: q["f"][level(t)], beta=q["beta"], n_t=5, CN=True,
+                             time_interval=q["time_interval"], bc_dofs=q["bdofs"])
+    capsys.readouterr()
+    k = c.non_linear_solve(lambda_v_bounds=q["lambda_v_bounds"], solver_parameters=quiet, max_non_linear_iter=2,
+                           print_error_non_linear=True, device_loop=False)
+    assert k == 2 and len(c.non_linear_history) == 3
+    assert capsys.readouterr().out.splitlines() == _loop_lines(c.non_linear_history)
+
+    q = kat.reference_navier_stokes_problem(False, nx=4, n_t=6)
+    sq = q["sq"]
+
+    def level(t):
+        return int(round(t / q["tau"]))
+    c = Control.Instationary(q["M"], lambda v_i, t, gn: q["D_v"](v_i, t),
+                             desired_state=lambda t: (q["v_d"][level(t)], q["v_hat"][level(t)]), beta=q["beta"],
+                             n_t=q["n_t"], CN=False, time_interval=q["time_interval"], bc_dofs=q["bdofs"],
+                             bc_values=lambda t: q["bc_values"][level(t)])
+    space_p = dict(B=q["B"], M_p=sq["M_p"], K_p=sq["L_p"], forward_matrix_p=lambda v_i, t, gn: q["D_p"](v_i, t))
+    capsys.readouterr()
+    k = c.incompressible_non_linear_solve("constant", space_p=space_p, solver_parameters=quiet, max_non_linear_iter=2,
+                                          lambda_v_bounds=q["lambda_v_bounds"], lambda_p_bounds=q["lambda_p_bounds"])
+    assert k == 2 and len(c.non_linear_history) == 3 and len(c.inner_iterations) == 2
+    assert capsys.readouterr().out.splitlines() == _loop_lines(c.non_linear_history)

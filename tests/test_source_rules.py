@@ -89,3 +89,14 @@ def test_device_resources_are_released_only_by_their_owning_types():
         assert "cudaEventDestroy" not in src, f"{name}: events are destroyed by EventPair ({owner})"
         assert not re.search(r"\b(pool|free_)\s*\.\s*(push_back|pop_back)\b", src), \
             f"{name}: scratch vectors are leased with ScratchPool::take ({owner})"
+
+
+def test_host_paths_are_written_once():
+    """The host layer has one outer-loop function (the first-residual print of every Picard / Gauss-Newton loop), one
+    callback trampoline, one mapping of a preconditioner choice to CTL_PC_CALLBACK and one print of the Krylov history,
+    shared by the heat and the Stokes systems and by every driver -- copies of them had drifted apart."""
+    pkg = os.path.join(ROOT, "control_b200")
+    srcs = {f: open(os.path.join(pkg, f)).read() for f in sorted(os.listdir(pkg)) if f.endswith(".py")}
+    for needle in ("Initial non-linear residual", "PC_CALLBACK(", "L.CTL_PC_CALLBACK", "KSP: iteration"):
+        counts = {f: s.count(needle) for f, s in srcs.items() if needle in s}
+        assert len(counts) == 1 and sum(counts.values()) == 1, f"{needle!r} written {counts}"
