@@ -312,10 +312,14 @@ class Control:
             """The ``StokesSystem`` of this instance, created on first use, with the forward matrices K, D_p."""
             from .stokes import StokesSystem
             if getattr(self, "_stokes", None) is None:
+                world = self._dev["world"]
+                ranks = dict(rank=self._dev["rank"], world=world) if world > 1 else {}
                 self._stokes = StokesSystem(self._M, K, space_p["B"], space_p["M_p"], space_p["K_p"], n_t=self._n_t,
                                             beta=self._beta, CN=self._CN, time_interval=self._time_interval,
                                             bc_dofs_v=self._bc_dofs, device=self._dev["device"], D_p=D_p,
-                                            **self._block_kw("velocity_block_size"))
+                                            **self._block_kw("velocity_block_size"), **ranks)
+                if world > 1:
+                    self._stokes.init_comm()
             elif not self._is_linear():
                 self._stokes.set_forward(K, D_p)
             return self._stokes
@@ -328,7 +332,10 @@ class Control:
             of the constructor, inhomogeneous and time dependent; a callable forward matrix is evaluated
             at the current ``_v`` per time level, with ``space_p["forward_matrix_p"]`` on the pressure space).  ``nullspace_p``: None or "constant" -- the pressure blocks
             carry ConstantNullspace as in every caller of the reference (test/test_control.py,
-            README.md).  Sets ``_v``, ``_zeta``, ``_p``, ``_mu`` and returns the KSP information."""
+            README.md).  Sets ``_v``, ``_zeta``, ``_p``, ``_mu`` and returns the KSP information.  On several ranks
+            each solves for its own rows and every rank receives the whole solution; ``P=`` runs on one rank."""
+            if P is not None and self._dev["world"] > 1:
+                raise ValueError("P= runs on one rank: the user preconditioner sees host block arrays of all rows")
             if space_p is None:
                 space_p = getattr(self, "_space_p", None)
                 if space_p is None:
@@ -368,10 +375,16 @@ class Control:
             if P is None:                                           # control.py:4686-4689: pc_fn = P or the in-built one
                 system.setup_preconditioner(lambda_v_bounds=lambda_v_bounds, lambda_p_bounds=lambda_p_bounds, amg=amg,
                                             amg_p=amg_p, Multigrid=Multigrid)
-            u_0 = np.zeros((2 * N, n))
-            u_1 = np.zeros((2 * N, n_p))
+            several = self._dev["world"] > 1
+            if several:                                         # this rank's rows in, every rank's rows out
+                b_0 = np.ascontiguousarray(b_0[:, system.velocity_rows])
+                b_1 = np.ascontiguousarray(b_1[:, system.pressure_rows])
+            u_0 = np.zeros(b_0.shape)
+            u_1 = np.zeros(b_1.shape)
             self.last_ksp = system.solve(u_0, u_1, b_0, b_1, solver_parameters=solver_parameters,
                                          pc_fn="builtin" if P is None else P)
+            if several:
+                u_0, u_1 = system.allgather_blocks(u_0, u_1)
             self._store_blocks(u_0[:N], u_0[N:], v_0 if check_f and check_v_d else None, g)     # 4705-4725
             self._p, self._mu = u_1[N:].copy(), u_1[:N].copy()
             return self.last_ksp
@@ -390,9 +403,14 @@ class Control:
             (``_incompressible_non_linear_solve_device``; in-built preconditioner only, so ``P=`` raises
             ``ValueError``); False or None runs the host loop, which evaluates the residual on the host and moves the
             whole outer vector both ways every iteration.  None stays the host loop for now because the stand-in
-            systems that exercise both loops on inhomogeneous data have no device methods."""
+            systems that exercise both loops on inhomogeneous data have no device methods.  On several ranks only the
+            host loop with the in-built preconditioner runs: ``device_loop=True`` or ``P=`` raise ``ValueError``."""
             if device_loop and P is not None:
                 raise ValueError("device_loop=True runs the in-built preconditioner; it does not take P=")
+            if device_loop and self._dev["world"] > 1:
+                raise ValueError("device_loop=True runs on one rank")
+            if P is not None and self._dev["world"] > 1:
+                raise ValueError("P= runs on one rank: the user preconditioner sees host block arrays of all rows")
             if space_p is None:
                 space_p = getattr(self, "_space_p", None)
                 if space_p is None:

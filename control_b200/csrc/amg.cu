@@ -24,8 +24,8 @@
 
 #include "cheb_coefficients.h"
 
-int amg_build_distributed(ctl_handle_s *h, const AmgParams &p, const std::shared_ptr<SellPattern> &fine_pattern,
-                          AmgHierarchyDev &H);      // halo.cu
+int amg_build_distributed(ctl_handle_s *h, PcState *xs, const AmgParams &p,
+                          const std::shared_ptr<SellPattern> &fine_pattern, AmgHierarchyDev &H);      // halo.cu
 
 static int dev_alloc(ctl_handle_s *h, double **p, size_t n)
 {
@@ -74,7 +74,7 @@ int64_t amg_cycle_bytes(const AmgHierarchyDev &H)
 }
 
 int amg_build(ctl_handle_s *h, const HostCSR &A0, const AmgParams &p,
-              const std::shared_ptr<SellPattern> &fine_pattern, AmgHierarchyDev &H)
+              const std::shared_ptr<SellPattern> &fine_pattern, AmgHierarchyDev &H, PcState *xs)
 {
     H.params = p;
     try {
@@ -88,7 +88,7 @@ int amg_build(ctl_handle_s *h, const HostCSR &A0, const AmgParams &p,
     CTL_CHECK(H.nc == 1 || h->cfg.world == 1, CTL_ERR_ARG, "amg_build: block hierarchies run on one GPU only");
     if (h->cfg.world > 1) {
         CTL_CHECK(nl > 1, CTL_ERR_ARG, "amg_build: the problem is too small for a multi-rank hierarchy (single level)");
-        CTL_TRY(amg_build_distributed(h, p, fine_pattern, H));
+        CTL_TRY(amg_build_distributed(h, xs, p, fine_pattern, H));
     } else {
         for (int l = 0; l < nl; ++l) {
             AmgLevelHost &Lh = H.host[l];

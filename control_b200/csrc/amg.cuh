@@ -32,9 +32,11 @@ struct AmgHierarchyDev {
 };
 
 // A0 on level 0 may share an existing SELL pattern (fine-level matrices all have the
-// mesh pattern); pass nullptr to build one.
+// mesh pattern); pass nullptr to build one.  Multi-GPU: `xs` holds the exchange state the hierarchy's plans join
+// (mesh geometry, level-0 plans, arena; see pc_mesh_exchange); null = the handle's preconditioner state.
+struct PcState;
 int amg_build(ctl_handle_s *h, const HostCSR &A0, const AmgParams &p,
-              const std::shared_ptr<SellPattern> &fine_pattern, AmgHierarchyDev &H);
+              const std::shared_ptr<SellPattern> &fine_pattern, AmgHierarchyDev &H, PcState *xs = nullptr);
 void amg_free(AmgHierarchyDev &H);
 // dense_inverse.cu: (A + shift shift^T)^-1 (- shift shift^T when shift is given: the pseudo-inverse of a singular
 // symmetric A with normalised kernel vector shift), computed on the device with the host algorithm's arithmetic;

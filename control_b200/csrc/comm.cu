@@ -22,8 +22,6 @@ void ctl_comm_free(ctl_handle_s *h)
 {
     if (!h->comm) return;
     CommState &c = *h->comm;
-    cudaFree(c.d_send_rows);
-    cudaFree(c.d_sendbuf);
     cudaFree(c.d_epoch);
     cudaFree(c.d_err);
     cudaFree(c.d_barrier);
@@ -32,13 +30,6 @@ void ctl_comm_free(ctl_handle_s *h)
 }
 
 namespace {
-
-void owner_range(int n, int world, int rank, int *begin, int *count)
-{
-    const int base = n / world, rem = n % world;
-    *count = base + (rank < rem ? 1 : 0);
-    *begin = rank * base + std::min(rank, rem);
-}
 
 // gather rows of a [rows x width] row-major array: out[i, :] = in[rows[i], :]
 __global__ void pack_rows_kernel(const double *__restrict__ in, const int *__restrict__ rows, int n_rows, int width,
@@ -52,72 +43,49 @@ __global__ void pack_rows_kernel(const double *__restrict__ in, const int *__res
 
 }  // namespace
 
-// plan: ghosts of every rank owned by me (send) and my ghosts owned by every rank (recv)
-static int build_plan(ctl_handle_s *h, CommState &c)
+int exchange_plan_build(ctl_handle_s *h, const int *ip, const int *ix, int n_rows, int n_cols, int world, int me,
+                        ExchangePlan &P)
 {
-    const int n = h->n, world = c.world, me = c.rank;
-    const std::vector<int> &ip = h->h_indptr, &ix = h->h_indices;
-    int my_b, my_c;
-    owner_range(n, world, me, &my_b, &my_c);
-    std::vector<int> send_rows;
-    for (int p = 0; p < world; ++p) {
-        if (p == me) continue;
-        int pb, pc;
-        owner_range(n, world, p, &pb, &pc);
-        // what p needs from me: columns in my range referenced by p's rows (sorted, unique):
-        // exactly the segment of p's ghost list that I own, in p's ghost order
-        std::vector<int> need;
-        for (int r = pb; r < pb + pc; ++r)
-            for (int k = ip[r]; k < ip[r + 1]; ++k)
-                if (ix[k] >= my_b && ix[k] < my_b + my_c) need.push_back(ix[k]);
-        std::sort(need.begin(), need.end());
-        need.erase(std::unique(need.begin(), need.end()), need.end());
-        // what I need from p: my ghosts in p's range (halo_global is sorted by global id)
-        const auto lo = std::lower_bound(h->halo_global.begin(), h->halo_global.end(), pb);
-        const auto hi = std::lower_bound(h->halo_global.begin(), h->halo_global.end(), pb + pc);
-        const int rc = (int)(hi - lo);
-        if (need.empty() && rc == 0) continue;
-        c.peers.push_back(p);
-        c.recv_off.push_back((int)(lo - h->halo_global.begin()));
-        c.recv_cnt.push_back(rc);
-        c.send_off.push_back((int)send_rows.size());
-        c.send_cnt.push_back((int)need.size());
-        for (int g : need) send_rows.push_back(g - my_b);
-    }
-    c.n_send = (int)send_rows.size();
-    CTL_TRY(ctl_upload(h, &c.d_send_rows, send_rows.data(), send_rows.size()));
-    if (c.n_send > 0)
-        CTL_CUDA(cudaMalloc((void **)&c.d_sendbuf, (size_t)2 * c.n_send * h->ld * sizeof(double)));
+    exchange_lists(ip, ix, n_rows, n_cols, world, me, P);
+    P.n_send = (int)P.send_rows.size();
+    CTL_TRY(ctl_upload(h, &P.d_send_rows, P.send_rows.data(), P.send_rows.size()));
+    if (P.n_send > 0)
+        CTL_CUDA(cudaMalloc((void **)&P.d_sendbuf, (size_t)2 * P.n_send * h->ld * sizeof(double)));
     return CTL_OK;
 }
 
-// exchange `panels` time-fastest panels: ghost rows land in h->d_halo[p]
-static int exchange_panels(ctl_handle_s *h, const double *x_tf, int panels)
+int exchange_plan_run(ctl_handle_s *h, ncclComm_t comm, const ExchangePlan &P, const double *x_tf,
+                      size_t panel_stride, int panels, double *ghost)
 {
-    CommState &c = *h->comm;
     const int ld = h->ld;
-    const size_t panel = (size_t)h->n_loc * ld;
+    const size_t n_ghost = P.ghosts.size();
     for (int p = 0; p < panels; ++p) {
-        if (c.n_send == 0) break;
-        const int64_t total = (int64_t)c.n_send * ld;
-        pack_rows_kernel<<<ceil_div(total, 256), 256, 0, h->stream>>>(x_tf + p * panel, c.d_send_rows, c.n_send, ld,
-                                                                     c.d_sendbuf + (size_t)p * c.n_send * ld);
+        if (P.n_send == 0) break;
+        const int64_t total = (int64_t)P.n_send * ld;
+        pack_rows_kernel<<<ceil_div(total, 256), 256, 0, h->stream>>>(x_tf + p * panel_stride, P.d_send_rows, P.n_send,
+                                                                     ld, P.d_sendbuf + (size_t)p * P.n_send * ld);
         h->launches++;
     }
     CTL_CUDA(cudaGetLastError());
     CTL_NCCL(ncclGroupStart());
-    for (size_t i = 0; i < c.peers.size(); ++i) {
+    for (size_t i = 0; i < P.peers.size(); ++i) {
         for (int p = 0; p < panels; ++p) {
-            if (c.send_cnt[i])
-                CTL_NCCL(ncclSend(c.d_sendbuf + ((size_t)p * c.n_send + c.send_off[i]) * ld, (size_t)c.send_cnt[i] * ld,
-                                  ncclDouble, c.peers[i], c.comm, h->stream));
-            if (c.recv_cnt[i])
-                CTL_NCCL(ncclRecv(h->d_halo + ((size_t)p * h->n_halo + c.recv_off[i]) * ld, (size_t)c.recv_cnt[i] * ld,
-                                  ncclDouble, c.peers[i], c.comm, h->stream));
+            if (P.send_cnt[i])
+                CTL_NCCL(ncclSend(P.d_sendbuf + ((size_t)p * P.n_send + P.send_off[i]) * ld, (size_t)P.send_cnt[i] * ld,
+                                  ncclDouble, P.peers[i], comm, h->stream));
+            if (P.recv_cnt[i])
+                CTL_NCCL(ncclRecv(ghost + ((size_t)p * n_ghost + P.recv_off[i]) * ld, (size_t)P.recv_cnt[i] * ld,
+                                  ncclDouble, P.peers[i], comm, h->stream));
         }
     }
     CTL_NCCL(ncclGroupEnd());
     return CTL_OK;
+}
+
+// exchange `panels` time-fastest panels through the mesh pattern: ghost rows land in h->d_halo[p]
+static int exchange_panels(ctl_handle_s *h, const double *x_tf, int panels)
+{
+    return exchange_plan_run(h, h->comm->comm, h->comm->mesh, x_tf, (size_t)h->n_loc * h->ld, panels, h->d_halo);
 }
 
 int ctl_halo_exchange(ctl_handle_s *h, const double *x_tf)
@@ -180,7 +148,8 @@ int ctl_comm_init(ctl_handle h, const void *id128)
     ncclUniqueId id;
     memcpy(&id, id128, sizeof(id));
     CTL_NCCL(ncclCommInitRank(&c.comm, c.world, id, c.rank));
-    CTL_TRY(build_plan(h, c));
+    CTL_TRY(exchange_plan_build(h, h->h_indptr.data(), h->h_indices.data(), h->n, h->n, c.world, c.rank, c.mesh));
+    CTL_CHECK(c.mesh.ghosts == h->halo_global, CTL_ERR_STATE, "ctl_comm_init: exchange plan and local pattern disagree");
     // device words of the in-kernel exchange (halo.cu)
     CTL_CUDA(cudaMalloc((void **)&c.d_epoch, sizeof(unsigned long long)));
     CTL_CUDA(cudaMemset(c.d_epoch, 0, sizeof(unsigned long long)));

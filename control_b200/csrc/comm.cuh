@@ -6,18 +6,37 @@
 #include <vector>
 
 #include "common.cuh"
+#include "exchange_plan.h"
 #include "halo.cuh"
+
+// NCCL exchange of time-fastest panels through a sparsity pattern (exchange_plan.h): the host lists, and the packed
+// row list and send buffer on the device
+struct ExchangePlan : ExchangeLists {
+    int n_send = 0;
+    int *d_send_rows = nullptr;           // send_rows on the device
+    double *d_sendbuf = nullptr;          // [2][n_send x ld]
+    ExchangePlan() = default;
+    ExchangePlan(const ExchangePlan &) = delete;
+    ExchangePlan &operator=(const ExchangePlan &) = delete;
+    ~ExchangePlan()
+    {
+        cudaFree(d_send_rows);
+        cudaFree(d_sendbuf);
+    }
+};
+
+// the plan of the rows [row split of n_rows] of a global CSR pattern over the columns [column split of n_cols]
+int exchange_plan_build(ctl_handle_s *h, const int *indptr, const int *indices, int n_rows, int n_cols, int world,
+                        int rank, ExchangePlan &P);
+// exchange `panels` time-fastest panels of x_tf (panel_stride doubles apart): the ghost rows land in
+// ghost[p][n_ghost x ld]
+int exchange_plan_run(ctl_handle_s *h, ncclComm_t comm, const ExchangePlan &P, const double *x_tf,
+                      size_t panel_stride, int panels, double *ghost);
 
 struct CommState {
     ncclComm_t comm = nullptr;
     int rank = 0, world = 1;
-    // ---- NCCL exchange of time-fastest panels (KKT apply, batched Chebyshev, Schur right-hand side)
-    std::vector<int> peers;               // ranks we exchange with
-    std::vector<int> recv_off, recv_cnt;  // ghost segment of each peer (rows)
-    std::vector<int> send_off, send_cnt;  // segment of each peer in the packed send list
-    int n_send = 0;
-    int *d_send_rows = nullptr;           // owned local rows to pack, peer after peer
-    double *d_sendbuf = nullptr;          // [2][n_send x ld]
+    ExchangePlan mesh;                    // KKT apply, batched Chebyshev, Schur right-hand side
     // ---- device-initiated exchange (halo.cu)
     unsigned long long *d_epoch = nullptr;    // bumped once per sweep replay, after a barrier across ranks
     int *d_err = nullptr;                     // a bounded wait gave up

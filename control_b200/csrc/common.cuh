@@ -237,10 +237,11 @@ void ctl_pc_free(ctl_handle_s *h);        // pc.cu
 void ctl_comm_free(ctl_handle_s *h);      // comm.cu
 int ctl_pc_invalidate(ctl_handle_s *h);   // pc.cu: matrices changed, rebuild on next setup
 void ctl_lift_invalidate(ctl_handle_s *h);   // lift.cu: M, K or the Dirichlet dofs changed
-// lift.cu: the constrained-velocity columns of the divergence matrix B (n_p x n_v host CSR, values before
-// elimination; columns in the ctl_set_bc list of the velocity handle h), and b_1_0 -= T_2(tau B g) on them
+// lift.cu: the constrained-velocity columns of the divergence matrix B (n_p x n_v global host CSR, values before
+// elimination; columns in the ctl_set_bc list of the velocity handle h) in the n_rows rows from row_begin (this rank's
+// pressure rows, numbered locally), and b_1_0 -= T_2(tau B g) on them
 int ctl_lift_div_setup(ctl_handle_s *h, const int32_t *B_indptr, const int32_t *B_indices, const double *B_values,
-                       int n_p, std::shared_ptr<struct LiftState> *out);
+                       int row_begin, int n_rows, std::shared_ptr<struct LiftState> *out);
 int ctl_lift_div_apply(ctl_handle_s *h, const struct LiftState *S, const double *g, double *b10, int n_p);
 // comm.cu
 int ctl_halo_exchange(ctl_handle_s *h, const double *x_tf);            // both panels -> d_halo

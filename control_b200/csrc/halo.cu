@@ -59,14 +59,47 @@ int halo_space_upload(ctl_handle_s *h, const std::shared_ptr<HaloGeom> &g, std::
 // ---------------------------------------------------------------------------------------------------------
 static size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
 
+// all ranks have drained their streams up to here: an all-reduce of one word, then a host wait.  Returns false (and
+// records why on h) when the barrier could not be enqueued or completed: the caller must then not release memory that
+// the peers may still write or map.
+static bool arena_barrier(ctl_handle_s *h)
+{
+    CommState &c = *h->comm;
+    const ncclResult_t r = ncclAllReduce(c.d_barrier, c.d_barrier, 1, ncclInt, ncclMax, c.comm, h->stream);
+    if (r != ncclSuccess) {
+        ctl_set_error(h, std::string("halo arena release: barrier failed: ") + ncclGetErrorString(r));
+        return false;
+    }
+    const cudaError_t e = cudaStreamSynchronize(h->stream);
+    if (e != cudaSuccess) {
+        ctl_set_error(h, std::string("halo arena release: barrier failed: ") + cudaGetErrorString(e));
+        return false;
+    }
+    return true;
+}
+
+// Collective on several ranks: every peer writes into this rank's arena, and this rank into theirs.  The first barrier
+// makes sure that no peer's last push into our slots is still in flight when the mappings go away; the second that no
+// peer still holds a mapping of our arena when it is freed (a set-up per Picard iteration makes this the common case).
+// When a barrier fails, the mappings and the arena are left in place (leaked) rather than released under a peer that
+// may still use them; the error text stays on h.
 void halo_arena_free(ctl_handle_s *h, HaloArena &a)
 {
+    const bool shared = a.finalized && h->comm && h->comm->comm;
     if (h->comm) {
         std::vector<HaloPlan *> &live = h->comm->plans;
         for (HaloArena::Inst &i : a.inst) live.erase(std::remove(live.begin(), live.end(), i.plan.get()), live.end());
     }
     for (HaloArena::Inst &i : a.inst) cudaFree(i.d_dsts);
+    if (shared && !arena_barrier(h)) {
+        a = HaloArena();
+        return;
+    }
     for (void *p : a.opened) cudaIpcCloseMemHandle(p);
+    if (shared && !arena_barrier(h)) {
+        a = HaloArena();
+        return;
+    }
     cudaFree(a.base);
     a = HaloArena();
 }
@@ -294,15 +327,16 @@ static void finish_matrix(const HostCSR &, int n_own_cols, SellMat &M)
     if (n_own_cols > 0) M.n_own = n_own_cols;      // columns behind it are ghosts
 }
 
-int amg_build_distributed(ctl_handle_s *h, const AmgParams &p, const std::shared_ptr<SellPattern> &fine_pattern,
-                          AmgHierarchyDev &H)
+int amg_build_distributed(ctl_handle_s *h, PcState *xs, const AmgParams &p,
+                          const std::shared_ptr<SellPattern> &fine_pattern, AmgHierarchyDev &H)
 {
-    CTL_CHECK(h->pc && h->pc->mesh_space, CTL_ERR_STATE, "amg_build: the exchange geometry of the mesh is missing");
+    if (!xs) xs = h->pc.get();
+    CTL_CHECK(xs && xs->mesh_space, CTL_ERR_STATE, "amg_build: the exchange geometry of the mesh is missing");
     CTL_CHECK(fine_pattern != nullptr, CTL_ERR_ARG, "amg_build: level 0 needs the mesh pattern");
     CTL_CHECK(p.nu >= 3 && (p.nu_fine == 0 || p.nu_fine >= 3), CTL_ERR_ARG,
               "amg_build: smoother degrees below 3 are not supported on several GPUs");
     CTL_CHECK(p.acc_lo <= 0.0, CTL_ERR_ARG, "amg_build: accelerated cycles are not supported on several GPUs");
-    PcState &st = *h->pc;
+    PcState &st = *xs;
     const int world = h->cfg.world, me = h->cfg.rank;
     const int nl = (int)H.host.size();
     // A coarse level with fewer matrix entries per rank than this (and everything below it) is replicated.  Measured

@@ -189,13 +189,13 @@ int lift_build(ctl_handle_s *h)
 void ctl_lift_invalidate(ctl_handle_s *h) { h->lift.reset(); }
 
 int ctl_lift_div_setup(ctl_handle_s *h, const int32_t *B_indptr, const int32_t *B_indices, const double *B_values,
-                       int n_p, std::shared_ptr<LiftState> *out)
+                       int row_begin, int n_rows, std::shared_ptr<LiftState> *out)
 {
     const std::vector<int> col_slot = bc_slots(h);
     std::vector<int> rows, ptr(1, 0), slot;
     std::vector<double> A;
-    for (int r = 0; r < n_p; ++r) {
-        for (int k = B_indptr[r]; k < B_indptr[r + 1]; ++k)
+    for (int r = 0; r < n_rows; ++r) {
+        for (int k = B_indptr[row_begin + r]; k < B_indptr[row_begin + r + 1]; ++k)
             if (col_slot[B_indices[k]] >= 0) {
                 slot.push_back(col_slot[B_indices[k]]);
                 A.push_back(B_values[k]);

@@ -174,6 +174,26 @@ int ctl_pc_invalidate(ctl_handle_s *h)
     return CTL_OK;
 }
 
+int pc_mesh_exchange(ctl_handle_s *h, PcState &st)
+{
+    std::vector<int> part0(h->cfg.world + 1, 0);
+    for (int r = 0; r < h->cfg.world; ++r) {
+        const int base = h->n / h->cfg.world, rem = h->n % h->cfg.world;
+        part0[r + 1] = part0[r] + base + (r < rem ? 1 : 0);
+    }
+    SpaceConsumer mesh;
+    mesh.n_rows = h->n;
+    mesh.indptr = h->h_indptr.data();
+    mesh.indices = h->h_indices.data();
+    mesh.row_part = part0.data();
+    auto geom = std::make_shared<HaloGeom>();
+    halo_geometry(h->cfg.world, h->cfg.rank, part0, {mesh}, false, *geom);
+    CTL_TRY(halo_space_upload(h, geom, st.mesh_space));
+    st.px0 = halo_arena_add(h, st.arena, st.mesh_space);
+    st.pb0 = halo_arena_add(h, st.arena, st.mesh_space);
+    return CTL_OK;
+}
+
 // a sweep vector with its ghosts behind the owned entries (multi-GPU: completed by halo_persist right after the
 // solve that produced it, so later products need not wait)
 static GVec ts_vec(const PcState &st, const double *v, int n_loc)
@@ -487,23 +507,7 @@ int ctl_pc_setup(ctl_handle h, const ctl_pc_options *opts)
     lap("transposition map, mass dinv");
     // multi-GPU: exchange geometry of everything that gathers through the mesh pattern, and the two level-0
     // exchange streams (iterates, right-hand sides) every hierarchy shares
-    if (h->cfg.world > 1) {
-        std::vector<int> part0(h->cfg.world + 1, 0);
-        for (int r = 0; r < h->cfg.world; ++r) {
-            const int base = h->n / h->cfg.world, rem = h->n % h->cfg.world;
-            part0[r + 1] = part0[r] + base + (r < rem ? 1 : 0);
-        }
-        SpaceConsumer mesh;
-        mesh.n_rows = h->n;
-        mesh.indptr = h->h_indptr.data();
-        mesh.indices = h->h_indices.data();
-        mesh.row_part = part0.data();
-        auto geom = std::make_shared<HaloGeom>();
-        halo_geometry(h->cfg.world, h->cfg.rank, part0, {mesh}, false, *geom);
-        CTL_TRY(halo_space_upload(h, geom, st.mesh_space));
-        st.px0 = halo_arena_add(h, st.arena, st.mesh_space);
-        st.pb0 = halo_arena_add(h, st.arena, st.mesh_space);
-    }
+    if (h->cfg.world > 1) CTL_TRY(pc_mesh_exchange(h, st));
     auto mesh_matrix = [&](SellMat &m) {
         if (h->cfg.world > 1) m.n_own = h->n_loc;
     };

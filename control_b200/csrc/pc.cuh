@@ -17,6 +17,11 @@ int pcb_bc_fixup(ctl_handle_s *h, const int *bc_rows, int n_bc, const double *wr
 int pcb_panel_to_ts(ctl_handle_s *h, const double *panel_tf, double *ts, size_t stride);
 int pcb_ts_to_panel(ctl_handle_s *h, const double *ts, double *panel_tf, size_t stride);
 
+struct PcState;
+// multi-GPU: the exchange geometry of the handle's mesh pattern and the two level-0 exchange streams (iterates,
+// right-hand sides) that every hierarchy built on `st` shares; finalise st.arena after the last amg_build
+int pc_mesh_exchange(ctl_handle_s *h, PcState &st);
+
 struct PcState {
     ctl_pc_options opts{};
     bool ready = false;

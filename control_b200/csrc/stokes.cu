@@ -13,9 +13,18 @@
 //   K_p solves     AMG cycles per time block on the Neumann Laplacian (4300-4309)
 //   M_p solves     batched Chebyshev/Jacobi on the pressure mass matrix (4311-4333)
 // Outer vectors in the internal layout: [velocity time-fastest vector | pressure one].
+//
+// Several ranks: the velocity and the pressure rows are each split over the ranks by PETSc's rule (the two handles'
+// own partitions).  Each rank keeps the rows of B for its pressure rows and the rows of B^T for its velocity rows;
+// before a divergence product the rows of the other space that its rows read and other ranks own ("ghosts") arrive
+// through NCCL (comm.cu: one exchange plan per product), and the ghost-aware product reads them from there.  The
+// per-block means of ConstantNullspace and the norm of the Picard residual add the ranks' partial sums in one
+// all-reduce; the K_p hierarchy is distributed like the sweep hierarchies, on an exchange state of its own.
+#include <cmath>
 #include <cstdlib>
 
 #include "cheb_coefficients.h"
+#include "comm.cuh"
 #include "krylov.cuh"
 #include "panel.cuh"
 
@@ -23,6 +32,7 @@ namespace {
 
 struct DevCSR {
     int n_rows = 0, n_cols = 0;
+    int n_own = 0;                // columns >= n_own are ghosts (several ranks)
     int *ptr = nullptr, *cols = nullptr;
     double *vals = nullptr;
 };
@@ -52,6 +62,11 @@ struct ctl_stokes_s {
     KrylovState ks;
     ctl_pc_callback pc_cb = nullptr;   // user preconditioner P= of incompressible_linear_solve (control/control.py:4686-4689)
     void *pc_cb_user = nullptr;
+    // several ranks
+    ExchangePlan xB, xBT;         // ghosts of tau B X_v (velocity rows) and of tau B^T X_p (pressure rows)
+    double *d_ghost_v = nullptr;  // [2 panels][xB.ghosts x ld]
+    double *d_ghost_p = nullptr;  // [2 panels][xBT.ghosts x ld]
+    std::unique_ptr<PcState> kp_x;   // exchange state (mesh geometry, level-0 plans, arena) of the K_p hierarchy
     int64_t len() const { return hv->vec_len() + hp->vec_len(); }
 };
 
@@ -59,13 +74,14 @@ namespace {
 
 constexpr int COLSUM_ROWS = 1024;   // rows per block of the column-sum kernel
 
-// out[r, :] (+)= T_inv( post * ( T_fwd(alpha * (A X)[r, :]) - sub[r, :] ) ), columns >= N zeroed
-template <int G, int CPL>
-__global__ void __launch_bounds__(256) panel_spmm_kernel(const int *__restrict__ ptr, const int *__restrict__ cols,
-                                                        const double *__restrict__ vals, const double *__restrict__ X,
-                                                        const double *__restrict__ sub, double *out, double alpha,
-                                                        double post, int t_fwd, int t_inv, int accumulate, int n_rows,
-                                                        int N, int ld)
+// out[r, :] (+)= T_inv( post * ( T_fwd(alpha * (A X)[r, :]) - sub[r, :] ) ), columns >= N zeroed.
+// HALO: columns >= n_own are ghost rows, read from the exchanged panel `ghost`.
+template <int G, int CPL, bool HALO>
+__device__ __forceinline__ void panel_spmm_rows(const int *__restrict__ ptr, const int *__restrict__ cols,
+                                                const double *__restrict__ vals, const double *__restrict__ X,
+                                                const double *__restrict__ ghost, int n_own,
+                                                const double *__restrict__ sub, double *out, double alpha, double post,
+                                                int t_fwd, int t_inv, int accumulate, int n_rows, int N, int ld)
 {
     const RowMap m = row_map<G, CPL>(n_rows);
     const size_t off = (size_t)m.r * ld + m.c0;
@@ -78,7 +94,8 @@ __global__ void __launch_bounds__(256) panel_spmm_kernel(const int *__restrict__
         const int col = __ldg(cols + k);
         const double v = __ldg(vals + k);
         double x[CPL];
-        load_cols<CPL>(X + (size_t)col * ld + m.c0, x);
+        if (HALO && col >= n_own) load_cols<CPL>(ghost + (size_t)(col - n_own) * ld + m.c0, x);
+        else load_cols<CPL>(X + (size_t)col * ld + m.c0, x);
 #pragma unroll
         for (int q = 0; q < CPL; ++q) acc[q] = fma(v, x[q], acc[q]);
     }
@@ -117,6 +134,29 @@ __global__ void __launch_bounds__(256) panel_spmm_kernel(const int *__restrict__
         }
     }
     store_cols<CPL>(out + off, acc);
+}
+
+template <int G, int CPL>
+__global__ void __launch_bounds__(256) panel_spmm_kernel(const int *__restrict__ ptr, const int *__restrict__ cols,
+                                                        const double *__restrict__ vals, const double *__restrict__ X,
+                                                        const double *__restrict__ sub, double *out, double alpha,
+                                                        double post, int t_fwd, int t_inv, int accumulate, int n_rows,
+                                                        int N, int ld)
+{
+    panel_spmm_rows<G, CPL, false>(ptr, cols, vals, X, nullptr, 0, sub, out, alpha, post, t_fwd, t_inv, accumulate,
+                                   n_rows, N, ld);
+}
+
+template <int G, int CPL>
+__global__ void __launch_bounds__(256) panel_spmm_halo_kernel(const int *__restrict__ ptr, const int *__restrict__ cols,
+                                                             const double *__restrict__ vals, const double *__restrict__ X,
+                                                             const double *__restrict__ ghost, int n_own,
+                                                             const double *__restrict__ sub, double *out, double alpha,
+                                                             double post, int t_fwd, int t_inv, int accumulate,
+                                                             int n_rows, int N, int ld)
+{
+    panel_spmm_rows<G, CPL, true>(ptr, cols, vals, X, ghost, n_own, sub, out, alpha, post, t_fwd, t_inv, accumulate,
+                                  n_rows, N, ld);
 }
 
 // in place: X[r, :] <- T_1^-1 / T_2^-1 X[r, :], columns >= N zeroed
@@ -161,7 +201,8 @@ __global__ void __launch_bounds__(256) colsum_partial_kernel(const double *__res
     }
 }
 
-// mean[panel][c] = sum_b part[panel][b][c] / n_rows   (one block per panel, ld threads)
+// mean[panel][c] = sum_b part[panel][b][c] / n_rows   (one block per panel, ld threads; several ranks: n_rows = 1,
+// the sums are all-reduced and then divided by mean_divide_kernel)
 __global__ void colsum_finish_kernel(const double *__restrict__ part, double *__restrict__ mean, int blocks, int ld,
                                      int n_rows)
 {
@@ -170,6 +211,13 @@ __global__ void colsum_finish_kernel(const double *__restrict__ part, double *__
     double s = 0.0;
     for (int b = 0; b < blocks; ++b) s += part[(size_t)b * ld + c];
     mean[blockIdx.x * ld + c] = s / (double)n_rows;
+}
+
+// mean[i] /= n for i < count: the means from the all-reduced sums of several ranks
+__global__ void mean_divide_kernel(double *mean, int count, double n)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < count) mean[i] /= n;
 }
 
 // Epilogue of ctl_stokes_nonlinear_residual, one pass over the four panels of an internal-layout outer vector
@@ -235,7 +283,9 @@ __global__ void __launch_bounds__(256) stokes_residual_kernel(const double *__re
     }
 }
 
-// out = sqrt(sum_b part[b]) in a fixed order (one block of 256 threads)
+// out = sqrt(sum_b part[b]) in a fixed order (one block of 256 threads); ROOT = false: the sum (several ranks add
+// theirs before the root is taken)
+template <bool ROOT>
 __global__ void __launch_bounds__(256) residual_finish_kernel(const double *__restrict__ part, int blocks,
                                                               double *__restrict__ out)
 {
@@ -248,7 +298,7 @@ __global__ void __launch_bounds__(256) residual_finish_kernel(const double *__re
         if (threadIdx.x < w) sh[threadIdx.x] += sh[threadIdx.x + w];
         __syncthreads();
     }
-    if (threadIdx.x == 0) *out = sqrt(sh[0]);
+    if (threadIdx.x == 0) *out = ROOT ? sqrt(sh[0]) : sh[0];
 }
 
 // out = v - mean_v (+ mean_w), both panels (2 * n_rows rows of ld columns)
@@ -275,10 +325,11 @@ __global__ void panel_rowscale_kernel(const double *__restrict__ in, const doubl
     out[i] = s * dinv[i / ld] * in[i];
 }
 
-int upload_csr(ctl_handle_s *h, const HostCSR &A, DevCSR &D)
+int upload_csr(ctl_handle_s *h, const HostCSR &A, int n_own, DevCSR &D)
 {
     D.n_rows = A.n_rows;
     D.n_cols = A.n_cols;
+    D.n_own = n_own;
     CTL_TRY(ctl_upload(h, &D.ptr, A.indptr.data(), A.indptr.size()));
     CTL_TRY(ctl_upload(h, &D.cols, A.indices.data(), A.indices.size()));
     CTL_TRY(ctl_upload(h, &D.vals, A.values.data(), A.values.size()));
@@ -293,15 +344,58 @@ void free_csr(DevCSR &D)
     D = DevCSR();
 }
 
-int panel_spmm(ctl_stokes_s *S, const DevCSR &A, const double *X, const double *sub, double *out, double alpha,
-               double post, int t_fwd, int t_inv, bool accumulate)
+// ghost: the exchanged panel of the ghost rows of X (matrices with ghost columns only)
+int panel_spmm(ctl_stokes_s *S, const DevCSR &A, const double *X, const double *ghost, const double *sub, double *out,
+               double alpha, double post, int t_fwd, int t_inv, bool accumulate)
 {
     ctl_handle_s *h = S->hv;
     const int ld = h->ld, nb = blocks_for(A.n_rows, ld);
-    DISPATCH_G(ld, (panel_spmm_kernel<GG, CC><<<nb, 256, 0, h->stream>>>(A.ptr, A.cols, A.vals, X, sub, out, alpha, post, t_fwd,
-                                                                   t_inv, accumulate ? 1 : 0, A.n_rows, h->N, ld)));
+    if (A.n_own < A.n_cols) {
+        DISPATCH_G(ld, (panel_spmm_halo_kernel<GG, CC><<<nb, 256, 0, h->stream>>>(A.ptr, A.cols, A.vals, X, ghost, A.n_own,
+                                                                            sub, out, alpha, post, t_fwd, t_inv,
+                                                                            accumulate ? 1 : 0, A.n_rows, h->N, ld)));
+    } else {
+        DISPATCH_G(ld, (panel_spmm_kernel<GG, CC><<<nb, 256, 0, h->stream>>>(A.ptr, A.cols, A.vals, X, sub, out, alpha, post,
+                                                                       t_fwd, t_inv, accumulate ? 1 : 0, A.n_rows, h->N,
+                                                                       ld)));
+    }
     h->launches++;
     CTL_CUDA(cudaGetLastError());
+    return CTL_OK;
+}
+
+// several ranks: the ghost rows of `panels` input panels of a divergence product (B: velocity rows, B^T: pressure rows)
+int div_exchange(ctl_stokes_s *S, bool transpose, const double *X, int panels)
+{
+    ctl_handle_s *h = S->hv;
+    if (h->cfg.world == 1) return CTL_OK;
+    const ExchangePlan &P = transpose ? S->xBT : S->xB;
+    if (P.peers.empty()) return CTL_OK;
+    const size_t panel = (size_t)(transpose ? S->hp->n_loc : h->n_loc) * h->ld;
+    return exchange_plan_run(h, h->comm->comm, P, X, panel, panels, transpose ? S->d_ghost_p : S->d_ghost_v);
+}
+
+// The divergence blocks on both panels q of X, each with its sub-block transform (preconditioner.py:471-525, CN only):
+//   B    (block_10): T_2 on panel 0, T_1 on panel 1     out[q] = T_inv(post (T(alpha B X[q]) - sub[q]))
+//   B^T  (block_01): T_1 on panel 0, T_2 on panel 1     out[q] (+)= T(alpha B^T X[q])
+// invert: T_inv = T (the Schur right-hand side of pc_fn), otherwise none.  X[q] are panels of the column space,
+// out[q] and sub[q] panels of the row space.
+int div_product(ctl_stokes_s *S, bool transpose, const double *X, const double *sub, double *out, double alpha,
+                double post, bool invert, bool accumulate)
+{
+    ctl_handle_s *hv = S->hv, *hp = S->hp;
+    const bool cn = hv->cfg.CN != 0;
+    const size_t pv = (size_t)hv->n_loc * hv->ld, pp = (size_t)hp->n_loc * hp->ld;
+    const size_t p_in = transpose ? pp : pv, p_out = transpose ? pv : pp;
+    const DevCSR &A = transpose ? S->BT : S->B;
+    const double *ghost = transpose ? S->d_ghost_p : S->d_ghost_v;
+    const size_t g_panel = (transpose ? S->xBT : S->xB).ghosts.size() * hv->ld;
+    CTL_TRY(div_exchange(S, transpose, X, 2));
+    for (int q = 0; q < 2; ++q) {
+        const int t = cn ? ((q == 0) == transpose ? T_ONE : T_TWO) : T_NONE;
+        CTL_TRY(panel_spmm(S, A, X + q * p_in, ghost ? ghost + q * g_panel : nullptr, sub ? sub + q * p_out : nullptr,
+                           out + q * p_out, alpha, post, t, invert ? t : T_NONE, accumulate));
+    }
     return CTL_OK;
 }
 
@@ -320,18 +414,29 @@ int panel_tinv(ctl_stokes_s *S, double *X, int t_inv, int n_rows) { return panel
 // ConstantNullspace on a pressure vector (both panels): out = v - mean(v) [+ mean(w)]
 //   project / pre_mult_corrected_lhs / pc_pre_mult_corrected: w = null
 //   post_mult_correct_lhs(x, y), pc_post_mult_correct(u, b):  w = x resp. b
+// Several ranks: the per-rank column sums (of v, and of w) go through one all-reduce in rank order, then are divided by
+// the global n_p, so every rank shifts by the same means and a run repeats bitwise for a given number of ranks.
 int pressure_center(ctl_stokes_s *S, const double *v, const double *w, double *out)
 {
     ctl_handle_s *h = S->hv;
+    const bool several = h->cfg.world > 1;
     const int n_p = S->hp->n_loc, ld = h->ld, nb = S->colsum_blocks;
+    const int div = several ? 1 : n_p;
     double *mean_v = S->d_mean, *mean_w = S->d_mean + 2 * ld;
     colsum_partial_kernel<<<dim3(nb, 2), 256, 0, h->stream>>>(v, S->d_part, n_p, ld, COLSUM_ROWS);
-    colsum_finish_kernel<<<2, ld, 0, h->stream>>>(S->d_part, mean_v, nb, ld, n_p);
+    colsum_finish_kernel<<<2, ld, 0, h->stream>>>(S->d_part, mean_v, nb, ld, div);
     h->launches += 2;
     if (w) {
         colsum_partial_kernel<<<dim3(nb, 2), 256, 0, h->stream>>>(w, S->d_part, n_p, ld, COLSUM_ROWS);
-        colsum_finish_kernel<<<2, ld, 0, h->stream>>>(S->d_part, mean_w, nb, ld, n_p);
+        colsum_finish_kernel<<<2, ld, 0, h->stream>>>(S->d_part, mean_w, nb, ld, div);
         h->launches += 2;
+    }
+    if (several) {
+        const int count = (w ? 4 : 2) * ld;
+        CTL_CUDA(cudaGetLastError());
+        CTL_TRY(ctl_allreduce_sum(h, S->d_mean, count));
+        mean_divide_kernel<<<ceil_div(count, 256), 256, 0, h->stream>>>(S->d_mean, count, (double)S->hp->n);
+        h->launches++;
     }
     const size_t total = 2 * (size_t)n_p * ld;
     panel_shift_kernel<<<ceil_div(total, 256), 256, 0, h->stream>>>(v, out, mean_v, w ? mean_w : nullptr, n_p, ld);
@@ -344,23 +449,15 @@ int pressure_center(ctl_stokes_s *S, const double *v, const double *w, double *o
 int stokes_apply_tf(ctl_stokes_s *S, const double *x, double *y)
 {
     ctl_handle_s *hv = S->hv, *hp = S->hp;
-    const bool cn = hv->cfg.CN != 0;
     const double tau = hv->cfg.tau;
-    const size_t pv = (size_t)hv->n_loc * hv->ld, pp = (size_t)hp->n_loc * hp->ld;
     const double *x0 = x, *x1 = x + hv->vec_len();
     double *y0 = y, *y1 = y + hv->vec_len();
     CTL_TRY(ctl_kkt_apply_tf(hv, x0, y0));                       // block_00 (constrained rows: y = x)
     Scratch xc1;
     CTL_TRY(hp->pool.take(&xc1));
     CTL_TRY(pressure_center(S, x1, nullptr, xc1));               // pre_mult_corrected_lhs
-    // block_01 = diag(tau B^T): rows [0, N) get T_1, rows [N, 2N) get T_2 (preconditioner.py:471-525)
-    for (int q = 0; q < 2; ++q)
-        CTL_TRY(panel_spmm(S, S->BT, xc1 + q * pp, nullptr, y0 + q * pv, tau, 1.0,
-                           cn ? (q == 0 ? T_ONE : T_TWO) : T_NONE, T_NONE, true));
-    // block_10 = diag(tau B): rows [0, N) get T_2, rows [N, 2N) get T_1
-    for (int q = 0; q < 2; ++q)
-        CTL_TRY(panel_spmm(S, S->B, x0 + q * pv, nullptr, y1 + q * pp, tau, 1.0,
-                           cn ? (q == 0 ? T_TWO : T_ONE) : T_NONE, T_NONE, false));
+    CTL_TRY(div_product(S, true, xc1, nullptr, y0, tau, 1.0, false, true));     // block_01 = diag(tau B^T)
+    CTL_TRY(div_product(S, false, x0, nullptr, y1, tau, 1.0, false, false));    // block_10 = diag(tau B)
     return pressure_center(S, y1, x1, y1);                       // post_mult_correct_lhs
 }
 
@@ -390,6 +487,7 @@ int mass_p_solve(ctl_stokes_s *S, const double *c, double *u, double *tmp)
     CTL_CUDA(cudaGetLastError());
     for (int k = 2; k <= steps; ++k) {
         const double w = om[k - 2];
+        if (hp->n_halo > 0) CTL_TRY(ctl_halo_exchange_panel(hp, buf[(k - 1) & 1]));
         CTL_TRY(pcb_cheb_step(hp, S->d_mp_dinv, c, k == 2 ? nullptr : buf[k & 1], buf[(k - 1) & 1], buf[k & 1],
                               k == 2 ? 0.0 : 1.0 - w, w, w * scale));
     }
@@ -427,12 +525,10 @@ int stokes_pc_run(ctl_stokes_s *S, const double *b, double *u, bool wrap)
     CTL_TRY(vec_zero(hv, u0, hv->vec_len()));
     CTL_TRY(ctl_solve_tf(hv, b0, u0, &io, &ir));
     // ---- u_1 = T^-1 ((T (tau B u_0) - b_1) / tau^2)
-    for (int q = 0; q < 2; ++q) {
-        const int t = cn ? (q == 0 ? T_TWO : T_ONE) : T_NONE;
-        CTL_TRY(panel_spmm(S, S->B, u0 + q * pv, rhs1 + q * pp, s1 + q * pp, tau, 1.0 / (tau * tau), t, t, false));
-    }
+    CTL_TRY(div_product(S, false, u0, rhs1, s1, tau, 1.0 / (tau * tau), true, false));
     // ---- AMG cycles on K_p, one solve per time block
     for (int q = 0; q < 2; ++q) CTL_TRY(pcb_panel_to_ts(hp, s1 + q * pp, S->ts_b + (size_t)q * N * n_p, (size_t)n_p));
+    CTL_TRY(halo_epoch_begin(hp));                              // several ranks: the K_p exchanges start a new epoch
     for (int j = 0; j < 2 * N; ++j) CTL_TRY(amg_solve(hp, S->Kp, S->ts_b + (size_t)j * n_p, S->ts_x + (size_t)j * n_p));
     for (int q = 0; q < 2; ++q) CTL_TRY(pcb_ts_to_panel(hp, S->ts_x + (size_t)q * N * n_p, s1 + q * pp, (size_t)n_p));
     // ---- multiply with the (untransformed) heat-type KKT blocks of the pressure space
@@ -490,6 +586,26 @@ struct StokesSolver : Solver {
     }
 };
 
+// the K_p hierarchy and, on several ranks, its exchange arena (collective: every rank frees it at the same point)
+void kp_free(ctl_stokes_s *S)
+{
+    if (S->kp_x) halo_arena_free(S->hp, S->kp_x->arena);
+    S->kp_x.reset();
+    if (S->have_Kp) amg_free(S->Kp);
+    S->have_Kp = false;
+}
+
+// has a bounded wait of either handle's device-initiated exchange given up (ctl_comm_check)?  Both report through the
+// velocity handle.
+int stokes_comm_check(ctl_stokes_s *S)
+{
+    ctl_handle_s *h = S->hv;
+    CTL_TRY(ctl_comm_check(h));
+    const int rc = ctl_comm_check(S->hp);
+    if (rc != CTL_OK) ctl_set_error(h, "pressure handle: " + S->hp->err);
+    return rc;
+}
+
 // with_internal for the Stokes system: the caller's vectors are block-major
 template <size_t K, class F>
 int with_tf(ctl_stokes_s *S, const double *const (&in)[K], double *out, F fn)
@@ -517,10 +633,11 @@ int ctl_stokes_create(ctl_handle velocity, ctl_handle pressure, const int32_t *B
               "ctl_stokes_create: assemble the velocity and pressure handles first");
     const ctl_config &a = velocity->cfg, &b = pressure->cfg;
     CTL_CHECK(a.n_t == b.n_t && a.CN == b.CN && a.tau == b.tau && a.beta == b.beta && a.device == b.device &&
-                  velocity->stream == pressure->stream,
-              CTL_ERR_ARG, "ctl_stokes_create: the two handles must share n_t, CN, tau, beta, device and stream");
-    CTL_CHECK(a.world == 1 && b.world == 1, CTL_ERR_ARG, "ctl_stokes_create: the Stokes path is single-GPU in this version");
-    CTL_CHECK(pressure->n_bc_all == 0, CTL_ERR_ARG, "ctl_stokes_create: the pressure handle must not carry Dirichlet dofs");
+                  a.rank == b.rank && a.world == b.world && velocity->stream == pressure->stream,
+              CTL_ERR_ARG, "ctl_stokes_create: the two handles must share n_t, CN, tau, beta, rank, world, device and stream");
+    CTL_CHECK(a.world == 1 || (velocity->comm && pressure->comm), CTL_ERR_STATE,
+              "ctl_stokes_create: call ctl_comm_init on both handles first (world > 1)");
+    CTL_CHECK(pressure->h_bc.empty(), CTL_ERR_ARG, "ctl_stokes_create: the pressure handle must not carry Dirichlet dofs");
     CTL_CUDA(cudaSetDevice(a.device));
     const int n_v = velocity->n, n_p = pressure->n;
     HostCSR B;
@@ -533,7 +650,7 @@ int ctl_stokes_create(ctl_handle velocity, ctl_handle pressure, const int32_t *B
     for (int64_t k = 0; k < nnz; ++k)
         CTL_CHECK(B.indices[k] >= 0 && B.indices[k] < n_v, CTL_ERR_ARG, "ctl_stokes_create: column index out of range");
     std::shared_ptr<LiftState> lift_div;       // kept for the lifting of inhomogeneous velocity data
-    CTL_TRY(ctl_lift_div_setup(velocity, B_indptr, B_indices, B_values, n_p, &lift_div));
+    CTL_TRY(ctl_lift_div_setup(velocity, B_indptr, B_indices, B_values, pressure->row_begin, pressure->n_loc, &lift_div));
     for (int64_t k = 0; k < nnz; ++k)
         if (velocity->h_bcmask[B.indices[k]]) B.values[k] = 0.0;      // the operator sees x with bcs zeroed
     HostCSR BT;
@@ -543,15 +660,29 @@ int ctl_stokes_create(ctl_handle velocity, ctl_handle pressure, const int32_t *B
     S->hp = pressure;
     S->pool.init(h, S->len());
     S->lift_div = lift_div;
-    int rc = upload_csr(h, B, S->B);
-    if (rc == CTL_OK) rc = upload_csr(h, BT, S->BT);
-    S->colsum_blocks = ceil_div(n_p, COLSUM_ROWS);
+    int rc = CTL_OK;
+    if (a.world == 1) {
+        rc = upload_csr(h, B, n_v, S->B);
+        if (rc == CTL_OK) rc = upload_csr(h, BT, n_p, S->BT);
+    } else {
+        // this rank's rows of B (pressure) and of B^T (velocity), each over the other space's split
+        const int vb = velocity->row_begin, nv = velocity->n_loc, pb = pressure->row_begin, np = pressure->n_loc;
+        rc = exchange_plan_build(h, B.indptr.data(), B.indices.data(), n_p, n_v, a.world, a.rank, S->xB);
+        if (rc == CTL_OK) rc = exchange_plan_build(h, BT.indptr.data(), BT.indices.data(), n_v, n_p, a.world, a.rank, S->xBT);
+        if (rc == CTL_OK) rc = upload_csr(h, local_rows(B, pb, np, vb, nv, S->xB.ghosts), nv, S->B);
+        if (rc == CTL_OK) rc = upload_csr(h, local_rows(BT, vb, nv, pb, np, S->xBT.ghosts), np, S->BT);
+        const size_t gv = 2 * S->xB.ghosts.size() * h->ld, gp = 2 * S->xBT.ghosts.size() * h->ld;
+        if (rc == CTL_OK && gv && cudaMalloc((void **)&S->d_ghost_v, gv * sizeof(double)) != cudaSuccess) rc = CTL_ERR_CUDA;
+        if (rc == CTL_OK && gp && cudaMalloc((void **)&S->d_ghost_p, gp * sizeof(double)) != cudaSuccess) rc = CTL_ERR_CUDA;
+    }
+    S->colsum_blocks = ceil_div(pressure->n_loc, COLSUM_ROWS);
     if (rc == CTL_OK && cudaMalloc((void **)&S->d_part, sizeof(double) * 2 * S->colsum_blocks * h->ld) != cudaSuccess) rc = CTL_ERR_CUDA;
     if (rc == CTL_OK && cudaMalloc((void **)&S->d_mean, sizeof(double) * 4 * h->ld) != cudaSuccess) rc = CTL_ERR_CUDA;
     S->res_blocks = blocks_for(2 * (velocity->n_loc + pressure->n_loc), h->ld);
     if (rc == CTL_OK && cudaMalloc((void **)&S->d_res_part, sizeof(double) * (S->res_blocks + 1)) != cudaSuccess)
         rc = CTL_ERR_CUDA;
     if (rc != CTL_OK) {
+        if (h->err.empty()) ctl_set_error(h, "ctl_stokes_create: device allocation failed");
         ctl_stokes_destroy(S);
         return rc;
     }
@@ -566,7 +697,9 @@ int ctl_stokes_destroy(ctl_stokes S)
     cudaStreamSynchronize(S->hv->stream);
     free_csr(S->B);
     free_csr(S->BT);
-    if (S->have_Kp) amg_free(S->Kp);
+    kp_free(S);
+    cudaFree(S->d_ghost_v);
+    cudaFree(S->d_ghost_p);
     cudaFree(S->d_mp_dinv);
     cudaFree(S->ts_b);
     cudaFree(S->ts_x);
@@ -586,7 +719,8 @@ int ctl_stokes_lift_bc(ctl_stokes S, const double *g, double *b)
     CTL_CHECK(g && b, CTL_ERR_ARG, "ctl_stokes_lift_bc: null g or b (the velocity handle has Dirichlet dofs)");
     CTL_TRY(ctl_lift_bc(h, g, b, CTL_LAYOUT_BLOCK_MAJOR));              // velocity rows: [2N blocks of n_v]
     CTL_CUDA(cudaSetDevice(h->cfg.device));
-    return ctl_lift_div_apply(h, S->lift_div.get(), g, b + 2 * (size_t)h->N * h->n_loc, S->hp->n_loc);   // b_1_0
+    CTL_TRY(ctl_lift_div_apply(h, S->lift_div.get(), g, b + 2 * (size_t)h->N * h->n_loc, S->hp->n_loc));   // b_1_0
+    return stokes_comm_check(S);
 }
 
 // Residual of the Navier-Stokes Picard loop (res_eval, control/control.py:4979-5072) on device vectors.  The
@@ -603,30 +737,32 @@ int ctl_stokes_nonlinear_residual(ctl_stokes S, const double *b, const double *x
     CTL_CHECK(h->assembled && hp->assembled, CTL_ERR_STATE,
               "ctl_stokes_nonlinear_residual: the velocity and pressure handles are not assembled");
     CTL_CUDA(cudaSetDevice(h->cfg.device));
-    const bool cn = h->cfg.CN != 0;
+    const bool cn = h->cfg.CN != 0, several = h->cfg.world > 1;
     const double tau = h->cfg.tau;
     const int n_v = h->n_loc, n_p = hp->n_loc, ld = h->ld;
-    const size_t pv = (size_t)n_v * ld, pp = (size_t)n_p * ld;
     const int64_t lv = h->vec_len();
     double *partials = nullptr, *scalars = nullptr;
     CTL_TRY(vec_workspace(h, &partials, &scalars));                             // pinned staging of vec_read_scalars
     CTL_TRY(with_tf(S, {b, x, nullptr}, r, [&](const double *bt, const double *xt, double *yt) -> int {
         CTL_TRY(ctl_kkt_apply_tf(h, xt, yt));                                    // block_00 with D_v at the iterate
-        for (int q = 0; q < 2; ++q)                                               // + tau T(B^T x_p), raw x_p
-            CTL_TRY(panel_spmm(S, S->BT, xt + lv + q * pp, nullptr, yt + q * pv, tau, 1.0,
-                               cn ? (q == 0 ? T_ONE : T_TWO) : T_NONE, T_NONE, true));
-        for (int q = 0; q < 2; ++q)                                               // r_p = b_p - tau T(B x_v)
-            CTL_TRY(panel_spmm(S, S->B, xt + q * pv, bt + lv + q * pp, yt + lv + q * pp, tau, -1.0,
-                               cn ? (q == 0 ? T_TWO : T_ONE) : T_NONE, T_NONE, false));
+        CTL_TRY(div_product(S, true, xt + lv, nullptr, yt, tau, 1.0, false, true));         // + tau T(B^T x_p), raw x_p
+        CTL_TRY(div_product(S, false, xt, bt + lv, yt + lv, tau, -1.0, false, false));      // r_p = b_p - tau T(B x_v)
         DISPATCH_G(ld, (stokes_residual_kernel<GG, CC><<<S->res_blocks, 256, 0, h->stream>>>(
                            bt, yt, h->d_bcmask, S->d_res_part, n_v, n_p, h->N, ld, cn ? 1 : 0, 1.0 / (tau * tau))));
-        residual_finish_kernel<<<1, 256, 0, h->stream>>>(S->d_res_part, S->res_blocks, S->d_res_part + S->res_blocks);
+        if (several)
+            residual_finish_kernel<false><<<1, 256, 0, h->stream>>>(S->d_res_part, S->res_blocks, S->d_res_part + S->res_blocks);
+        else
+            residual_finish_kernel<true><<<1, 256, 0, h->stream>>>(S->d_res_part, S->res_blocks, S->d_res_part + S->res_blocks);
         h->launches += 2;
         CTL_CHECK(cudaGetLastError() == cudaSuccess, CTL_ERR_CUDA,
                   "ctl_stokes_nonlinear_residual: kernel launch failed");
+        // several ranks: the sum of the squares over all rows, then the root of the same sum on every rank
+        if (several) CTL_TRY(ctl_allreduce_sum(h, S->d_res_part + S->res_blocks, 1));
         return CTL_OK;
     }));
-    return vec_read_scalars(h, S->d_res_part + S->res_blocks, 1, norm_host);
+    CTL_TRY(vec_read_scalars(h, S->d_res_part + S->res_blocks, 1, norm_host));
+    if (several) *norm_host = std::sqrt(*norm_host);
+    return stokes_comm_check(S);
 }
 
 int64_t ctl_stokes_vec_len(ctl_stokes S) { return S ? 2ll * S->hv->N * ((int64_t)S->hv->n_loc + S->hp->n_loc) : 0; }
@@ -688,8 +824,11 @@ int ctl_stokes_pc_setup(ctl_stokes S, const ctl_stokes_pc_options *opts)
     S->opts = *opts;
     CTL_TRY(ctl_pc_setup(h, &opts->velocity));
     // K_p hierarchy: K_p is singular (kernel = constants), the coarsest level gets a pseudo-inverse
-    if (S->have_Kp) amg_free(S->Kp);
-    S->have_Kp = false;
+    kp_free(S);
+    auto from_hp = [&](int rc, const char *what) {       // errors of the pressure handle, reported on the velocity one
+        if (rc != CTL_OK) ctl_set_error(h, std::string("ctl_stokes_pc_setup (") + what + "): " + hp->err);
+        return rc;
+    };
     AmgParams p;
     p.theta = opts->amg_p_theta;
     p.max_levels = opts->amg_p_max_levels;
@@ -706,40 +845,37 @@ int ctl_stokes_pc_setup(ctl_stokes S, const ctl_stokes_pc_options *opts)
         Kp.indptr = hp->h_indptr;
         Kp.indices = hp->h_indices;
         Kp.values = S->h_Kp_solver.empty() ? hp->h_K[0] : S->h_Kp_solver;
-        if (!S->fine_p) {
-            const int rc = sell_build_pattern(hp, hp->loc, S->fine_p);
-            if (rc != CTL_OK) {
-                ctl_set_error(h, std::string("ctl_stokes_pc_setup: ") + hp->err);
-                return rc;
-            }
+        if (!S->fine_p) CTL_TRY(from_hp(sell_build_pattern(hp, hp->loc, S->fine_p), "SELL pattern"));
+        if (h->cfg.world > 1) {                        // the exchange state the distributed hierarchy joins
+            S->kp_x.reset(new PcState());
+            CTL_TRY(from_hp(pc_mesh_exchange(hp, *S->kp_x), "K_p exchange geometry"));
         }
         S->Kp = AmgHierarchyDev();
-        const int rc = amg_build(hp, Kp, p, S->fine_p, S->Kp);
-        if (rc != CTL_OK) {
-            ctl_set_error(h, std::string("ctl_stokes_pc_setup (K_p hierarchy): ") + hp->err);
-            return rc;
-        }
         S->have_Kp = true;
+        CTL_TRY(from_hp(amg_build(hp, Kp, p, S->fine_p, S->Kp, S->kp_x.get()), "K_p hierarchy"));
+        if (S->kp_x) CTL_TRY(from_hp(halo_arena_finalize(hp, S->kp_x->arena), "K_p exchange arena"));
     }
     {
-        std::vector<double> dinv(n_p);
-        for (int r = 0; r < n_p; ++r) {
+        const int rb = hp->row_begin, nl = hp->n_loc;
+        std::vector<double> dinv(nl);
+        for (int i = 0; i < nl; ++i) {
+            const int r = rb + i;
             double d = 0.0;
             for (int k = hp->h_indptr[r]; k < hp->h_indptr[r + 1]; ++k)
                 if (hp->h_indices[k] == r) d = hp->h_M[k];
             CTL_CHECK(d != 0.0, CTL_ERR_ARG, "ctl_stokes_pc_setup: pressure mass matrix has a zero diagonal entry");
-            dinv[r] = 1.0 / d;
+            dinv[i] = 1.0 / d;
         }
         CTL_TRY(ctl_upload(h, &S->d_mp_dinv, dinv.data(), dinv.size()));
     }
-    const size_t ts_bytes = 2ull * h->N * n_p * sizeof(double);
+    const size_t ts_bytes = 2ull * h->N * hp->n_loc * sizeof(double);
     if (!S->ts_b) CTL_CUDA(cudaMalloc((void **)&S->ts_b, ts_bytes));
     if (!S->ts_x) CTL_CUDA(cudaMalloc((void **)&S->ts_x, ts_bytes));
     CTL_CUDA(cudaMemsetAsync(S->ts_b, 0, ts_bytes, h->stream));
     CTL_CUDA(cudaMemsetAsync(S->ts_x, 0, ts_bytes, h->stream));
     CTL_CUDA(cudaStreamSynchronize(h->stream));
     S->pc_ready = true;
-    return CTL_OK;
+    return stokes_comm_check(S);
 }
 
 int ctl_stokes_apply(ctl_stokes S, const double *x, double *y)
@@ -747,7 +883,8 @@ int ctl_stokes_apply(ctl_stokes S, const double *x, double *y)
     if (!S) return CTL_ERR_ARG;
     ctl_handle_s *h = S->hv;
     CTL_CHECK(x && y, CTL_ERR_ARG, "ctl_stokes_apply: null argument");
-    return with_tf(S, {x, nullptr}, y, [&](const double *xt, double *yt) { return stokes_apply_tf(S, xt, yt); });
+    CTL_TRY(with_tf(S, {x, nullptr}, y, [&](const double *xt, double *yt) { return stokes_apply_tf(S, xt, yt); }));
+    return stokes_comm_check(S);
 }
 
 int ctl_stokes_pc_apply(ctl_stokes S, const double *b, double *u)
@@ -755,7 +892,8 @@ int ctl_stokes_pc_apply(ctl_stokes S, const double *b, double *u)
     if (!S) return CTL_ERR_ARG;
     ctl_handle_s *h = S->hv;
     CTL_CHECK(b && u, CTL_ERR_ARG, "ctl_stokes_pc_apply: null argument");
-    return with_tf(S, {b, nullptr}, u, [&](const double *bt, double *ut) { return stokes_pc_tf(S, bt, ut, true); });
+    CTL_TRY(with_tf(S, {b, nullptr}, u, [&](const double *bt, double *ut) { return stokes_pc_tf(S, bt, ut, true); }));
+    return stokes_comm_check(S);
 }
 
 int ctl_stokes_pc_fn(ctl_stokes S, const double *b, double *u)
@@ -763,7 +901,8 @@ int ctl_stokes_pc_fn(ctl_stokes S, const double *b, double *u)
     if (!S) return CTL_ERR_ARG;
     ctl_handle_s *h = S->hv;
     CTL_CHECK(b && u, CTL_ERR_ARG, "ctl_stokes_pc_fn: null argument");
-    return with_tf(S, {b, nullptr}, u, [&](const double *bt, double *ut) { return stokes_pc_tf(S, bt, ut, false); });
+    CTL_TRY(with_tf(S, {b, nullptr}, u, [&](const double *bt, double *ut) { return stokes_pc_tf(S, bt, ut, false); }));
+    return stokes_comm_check(S);
 }
 
 int ctl_stokes_set_pc_callback(ctl_stokes S, ctl_pc_callback fn, void *user)
@@ -784,10 +923,11 @@ int ctl_stokes_solve(ctl_stokes S, const double *b, double *u, const ctl_krylov_
     CTL_CHECK(opts->pc >= CTL_PC_NONE && opts->pc <= CTL_PC_CALLBACK, CTL_ERR_ARG, "ctl_stokes_solve: unknown pc kind");
     if (opts->pc == CTL_PC_CALLBACK) CTL_CHECK(S->pc_cb, CTL_ERR_STATE, "ctl_stokes_solve: call ctl_stokes_set_pc_callback first");
     if (opts->pc == CTL_PC_BUILTIN) CTL_CHECK(S->pc_ready, CTL_ERR_STATE, "ctl_stokes_solve: call ctl_stokes_pc_setup first");
-    return with_tf(S, {b, u}, u, [&](const double *bt, double *ut) {
+    CTL_TRY(with_tf(S, {b, u}, u, [&](const double *bt, double *ut) {
         StokesSolver K(S, *opts, *result);
         return krylov_solve(K, bt, ut);
-    });
+    }));
+    return stokes_comm_check(S);
 }
 
 int ctl_stokes_time(ctl_stokes S, int reps, double *out)
@@ -810,9 +950,12 @@ int ctl_stokes_time(ctl_stokes S, int reps, double *out)
     for (int which = 0; which < 2 && rc == CTL_OK; ++which) {
         for (int pass = 0; pass < 2 && rc == CTL_OK; ++pass) {        // pass 0 warms up
             cudaEventRecord(ev.begin, h->stream);
-            for (int r = 0; r < reps && rc == CTL_OK; ++r)
-                rc = which == 0 ? panel_spmm(S, S->B, xv, nullptr, xp, tau, 1.0, T_TWO, T_NONE, false)
-                                : panel_spmm(S, S->BT, xp, nullptr, yv, tau, 1.0, T_ONE, T_NONE, true);
+            for (int r = 0; r < reps && rc == CTL_OK; ++r) {        // several ranks: with the exchange of the ghosts
+                rc = div_exchange(S, which == 1, which == 0 ? (const double *)xv : xp, 1);
+                if (rc == CTL_OK)
+                    rc = which == 0 ? panel_spmm(S, S->B, xv, S->d_ghost_v, nullptr, xp, tau, 1.0, T_TWO, T_NONE, false)
+                                    : panel_spmm(S, S->BT, xp, S->d_ghost_p, nullptr, yv, tau, 1.0, T_ONE, T_NONE, true);
+            }
             cudaEventRecord(ev.end, h->stream);
             cudaEventSynchronize(ev.end);
             cudaEventElapsedTime(&ms[which], ev.begin, ev.end);
@@ -826,7 +969,8 @@ int ctl_stokes_time(ctl_stokes S, int reps, double *out)
     out[1] = 12.0 * nnz + 4.0 * (n_p + 1) + 8.0 * N * (n_v + n_p);
     out[2] = ms[1] / reps;
     out[3] = 12.0 * nnz + 4.0 * (n_v + 1) + 8.0 * N * (n_v + n_p) + 8.0 * N * n_v;
-    return rc;
+    CTL_TRY(rc);
+    return stokes_comm_check(S);
 }
 
 }  // extern "C"

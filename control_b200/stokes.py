@@ -9,7 +9,9 @@ blocks and ConstantNullspace on the pressure blocks.  It is constructed from the
 spatial matrices the blocks are made of; every numeric operation runs in libctl_b200.so.
 
 Vectors at this boundary are block-major: ``x_0`` of shape (2N, n_v) = [v | zeta] and ``x_1``
-of shape (2N, n_p) = [mu | p], or one flat device vector [x_0 | x_1].
+of shape (2N, n_p) = [mu | p], or one flat device vector [x_0 | x_1].  On several ranks (``world > 1``)
+each rank holds its own rows of both spaces, PETSc's split of each (``velocity_rows``,
+``pressure_rows``): ``x_0`` of shape (2N, n_v_local), ``x_1`` of shape (2N, n_p_local).
 """
 import ctypes as C
 
@@ -26,35 +28,59 @@ class StokesSystem(_DeviceSystem):
     _SET_CALLBACK = "ctl_stokes_set_pc_callback"
 
     def __init__(self, M_v, K_v, B, M_p, K_p, *, n_t, beta, CN, time_interval=(0.0, 1.0), bc_dofs_v=(),
-                 epsilon=1e-3, device=None, D_p=None, velocity_block_size=1):
+                 epsilon=1e-3, device=None, D_p=None, velocity_block_size=1, rank=0, world=1):
         """``K_v``: the forward matrix on the velocity space (one matrix or n_t matrices ``D_v_i``).  ``K_p``: the
         pressure Laplacian ``solver_K_p`` inverts (control/control.py:3746, 4300-4309).  ``D_p``: the forward
         form on the PRESSURE space (``D_p_i``, control/control.py:3787-3789; one matrix or n_t matrices) of the
         pressure-space KKT multiply; default ``K_p`` (the Stokes forward operator).  ``velocity_block_size``: block
         size of the velocity space (2 for a 2-D ``VectorFunctionSpace``): the velocity sweeps then run on the scalar
-        block of ``I_2 (x) S`` (``MultiBlockSystem(block_size=)``)."""
+        block of ``I_2 (x) S`` (``MultiBlockSystem(block_size=)``); one GPU only.  ``rank`` / ``world``: this
+        process's rank of ``world`` (one GPU each); with ``world > 1`` call ``init_comm`` before anything else."""
+        if int(velocity_block_size) > 1 and world > 1:
+            raise ValueError("velocity_block_size > 1 runs on one GPU: block-scalar sweeps are not available with "
+                             "world > 1")
         self.velocity = MultiBlockSystem(M_v, K_v, n_t=n_t, beta=beta, CN=CN, time_interval=time_interval,
                                          bc_dofs=bc_dofs_v, epsilon=epsilon, device=device,
-                                         block_size=velocity_block_size)
+                                         block_size=velocity_block_size, rank=rank, world=world)
         self.pressure = MultiBlockSystem(M_p, K_p if D_p is None else D_p, n_t=n_t, beta=beta, CN=CN,
                                          time_interval=time_interval, bc_dofs=(), epsilon=epsilon,
-                                         device=self.velocity.device.index, stream=self.velocity.stream)
+                                         device=self.velocity.device.index, stream=self.velocity.stream,
+                                         rank=rank, world=world)
+        self.rank, self.world = rank, world
         self._K_p_solver = None if D_p is None else np.ascontiguousarray(self.pressure._same_pattern(K_p))
         self._lib = self.velocity._lib
         self.device = self.velocity.device
         self._stream = self.velocity.stream
         self.N = self.velocity.N
         self.n_v, self.n_p = self.velocity.n, self.pressure.n
+        self.n_v_local, self.n_p_local = self.velocity.n_local, self.pressure.n_local
+        self.velocity_rows = slice(self.velocity.row_begin, self.velocity.row_begin + self.n_v_local)
+        self.pressure_rows = slice(self.pressure.row_begin, self.pressure.row_begin + self.n_p_local)
         self.tau = self.velocity.tau
         indptr, indices, data = csr_arrays(B)
         if indptr.size != self.n_p + 1 or (indices.size and int(indices.max()) >= self.n_v):
             raise ValueError("B must be the n_p x n_v divergence matrix")
+        self._B = (indptr, indices, data)
         self._s = C.c_void_p()
+        self._pc_ready = False
+        if world == 1:
+            self._create()
+
+    def _create(self):
+        indptr, indices, data = self._B
         self._check(self._lib.ctl_stokes_create(self.velocity._h, self.pressure._h, indptr.ctypes.data,
                                                 indices.ctypes.data, data.ctypes.data, C.byref(self._s)))
         if self._K_p_solver is not None:
             self._check(self._lib.ctl_stokes_set_laplacian_p(self._s, self._K_p_solver.ctypes.data))
-        self._pc_ready = False
+
+    def init_comm(self, dist=None):
+        """Several ranks: the NCCL communicators of both spaces (``MultiBlockSystem.init_comm``), then the outer
+        system, whose divergence products exchange rows through them.  Every rank passes the global matrices."""
+        if self.world == 1:
+            return
+        self.velocity.init_comm(dist)
+        self.pressure.init_comm(dist)
+        self._create()
 
     def set_forward(self, K_v, D_p=None):
         """New forward matrices of a Picard iteration (control/control.py:5109-5118: every outer iteration
@@ -76,6 +102,7 @@ class StokesSystem(_DeviceSystem):
         self.velocity._check(rc)            # the library records the Stokes system's errors on the velocity handle
 
     def close(self):
+        """Release the outer system and both handles; collective with world > 1 (see ``MultiBlockSystem.close``)."""
         if getattr(self, "_s", None) is not None and self._s:
             self._lib.ctl_stokes_destroy(self._s)
             self._s = C.c_void_p()
@@ -94,14 +121,19 @@ class StokesSystem(_DeviceSystem):
 
     def to_host_blocks(self, x_dev):
         a = x_dev.detach().cpu().numpy()
-        L0 = 2 * self.N * self.n_v
-        return a[:L0].reshape(2 * self.N, self.n_v), a[L0:].reshape(2 * self.N, self.n_p)
+        L0 = 2 * self.N * self.n_v_local
+        return a[:L0].reshape(2 * self.N, self.n_v_local), a[L0:].reshape(2 * self.N, self.n_p_local)
+
+    def allgather_blocks(self, x_0, x_1):
+        """This rank's block arrays (2N, n_v_local), (2N, n_p_local) -> the global (2N, n_v), (2N, n_p) on every
+        rank."""
+        return self.velocity.allgather_blocks(x_0), self.pressure.allgather_blocks(x_1)
 
     def velocity_state_to_host(self, x_dev):
-        """The N velocity-state blocks of an outer device vector (its first N n_v entries) as a host array of shape
-        (N, n_v): all a Picard loop needs to assemble ``D_v_i`` / ``D_p_i`` at the iterate."""
+        """The N velocity-state blocks of an outer device vector (its first N n_v_local entries) as a host array of
+        shape (N, n_v_local): all a Picard loop needs to assemble ``D_v_i`` / ``D_p_i`` at the iterate."""
         self._check_vecs("velocity_state_to_host", x_dev)
-        return x_dev[:self.N * self.n_v].cpu().numpy().reshape(self.N, self.n_v)
+        return x_dev[:self.N * self.n_v_local].cpu().numpy().reshape(self.N, self.n_v_local)
 
     # ------------------------------------------------------------------ operator / preconditioner
     def apply(self, x_dev, y_dev=None):

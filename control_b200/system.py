@@ -330,6 +330,8 @@ class MultiBlockSystem(_DeviceSystem):
         L.check(self._h, rc)
 
     def close(self):
+        """Release the handle.  With world > 1 this is collective (ctl_destroy): call it on every rank at the same
+        point rather than leaving it to garbage collection, whose timing differs between processes."""
         if getattr(self, "_h", None) is not None and self._h:
             self._lib.ctl_destroy(self._h)
             self._h = C.c_void_p()

@@ -132,6 +132,8 @@ typedef int (*ctl_pc_callback)(void *user, const double *b, double *u);
 /* ---- lifetime: MultiBlockSystem.__init__ / `del system` (preconditioner.py:217-335,
  *      control/control.py:3323-3326) */
 int ctl_create(const ctl_config *cfg, ctl_handle *out);
+/* world > 1: collective once ctl_pc_setup has run (the preconditioner's exchange arena is released behind two
+ * barriers across the ranks): every rank destroys its handle at the same point of its call sequence */
 int ctl_destroy(ctl_handle h);
 const char *ctl_last_error(ctl_handle h);     /* h may be NULL: error of a failed create  */
 const char *ctl_version(void);
@@ -157,7 +159,8 @@ int ctl_set_bc(ctl_handle h, const int32_t *dofs_host, int32_t count);
  * change.  CTL_ERR_ARG unless bs is 1, 2 or 3 and divides n, and for bs > 1 with world > 1 (block-scalar sweeps
  * run on one GPU).  Drops a preconditioner that is already set up (call ctl_pc_setup again). */
 int ctl_set_block_size(ctl_handle h, int32_t bs);
-/* finish setup (uploads, eliminations); must precede apply/solve */
+/* finish setup (uploads, eliminations); must precede apply/solve.  Drops a set-up preconditioner: with world > 1
+ * that release is collective like ctl_destroy, so every rank assembles at the same point */
 int ctl_assemble(ctl_handle h);
 
 /* ---- sizes */
@@ -264,7 +267,14 @@ int ctl_amg_solve(ctl_handle h, int32_t hierarchy, const double *b, double *x);
  *      velocity Dirichlet dofs) and `pressure` (M_p, K_p, no bcs), same n_t / tau / beta / CN /
  *      device / stream -- plus the divergence matrix B (n_p x n_v CSR, host).  Vectors are
  *      DEVICE pointers, block-major: [2N blocks of n_v (v | zeta) | 2N blocks of n_p (mu | p)].
- *      Errors are reported through ctl_last_error(velocity).  Single GPU in this round. */
+ *      Errors are reported through ctl_last_error(velocity).
+ *      Several GPUs (one process each): both handles carry the same rank / world > 1 and have been through
+ *      ctl_comm_init.  Every rank passes the GLOBAL B; velocity and pressure rows are each split by PETSc's rule
+ *      (the handles' own partitions), and every entry point works on this rank's rows: the outer vector is
+ *      [2N blocks of n_v_local | 2N blocks of n_p_local] and ctl_stokes_vec_len is that local length.  The
+ *      divergence products exchange the rows of the other space they read through NCCL; the pressure means, the
+ *      Krylov dots and the residual norm are summed over all ranks, so every rank receives the same global values.
+ *      All calls are collective.  Block-scalar velocity sweeps (ctl_set_block_size > 1) stay on one GPU. */
 typedef struct ctl_stokes_s *ctl_stokes;
 
 /* the in-built pressure-Schur preconditioner (control/control.py:4299-4687) */
@@ -280,10 +290,13 @@ typedef struct {
     double amg_p_theta, amg_p_lo, amg_p_hi;
 } ctl_stokes_pc_options;
 
+/* CTL_ERR_ARG: the handles differ in n_t, CN, tau, beta, rank, world, device or stream, the pressure handle has
+ * Dirichlet dofs, or B has a column out of range; CTL_ERR_STATE: a handle is not assembled, or (world > 1) has not
+ * been through ctl_comm_init */
 int ctl_stokes_create(ctl_handle velocity, ctl_handle pressure, const int32_t *B_indptr_host,
                       const int32_t *B_indices_host, const double *B_values_host, ctl_stokes *out);
 int ctl_stokes_destroy(ctl_stokes s);
-int64_t ctl_stokes_vec_len(ctl_stokes s);      /* 2 N (n_v + n_p) */
+int64_t ctl_stokes_vec_len(ctl_stokes s);      /* 2 N (n_v_local + n_p_local); n_v + n_p on one GPU */
 /* y = A x: MultiBlockSystemMatrix.mult with sub_n_blocks = 2 (preconditioner.py:375-543) */
 int ctl_stokes_apply(ctl_stokes s, const double *x, double *y);
 int ctl_stokes_pc_default_options(ctl_stokes_pc_options *opts);
@@ -340,7 +353,10 @@ int ctl_amg_setup_probe(const int32_t *indptr_host, const int32_t *indices_host,
                         int64_t *level_nnz16, double *level_rho16, int32_t *aggregates_n);
 
 /* ---- multi-GPU (one process per GPU): the 128-byte ncclUniqueId is created on rank 0
- *      with ctl_comm_unique_id and distributed by the caller (torch.distributed) */
+ *      with ctl_comm_unique_id and distributed by the caller (torch.distributed).  With world > 1 every call that
+ *      communicates is collective -- the entry points that apply, precondition or solve, ctl_pc_setup,
+ *      ctl_stokes_create / _pc_setup, and the releases of ctl_destroy, ctl_assemble, ctl_set_block_size and
+ *      ctl_stokes_destroy: all ranks make them in the same order */
 int ctl_comm_unique_id(void *id128_host);
 int ctl_comm_init(ctl_handle h, const void *id128_host);
 
