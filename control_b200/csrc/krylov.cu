@@ -3,6 +3,11 @@
 // oracle/krylov.py (SURVEY.md Appendix A.3): initial guess always non-zero (743), default
 // convergence test against ||b|| (||P^-1 b|| for the preconditioned norm), classical
 // Gram-Schmidt without refinement, iteration counter across restarts, max_it -> DIVERGED_ITS.
+// PETSc's call sequence with one exception: when the guess is zero and the preconditioner is
+// not a user callback, the start skips the apply A 0 and, for MINRES and left-preconditioned
+// GMRES, the second preconditioner application to b - A 0 = b (krylov_solve).  The preconditioner
+// is deterministic, so iterates, history and counts of iterations are those of the full start;
+// only n_mult and n_pc are lower.
 // Vectors never leave the device; per iteration the host reads the k+1 Gram-Schmidt
 // scalars once (Hessenberg / Givens bookkeeping is host work on a handful of doubles).
 #include <cmath>

@@ -152,7 +152,8 @@ struct Solver {
         return CTL_OK;
     }
 
-    int gmres(const double *b, double *x)
+    // zero_guess: x is zero (see krylov_solve), so the first residual b - A x is b bit for bit
+    int gmres(const double *b, double *x, bool zero_guess)
     {
         const bool flexible = o.ksp_type == CTL_KSP_FGMRES;
         // a restart length beyond max_it is never reached: do not allocate basis vectors for it
@@ -165,27 +166,35 @@ struct Solver {
         CTL_TRY(pool.take(&t));
         double *partials, *scal;
         CTL_TRY(vec_workspace(h, &partials, &scal));
+        // the reference norm ||b|| (left PC: ||P^-1 b||); from a zero guess its vector is the first V[0]
         double ref = 0.0;
         if (flexible) {
             CTL_TRY(norm(b, &ref));
+            if (zero_guess) CTL_TRY(vec_copy(h, V[0], b, len));
         } else {
-            CTL_TRY(prec(b, t));
-            CTL_TRY(norm(t, &ref));
+            double *pb = zero_guess ? V[0] : t;
+            CTL_TRY(prec(b, pb));
+            CTL_TRY(norm(pb, &ref));
         }
         res.ref_norm = ref;
         const Conv conv(o.rtol, o.atol, o.divtol, ref);
         std::vector<double> H((size_t)(m + 1) * m), g(m + 1), cs(m), sn(m), hcol(m + 2);
+        bool first_residual_ready = zero_guess;
         while (res.reason == 0) {
-            // r = b - A x (left PC: P^-1 (b - A x)) -> V[0]
-            CTL_TRY(op(x, t));
-            if (flexible) {
-                CTL_TRY(vec_lincomb(h, V[0], 1.0, b, -1.0, t, 0.0, nullptr, nullptr, len));
+            double rnorm = ref;
+            if (first_residual_ready) {
+                first_residual_ready = false;
             } else {
-                CTL_TRY(vec_lincomb(h, t, 1.0, b, -1.0, t, 0.0, nullptr, nullptr, len));
-                CTL_TRY(prec(t, V[0]));
+                // r = b - A x (left PC: P^-1 (b - A x)) -> V[0]
+                CTL_TRY(op(x, t));
+                if (flexible) {
+                    CTL_TRY(vec_lincomb(h, V[0], 1.0, b, -1.0, t, 0.0, nullptr, nullptr, len));
+                } else {
+                    CTL_TRY(vec_lincomb(h, t, 1.0, b, -1.0, t, 0.0, nullptr, nullptr, len));
+                    CTL_TRY(prec(t, V[0]));
+                }
+                CTL_TRY(norm(V[0], &rnorm));
             }
-            double rnorm = 0.0;
-            CTL_TRY(norm(V[0], &rnorm));
             if (res.its == 0) record(rnorm);
             res.reason = conv(rnorm);
             if (res.reason) break;
@@ -253,7 +262,7 @@ struct Solver {
         return CTL_OK;
     }
 
-    int minres(const double *b, double *x)
+    int minres(const double *b, double *x, bool zero_guess)
     {
         Scratch vecs[7];
         for (Scratch &s : vecs) CTL_TRY(pool.take(&s));
@@ -267,14 +276,18 @@ struct Solver {
         }
         res.ref_norm = std::sqrt(bb);
         const Conv conv(o.rtol, o.atol, o.divtol, res.ref_norm);
-        CTL_TRY(op(x, r1));
-        CTL_TRY(vec_lincomb(h, r1, 1.0, b, -1.0, r1, 0.0, nullptr, nullptr, len));
-        CTL_TRY(prec(r1, y));
-        double beta1 = 0.0;
-        CTL_TRY(dot(r1, y, &beta1));
-        if (beta1 < 0.0) {
-            res.reason = CTL_DIVERGED_INDEFINITE_PC;
-            return CTL_OK;
+        double beta1 = bb;          // from a zero guess r1 = b, y = P^-1 b and r1 . y = bb
+        if (zero_guess) {
+            CTL_TRY(vec_copy(h, r1, b, len));
+        } else {
+            CTL_TRY(op(x, r1));
+            CTL_TRY(vec_lincomb(h, r1, 1.0, b, -1.0, r1, 0.0, nullptr, nullptr, len));
+            CTL_TRY(prec(r1, y));
+            CTL_TRY(dot(r1, y, &beta1));
+            if (beta1 < 0.0) {
+                res.reason = CTL_DIVERGED_INDEFINITE_PC;
+                return CTL_OK;
+            }
         }
         beta1 = std::sqrt(beta1);
         record(beta1);
@@ -288,12 +301,16 @@ struct Solver {
         CTL_TRY(vec_zero(h, w2, len));
         CTL_TRY(vec_copy(h, r2, r1, len));
         const double eps = std::numeric_limits<double>::epsilon();
+        // the first v = y / beta; each later one is written with the w and x updates of the iteration before
+        if (o.max_it > 0) CTL_TRY(vec_lincomb(h, v, 1.0 / beta, y, 0.0, nullptr, 0.0, nullptr, nullptr, len));
         while (res.reason == 0 && res.its < o.max_it) {
-            CTL_TRY(vec_lincomb(h, v, 1.0 / beta, y, 0.0, nullptr, 0.0, nullptr, nullptr, len));
             CTL_TRY(op(v, y));
-            if (res.its >= 1) CTL_TRY(vec_lincomb(h, y, 1.0, y, -(beta / oldb), r1, 0.0, nullptr, nullptr, len));
             double alfa = 0.0;
-            CTL_TRY(dot(v, y, &alfa));
+            if (res.its >= 1) {
+                CTL_TRY(vec_axpy_dot_host(h, y, -(beta / oldb), r1, v, len, &alfa));
+            } else {
+                CTL_TRY(dot(v, y, &alfa));
+            }
             CTL_TRY(vec_lincomb(h, y, 1.0, y, -(alfa / beta), r2, 0.0, nullptr, nullptr, len));
             double *freed = r1;
             r1 = r2;
@@ -317,18 +334,20 @@ struct Solver {
             sn = beta / gamma;
             const double phi = cs * phibar;
             phibar = sn * phibar;
-            // w <- (v - oldeps w2_old - delta w_old) / gamma, written into the retired w1 buffer
-            CTL_TRY(vec_lincomb(h, w1, 1.0 / gamma, v, -oldeps / gamma, w2, -delta / gamma, w, nullptr, len));
-            double *neww = w1;
-            w1 = w2;
-            w2 = w;
-            w = neww;
-            CTL_TRY(vec_lincomb(h, x, 1.0, x, phi, w, 0.0, nullptr, nullptr, len));
             ++res.its;
             const double rnorm = std::fabs(phibar);
             record(rnorm);
             res.reason = conv(rnorm);
             if (beta == 0.0 && res.reason == 0) res.reason = CTL_CONVERGED_HAPPY_BREAKDOWN;
+            const bool more = res.reason == 0 && res.its < o.max_it;
+            // w <- (v - oldeps w2_old - delta w_old) / gamma, written into the retired w1 buffer; x += phi w; and,
+            // if there is a next iteration, its v = y / beta
+            CTL_TRY(vec_minres_update(h, w1, 1.0 / gamma, v, -oldeps / gamma, w2, -delta / gamma, w, x, phi, v,
+                                      1.0 / beta, more ? y : nullptr, len));
+            double *neww = w1;
+            w1 = w2;
+            w2 = w;
+            w = neww;
         }
         if (res.its >= o.max_it && res.reason == 0) res.reason = CTL_DIVERGED_ITS;
         return CTL_OK;
@@ -355,7 +374,14 @@ int krylov_solve(Solver &K, const double *b_in, double *u)
         if (rc == CTL_OK) rc = vec_copy(h, b, b_in, K.len);
         if (rc == CTL_OK) rc = K.project(b, nullptr);
         if (rc == CTL_OK) rc = K.project(u, nullptr);
-        if (rc == CTL_OK) rc = (K.o.ksp_type == CTL_KSP_MINRES) ? K.minres(b, u) : K.gmres(b, u);
+        // From a zero guess the first residual b - A u is b, so the solvers skip that operator apply and reuse the
+        // preconditioned b of the reference norm instead of applying the preconditioner to the same bits again:
+        // the in-built preconditioner and the copy of CTL_PC_NONE are deterministic, so the values are those of the
+        // full start.  A user callback may keep state and sees the full sequence of calls.
+        bool zero_guess = false;
+        if (rc == CTL_OK && K.o.pc != CTL_PC_CALLBACK) rc = vec_is_zero_host(h, u, K.len, &zero_guess);
+        if (rc == CTL_OK)
+            rc = (K.o.ksp_type == CTL_KSP_MINRES) ? K.minres(b, u, zero_guess) : K.gmres(b, u, zero_guess);
         if (rc == CTL_OK) rc = K.project(u, nullptr);                   // 761-766
         if (rc == CTL_OK) rc = ctl_comm_check(h);
     }

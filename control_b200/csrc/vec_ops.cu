@@ -151,6 +151,67 @@ __global__ void __launch_bounds__(RT) lincomb_kernel(double *dst, double a, cons
     }
 }
 
+// y += c r, then partial[block] = sum over the block of v * y_new: the update of vec_lincomb(y, 1, y, c, r) (1 * y is
+// exact) followed by multi_dot_kernel's loop for V = {v}, w = y; block_sum<1> adds what block_sum<8> adds for j = 0
+__global__ void __launch_bounds__(RT) axpy_dot_kernel(double *y, double c, const double *r, const double *v,
+                                                     int64_t len2, double *__restrict__ partial)
+{
+    __shared__ double smem[RT / 32];
+    double acc[1] = {0.0};
+    double2 *y2 = reinterpret_cast<double2 *>(y);
+    for (int64_t i = (int64_t)blockIdx.x * RT + threadIdx.x; i < len2; i += (int64_t)gridDim.x * RT) {
+        double2 yi = y2[i];
+        const double2 ri = reinterpret_cast<const double2 *>(r)[i];
+        yi.x = fma(c, ri.x, yi.x);
+        yi.y = fma(c, ri.y, yi.y);
+        y2[i] = yi;
+        const double2 vi = reinterpret_cast<const double2 *>(v)[i];
+        acc[0] = fma(vi.x, yi.x, fma(vi.y, yi.y, acc[0]));
+    }
+    block_sum<1>(acc, smem);
+    if (threadIdx.x == 0) partial[blockIdx.x] = acc[0];
+}
+
+// MINRES direction, iterate and next Lanczos vector in one pass, each as its own vec_lincomb computes it:
+// w_new = a v + b w2 + c w; x += phi w_new; then, when y is given, v = s y.  Every element of v is read before the
+// same thread overwrites it.
+__global__ void __launch_bounds__(RT) minres_update_kernel(double *w_new, double a, const double *v, double b,
+                                                          const double *w2, double c, const double *w, double *x,
+                                                          double phi, double *v_next, double s, const double *y,
+                                                          int64_t len2)
+{
+    for (int64_t i = (int64_t)blockIdx.x * RT + threadIdx.x; i < len2; i += (int64_t)gridDim.x * RT) {
+        const double2 vi = reinterpret_cast<const double2 *>(v)[i];
+        const double2 w2i = reinterpret_cast<const double2 *>(w2)[i];
+        const double2 wi = reinterpret_cast<const double2 *>(w)[i];
+        double2 r;
+        r.x = fma(c, wi.x, fma(b, w2i.x, a * vi.x));
+        r.y = fma(c, wi.y, fma(b, w2i.y, a * vi.y));
+        reinterpret_cast<double2 *>(w_new)[i] = r;
+        double2 xi = reinterpret_cast<double2 *>(x)[i];
+        xi.x = fma(phi, r.x, xi.x);
+        xi.y = fma(phi, r.y, xi.y);
+        reinterpret_cast<double2 *>(x)[i] = xi;
+        if (y) {
+            const double2 yi = reinterpret_cast<const double2 *>(y)[i];
+            reinterpret_cast<double2 *>(v_next)[i] = make_double2(s * yi.x, s * yi.y);
+        }
+    }
+}
+
+// partial[block] = sum over the block of |x|
+__global__ void __launch_bounds__(RT) asum_kernel(const double *x, int64_t len2, double *__restrict__ partial)
+{
+    __shared__ double smem[RT / 32];
+    double acc[1] = {0.0};
+    for (int64_t i = (int64_t)blockIdx.x * RT + threadIdx.x; i < len2; i += (int64_t)gridDim.x * RT) {
+        const double2 xi = reinterpret_cast<const double2 *>(x)[i];
+        acc[0] += fabs(xi.x) + fabs(xi.y);
+    }
+    block_sum<1>(acc, smem);
+    if (threadIdx.x == 0) partial[blockIdx.x] = acc[0];
+}
+
 int grid_for(int64_t len2)
 {
     int64_t b = (len2 + RT - 1) / RT;
@@ -301,5 +362,52 @@ int vec_norm_host(ctl_handle_s *h, const double *x, int64_t len, double *out)
     double d = 0;
     CTL_TRY(vec_dot_host(h, x, x, len, &d));
     *out = sqrt(d);
+    return CTL_OK;
+}
+
+// the block partials in partials[0, nb) -> their sum on the host, all-reduced over the ranks
+static int sum_partials_host(ctl_handle_s *h, int nb, double *out)
+{
+    double *partials, *scalars;
+    CTL_TRY(vec_workspace(h, &partials, &scalars));
+    final_sum_kernel<<<1, RT, 0, h->stream>>>(partials, nb, scalars, nullptr);
+    h->launches++;
+    CTL_CUDA(cudaGetLastError());
+    if (h->comm) CTL_TRY(ctl_allreduce_sum(h, scalars, 1));
+    return vec_read_scalars(h, scalars, 1, out);
+}
+
+int vec_axpy_dot_host(ctl_handle_s *h, double *y, double c, const double *r, const double *v, int64_t len,
+                      double *out)
+{
+    double *partials, *scalars;
+    CTL_TRY(vec_workspace(h, &partials, &scalars));
+    const int64_t len2 = len / 2;
+    axpy_dot_kernel<<<grid_for(len2), RT, 0, h->stream>>>(y, c, r, v, len2, partials);
+    h->launches++;
+    return sum_partials_host(h, grid_for(len2), out);
+}
+
+int vec_minres_update(ctl_handle_s *h, double *w_new, double a, const double *v, double b, const double *w2,
+                      double c, const double *w, double *x, double phi, double *v_next, double s, const double *y,
+                      int64_t len)
+{
+    const int64_t len2 = len / 2;
+    minres_update_kernel<<<grid_for(len2), RT, 0, h->stream>>>(w_new, a, v, b, w2, c, w, x, phi, v_next, s, y, len2);
+    h->launches++;
+    CTL_CUDA(cudaGetLastError());
+    return CTL_OK;
+}
+
+int vec_is_zero_host(ctl_handle_s *h, const double *x, int64_t len, bool *out)
+{
+    double *partials, *scalars;
+    CTL_TRY(vec_workspace(h, &partials, &scalars));
+    const int64_t len2 = len / 2;
+    asum_kernel<<<grid_for(len2), RT, 0, h->stream>>>(x, len2, partials);
+    h->launches++;
+    double s = 0.0;
+    CTL_TRY(sum_partials_host(h, grid_for(len2), &s));
+    *out = s == 0.0;
     return CTL_OK;
 }

@@ -20,6 +20,17 @@ int vec_sqrt_dev(ctl_handle_s *h, const double *in, double *out, int k);
 int vec_read_scalars(ctl_handle_s *h, const double *dev, int k, double *host_out);
 int vec_dot_host(ctl_handle_s *h, const double *x, const double *y, int64_t len, double *out);
 int vec_norm_host(ctl_handle_s *h, const double *x, int64_t len, double *out);
+// y += c r, then *out = v . y, with the update of vec_lincomb and the reduction of vec_dot_host, bit for bit
+int vec_axpy_dot_host(ctl_handle_s *h, double *y, double c, const double *r, const double *v, int64_t len,
+                      double *out);
+// MINRES: w_new = a v + b w2 + c w; x += phi w_new; then v_next = s y unless y is null (v_next may be v), each
+// bit for bit as the corresponding vec_lincomb
+int vec_minres_update(ctl_handle_s *h, double *w_new, double a, const double *v, double b, const double *w2,
+                      double c, const double *w, double *x, double phi, double *v_next, double s, const double *y,
+                      int64_t len);
+// is every entry of x (on every rank) +0 or -0?  A sum of magnitudes, not of squares: squares of entries below
+// 1e-162 underflow to zero
+int vec_is_zero_host(ctl_handle_s *h, const double *x, int64_t len, bool *out);
 
 // with_internal for the heat-type handle: the caller's vectors are block-major, or time-fastest (copied)
 template <size_t K, class F>

@@ -2,6 +2,7 @@
 import argparse
 import json
 import os
+import subprocess
 import sys
 import time
 
@@ -47,6 +48,9 @@ def main():
     b0, b1 = build_rhs(q["M"], q["K"], q["tau"], q["n_t"], not args.be, q["bdofs"], q["v_d"], q["f"],
                            np.zeros(s.n))
     b = s.to_device(b0, b1)
+    gpu = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i",
+                          str(torch.cuda.current_device())], capture_output=True, text=True).stdout.strip()
+    print(f"gpu: {gpu}", flush=True)
     sp_ = {"linear_solver": args.ksp, "gmres_restart": args.restart, "maximum_iterations": 60, "preconditioner": True,
            "relative_tolerance": args.rtol, "absolute_tolerance": 0.0}
     for rep in range(args.reps):
@@ -54,7 +58,8 @@ def main():
         l0 = s.kernel_launches()
         info = s.solve_device(b, u, solver_parameters=sp_, pc="builtin")
         print(json.dumps({"its": info.its, "reason": info.reason, "seconds": info.seconds_total,
-                          "mult_s": info.seconds_mult, "pc_s": info.seconds_pc, "n_mult": info.n_mult,
+                          "mult_s": info.seconds_mult, "pc_s": info.seconds_pc,
+                          "vector_s": info.seconds_total - info.seconds_mult - info.seconds_pc, "n_mult": info.n_mult,
                           "n_pc": info.n_pc, "launches": s.kernel_launches() - l0,
                           "res": s.residual_norm(b, u), "hist": info.history[:3] + info.history[-2:]}), flush=True)
     print("mem GB", torch.cuda.max_memory_allocated() / 1e9, torch.cuda.mem_get_info())
